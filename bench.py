@@ -2,6 +2,7 @@
 """Headline benchmark: simulated plays/s (and games/s) of the play-by-play Monte Carlo engine.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--games G] [--memo on|off]
+                    [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): Kansas State vs Iowa State from the 2025 week-1 SP+ priors,
 10,000,000 simulated games per GPU per step (weak scaling: rank r plays game ids
@@ -72,7 +73,20 @@ def parse():
     ap.add_argument("--no-roofline", action="store_true")
     ap.add_argument("--no-tree-eval", action="store_true")
     ap.add_argument("--tree-states", type=int, default=1 << 26, help="states of the configs[2] tree-eval sub-record")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, rank 0 writes what the last timed step computed as DIR/<name>.npy: "
+                         "scores float32[games, 2] (points of team A, team B) and, with --players, players "
+                         "float64[games, 2, slots, 6] of rank 0's games; hist float64[matchups, 2, 128, 128] and "
+                         "counters float64[15] (games, plays, iters, pass, comp, inc, int, sack, run, td, fga, fg, punt, "
+                         "go, hist_overflow) summed over all ranks, as every rank receives them. Larger outputs are "
+                         "sampled with a fixed seed: scores of 2^20 games, the boxes of the first of those that fit "
+                         "in 24 MiB, histograms of 64 matchups")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return args
 
 
 def slate_pairs():
@@ -433,6 +447,47 @@ def tree_eval_record(eng, ms, local, n_total=1 << 26, batch=1 << 22):
 
 
 # ----------------------------------------------------------------------------------------------
+# outputs of the timed path (--dump-outputs): the same arguments give the same inputs, so that two builds
+# can be compared output for output
+# ----------------------------------------------------------------------------------------------
+DUMP_GAMES = 1 << 20          # per-game scores: seeded sample of at most this many games (8 MiB)
+DUMP_BOX_BYTES = 24 << 20     # per-game player boxes: the first games of that sample that fit in 24 MiB
+DUMP_MATCHUPS = 64            # histograms: seeded sample of at most this many matchups (16 MiB)
+DUMP_BYTES = 64 << 20
+DUMP_COUNTERS = 15            # games .. hist_overflow: what the games did, not how the kernel scheduled them
+
+
+def sample_ids(n: int, k: int):
+    """Sorted, seeded sample of k of range(n); all of range(n) when n <= k."""
+    import numpy as np
+    if n <= k:
+        return np.arange(n)
+    return np.sort(np.random.default_rng(SEED).choice(n, size=k, replace=False))
+
+
+def dump_outputs(path, scores, hist, counters, box):
+    """Writes the device buffers of the last timed step as float32 / float64 .npy files under `path`."""
+    import numpy as np
+    import torch
+    from fast_monte_carlo_b200 import native
+    games = torch.from_numpy(sample_ids(scores.shape[0], DUMP_GAMES)).to(scores.device)
+    words = scores[games].cpu().numpy().view(np.uint32)                  # points A | points B << 16
+    out = {"scores": np.stack([words & 0xFFFF, words >> 16], axis=1).astype(np.float32),
+           "hist": hist[torch.from_numpy(sample_ids(hist.shape[0], DUMP_MATCHUPS)).to(hist.device)].cpu().numpy()
+           .astype(np.float64),
+           "counters": counters[:DUMP_COUNTERS].cpu().numpy().astype(np.float64)}
+    if box is not None:                                                  # int64 pairs = fmc_player_rec
+        per_game = 2 * box.shape[2] * 6 * 8                              # float64 [2, slots, 6]
+        rec = np.ascontiguousarray(box[games[:DUMP_BOX_BYTES // per_game]].cpu().numpy()).view(native.PLAYER_REC)[..., 0]
+        out["players"] = native.unpack_player_box(rec)
+    total = sum(a.nbytes for a in out.values())
+    assert total <= DUMP_BYTES, total
+    os.makedirs(path, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(path, f"{name}.npy"), a)
+
+
+# ----------------------------------------------------------------------------------------------
 # GPU arm
 # ----------------------------------------------------------------------------------------------
 def run_ours(args):
@@ -533,6 +588,8 @@ def run_ours(args):
     games_step = step_counters["games"]
     assert games_step == total_games, (games_step, total_games)
     value = plays_step * args.steps / (total_ms / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, scores, hist64 if world > 1 else hist, counters, box)
 
     # ---- end to end through the reference's Python entry point (FMC:1467-1521 simulate_matchup), host buffers ----
     # every sample: api.simulate_matchup -> fmc_simulate_host (tables specialised + uploaded when the pair changes,

@@ -1,4 +1,4 @@
-"""ORACLE (test infrastructure only; needs /root/reference, so it only runs in the build container).
+"""ORACLE (test infrastructure only; needs the original project in the directory named by FMC_REFERENCE_DIR).
 
 Imports the UNMODIFIED reference module fast_monte_carlo_cfb.py with
   * `xgboost` replaced by oracle/fake_xgboost.py (xgboost is not installed here),
@@ -23,7 +23,7 @@ import tempfile
 
 import numpy as np
 
-REFERENCE_DIR = "/root/reference"
+REFERENCE_DIR = os.environ.get("FMC_REFERENCE_DIR", "")     # the original project's directory; "" = not available
 
 # slot layout (grouped so that one Philox4x32 call serves the common case)
 SLOT = dict(U_call=0, U_comp=1, Z_yards=2, U_ex=3,

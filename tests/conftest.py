@@ -9,7 +9,16 @@ for p in (ROOT, os.path.join(ROOT, "tests")):
         sys.path.insert(0, p)
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
-REFERENCE = "/root/reference"
+# The original project (fast_monte_carlo_cfb.py, sim_helpers.py, edge_finder.py, PregameSPPlus2025_1.csv and its model
+# artifacts) is not part of this repository; the tests that run it side by side with ours need FMC_REFERENCE_DIR.
+from oracle.ref_harness import REFERENCE_DIR as REFERENCE   # noqa: E402
+
+
+def has_reference(name: str) -> bool:
+    return bool(REFERENCE) and os.path.exists(os.path.join(REFERENCE, name))
+
+
+NO_REFERENCE = "the original project is not here: set FMC_REFERENCE_DIR to its directory"
 
 
 def pytest_configure(config):

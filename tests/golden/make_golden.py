@@ -1,6 +1,6 @@
 """Regenerates every fixture under tests/golden/ from the REAL reference objects.
 
-Runs only in the build container (needs /root/reference):   python tests/golden/make_golden.py
+Needs the original project (FMC_REFERENCE_DIR=<its directory>):   python tests/golden/make_golden.py
 
   sklearn_quantiles.npz   live `Pipeline.predict` of the nine quantile pipelines (FMC:658-668) on random
                           rows, incl. exact-zero features, down >= 5 and real player names
@@ -26,10 +26,10 @@ import pandas as pd
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
-REF = "/root/reference"
-
 from fast_monte_carlo_b200 import artifacts as art   # noqa: E402
 from oracle import ref_harness as rh                  # noqa: E402
+
+REF = rh.REFERENCE_DIR
 
 NUM = art.NUM_FEATURES
 

@@ -1,7 +1,7 @@
 """Golden trajectories of the UNMODIFIED reference simulate_game under ADVERSARIAL injected draws
 (tests/streams.py: all-zero / all-one uniforms, +-4 sigma normals, mixtures) -- pins the oracle on the rare
 branches (touchback punts, missed field goals, sacks past the 100, down >= 5 chains, late-game go-for-it).
-Runs only in the build container (needs /root/reference):   python tests/golden/make_golden_adversarial.py
+Needs the original project (FMC_REFERENCE_DIR=<its directory>):   python tests/golden/make_golden_adversarial.py
 """
 import json
 import os

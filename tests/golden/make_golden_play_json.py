@@ -1,6 +1,6 @@
 """Golden fixtures for the binary play-call model path (SURVEY 8a row a4 / 8f row 3), from the UNMODIFIED reference.
 
-Runs only in the build container (needs /root/reference):   python tests/golden/make_golden_play_json.py
+Needs the original project (FMC_REFERENCE_DIR=<its directory>):   python tests/golden/make_golden_play_json.py
 
 `play_model.json` and `calibration.json` are not in the reference snapshot, so the reference falls back to
 `pass_prob_v1` (FMC:326-328).  This script gives the reference module a SYNTHETIC `play_model.json` of the trained

@@ -1,6 +1,6 @@
 """Golden fixtures for the per-player path (SURVEY 8a row a16 / 8f row 1), from the UNMODIFIED reference.
 
-Runs only in the build container (needs /root/reference):   python tests/golden/make_golden_players.py
+Needs the original project (FMC_REFERENCE_DIR=<its directory>):   python tests/golden/make_golden_players.py
 
 The shipped reference has no usage data (every name is "Unknown", nothing is tracked, FMC:246-249), so
 the fixture gives the reference module a synthetic focus sheet (`players_focus.csv`, the format of

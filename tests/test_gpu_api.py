@@ -106,6 +106,31 @@ def test_bench_json_line_contract(tmp_path):
     assert "workload" in d["config"] and "model" not in d["config"]
 
 
+def test_bench_dump_outputs_equal_the_oracle(tmp_path):
+    """`bench.py --dump-outputs` writes the last timed step's games: scores, boxes and event counters are the C
+    oracle's games of the same seed, and the histogram is that of the dumped scores."""
+    import subprocess, sys
+    from conftest import ROOT
+    from test_gpu_players import _box_equal_philox
+    import bench
+    n = 4000
+    out = tmp_path / "out"
+    r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--players", "--games", str(n), "--steps", "2",
+                        "--warmup", "1", "--e2e-steps", "1", "--no-roofline", "--no-tree-eval", "--no-cpu-baseline",
+                        "--dump-outputs", str(out)], capture_output=True, text=True, timeout=900, cwd=ROOT)
+    assert r.returncode == 0, r.stderr[-2000:]
+    got = {p.stem: np.load(p) for p in out.iterdir()}
+    assert sorted(got) == ["counters", "hist", "players", "scores"]
+    assert got["scores"].dtype == np.float32 and got["scores"].shape == (n, 2)
+    assert all(got[k].dtype == np.float64 for k in ("counters", "hist", "players"))
+    assert got["hist"].shape == (1, 2, 128, 128) and got["counters"].shape == (15,) and got["counters"][0] == n
+    assert np.array_equal(got["hist"][0], outputs.histogram_from_scores(got["scores"].astype(np.int64)))
+    ref, _, _ = bench.cpu_run(bench.load_models("synthetic"), n, "synthetic", players=True)
+    assert np.array_equal(got["scores"], ref["scores"])
+    _box_equal_philox(got["players"], ref["players"])
+    assert got["counters"][1:14].tolist() == list(ref["counters"].values())
+
+
 def test_simulate_upcoming_matchup_players(engine, oracle, models_s2, tmp_path, monkeypatch):
     """collect_players=True with a focus sheet: players_df / players_<base>.csv carry the reference's rows, and
     they equal the oracle's on the same Philox seed."""

@@ -6,11 +6,11 @@ import sys
 import numpy as np
 import pytest
 
-from conftest import REFERENCE
+from conftest import NO_REFERENCE, REFERENCE, has_reference
 from fast_monte_carlo_b200 import helpers
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REFERENCE, "sim_helpers.py")), reason="reference not mounted")
+@pytest.mark.skipif(not has_reference("sim_helpers.py"), reason=NO_REFERENCE)
 def test_softmax_equals_reference():
     import oracle.fake_xgboost as fx
     saved = sys.modules.get("xgboost")

@@ -7,7 +7,7 @@ import numpy as np
 import pandas as pd
 import pytest
 
-from conftest import REFERENCE
+from conftest import NO_REFERENCE, REFERENCE, has_reference
 from fast_monte_carlo_b200 import outputs
 
 
@@ -69,7 +69,7 @@ def test_histogram_adapter_equals_direct(n):
             assert got["total"]["median_total"] == d["median_total"]
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REFERENCE, "edge_finder.py")), reason="reference not mounted")
+@pytest.mark.skipif(not has_reference("edge_finder.py"), reason=NO_REFERENCE)
 def test_unmodified_edge_finder_reads_our_files(tmp_path):
     """Gate G9: edge_finder.game_market_odds / moneyline_from_sims on a materialised scores_*.csv
     equal the histogram adapter."""

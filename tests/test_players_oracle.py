@@ -8,7 +8,7 @@ import numpy as np
 import pandas as pd
 import pytest
 
-from conftest import GOLDEN
+from conftest import GOLDEN, NO_REFERENCE, REFERENCE, has_reference
 
 from fast_monte_carlo_b200 import priors, usage
 
@@ -109,12 +109,12 @@ def test_oracle_trivial_usage_equals_plain_run(models, oracle):
     assert np.array_equal(a["scores"], b["scores"]) and np.array_equal(a["iters"], b["iters"])
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/edge_finder.py"), reason="reference not mounted")
+@pytest.mark.skipif(not has_reference("edge_finder.py"), reason=NO_REFERENCE)
 def test_unmodified_edge_finder_reads_our_players_file(models, oracle, contexts, tmp_path, monkeypatch):
     """`players_<base>.csv` written from the per-game box is what edge_finder.player_prop_odds /
     scan_props_for_matchup expect (edge_finder.py:131-231, 340-390), and the box adapter returns the same odds."""
     import importlib.util
-    spec = importlib.util.spec_from_file_location("edge_finder_ref", "/root/reference/edge_finder.py")
+    spec = importlib.util.spec_from_file_location("edge_finder_ref", os.path.join(REFERENCE, "edge_finder.py"))
     ef = importlib.util.module_from_spec(spec)
     spec.loader.exec_module(ef)
     monkeypatch.chdir(tmp_path)                      # edge_finder drops a scratch `testings.csv` into the cwd

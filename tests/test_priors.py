@@ -4,7 +4,7 @@ import os
 
 import pytest
 
-from conftest import GOLDEN, REFERENCE
+from conftest import GOLDEN, NO_REFERENCE, REFERENCE, has_reference
 from fast_monte_carlo_b200 import priors
 
 
@@ -58,7 +58,7 @@ def test_bad_schema(tmp_path):
         priors.load_sp_flex(str(p))
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REFERENCE, "PregameSPPlus2025_1.csv")), reason="reference not mounted")
+@pytest.mark.skipif(not has_reference("PregameSPPlus2025_1.csv"), reason=NO_REFERENCE)
 def test_real_csv(golden):
     sp = priors.load_sp_flex(os.path.join(REFERENCE, "PregameSPPlus2025_1.csv"))
     assert [r.team for r in sp.itertuples()] == [r["team"] for r in golden["table"]]

@@ -7,7 +7,7 @@ import numpy as np
 import pandas as pd
 import pytest
 
-from conftest import REFERENCE
+from conftest import NO_REFERENCE, REFERENCE, has_reference
 from fast_monte_carlo_b200 import outputs, store
 
 
@@ -50,7 +50,7 @@ def test_bundle_layout_and_signature(tmp_path):
     assert sig == hashlib.sha256(json.dumps(meta, sort_keys=True, separators=(",", ":")).encode()).hexdigest()
 
 
-@pytest.mark.skipif(not os.path.exists(os.path.join(REFERENCE, "edge_finder.py")), reason="reference not mounted")
+@pytest.mark.skipif(not has_reference("edge_finder.py"), reason=NO_REFERENCE)
 def test_unmodified_edge_finder_reads_the_parquet(tmp_path, monkeypatch):
     spec = importlib.util.spec_from_file_location("edge_finder_ref", os.path.join(REFERENCE, "edge_finder.py"))
     ef = importlib.util.module_from_spec(spec)

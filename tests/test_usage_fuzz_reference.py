@@ -1,17 +1,14 @@
-"""Host usage loaders against the UNMODIFIED reference on random inputs (runs only where /root/reference is
-mounted: the build container).  `usage.build_focus_usage_tables` / `usage.load_usage_table` must return the
+"""Host usage loaders against the UNMODIFIED reference on random inputs (runs only where FMC_REFERENCE_DIR names
+the original project).  `usage.build_focus_usage_tables` / `usage.load_usage_table` must return the
 reference's tables bit for bit: names, order, float64 shares, track sets."""
-import os
-
 import numpy as np
 import pandas as pd
 import pytest
 
-from conftest import REFERENCE
+from conftest import NO_REFERENCE, has_reference
 from fast_monte_carlo_b200 import usage
 
-pytestmark = pytest.mark.skipif(not os.path.exists(os.path.join(REFERENCE, "fast_monte_carlo_cfb.py")),
-                                reason="reference not mounted")
+pytestmark = pytest.mark.skipif(not has_reference("fast_monte_carlo_cfb.py"), reason=NO_REFERENCE)
 
 
 @pytest.fixture(scope="module")
