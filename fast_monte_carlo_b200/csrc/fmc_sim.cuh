@@ -18,6 +18,10 @@
 // Finished games are replaced at once from a global per-matchup game counter, so lanes stay busy
 // until the matchup is exhausted (the warp-level compaction of finished games the north star asks
 // for is the same mechanism: a parked lane is either refilled or absent from every request list).
+//
+// The game rules live here once, as step functions ("the game rules, one step at a time": new_game ... after_yards),
+// and so do the pieces of a round (next_matchup, request_rank, plan_round, walk_requests).  advance_lane below and the
+// trip loop of sim_memo_kernel (fmc_sim_memo.cuh) both call them: a rule is changed in one place for both kernels.
 #pragma once
 
 #include "fmc_device.cuh"
@@ -121,15 +125,6 @@ struct Lane {
 
 // A game's state between rounds: nine registers instead of sixteen, so that the tree walk (which runs with
 // every lane's game parked) has room for its eight gather chains.
-#ifndef FMC_PACK_LANE
-#define FMC_PACK_LANE 1
-#endif
-#if !FMC_PACK_LANE
-typedef Lane PackedLane;
-__device__ __forceinline__ PackedLane pack_lane(const Lane &L) { return L; }
-__device__ __forceinline__ Lane unpack_lane(const PackedLane &P) { return P; }
-__device__ __forceinline__ void set_stage(PackedLane &P, int stage) { P.stage = stage; }
-#else
 struct PackedLane {
     unsigned long long game;
     double dist, ytg;
@@ -157,7 +152,14 @@ __device__ __forceinline__ Lane unpack_lane(const PackedLane &P) {
     return L;
 }
 __device__ __forceinline__ void set_stage(PackedLane &P, int stage) { P.a = (P.a & 0x07FFFFFFu) | ((uint32_t)stage << 27); }
-#endif
+// the state of a lane without a game
+__device__ __forceinline__ PackedLane idle_lane() {
+    Lane L0;
+    L0.game = 0; L0.dist = 0.0; L0.ytg = 0.0; L0.sec = 0; L0.down = 0; L0.offense = 0; L0.period = 0; L0.going = 0;
+    L0.iter = 0; L0.score[0] = 0; L0.score[1] = 0; L0.plays = 0; L0.p1 = 0; L0.wr = 0; L0.home = 0;
+    L0.stage = ST_IDLE;
+    return pack_lane(L0);
+}
 
 // python semantics helpers (FMC:97 softclip = max(lo, min(hi, x)))
 __device__ __forceinline__ double pymax(double a, double b) { return (b > a) ? b : a; }
@@ -174,7 +176,6 @@ struct Draws {
     const SimKernelArgs &a;
     const double *rec;        // injected record base for this game (or nullptr)
     uint4 ctr;                // x,y = game; z = matchup; w = iter << 2 | block
-#ifndef FMC_DRAWS_ALL_BLOCKS
     // ONE cached Philox block: the draw sites of an iteration visit the record block by block (play call /
     // completion / yards / explosive in block 0, boost / finish / stage 2 / return in block 1, fourth down in 2-3),
     // so a single block costs no extra Philox calls and twelve registers less than caching all four.
@@ -197,28 +198,6 @@ struct Draws {
         const int j = slot & 3;
         return j == 0 ? w.x : (j == 1 ? w.y : (j == 2 ? w.z : w.w));
     }
-#else
-    uint32_t have;            // bit b: block b cached
-    uint4 w[4];
-    __device__ Draws(const SimKernelArgs &a_, const MatchupDev &M, int matchup, const Lane &L) : a(a_) {
-        rec = (TEST && a.stream) ? a.stream + ((size_t)(M.out_offset + (L.game - M.game_begin)) * FMC_MAX_ITERS + (size_t)L.iter) * FMC_N_SLOTS
-                                 : nullptr;
-        ctr = make_uint4((uint32_t)L.game, (uint32_t)(L.game >> 32), (uint32_t)matchup, (uint32_t)L.iter << 2);
-        have = 0;
-    }
-    __device__ __forceinline__ uint32_t word(int slot) {
-        const int b = slot >> 2;
-        if (!((have >> b) & 1u)) {
-            uint4 c = ctr;
-            c.w |= (uint32_t)b;
-            w[b] = philox4x32_10(c, make_uint2(a.seed_lo, a.seed_hi));
-            have |= 1u << b;
-        }
-        const uint4 v = w[b];
-        const int j = slot & 3;
-        return j == 0 ? v.x : (j == 1 ? v.y : (j == 2 ? v.z : v.w));
-    }
-#endif
     __device__ __forceinline__ double u(int slot) { return (TEST && rec) ? rec[slot] : u01(word(slot)); }
     __device__ __forceinline__ double z(int slot) { return (TEST && rec) ? rec[slot] : ppnd16(u01(word(slot))); }
 };
@@ -320,7 +299,8 @@ __device__ __forceinline__ double sample_yards(const SimKernelArgs &a, Draws<TES
 #endif
 constexpr int kSlateWave = FMC_SLATE_WAVE;
 
-struct SimShared {
+// Shared-memory state of the rounds, common to sim_kernel (SimShared) and sim_memo_kernel (MemoShared).
+struct RoundShared {
     MatchupDev M;
     int cur_matchup;
     int scan_from;                    // no matchup below this index has games left
@@ -330,10 +310,11 @@ struct SimShared {
     unsigned int aged[kNumKeys];      // the key's tail was held back last round: evaluate everything now
     unsigned int item_prefix[kNumKeys + 1];
     unsigned int item_next;
+    unsigned long long stat[FMC_N_COUNTERS];
+};
+struct SimShared : RoundShared {
     unsigned int dense_off[kNumKeys];  // first thread of each key's evaluated requests after the regrouping
     unsigned int n_eval, rest;         // evaluated requests this round; counter for the other lanes
-    unsigned int done[kSimThreads / 32 + kNumKeys];   // outputs finished per request chunk this round (FMC_EARLY_RESUME)
-    unsigned long long stat[FMC_N_COUNTERS];
 };
 
 // A key whose last chunk would hold fewer than this many requests holds that tail back for one round (the
@@ -350,22 +331,11 @@ __host__ __device__ constexpr int chunk_floats(bool players) { return (kSimRows 
 constexpr size_t kSimSharedBytes = ((sizeof(SimShared) + 15) / 16) * 16;
 __host__ __device__ constexpr size_t sim_feat_bytes(bool players) { return (size_t)kSimChunks * chunk_floats(players) * 4; }
 constexpr size_t kSimResultBytes = (size_t)kSimChunks * 32 * 3 * 8;
-// Regrouping (FMC_REGROUP): after the compaction every game moves to the thread at its request's rank, so that a
-// warp resumes games of ONE (family, orientation) next round instead of six different stages.  The ten words of a
-// game's record travel through shared memory: eight in the result buffer (free between the read-back and the walk),
-// two in kSimXchgExtraBytes.
-#ifndef FMC_REGROUP
-#define FMC_REGROUP 1
-#endif
-// FMC_EARLY_RESUME: no barrier after the walk.  A warp that finds the work queue empty waits only until the chunks
-// of ITS OWN games are finished (per-chunk completion counters) and starts the state machine of the next round while
-// other warps still walk: the tail of the walk phase overlaps the state-machine phase.  Needs FMC_REGROUP.
-// Measured +0.4 % (bit-identical results): off by default -- not worth a spin-wait on shared-memory flags.
-#ifndef FMC_EARLY_RESUME
-#define FMC_EARLY_RESUME 0
-#endif
-static_assert(!FMC_EARLY_RESUME || FMC_REGROUP, "FMC_EARLY_RESUME needs FMC_REGROUP");
-constexpr size_t kSimXchgExtraBytes = FMC_REGROUP ? (size_t)2 * kSimThreads * 4 : 0;
+// Regrouping: after the compaction every game moves to the thread at its request's rank, so that a warp resumes
+// games of ONE (family, orientation) next round instead of six different stages.  The ten words of a game's record
+// travel through shared memory: eight in the result buffer (free between the read-back and the walk), two in
+// kSimXchgExtraBytes.
+constexpr size_t kSimXchgExtraBytes = (size_t)2 * kSimThreads * 4;
 static_assert(kSimResultBytes >= (size_t)8 * kSimThreads * 4, "the result buffer must hold eight exchange words per thread");
 
 // keys in processing order, heaviest family first (LPT-style dynamic scheduling):
@@ -448,20 +418,6 @@ __device__ __noinline__ void flush_box(fmc_player_rec *box, fmc_player_rec *out,
         }
     }
 }
-// a pass call: sample_qb, sample_target, tgt += 1 (FMC:1058-1075); a run call: sample_rusher, att += 1 (FMC:1203-1208)
-template <bool TEST>
-__device__ __forceinline__ void call_pass(Lane &L, const SimKernelArgs &a, const MatchupDev &M, Draws<TEST> &D, int team) {
-    L.p1 = sample_usage(M.usage[team], 0, D.u(S_U_P1));
-    L.wr = sample_usage(M.usage[team], 2, D.u(S_U_WR));
-    credit(a, M, L, team, 2, L.wr, PC_ATT, false, 0.0);
-}
-template <bool TEST>
-__device__ __forceinline__ void call_run(Lane &L, const SimKernelArgs &a, const MatchupDev &M, Draws<TEST> &D, int team) {
-    L.p1 = sample_usage(M.usage[team], 1, D.u(S_U_P1));
-    L.wr = 0;
-    credit(a, M, L, team, 1, L.p1, PC_ATT, false, 0.0);
-}
-
 // FMC:420-425: float32 softmax of the play model's margins / T; returns exp of the "pass" class and the sum.
 // Out of line: only the model policies reach it, and its registers stay out of the heuristic path.
 __device__ __noinline__ void play_softmax(const float *m, int nc, int pass_class, float temp, float &e_pass, float &sum) {
@@ -475,239 +431,324 @@ __device__ __noinline__ void play_softmax(const float *m, int nc, int pass_class
         if (k < nc) { const float e = expf_cr(zv[k] - zmax); sum += e; if (k == pass_class) e_pass = e; }
 }
 
-// Advance one lane until it posts a request (returns key = family * 2 + offense) or has nothing
+// ---- the game rules, one step at a time ----------------------------------------------------------------------------
+// sim_kernel (advance_lane) and sim_memo_kernel (its trip loop) schedule a game's steps differently but play them with
+// these functions, so the two kernels share one copy of the rules, draws and arithmetic.  A step counts the game events
+// it sees through the kernel's event sink: any type with a method hit(EV_*).
+
+// game events, then the memo hits per family (sim_memo_kernel)
+enum { EV_GO = 0, EV_FGA, EV_FG, EV_PUNT, EV_RUN, EV_PASS, EV_COMP, EV_INC, EV_INT, EV_SACK, EV_TD, EV_GAMES,
+       EV_HIT0, EV_HIT1, EV_HIT2, EV_HIT3, EV_HIT4, EV_HIT5, EV_N };
+__host__ __device__ constexpr int ev_counter(int ev) {      // the FMC_C_* counter of an event
+    switch (ev) {
+    case EV_GO: return FMC_C_GO;
+    case EV_FGA: return FMC_C_FGA;
+    case EV_FG: return FMC_C_FG;
+    case EV_PUNT: return FMC_C_PUNT;
+    case EV_RUN: return FMC_C_RUN;
+    case EV_PASS: return FMC_C_PASS;
+    case EV_COMP: return FMC_C_COMP;
+    case EV_INC: return FMC_C_INC;
+    case EV_INT: return FMC_C_INT;
+    case EV_SACK: return FMC_C_SACK;
+    case EV_TD: return FMC_C_TD;
+    case EV_GAMES: return FMC_C_GAMES;
+    default: return FMC_C_MEMO_HITS_FAM0 + (ev - EV_HIT0);
+    }
+}
+// sim_kernel's event sink: one shared-memory atomic per event
+struct StatEvents {
+    unsigned long long *stat;
+    __device__ __forceinline__ void hit(int ev) { atomicAdd(&stat[ev_counter(ev)], 1ULL); }
+};
+
+__device__ __forceinline__ int stage_family(int stage) {      // ST_WAIT_* -> model id
+    return stage == ST_WAIT_PM ? 5 : stage - ST_WAIT_S1;      // S1, S2, PQ, RQ, SQ are consecutive
+}
+static_assert(ST_WAIT_S2 == ST_WAIT_S1 + 1 && ST_WAIT_PQ == ST_WAIT_S1 + 2 && ST_WAIT_RQ == ST_WAIT_S1 + 3 && ST_WAIT_SQ == ST_WAIT_S1 + 4,
+              "stage_family assumes consecutive wait stages");
+// key (family * 2 + team on offense) of the request a lane at a ST_WAIT_* stage waits for
+__device__ __forceinline__ int request_key(const Lane &L) { return stage_family(L.stage) * 2 + L.offense; }
+
+// game g of the matchup starts (simulate_game FMC:1428-1464); the parity of its id picks the team that receives first
+__device__ __forceinline__ void new_game(Lane &L, unsigned long long g) {
+    L.game = g;
+    L.offense = (int)(g & 1ULL);
+    L.sec = 3600; L.down = 1; L.dist = 10.0; L.ytg = 75.0; L.period = 1; L.going = 0;
+    L.score[0] = 0; L.score[1] = 0; L.iter = 0; L.plays = 0; L.p1 = 0; L.wr = 0;
+    L.stage = ST_ITER;
+}
+
+// Game over (FMC:1456-1464, 1501-1503): score word, iteration count and player box to the outputs.  Returns the game's
+// bin in the score histogram of its matchup ([orientation][score 0][score 1]; a score past the last bin is clamped into
+// it and counted as an overflow); the kernel adds it.
+template <bool PLAYERS, class Ev>
+__device__ __forceinline__ unsigned int end_game_record(const Lane &L, const SimKernelArgs &a, const MatchupDev &M, int matchup,
+                                                        unsigned long long *stat, Ev &ev) {
+    const size_t oi = (size_t)(M.out_offset + (L.game - M.game_begin));
+    if (a.scores) a.scores[oi] = (uint32_t)L.score[0] | ((uint32_t)L.score[1] << 16);
+    if (a.iters) a.iters[oi] = (uint16_t)L.iter;
+    const int ha = L.score[0] < FMC_HIST_BINS ? L.score[0] : FMC_HIST_BINS - 1;
+    const int hb = L.score[1] < FMC_HIST_BINS ? L.score[1] : FMC_HIST_BINS - 1;
+    if (a.hist && (L.score[0] >= FMC_HIST_BINS || L.score[1] >= FMC_HIST_BINS)) atomicAdd(&stat[FMC_C_HIST_OVERFLOW], 1ULL);
+    if (PLAYERS && a.n_slots > 0) {
+        const int lines = 2 * a.n_slots;
+        flush_box(lane_box(a, L.home), a.players ? a.players + oi * (size_t)lines : nullptr,
+                  a.player_hist ? a.player_hist + (size_t)matchup * (size_t)lines * FMC_PH_BINS : nullptr, lines,
+                  &stat[FMC_C_PH_OVERFLOW]);
+    }
+    ev.hit(EV_GAMES);
+    return (unsigned int)(((L.game & 1ULL) * FMC_HIST_BINS + ha) * FMC_HIST_BINS + hb);
+}
+
+// TEST: the state at the start of iteration L.iter into the per-iteration trace (parity tests)
+template <bool TEST>
+__device__ __forceinline__ void write_trace(const Lane &L, const SimKernelArgs &a, const MatchupDev &M) {
+    if (TEST && a.trace && L.iter < FMC_MAX_ITERS) {
+        const int first = (int)(L.game & 1ULL);
+        double *t = a.trace + ((size_t)(M.out_offset + (L.game - M.game_begin)) * FMC_MAX_ITERS + (size_t)L.iter) * FMC_TRACE_COLS;
+        t[0] = (L.offense == first) ? 1.0 : 0.0; t[1] = (double)L.down; t[2] = (double)L.sec;
+        t[3] = (double)L.score[first]; t[4] = (double)L.score[first ^ 1]; t[5] = L.dist; t[6] = L.ytg;
+        t[7] = (double)L.going;
+    }
+}
+
+// Fourth down (handle_fourth FMC:1382-1421): go for it, kick a field goal or punt (attempt_punt FMC:876-896).  Returns
+// whether a play follows; sd = score difference for the team on offense.
+template <bool TEST, class Ev>
+__device__ __forceinline__ bool fourth_down(Lane &L, Draws<TEST> &D, int sd, Ev &ev) {
+    if (L.down != 4) return true;
+    const int team = L.offense;
+    const double ytg = L.ytg, dist = L.dist;
+    const double p_go = pymin(1.0, go_for_it_prob(ytg, dist, sd, L.sec) * 1.15);
+    if (D.u(S_U_GO) < p_go) {
+        L.going = 1;
+        ev.hit(EV_GO);
+        return true;
+    }
+    if (ytg <= 38.0) {
+        ev.hit(EV_FGA);
+        const bool good = D.u(S_U_FG) < field_goal_prob(ytg + 17.0);
+        tick_clock(L, 12);
+        if (good) { ev.hit(EV_FG); L.score[team] += 3; change_possession(L, true, 75.0); }
+        else change_possession(L, true, 100.0 - ytg);
+        return false;
+    }
+    ev.hit(EV_PUNT);
+    const double gross = pymax(30.0, 43.0 + 6.0 * D.z(S_Z_GROSS));
+    const double ret = pymax(0.0, 6.0 + 3.0 * D.z(S_Z_RET));
+    double net = gross - ret;
+    if (ytg <= 60.0) {
+        const double tb = softclip((60.0 - ytg) / 60.0, 0.10, 0.55);
+        if (D.u(S_U_TB) < tb) net = ytg - 25.0;
+    }
+    net = softclip(net, 15.0, ytg - 1.0);
+    const int inet = (int)net;
+    tick_clock(L, 16);
+    change_possession(L, true, softclip(100.0 - (ytg - (double)inet), 1.0, 99.0));
+    return false;
+}
+
+// The play call from P(pass) (FMC:1058-1075, 1203-1208; P(run) after the two normalisations of FMC:1064-1066).  Returns
+// the stage the play waits at.  Player mode samples the passer and target (credits the target) or the rusher (credits
+// the carry).
+template <bool TEST, bool PLAYERS, class Ev>
+__device__ __forceinline__ int call_play(Lane &L, const SimKernelArgs &a, const MatchupDev &M, Draws<TEST> &D, int team,
+                                         double p_pass, Ev &ev) {
+    double a0 = 1.0 - p_pass, a1 = p_pass;
+    const double s = a0 + a1;
+    a0 = a0 / s; a1 = a1 / s;
+    const double c0 = a0 / (a0 + a1);
+    if (D.u(S_U_CALL) < c0) {
+        ev.hit(EV_RUN);
+        if (PLAYERS) {
+            L.p1 = sample_usage(M.usage[team], 1, D.u(S_U_P1));
+            L.wr = 0;
+            credit(a, M, L, team, 1, L.p1, PC_ATT, false, 0.0);
+        }
+        return ST_WAIT_RQ;
+    }
+    ev.hit(EV_PASS);
+    if (PLAYERS) {
+        L.p1 = sample_usage(M.usage[team], 0, D.u(S_U_P1));
+        L.wr = sample_usage(M.usage[team], 2, D.u(S_U_WR));
+        credit(a, M, L, team, 2, L.wr, PC_ATT, false, 0.0);
+    }
+    return ST_WAIT_S1;
+}
+
+// A play starts (simulate_play FMC:1026-...).  Returns the stage it waits at: the play model's margins (policy 1), or
+// the model of the play called with the heuristic P(pass).
+template <bool TEST, bool PLAYERS, class Ev>
+__device__ __forceinline__ int start_play(Lane &L, const SimKernelArgs &a, const MatchupDev &M, Draws<TEST> &D, int sd, Ev &ev) {
+    L.plays += 1;
+    if (a.policy == 1) return ST_WAIT_PM;
+    return call_play<TEST, PLAYERS>(L, a, M, D, L.offense, pass_prob_v1(L.down, L.dist, L.ytg, L.sec, sd), ev);
+}
+
+// P(pass) from the play model's nc margins m (FMC:420-425): float32 softmax of m / T, clipped to [.02, .98]
+__device__ __forceinline__ double p_pass_from_play_model(const float *m, int nc, const SimKernelArgs &a) {
+    float e1, sum;
+    play_softmax(m, nc, a.pass_class, a.play_temp, e1, sum);
+    return softclip((double)(e1 / sum), 0.02, 0.98);
+}
+
+// Stage-1 result from the stage-1 model's margin m1 (FMC:1086-1087): a completed pass waits for its yards, an incomplete
+// one for the stage-2 model.  Returns true when the launch has no stage-2 model: the stage stays ST_WAIT_S1 and stage 2
+// is decided at once from the stand-in probabilities.
+template <bool TEST, class Ev>
+__device__ __forceinline__ bool after_stage1(Lane &L, const SimKernelArgs &a, const MatchupDev &M, Draws<TEST> &D, int team,
+                                             float m1, Ev &ev) {
+    const double p1 = (double)(1.0f / (expf_cr(-m1) + 1.0f));                 // xgboost sigmoid, float32
+    const double p_complete = softclip(p1 + M.bias[team], 0.02, 0.98);
+    if (D.u(S_U_COMP) < p_complete) { ev.hit(EV_COMP); L.stage = ST_WAIT_PQ; return false; }
+    if (a.stage2_mode == 1) { L.stage = ST_WAIT_S2; return false; }
+    return true;
+}
+
+// Stage-2 class probabilities (incomplete, interception, sack): the stage-2 model's margins m through xgboost's Softmax
+// (f32 exp, double sum), or the stand-in probabilities
+__device__ __forceinline__ void stage2_raw(bool model, const float *m, const SimKernelArgs &a, double raw[3]) {
+    if (model) {
+        float wmax = m[0];
+        wmax = fmaxf(m[1], wmax); wmax = fmaxf(m[2], wmax);
+        float e[3];
+        double wsum = 0.0;
+#pragma unroll
+        for (int k = 0; k < 3; ++k) { e[k] = expf_cr(m[k] - wmax); wsum += (double)e[k]; }
+#pragma unroll
+        for (int k = 0; k < 3; ++k) raw[k] = (double)(e[k] / (float)wsum);
+    } else {
+        raw[0] = a.standin[0]; raw[1] = a.standin[1]; raw[2] = a.standin[2];
+    }
+}
+
+// The not-complete outcome (FMC:1157-1199): incomplete, interception, or a sack that waits for its yards
+template <bool TEST, bool PLAYERS, class Ev>
+__device__ __forceinline__ void after_stage2(Lane &L, const SimKernelArgs &a, const MatchupDev &M, Draws<TEST> &D, int team,
+                                             const double raw[3], Ev &ev) {
+    const int outcome = stage2_outcome(raw, D.u(S_U_S2));
+    if (outcome == 0) {                                   // incomplete FMC:1160-1168
+        ev.hit(EV_INC);
+        if (PLAYERS) credit(a, M, L, team, 0, L.p1, PC_ATT, false, 0.0);
+        L.down += 1; L.going = 0;
+        tick_clock(L, 10);
+        L.stage = ST_ITER;
+    } else if (outcome == 2) {                            // sack FMC:1170-1174
+        ev.hit(EV_SACK);
+        if (PLAYERS) credit(a, M, L, team, 0, L.p1, PC_SACK, false, 0.0);
+        L.stage = ST_WAIT_SQ;
+    } else {                                              // intercepted FMC:1186-1199
+        ev.hit(EV_INT);
+        if (PLAYERS) credit(a, M, L, team, 0, L.p1, PC_ATT | PC_INT, false, 0.0);
+        const double ret = softclip(6.0 + 5.0 * D.z(S_Z_INT), 0.0, L.ytg);
+        const double spot = 100.0 - (L.ytg - ret);
+        L.going = 0;
+        change_possession(L, true, spot);
+        tick_clock(L, 12);
+        L.stage = ST_ITER;
+    }
+}
+
+// The yards of a play from the quantiles q of its yardage model: sack FMC:1170-1184, completed pass FMC:1089-1152 and
+// run FMC:1201-1257 (the same steps with different constants).  The play ends.
+template <bool TEST, bool PLAYERS, class Ev>
+__device__ __forceinline__ void after_yards(Lane &L, const SimKernelArgs &a, const MatchupDev &M, Draws<TEST> &D, int team,
+                                            const double q[3], Ev &ev) {
+    if (L.stage == ST_WAIT_SQ) {
+        double loss = -sample_yards(a, D, q, 0.25, -20.0, 0.0);
+        loss = pymax(0.0, loss);
+        loss = pymin(loss, 100.0 - (100.0 - L.ytg));
+        L.ytg += loss; L.dist += loss; L.down += 1; L.going = 0;
+        tick_clock(L, 24);
+    } else {
+        const bool pass = L.stage == ST_WAIT_PQ;
+        const double ytg0 = L.ytg, mz = M.mz[team];
+        double yards = sample_yards(a, D, q, pass ? 0.4 : 0.35, pass ? 0.0 : -4.0, ytg0) * M.ymul[team];
+        if (ytg0 > 25.0 && D.u(S_U_EX) < (pass ? 0.60 : 0.5) * explosive_prob(mz, ytg0)) {
+            const double ub = pass ? 0.35 + (0.95 - 0.35) * D.u(S_U_BOOST) : 0.2 + (0.5 - 0.2) * D.u(S_U_BOOST);
+            yards *= 1.0 + ub * (1.0 + (pass ? 0.7 : 0.6) * mz);
+            yards = pymin(yards, ytg0);
+        }
+        if (ytg0 <= (pass ? 12.0 : 9.0) && L.down <= 3) {
+            if (D.u(S_U_FIN) < rz_finish_prob(ytg0, M.tanh35[team], L.down, pass)) yards = ytg0;
+        }
+        const bool td = yards + 1e-9 >= ytg0;
+        if (PLAYERS) {                  // FMC:1108-1127, 1140-1145 (pass), 1232-1234, 1246-1247 (run)
+            const double y = td ? ytg0 : yards;
+            const unsigned long long c_td = td ? PC_TD : 0ULL;
+            if (pass) {
+                credit(a, M, L, team, 0, L.p1, PC_ATT | PC_COMP | c_td, true, y);
+                credit(a, M, L, team, 2, L.wr, PC_COMP | c_td, true, y);
+            } else {
+                credit(a, M, L, team, 1, L.p1, c_td, true, y);
+            }
+        }
+        if (td) {
+            ev.hit(EV_TD);
+            L.score[team] += 7; L.going = 0;
+            tick_clock(L, pass ? 20 : 28);
+            change_possession(L, true, 75.0);
+        } else {
+            L.going = 0;
+            advance_down(L, yards);
+            tick_clock(L, pass ? 26 : 28);
+        }
+    }
+    L.stage = ST_ITER;
+}
+
+// Advance one lane until it posts a request (returns its key, family * 2 + offense) or has nothing
 // left to do (returns -1).  `res` points at this lane's result record of the previous round.
 template <bool TEST, bool PLAYERS>
 __device__ __forceinline__ int advance_lane(Lane &L, const SimKernelArgs &a, SimShared &sh, const double *res) {
     const MatchupDev &M = sh.M;
     const int matchup = sh.cur_matchup;
+    StatEvents ev{sh.stat};
     for (;;) {
         if (L.stage == ST_IDLE) return -1;
         if (L.stage == ST_NEED_GAME) {
             const unsigned long long g = atomicAdd(&a.next_game[matchup], 1ULL);
             if (g >= M.game_end) { L.stage = ST_IDLE; return -1; }
-            L.game = g;
-            L.offense = (int)(g & 1ULL);
-            L.sec = 3600; L.down = 1; L.dist = 10.0; L.ytg = 75.0; L.period = 1; L.going = 0;
-            L.score[0] = 0; L.score[1] = 0; L.iter = 0; L.plays = 0; L.p1 = 0; L.wr = 0;
-            L.stage = ST_ITER;
+            new_game(L, g);
         }
         if (L.stage == ST_ITER) {
             if (L.sec <= 0) {
-                // game over: outputs (FMC:1456-1464, 1501-1503)
-                const size_t oi = (size_t)(M.out_offset + (L.game - M.game_begin));
-                if (a.scores) a.scores[oi] = (uint32_t)L.score[0] | ((uint32_t)L.score[1] << 16);
-                if (a.iters) a.iters[oi] = (uint16_t)L.iter;
-                if (a.hist) {
-                    const int ha = L.score[0] < FMC_HIST_BINS ? L.score[0] : FMC_HIST_BINS - 1;
-                    const int hb = L.score[1] < FMC_HIST_BINS ? L.score[1] : FMC_HIST_BINS - 1;
-                    if (L.score[0] >= FMC_HIST_BINS || L.score[1] >= FMC_HIST_BINS) atomicAdd(&sh.stat[FMC_C_HIST_OVERFLOW], 1ULL);
-                    atomicAdd(&a.hist[(((size_t)matchup * 2 + (size_t)(L.game & 1ULL)) * FMC_HIST_BINS + ha) * FMC_HIST_BINS + hb], 1u);
-                }
-                if (PLAYERS && a.n_slots > 0) {
-                    const int lines = 2 * a.n_slots;
-                    flush_box(lane_box(a, L.home), a.players ? a.players + oi * (size_t)lines : nullptr,
-                              a.player_hist ? a.player_hist + (size_t)matchup * (size_t)lines * FMC_PH_BINS : nullptr, lines,
-                              &sh.stat[FMC_C_PH_OVERFLOW]);
-                }
-                atomicAdd(&sh.stat[FMC_C_GAMES], 1ULL);
+                const unsigned int bin = end_game_record<PLAYERS>(L, a, M, matchup, sh.stat, ev);
+                if (a.hist) atomicAdd(&a.hist[(size_t)matchup * 2 * FMC_HIST_BINS * FMC_HIST_BINS + bin], 1u);
                 atomicAdd(&sh.stat[FMC_C_PLAYS], (unsigned long long)L.plays);
                 atomicAdd(&sh.stat[FMC_C_ITERS], (unsigned long long)L.iter);
                 L.stage = ST_NEED_GAME;
                 continue;
             }
-            if (TEST && a.trace && L.iter < FMC_MAX_ITERS) {
-                const int first = (int)(L.game & 1ULL);
-                double *t = a.trace + ((size_t)(M.out_offset + (L.game - M.game_begin)) * FMC_MAX_ITERS + (size_t)L.iter) * FMC_TRACE_COLS;
-                t[0] = (L.offense == first) ? 1.0 : 0.0; t[1] = (double)L.down; t[2] = (double)L.sec;
-                t[3] = (double)L.score[first]; t[4] = (double)L.score[first ^ 1]; t[5] = L.dist; t[6] = L.ytg;
-                t[7] = (double)L.going;
-            }
+            write_trace<TEST>(L, a, M);
             Draws<TEST> D(a, M, matchup, L);
             L.iter += 1;
-            const int team = L.offense;
-            const int sd = L.score[team] - L.score[team ^ 1];
-            if (L.down == 4) {                                   // handle_fourth FMC:1382-1421
-                const double ytg = L.ytg, dist = L.dist;
-                const double p_go = pymin(1.0, go_for_it_prob(ytg, dist, sd, L.sec) * 1.15);
-                if (D.u(S_U_GO) < p_go) {
-                    L.going = 1;
-                    atomicAdd(&sh.stat[FMC_C_GO], 1ULL);
-                } else if (ytg <= 38.0) {
-                    atomicAdd(&sh.stat[FMC_C_FGA], 1ULL);
-                    const bool good = D.u(S_U_FG) < field_goal_prob(ytg + 17.0);
-                    tick_clock(L, 12);
-                    if (good) { atomicAdd(&sh.stat[FMC_C_FG], 1ULL); L.score[team] += 3; change_possession(L, true, 75.0); }
-                    else change_possession(L, true, 100.0 - ytg);
-                    continue;
-                } else {
-                    atomicAdd(&sh.stat[FMC_C_PUNT], 1ULL);
-                    const double gross = pymax(30.0, 43.0 + 6.0 * D.z(S_Z_GROSS));      // attempt_punt FMC:876-896
-                    const double ret = pymax(0.0, 6.0 + 3.0 * D.z(S_Z_RET));
-                    double net = gross - ret;
-                    if (ytg <= 60.0) {
-                        const double tb = softclip((60.0 - ytg) / 60.0, 0.10, 0.55);
-                        if (D.u(S_U_TB) < tb) net = ytg - 25.0;
-                    }
-                    net = softclip(net, 15.0, ytg - 1.0);
-                    const int inet = (int)net;
-                    tick_clock(L, 16);
-                    change_possession(L, true, softclip(100.0 - (ytg - (double)inet), 1.0, 99.0));
-                    continue;
-                }
-            }
-            // simulate_play FMC:1026-...: the play call
-            L.plays += 1;
-            if (a.policy == 1) { L.stage = ST_WAIT_PM; return 5 * 2 + team; }
-            const double p_pass = pass_prob_v1(L.down, L.dist, L.ytg, L.sec, sd);
-            double a0 = 1.0 - p_pass, a1 = p_pass;
-            const double s = a0 + a1;
-            a0 = a0 / s; a1 = a1 / s;
-            const double c0 = a0 / (a0 + a1);
-            if (D.u(S_U_CALL) < c0) {
-                atomicAdd(&sh.stat[FMC_C_RUN], 1ULL);
-                if (PLAYERS) call_run<TEST>(L, a, M, D, team);
-                L.stage = ST_WAIT_RQ;
-                return 3 * 2 + team;
-            }
-            atomicAdd(&sh.stat[FMC_C_PASS], 1ULL);
-            if (PLAYERS) call_pass<TEST>(L, a, M, D, team);
-            L.stage = ST_WAIT_S1;
-            return 0 * 2 + team;
+            const int sd = L.score[L.offense] - L.score[L.offense ^ 1];
+            if (!fourth_down(L, D, sd, ev)) continue;
+            L.stage = start_play<TEST, PLAYERS>(L, a, M, D, sd, ev);
+            return request_key(L);
         }
         // ---- resuming a parked play: the iteration counter already points past this iteration
         Lane Lv = L;
         Lv.iter = L.iter - 1;
         Draws<TEST> D(a, M, matchup, Lv);
         const int team = L.offense;
-        const int sd = L.score[team] - L.score[team ^ 1];
-        const double mz = M.mz[team];
-        const double ytg0 = L.ytg;
+        const float *mg = reinterpret_cast<const float *>(res);
         if (L.stage == ST_WAIT_PM) {
-            // FMC:420-425: float32 softmax of margins / T, P(pass) clipped to [.02, .98]
-            float e1, sum;
-            play_softmax(reinterpret_cast<const float *>(res), M.tbl[5][team].n_outputs, a.pass_class, a.play_temp, e1, sum);
-            const double p_pass = softclip((double)(e1 / sum), 0.02, 0.98);
-            double a0 = 1.0 - p_pass, a1 = p_pass;
-            const double s = a0 + a1;
-            a0 = a0 / s; a1 = a1 / s;
-            const double c0 = a0 / (a0 + a1);
-            if (D.u(S_U_CALL) < c0) {
-                atomicAdd(&sh.stat[FMC_C_RUN], 1ULL);
-                if (PLAYERS) call_run<TEST>(L, a, M, D, team);
-                L.stage = ST_WAIT_RQ;
-                return 3 * 2 + team;
-            }
-            atomicAdd(&sh.stat[FMC_C_PASS], 1ULL);
-            if (PLAYERS) call_pass<TEST>(L, a, M, D, team);
-            L.stage = ST_WAIT_S1;
-            return 0 * 2 + team;
+            L.stage = call_play<TEST, PLAYERS>(L, a, M, D, team, p_pass_from_play_model(mg, M.tbl[5][team].n_outputs, a), ev);
+            return request_key(L);
         }
-        if (L.stage == ST_WAIT_S1) {
-            const float m1 = *reinterpret_cast<const float *>(res);
-            const double p1 = (double)(1.0f / (expf_cr(-m1) + 1.0f));                 // xgboost sigmoid, float32
-            const double p_complete = softclip(p1 + M.bias[team], 0.02, 0.98);        // FMC:1086-1087
-            if (D.u(S_U_COMP) < p_complete) { atomicAdd(&sh.stat[FMC_C_COMP], 1ULL); L.stage = ST_WAIT_PQ; return 2 * 2 + team; }
-            if (a.stage2_mode == 1) { L.stage = ST_WAIT_S2; return 1 * 2 + team; }
-        }
+        if (L.stage == ST_WAIT_S1 && !after_stage1(L, a, M, D, team, mg[0], ev)) return request_key(L);
         if (L.stage == ST_WAIT_S1 || L.stage == ST_WAIT_S2) {
             double raw[3];
-            if (L.stage == ST_WAIT_S2) {
-                const float *m = reinterpret_cast<const float *>(res);           // xgboost Softmax: f32 exp, double sum
-                float wmax = m[0];
-                wmax = fmaxf(m[1], wmax); wmax = fmaxf(m[2], wmax);
-                float e[3];
-                double wsum = 0.0;
-#pragma unroll
-                for (int k = 0; k < 3; ++k) { e[k] = expf_cr(m[k] - wmax); wsum += (double)e[k]; }
-#pragma unroll
-                for (int k = 0; k < 3; ++k) raw[k] = (double)(e[k] / (float)wsum);
-            } else {
-                raw[0] = a.standin[0]; raw[1] = a.standin[1]; raw[2] = a.standin[2];
-            }
-            const int outcome = stage2_outcome(raw, D.u(S_U_S2));
-            if (outcome == 0) {                                   // incomplete FMC:1160-1168
-                atomicAdd(&sh.stat[FMC_C_INC], 1ULL);
-                if (PLAYERS) credit(a, M, L, team, 0, L.p1, PC_ATT, false, 0.0);                    // FMC:1163-1164
-                L.down += 1; L.going = 0;
-                tick_clock(L, 10);
-                L.stage = ST_ITER;
-                continue;
-            }
-            if (outcome == 2) {
-                atomicAdd(&sh.stat[FMC_C_SACK], 1ULL);
-                if (PLAYERS) credit(a, M, L, team, 0, L.p1, PC_SACK, false, 0.0);                   // FMC:1173-1174
-                L.stage = ST_WAIT_SQ;
-                return 4 * 2 + team;
-            }
-            atomicAdd(&sh.stat[FMC_C_INT], 1ULL);                 // intercepted FMC:1186-1199
-            if (PLAYERS) credit(a, M, L, team, 0, L.p1, PC_ATT | PC_INT, false, 0.0);               // FMC:1190-1192
-            const double ret = softclip(6.0 + 5.0 * D.z(S_Z_INT), 0.0, L.ytg);
-            const double spot = 100.0 - (L.ytg - ret);
-            L.going = 0;
-            change_possession(L, true, spot);
-            tick_clock(L, 12);
-            L.stage = ST_ITER;
+            stage2_raw(L.stage == ST_WAIT_S2, mg, a, raw);
+            after_stage2<TEST, PLAYERS>(L, a, M, D, team, raw, ev);
+            if (L.stage == ST_WAIT_SQ) return request_key(L);
             continue;
         }
         const double q[3] = {res[0], res[1], res[2]};
-        if (L.stage == ST_WAIT_PQ) {                              // completed pass FMC:1089-1152
-            double yards = sample_yards(a, D, q, 0.4, 0.0, L.ytg) * M.ymul[team];
-            if (ytg0 > 25.0 && D.u(S_U_EX) < 0.60 * explosive_prob(mz, ytg0)) {
-                const double ub = 0.35 + (0.95 - 0.35) * D.u(S_U_BOOST);
-                yards *= 1.0 + ub * (1.0 + 0.7 * mz);
-                yards = pymin(yards, ytg0);
-            }
-            if (ytg0 <= 12.0 && L.down <= 3 && D.u(S_U_FIN) < rz_finish_prob(ytg0, M.tanh35[team], L.down, true)) yards = ytg0;
-            if (yards + 1e-9 >= L.ytg) {
-                atomicAdd(&sh.stat[FMC_C_TD], 1ULL);
-                if (PLAYERS) {                                                                        // FMC:1108-1127
-                    credit(a, M, L, team, 0, L.p1, PC_ATT | PC_COMP | PC_TD, true, L.ytg);
-                    credit(a, M, L, team, 2, L.wr, PC_COMP | PC_TD, true, L.ytg);
-                }
-                L.score[team] += 7; L.going = 0;
-                tick_clock(L, 20);
-                change_possession(L, true, 75.0);
-            } else {
-                if (PLAYERS) {                                                                        // FMC:1108-1109, 1140-1145
-                    credit(a, M, L, team, 0, L.p1, PC_ATT | PC_COMP, true, yards);
-                    credit(a, M, L, team, 2, L.wr, PC_COMP, true, yards);
-                }
-                L.going = 0;
-                advance_down(L, yards);
-                tick_clock(L, 26);
-            }
-        } else if (L.stage == ST_WAIT_RQ) {                       // run FMC:1201-1257
-            double yards = sample_yards(a, D, q, 0.35, -4.0, L.ytg) * M.ymul[team];
-            if (ytg0 > 25.0 && D.u(S_U_EX) < 0.5 * explosive_prob(mz, ytg0)) {
-                const double ub = 0.2 + (0.5 - 0.2) * D.u(S_U_BOOST);
-                yards *= 1.0 + ub * (1.0 + 0.6 * mz);
-                yards = pymin(yards, ytg0);
-            }
-            if (ytg0 <= 9.0 && L.down <= 3) {
-                if (D.u(S_U_FIN) < rz_finish_prob(ytg0, M.tanh35[team], L.down, false)) yards = ytg0;
-            }
-            if (yards + 1e-9 >= ytg0) {
-                atomicAdd(&sh.stat[FMC_C_TD], 1ULL);
-                if (PLAYERS) credit(a, M, L, team, 1, L.p1, PC_TD, true, L.ytg);                     // FMC:1232-1234
-                L.score[team] += 7;
-                tick_clock(L, 28);
-                change_possession(L, true, 75.0);
-                L.going = 0;
-            } else {
-                if (PLAYERS) credit(a, M, L, team, 1, L.p1, 0ULL, true, yards);                      // FMC:1246-1247
-                advance_down(L, yards);
-                tick_clock(L, 28);
-                L.going = 0;
-            }
-        } else {                                                  // sack FMC:1170-1184
-            double loss = -sample_yards(a, D, q, 0.25, -20.0, 0.0);
-            loss = pymax(0.0, loss);
-            loss = pymin(loss, 100.0 - (100.0 - L.ytg));
-            L.ytg += loss; L.dist += loss; L.down += 1; L.going = 0;
-            tick_clock(L, 24);
-        }
-        L.stage = ST_ITER;
+        after_yards<TEST, PLAYERS>(L, a, M, D, team, q, ev);
     }
 }
 
@@ -777,10 +818,6 @@ __device__ __forceinline__ void write_features(float *col, const Lane &L, int fa
 
 __device__ __forceinline__ double eval_output(int fam, const TableRef &T, int out, const SimKernelArgs &a,
                                               uint32_t fcol, int lane, uint32_t &levels) {
-#ifdef FMC_SKIP_WALK      // measurement only (results are wrong): the kernel without its tree walk
-    levels = 0;
-    return (fam >= 2 && fam <= 4) ? T.base64[out] + 3.0 * out : (double)T.base[out];
-#endif
     ForestView F;
     F.win_lo = T.win_lo; F.win_hi = T.win_hi;
     F.stream = a.root_stream + T.stream_off[out];
@@ -793,6 +830,119 @@ __device__ __forceinline__ double eval_output(int fam, const TableRef &T, int ou
     }
     if (fam >= 2 && fam <= 4) return walk_output<true, false>(F, fcol, lane, T.base64[out], levels);
     return walk_output<false, false>(F, fcol, lane, (double)T.base[out], levels);
+}
+
+// ---- the rounds of both kernels ------------------------------------------------------------------------------------
+
+// Round state at kernel start, and the -inf feature row of every chunk (leaves keep lanes in place by testing it,
+// fmc_pack.hpp).  The kernel initialises its own fields and then synchronises.
+template <int THREADS>
+__device__ __forceinline__ void init_rounds(RoundShared &sh, float *feats, int chunk_floats) {
+    const int tid = threadIdx.x;
+    for (int i = tid; i < (THREADS / 32 + kNumKeys) * 32; i += THREADS)
+        feats[(size_t)(i >> 5) * chunk_floats + kSimNinfRow * 32 + (i & 31)] = __int_as_float(0xff800000);
+    if (tid < FMC_N_COUNTERS) sh.stat[tid] = 0ULL;
+    if (tid < kNumKeys) { sh.cnt[0][tid] = 0; sh.cnt[1][tid] = 0; sh.aged[tid] = 0; }
+    if (tid == 0) { sh.cur_matchup = -1; sh.scan_from = 0; }
+}
+
+// The next matchup that still has games (-1: none), its MatchupDev copied to shared memory, its request lists empty.
+// The kernel resets its own fields and then synchronises.
+template <int THREADS>
+__device__ __forceinline__ int next_matchup(RoundShared &sh, const SimKernelArgs &a) {
+    const int tid = threadIdx.x;
+    if (tid == 0) {
+        // Waves: the CTAs of the grid share the kSlateWave lowest-numbered matchups that still have games (CTA b takes
+        // the (b mod kSlateWave)-th of them), and move up as matchups drain -- so a slate keeps a handful of node
+        // tables (and their memo entries) live at a time instead of one per CTA (720 x 0.6 MB for a season).
+        int found = -1, last = -1, seen = 0;
+        const int want = (int)(blockIdx.x % (unsigned)kSlateWave);
+        for (int m = sh.scan_from; m < a.n_matchups; ++m) {
+            if (*((volatile unsigned long long *)&a.next_game[m]) < a.matchups[m].game_end) {
+                if (seen == 0) sh.scan_from = m;          // everything below is finished for good
+                last = m;
+                if (seen == want) { found = m; break; }
+                if (++seen >= kSlateWave) break;
+            }
+        }
+        if (found < 0) found = last;                      // fewer unfinished matchups than the wave is wide
+        sh.cur_matchup = found;
+    }
+    __syncthreads();
+    const int m = sh.cur_matchup;
+    if (m < 0) return m;
+    {
+        const uint32_t *src = reinterpret_cast<const uint32_t *>(a.matchups + m);
+        uint32_t *dst = reinterpret_cast<uint32_t *>(&sh.M);
+        for (int i = tid; i < (int)(sizeof(MatchupDev) / 4); i += THREADS) dst[i] = src[i];
+    }
+    // the last round of the previous matchup leaves its counts in one of the two buffers (the loop ends
+    // before it would clear them): start every matchup from empty lists
+    if (tid < kNumKeys) { sh.cnt[0][tid] = 0; sh.cnt[1][tid] = 0; sh.aged[tid] = 0; }
+    return m;
+}
+
+// B: rank of the lane's request in the list of its key (key < 0: no request); warp match, one shared atomic per key
+__device__ __forceinline__ unsigned int request_rank(unsigned int *cnt, int key, int lane) {
+    const unsigned int peers = __match_any_sync(0xFFFFFFFFu, key);
+    const int leader = __ffs(peers) - 1;
+    unsigned int base = 0;
+    if (key >= 0 && lane == leader) base = atomicAdd(&cnt[key], (unsigned int)__popc(peers));
+    base = __shfl_sync(0xFFFFFFFFu, base, leader);
+    return base + (unsigned int)__popc(peers & ((1u << lane) - 1u));
+}
+
+// Thread 0 plans the walk of a round from the request counts: the requests of each key walked now (evalc; the tail
+// hold-back), the first position of each key's list (off) and the work items of each key (item_prefix).
+__device__ __forceinline__ void plan_round(RoundShared &sh, int parity) {
+    unsigned int o = 0, it = 0;
+    for (int j = 0; j < kNumKeys; ++j) {
+        const int k = kKeyOrder[j];
+        unsigned int c = sh.cnt[parity][k];
+        const unsigned int tail = c & 31u;
+        if (tail != 0 && tail < kDeferBelow && !sh.aged[k]) { c -= tail; sh.aged[k] = 1; }
+        else sh.aged[k] = 0;
+        sh.evalc[k] = c;
+        sh.off[k] = o;
+        o += (c + 31u) & ~31u;          // lists start on chunk boundaries
+        sh.item_prefix[j] = it;
+        it += ((c + 31u) >> 5) * (unsigned int)splits_of(k >> 1);
+    }
+    sh.item_prefix[kNumKeys] = it;
+    sh.item_next = 0;
+}
+
+// C: walk the planned requests.  Work item = (key, chunk of 32 requests, output), handed to warps dynamically in key
+// order; each output goes to the request's result record.  Returns the node slots gathered for live requests.
+__device__ __forceinline__ void walk_requests(RoundShared &sh, const SimKernelArgs &a, uint32_t feats_saddr,
+                                                            int chunk_floats, double *results, int lane, unsigned long long &visits) {
+    const unsigned int n_items = sh.item_prefix[kNumKeys];
+    for (;;) {
+        unsigned int it = 0;
+        if (lane == 0) it = atomicAdd(&sh.item_next, 1u);
+        it = __shfl_sync(0xFFFFFFFFu, it, 0);
+        if (it >= n_items) break;
+        int j = 0;
+        while (it >= sh.item_prefix[j + 1]) ++j;
+        const int k = kKeyOrder[j];
+        const int fam = k >> 1;
+        const unsigned int local = it - sh.item_prefix[j];
+        const int ns = splits_of(fam);
+        const unsigned int chunk = local / (unsigned int)ns;
+        const int out = (int)(local - chunk * (unsigned int)ns);
+        const unsigned int c = sh.evalc[k];
+        const unsigned int idx = chunk * 32u + (unsigned int)lane;
+        const bool live = idx < c;
+        const unsigned int p = sh.off[k] + idx;      // idle lanes walk whatever their column holds
+        uint32_t levels;
+        const double v = eval_output(fam, sh.M.tbl[fam][k & 1], out, a,
+                                     feats_saddr + (p >> 5) * (uint32_t)(chunk_floats * 4) + (uint32_t)lane * 4u, lane, levels);
+        visits += (unsigned long long)levels * (live ? kIlp : 0);
+        if (live) {
+            if (fam >= 2 && fam <= 4) results[(size_t)p * 3 + out] = v;
+            else reinterpret_cast<float *>(results + (size_t)p * 3)[out] = (float)v;
+        }
+    }
 }
 
 // PLAYERS = true: usage tables are set (fmc_set_usage): names are sampled per play, requests carry kDynRows
@@ -811,59 +961,20 @@ __global__ void __launch_bounds__(kSimThreads, kSimCtasPerSm) sim_kernel(const S
     const uint32_t feats_saddr = (uint32_t)__cvta_generic_to_shared(feats);
     const int tid = threadIdx.x;
     const int lane = tid & 31;
-    // the -inf feature row of every chunk (leaves keep lanes in place by testing it, fmc_pack.hpp)
-    for (int i = tid; i < kSimChunks * 32; i += kSimThreads)
-        feats[(size_t)(i >> 5) * kChunkFloats + kSimNinfRow * 32 + (i & 31)] = __int_as_float(0xff800000);
-    if (tid < FMC_N_COUNTERS) sh.stat[tid] = 0ULL;
-    if (tid < kNumKeys) { sh.cnt[0][tid] = 0; sh.cnt[1][tid] = 0; sh.aged[tid] = 0; }
-    if (tid == 0) { sh.cur_matchup = -1; sh.scan_from = 0; }
+    init_rounds<kSimThreads>(sh, feats, kChunkFloats);
     __syncthreads();
 
-    PackedLane P;
-    {
-        Lane L0;
-        L0.game = 0; L0.dist = 0.0; L0.ytg = 0.0; L0.sec = 0; L0.down = 0; L0.offense = 0; L0.period = 0; L0.going = 0;
-        L0.iter = 0; L0.score[0] = 0; L0.score[1] = 0; L0.plays = 0; L0.p1 = 0; L0.wr = 0; L0.home = 0;
-        L0.stage = ST_IDLE;
-        P = pack_lane(L0);
-    }
+    PackedLane P = idle_lane();
     unsigned long long rounds = 0, requests = 0, visits = 0;
     int home = tid;        // running player box of the game this thread holds (travels with the game when games regroup)
     uint32_t *xchg = reinterpret_cast<uint32_t *>(results);                                   // words 0..7
     uint32_t *xchg2 = reinterpret_cast<uint32_t *>(smem_raw + kSimSharedBytes + kSimFeatBytes + kSimResultBytes);   // words 8..9
-    (void)xchg; (void)xchg2;
 
-    for (int visit = 0;; ++visit) {
-        // ---- pick the next matchup that still has games; CTAs start at different matchups so that a
-        // slate is spread over the SMs and each CTA drains only when its matchup runs dry
-        if (tid == 0) {
-            // Waves: the CTAs of the grid share the kSlateWave lowest-numbered matchups that still have games (CTA b takes
-            // the (b mod kSlateWave)-th of them), and move up as matchups drain -- so a slate keeps a handful of node
-            // tables (and their memo entries) live at a time instead of one per CTA (720 x 0.6 MB for a season).
-            int found = -1, last = -1, seen = 0;
-            const int want = (int)(blockIdx.x % (unsigned)kSlateWave);
-            for (int m = sh.scan_from; m < a.n_matchups; ++m) {
-                if (*((volatile unsigned long long *)&a.next_game[m]) < a.matchups[m].game_end) {
-                    if (seen == 0) sh.scan_from = m;          // everything below is finished for good
-                    last = m;
-                    if (seen == want) { found = m; break; }
-                    if (++seen >= kSlateWave) break;
-                }
-            }
-            if (found < 0) found = last;                      // fewer unfinished matchups than the wave is wide
-            sh.cur_matchup = found;
-        }
-        __syncthreads();
-        const int m = sh.cur_matchup;
+    for (;;) {
+        // ---- the next matchup that still has games; CTAs start at different matchups so that a slate is spread over
+        // the SMs and each CTA drains only when its matchup runs dry
+        const int m = next_matchup<kSimThreads>(sh, a);
         if (m < 0) break;
-        {
-            const uint32_t *src = reinterpret_cast<const uint32_t *>(a.matchups + m);
-            uint32_t *dst = reinterpret_cast<uint32_t *>(&sh.M);
-            for (int i = tid; i < (int)(sizeof(MatchupDev) / 4); i += kSimThreads) dst[i] = src[i];
-        }
-        // the last round of the previous matchup leaves its counts in one of the two buffers (the loop ends
-        // before it would clear them): start every matchup from empty lists
-        if (tid < kNumKeys) { sh.cnt[0][tid] = 0; sh.cnt[1][tid] = 0; sh.aged[tid] = 0; }
         __syncthreads();
         set_stage(P, ST_NEED_GAME);
         int pos = 0;
@@ -876,44 +987,22 @@ __global__ void __launch_bounds__(kSimThreads, kSimCtasPerSm) sim_kernel(const S
             const int key = held >= 0 ? held : advance_lane<TEST, PLAYERS>(L, a, sh, results + (size_t)pos * 3);
             __syncwarp();
             // ---- B: compaction
-            unsigned int rank = 0;
-            {
-                const unsigned int peers = __match_any_sync(0xFFFFFFFFu, key);
-                const int leader = __ffs(peers) - 1;
-                unsigned int base = 0;
-                if (key >= 0 && lane == leader) base = atomicAdd(&sh.cnt[parity][key], (unsigned int)__popc(peers));
-                base = __shfl_sync(0xFFFFFFFFu, base, leader);
-                rank = base + (unsigned int)__popc(peers & ((1u << lane) - 1u));
-            }
+            const unsigned int rank = request_rank(sh.cnt[parity], key, lane);
             const int total = __syncthreads_count(key >= 0);
             if (total == 0) break;
             if (tid == 0) {
-                unsigned int o = 0, it = 0, dn = 0;
+                plan_round(sh, parity);
+                unsigned int dn = 0;
                 for (int j = 0; j < kNumKeys; ++j) {
                     const int k = kKeyOrder[j];
-                    unsigned int c = sh.cnt[parity][k];
-                    const unsigned int tail = c & 31u;
-                    if (tail != 0 && tail < kDeferBelow && !sh.aged[k]) { c -= tail; sh.aged[k] = 1; }
-                    else sh.aged[k] = 0;
-                    sh.evalc[k] = c;
-                    sh.off[k] = o;
-                    o += (c + 31u) & ~31u;          // lists start on chunk boundaries
-                    sh.item_prefix[j] = it;
-                    it += ((c + 31u) >> 5) * (unsigned int)splits_of(k >> 1);
                     sh.dense_off[k] = dn;
-                    dn += c;
+                    dn += sh.evalc[k];
                 }
-                sh.item_prefix[kNumKeys] = it;
-                sh.item_next = 0;
                 sh.n_eval = dn;
                 sh.rest = 0;
             }
-#if FMC_EARLY_RESUME
-            if (tid < kSimChunks) sh.done[tid] = 0;
-#endif
             if (tid < kNumKeys) sh.cnt[parity ^ 1][tid] = 0;
             __syncthreads();
-#if FMC_REGROUP
             // ---- B2: regroup.  The game goes to thread dense_off[key] + rank (evaluated requests, key-major in the
             // order the keys are walked), every other game to the threads behind them.
             bool evald = key >= 0 && rank < sh.evalc[key];
@@ -952,71 +1041,13 @@ __global__ void __launch_bounds__(kSimThreads, kSimCtasPerSm) sim_kernel(const S
                 const Lane Ln = unpack_lane(P);
                 write_features<PLAYERS>(feats + (size_t)(pos >> 5) * kChunkFloats + (pos & 31), Ln, mykey >> 1, a, sh.M);
             }
-            const bool posted = evald;
             __syncthreads();
-#else
-            held = -1;
-            if (key >= 0) {
-                if (rank < sh.evalc[key]) {
-                    pos = (int)(sh.off[key] + rank);
-                    write_features<PLAYERS>(feats + (size_t)(pos >> 5) * kChunkFloats + (pos & 31), L, key >> 1, a, sh.M);
-                } else {
-                    held = key;
-                }
-            }
-            P = pack_lane(L);
-            const bool posted = key >= 0 && held < 0;
+            // ---- C: evaluate
+            walk_requests(sh, a, feats_saddr, kChunkFloats, results, lane, visits);
             __syncthreads();
-#endif
-            // ---- C: evaluate.  Work item = (key, chunk of 32 requests, output)
-            const unsigned int n_items = sh.item_prefix[kNumKeys];
-            for (;;) {
-                unsigned int it = 0;
-                if (lane == 0) it = atomicAdd(&sh.item_next, 1u);
-                it = __shfl_sync(0xFFFFFFFFu, it, 0);
-                if (it >= n_items) break;
-                int j = 0;
-                while (it >= sh.item_prefix[j + 1]) ++j;
-                const int k = kKeyOrder[j];
-                const int fam = k >> 1;
-                const unsigned int local = it - sh.item_prefix[j];
-                const int ns = splits_of(fam);
-                const unsigned int chunk = local / (unsigned int)ns;
-                const int out = (int)(local - chunk * (unsigned int)ns);
-                const unsigned int c = sh.evalc[k];
-                const unsigned int idx = chunk * 32u + (unsigned int)lane;
-                const bool live = idx < c;
-                const unsigned int p = sh.off[k] + idx;      // idle lanes walk whatever their column holds
-                uint32_t levels;
-                const double v = eval_output(fam, sh.M.tbl[fam][k & 1], out, a,
-                                             feats_saddr + (p >> 5) * (uint32_t)(kChunkFloats * 4) + (uint32_t)lane * 4u, lane, levels);
-                visits += (unsigned long long)levels * (live ? kIlp : 0);
-                if (live) {
-                    if (fam >= 2 && fam <= 4) results[(size_t)p * 3 + out] = v;
-                    else reinterpret_cast<float *>(results + (size_t)p * 3)[out] = (float)v;
-                }
-#if FMC_EARLY_RESUME
-                __syncwarp();                                   // the lanes' result stores are ordered before lane 0's release
-                if (lane == 0) {
-                    __threadfence_block();
-                    atomicAdd(&sh.done[(sh.off[k] >> 5) + chunk], 1u);
-                }
-#endif
-            }
-#if FMC_EARLY_RESUME
-            {
-                // wait for the outputs of this thread's own request only (every other warp may still be walking)
-                const unsigned int need = posted ? (unsigned int)splits_of(mykey >> 1) : 0u;
-                const volatile unsigned int *flag = &sh.done[posted ? (pos >> 5) : 0];
-                while (!__all_sync(0xFFFFFFFFu, need == 0u || *flag >= need)) { }
-                __threadfence_block();
-            }
-#else
-            __syncthreads();
-#endif
             parity ^= 1;
             rounds += 1;
-            requests += posted ? 1ULL : 0ULL;
+            requests += evald ? 1ULL : 0ULL;
         }
     }
     // ---- flush counters

@@ -1,7 +1,8 @@
 // Persistent simulation kernel with the exact rank-keyed memo (fmc_memo.hpp) in front of the tree walk.
 //
-// Same game rules, same draws, same arithmetic as sim_kernel (fmc_sim.cuh) -- results are bit-identical, the
-// parity tests run both.  What changes is the schedule:
+// The game rules are sim_kernel's own code: the trip loop calls the step functions of fmc_sim.cuh (new_game ...
+// after_yards) and its rounds use the same matchup pick, compaction, round plan and walk.  Results are bit-identical
+// to sim_kernel's; the parity tests run both.  What changes is the schedule:
 //
 //   * a request first computes its memo key (threshold ranks of its features on the specialised forest) and
 //     probes the table in HBM/L2; a hit continues the play at once, so a lane plays several plays per round;
@@ -31,42 +32,6 @@ __device__ __forceinline__ void memo_st(unsigned long long addr, unsigned long l
                  :: "l"(addr), "l"(k), "l"(v) : "memory");
 }
 
-__device__ __forceinline__ int stage_family(int stage) {      // ST_WAIT_* -> model id
-    return stage == ST_WAIT_PM ? 5 : stage - ST_WAIT_S1;      // S1, S2, PQ, RQ, SQ are consecutive
-}
-static_assert(ST_WAIT_S2 == ST_WAIT_S1 + 1 && ST_WAIT_PQ == ST_WAIT_S1 + 2 && ST_WAIT_RQ == ST_WAIT_S1 + 3 && ST_WAIT_SQ == ST_WAIT_S1 + 4,
-              "stage_family assumes consecutive wait stages");
-
-// Out-of-line copies of the pure scalar helpers for the trip loop: its code is several times the instruction cache that
-// 32 warps at different stages share (ncu: `stall_no_instruction` is the top stall of this kernel, 7.4 per issue), so the
-// helpers that are called from one or two places each are kept out of the loop body (FMC_MEMO_OUTLINE=1; measured 14 % SLOWER than inlining them -- 447 vs 393 ms at 4 M games: the calls cost more than the cache misses they save -- so the default keeps them inline).
-#ifndef FMC_MEMO_OUTLINE
-#define FMC_MEMO_OUTLINE 0
-#endif
-#if FMC_MEMO_OUTLINE
-#define FMC_MEMO_HELPER __device__ __noinline__
-#else
-#define FMC_MEMO_HELPER __device__ __forceinline__
-#endif
-FMC_MEMO_HELPER double m_pass_prob_v1(int down, double distance, double ytg, int sec, int sd) { return pass_prob_v1(down, distance, ytg, sec, sd); }
-FMC_MEMO_HELPER double m_go_for_it_prob(double ytg, double dist, int sd, int sec) { return go_for_it_prob(ytg, dist, sd, sec); }
-FMC_MEMO_HELPER int m_stage2_outcome(double r0, double r1, double r2, double u2) { const double raw[3] = {r0, r1, r2}; return stage2_outcome(raw, u2); }
-FMC_MEMO_HELPER double m_rz_finish_prob(double ytg, double tanh35, int down, bool pass) { return rz_finish_prob(ytg, tanh35, down, pass); }
-FMC_MEMO_HELPER double m_call_cut(double p_pass) {       // FMC:1064-1066: P(run) after the two normalisations of the play call
-    double a0 = 1.0 - p_pass, a1 = p_pass;
-    const double s = a0 + a1;
-    a0 = a0 / s; a1 = a1 / s;
-    return a0 / (a0 + a1);
-}
-FMC_MEMO_HELPER unsigned long long m_memo_key_xgb(const RankSpec *rs, int fam, int team, int matchup, int down, double dist, double ytg,
-                                                  int sd, int sec, float v1, float v2) {
-    return memo_key<true>(rs, fam, team, matchup, down, dist, ytg, sd, sec, v1, v2);
-}
-FMC_MEMO_HELPER unsigned long long m_memo_key_skl(const RankSpec *rs, int fam, int team, int matchup, int down, double dist, double ytg,
-                                                  int sd, int sec, float v1, float v2) {
-    return memo_key<false>(rs, fam, team, matchup, down, dist, ytg, sd, sec, v1, v2);
-}
-
 // Key of the request (family, team on offense) a lane is about to post.  The feature values are formed exactly as
 // write_features forms them (same float conversions, same play-model standardisation).
 template <bool XGB>
@@ -78,8 +43,7 @@ __device__ __forceinline__ unsigned long long lane_memo_key(const RankSpec *rs, 
         if (a.pm_scaled[1]) v1 = (float)((L.dist - a.pm_mean[1]) / a.pm_scale[1]);
         if (a.pm_scaled[2]) v2 = (float)((L.ytg - a.pm_mean[2]) / a.pm_scale[2]);
     }
-    return XGB ? m_memo_key_xgb(rs, fam, team, matchup, L.down, L.dist, L.ytg, sd, L.sec, v1, v2)
-               : m_memo_key_skl(rs, fam, team, matchup, L.down, L.dist, L.ytg, sd, L.sec, v1, v2);
+    return memo_key<XGB>(rs, fam, team, matchup, L.down, L.dist, L.ytg, sd, L.sec, v1, v2);
 }
 
 __device__ __forceinline__ unsigned long long memo_slot_addr(const MemoRegion &R, unsigned long long key) {
@@ -107,12 +71,6 @@ __device__ __forceinline__ void memo_insert(unsigned long long addr, unsigned lo
 
 // warp-level event tally of one trip: four words of five 6-bit fields each (a lane adds at most one per field and
 // trip, a field's warp sum is at most 32) -- except the probe count, which has a word of its own
-enum { EV_GO = 0, EV_FGA, EV_FG, EV_PUNT, EV_RUN, EV_PASS, EV_COMP, EV_INC, EV_INT, EV_SACK, EV_TD, EV_GAMES,
-       EV_HIT0, EV_HIT1, EV_HIT2, EV_HIT3, EV_HIT4, EV_HIT5, EV_N };
-__device__ __constant__ int kEvCounter[EV_N] = {FMC_C_GO, FMC_C_FGA, FMC_C_FG, FMC_C_PUNT, FMC_C_RUN, FMC_C_PASS, FMC_C_COMP,
-                                                FMC_C_INC, FMC_C_INT, FMC_C_SACK, FMC_C_TD, FMC_C_GAMES,
-                                                FMC_C_MEMO_HITS_FAM0, FMC_C_MEMO_HITS_FAM0 + 1, FMC_C_MEMO_HITS_FAM0 + 2,
-                                                FMC_C_MEMO_HITS_FAM0 + 3, FMC_C_MEMO_HITS_FAM0 + 4, FMC_C_MEMO_HITS_FAM0 + 5};
 constexpr int kEvWords = (EV_N + 4) / 5;
 constexpr int kWstat = 24;             // EV_N event totals, then plays, iters, probes
 static_assert(EV_N + 3 <= kWstat && EV_N + 3 <= 32, "one lane per tally");
@@ -139,16 +97,8 @@ constexpr int kMemoChunks = kMemoThreads / 32 + kNumKeys;        // every key's 
 constexpr size_t kMemoFeatBytes = (size_t)kMemoChunks * chunk_floats(false) * 4;
 constexpr size_t kMemoResultBytes = (size_t)kMemoChunks * 32 * 3 * 8;
 
-struct MemoShared {
-    MatchupDev M;
-    int cur_matchup;
-    int scan_from;                       // no matchup below this index has games left
-    unsigned int cnt[2][kNumKeys];
-    unsigned int off[kNumKeys], evalc[kNumKeys], aged[kNumKeys];
-    unsigned int item_prefix[kNumKeys + 1];
-    unsigned int item_next;
+struct MemoShared : RoundShared {
     unsigned int alive[2];
-    unsigned long long stat[FMC_N_COUNTERS];
     unsigned int waiting[2];             // warps that have left the trip loop this round (by round parity)
     unsigned long long wstat[kMemoThreads / 32][kWstat];  // per-warp event totals (EV_*, then plays, iters, probes), no atomics
 };
@@ -172,52 +122,18 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
 
     const uint32_t feats_saddr = (uint32_t)__cvta_generic_to_shared(feats);
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    for (int i = tid; i < kMemoChunks * 32; i += kMemoThreads)
-        feats[(size_t)(i >> 5) * kChunkFloats + kSimNinfRow * 32 + (i & 31)] = __int_as_float(0xff800000);
-    if (tid < FMC_N_COUNTERS) sh.stat[tid] = 0ULL;
+    init_rounds<kMemoThreads>(sh, feats, kChunkFloats);
     for (int i = tid; i < (kMemoThreads / 32) * kWstat; i += kMemoThreads) (&sh.wstat[0][0])[i] = 0ULL;
-    if (tid < kNumKeys) { sh.cnt[0][tid] = 0; sh.cnt[1][tid] = 0; sh.aged[tid] = 0; }
-    if (tid == 0) { sh.cur_matchup = -1; sh.scan_from = 0; sh.alive[0] = 0; sh.alive[1] = 0; sh.waiting[0] = 0; sh.waiting[1] = 0; }
+    if (tid == 0) { sh.alive[0] = 0; sh.alive[1] = 0; sh.waiting[0] = 0; sh.waiting[1] = 0; }
     __syncthreads();
 
-    PackedLane P;
-    {
-        Lane L0;
-        L0.game = 0; L0.dist = 0.0; L0.ytg = 0.0; L0.sec = 0; L0.down = 0; L0.offense = 0; L0.period = 0; L0.going = 0;
-        L0.iter = 0; L0.score[0] = 0; L0.score[1] = 0; L0.plays = 0; L0.p1 = 0; L0.wr = 0; L0.home = 0;
-        L0.stage = ST_IDLE;
-        P = pack_lane(L0);
-    }
+    PackedLane P = idle_lane();
     unsigned long long visits = 0;
     unsigned int rounds = 0, requests = 0, trips = 0;
 
     for (;;) {
-        if (tid == 0) {
-            // Waves: the CTAs of the grid share the kSlateWave lowest-numbered matchups that still have games (CTA b takes
-            // the (b mod kSlateWave)-th of them), and move up as matchups drain -- so a slate keeps a handful of node
-            // tables (and their memo entries) live at a time instead of one per CTA (720 x 0.6 MB for a season).
-            int found = -1, last = -1, seen = 0;
-            const int want = (int)(blockIdx.x % (unsigned)kSlateWave);
-            for (int m = sh.scan_from; m < a.n_matchups; ++m) {
-                if (*((volatile unsigned long long *)&a.next_game[m]) < a.matchups[m].game_end) {
-                    if (seen == 0) sh.scan_from = m;          // everything below is finished for good
-                    last = m;
-                    if (seen == want) { found = m; break; }
-                    if (++seen >= kSlateWave) break;
-                }
-            }
-            if (found < 0) found = last;                      // fewer unfinished matchups than the wave is wide
-            sh.cur_matchup = found;
-        }
-        __syncthreads();
-        const int m = sh.cur_matchup;
+        const int m = next_matchup<kMemoThreads>(sh, a);
         if (m < 0) break;
-        {
-            const uint32_t *src = reinterpret_cast<const uint32_t *>(a.matchups + m);
-            uint32_t *dst = reinterpret_cast<uint32_t *>(&sh.M);
-            for (int i = tid; i < (int)(sizeof(MatchupDev) / 4); i += kMemoThreads) dst[i] = src[i];
-        }
-        if (tid < kNumKeys) { sh.cnt[0][tid] = 0; sh.cnt[1][tid] = 0; sh.aged[tid] = 0; }
         if (tid == 0) { sh.alive[0] = 0; sh.alive[1] = 0; sh.waiting[0] = 0; sh.waiting[1] = 0; }
         __syncthreads();
         const MatchupDev &M = sh.M;
@@ -246,24 +162,17 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                 trips += 1;
                 EvTally ev;
                 uint32_t fin_plays = 0, fin_iters = 0, n_probes = 0;
-                // -- game over (FMC:1456-1464, 1501-1503)
+                // -- game over
                 const bool over = !parked && L.stage == ST_ITER && L.sec <= 0;
                 const unsigned int over_mask = __ballot_sync(FULL, over);
                 if (over) {
-                    const size_t oi = (size_t)(M.out_offset + (L.game - M.game_begin));
-                    if (a.scores) a.scores[oi] = (uint32_t)L.score[0] | ((uint32_t)L.score[1] << 16);
-                    if (a.iters) a.iters[oi] = (uint16_t)L.iter;
+                    const unsigned int bin = end_game_record<false>(L, a, M, m, sh.stat, ev);
                     if (a.hist) {
-                        const int ha = L.score[0] < FMC_HIST_BINS ? L.score[0] : FMC_HIST_BINS - 1;
-                        const int hb = L.score[1] < FMC_HIST_BINS ? L.score[1] : FMC_HIST_BINS - 1;
-                        if (L.score[0] >= FMC_HIST_BINS || L.score[1] >= FMC_HIST_BINS) atomicAdd(&sh.stat[FMC_C_HIST_OVERFLOW], 1ULL);
-                        const unsigned int bin = (unsigned int)(((L.game & 1ULL) * FMC_HIST_BINS + ha) * FMC_HIST_BINS + hb);
                         // warp-level reduce: lanes finishing in the same bin add once
                         const unsigned int peers = __match_any_sync(over_mask, bin);
                         if (lane == __ffs(peers) - 1)
                             atomicAdd(&a.hist[(size_t)m * 2 * FMC_HIST_BINS * FMC_HIST_BINS + bin], (unsigned int)__popc(peers));
                     }
-                    ev.hit(EV_GAMES);
                     fin_plays = (uint32_t)L.plays; fin_iters = (uint32_t)L.iter;
                     L.stage = ST_NEED_GAME;
                 }
@@ -279,13 +188,7 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                         if (need) {
                             const unsigned long long g = base + (unsigned long long)__popc(nm & ((1u << lane) - 1u));
                             if (g >= M.game_end) L.stage = ST_IDLE;
-                            else {
-                                L.game = g;
-                                L.offense = (int)(g & 1ULL);
-                                L.sec = 3600; L.down = 1; L.dist = 10.0; L.ytg = 75.0; L.period = 1; L.going = 0;
-                                L.score[0] = 0; L.score[1] = 0; L.iter = 0; L.plays = 0; L.p1 = 0; L.wr = 0;
-                                L.stage = ST_ITER;
-                            }
+                            else new_game(L, g);
                         }
                     }
                 }
@@ -296,60 +199,15 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                 Draws<TEST> D(a, M, m, Lv);
                 const int team = L.offense;
                 const int sd = L.score[team] - L.score[team ^ 1];
-                const double ytg0 = L.ytg;
                 __syncwarp();      // every stage of the trip is entered by the whole warp together
-                // -- iteration start: fourth down (handle_fourth FMC:1382-1421) and the play call
+                // -- iteration start: fourth down and the play call
                 if (!parked && L.stage == ST_ITER) {
-                    if (TEST && a.trace && L.iter < FMC_MAX_ITERS) {
-                        const int first = (int)(L.game & 1ULL);
-                        double *t = a.trace + ((size_t)(M.out_offset + (L.game - M.game_begin)) * FMC_MAX_ITERS + (size_t)L.iter) * FMC_TRACE_COLS;
-                        t[0] = (L.offense == first) ? 1.0 : 0.0; t[1] = (double)L.down; t[2] = (double)L.sec;
-                        t[3] = (double)L.score[first]; t[4] = (double)L.score[first ^ 1]; t[5] = L.dist; t[6] = L.ytg;
-                        t[7] = (double)L.going;
-                    }
+                    write_trace<TEST>(L, a, M);
                     L.iter += 1;
-                    bool play = true;
-                    if (L.down == 4) {
-                        const double ytg = L.ytg, dist = L.dist;
-                        const double p_go = pymin(1.0, m_go_for_it_prob(ytg, dist, sd, L.sec) * 1.15);
-                        if (D.u(S_U_GO) < p_go) {
-                            L.going = 1;
-                            ev.hit(EV_GO);
-                        } else if (ytg <= 38.0) {
-                            ev.hit(EV_FGA);
-                            const bool good = D.u(S_U_FG) < field_goal_prob(ytg + 17.0);
-                            tick_clock(L, 12);
-                            if (good) { ev.hit(EV_FG); L.score[team] += 3; change_possession(L, true, 75.0); }
-                            else change_possession(L, true, 100.0 - ytg);
-                            play = false;
-                        } else {
-                            ev.hit(EV_PUNT);
-                            const double gross = pymax(30.0, 43.0 + 6.0 * D.z(S_Z_GROSS));      // attempt_punt FMC:876-896
-                            const double ret = pymax(0.0, 6.0 + 3.0 * D.z(S_Z_RET));
-                            double net = gross - ret;
-                            if (ytg <= 60.0) {
-                                const double tb = softclip((60.0 - ytg) / 60.0, 0.10, 0.55);
-                                if (D.u(S_U_TB) < tb) net = ytg - 25.0;
-                            }
-                            net = softclip(net, 15.0, ytg - 1.0);
-                            const int inet = (int)net;
-                            tick_clock(L, 16);
-                            change_possession(L, true, softclip(100.0 - (ytg - (double)inet), 1.0, 99.0));
-                            play = false;
-                        }
-                    }
-                    if (play) {                                   // simulate_play FMC:1026-...: the play call
-                        L.plays += 1;
-                        if (a.policy == 1) L.stage = ST_WAIT_PM;
-                        else {
-                            const double c0 = m_call_cut(m_pass_prob_v1(L.down, L.dist, L.ytg, L.sec, sd));
-                            if (D.u(S_U_CALL) < c0) { ev.hit(EV_RUN); L.stage = ST_WAIT_RQ; }
-                            else { ev.hit(EV_PASS); L.stage = ST_WAIT_S1; }
-                        }
-                    }
+                    if (fourth_down(L, D, sd, ev)) L.stage = start_play<TEST, false>(L, a, M, D, sd, ev);
                 }
                 __syncwarp();      // every stage of the trip is entered by the whole warp together
-                // -- play model (policy 1): probe, then FMC:420-425
+                // -- play model (policy 1): probe, then the play call
                 if (a.policy == 1) {
                     if (!parked && !have && L.stage == ST_WAIT_PM) {
                         const RankSpec *rs = specs + 5 * 2 + team;
@@ -367,16 +225,12 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                         mg[0] = __uint_as_float((uint32_t)r[0]); mg[1] = __uint_as_float((uint32_t)(r[0] >> 32));
                         mg[2] = __uint_as_float((uint32_t)r[1]); mg[3] = __uint_as_float((uint32_t)(r[1] >> 32));
                         mg[4] = __uint_as_float((uint32_t)r[2]); mg[5] = 0.f;
-                        float e1, sum;
-                        play_softmax(mg, M.tbl[5][team].n_outputs, a.pass_class, a.play_temp, e1, sum);
-                        const double c0 = m_call_cut(softclip((double)(e1 / sum), 0.02, 0.98));
-                        if (D.u(S_U_CALL) < c0) { ev.hit(EV_RUN); L.stage = ST_WAIT_RQ; }
-                        else { ev.hit(EV_PASS); L.stage = ST_WAIT_S1; }
+                        L.stage = call_play<TEST, false>(L, a, M, D, team, p_pass_from_play_model(mg, M.tbl[5][team].n_outputs, a), ev);
                         have = false;
                     }
                 }
                 __syncwarp();      // every stage of the trip is entered by the whole warp together
-                // -- stage 1: probe, then FMC:1086-1087
+                // -- stage 1: probe, then the result
                 if (!parked && !have && L.stage == ST_WAIT_S1) {
                     const RankSpec *rs = specs + 0 * 2 + team;
                     unsigned long long key = 0ULL;
@@ -391,16 +245,11 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                 __syncwarp();      // every stage of the trip is entered by the whole warp together
                 bool s2_standin = false;
                 if (have && L.stage == ST_WAIT_S1) {
-                    const float m1 = __uint_as_float((uint32_t)r[0]);
-                    const double p1 = (double)(1.0f / (expf_cr(-m1) + 1.0f));                 // xgboost sigmoid, float32
-                    const double p_complete = softclip(p1 + M.bias[team], 0.02, 0.98);
                     have = false;
-                    if (D.u(S_U_COMP) < p_complete) { ev.hit(EV_COMP); L.stage = ST_WAIT_PQ; }
-                    else if (a.stage2_mode == 1) L.stage = ST_WAIT_S2;
-                    else s2_standin = true;
+                    s2_standin = after_stage1(L, a, M, D, team, __uint_as_float((uint32_t)r[0]), ev);
                 }
                 __syncwarp();      // every stage of the trip is entered by the whole warp together
-                // -- stage 2: probe, then the not-complete outcome FMC:751-770, 1157-1199
+                // -- stage 2: probe, then the not-complete outcome
                 if (!parked && !have && L.stage == ST_WAIT_S2) {
                     const RankSpec *rs = specs + 1 * 2 + team;
                     unsigned long long key = 0ULL;
@@ -414,40 +263,12 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                 }
                 __syncwarp();      // every stage of the trip is entered by the whole warp together
                 if ((have && L.stage == ST_WAIT_S2) || s2_standin) {
+                    const float mg[3] = {__uint_as_float((uint32_t)r[0]), __uint_as_float((uint32_t)(r[0] >> 32)),
+                                         __uint_as_float((uint32_t)r[1])};
                     double raw[3];
-                    if (!s2_standin) {
-                        float mg[3];
-                        mg[0] = __uint_as_float((uint32_t)r[0]); mg[1] = __uint_as_float((uint32_t)(r[0] >> 32)); mg[2] = __uint_as_float((uint32_t)r[1]);
-                        float wmax = mg[0];
-                        wmax = fmaxf(mg[1], wmax); wmax = fmaxf(mg[2], wmax);
-                        float e[3];
-                        double wsum = 0.0;
-#pragma unroll
-                        for (int k = 0; k < 3; ++k) { e[k] = expf_cr(mg[k] - wmax); wsum += (double)e[k]; }
-#pragma unroll
-                        for (int k = 0; k < 3; ++k) raw[k] = (double)(e[k] / (float)wsum);
-                    } else {
-                        raw[0] = a.standin[0]; raw[1] = a.standin[1]; raw[2] = a.standin[2];
-                    }
+                    stage2_raw(!s2_standin, mg, a, raw);
                     have = false;
-                    const int outcome = m_stage2_outcome(raw[0], raw[1], raw[2], D.u(S_U_S2));
-                    if (outcome == 0) {                                   // incomplete FMC:1160-1168
-                        ev.hit(EV_INC);
-                        L.down += 1; L.going = 0;
-                        tick_clock(L, 10);
-                        L.stage = ST_ITER;
-                    } else if (outcome == 2) {
-                        ev.hit(EV_SACK);
-                        L.stage = ST_WAIT_SQ;
-                    } else {                                              // intercepted FMC:1186-1199
-                        ev.hit(EV_INT);
-                        const double ret = softclip(6.0 + 5.0 * D.z(S_Z_INT), 0.0, L.ytg);
-                        const double spot = 100.0 - (L.ytg - ret);
-                        L.going = 0;
-                        change_possession(L, true, spot);
-                        tick_clock(L, 12);
-                        L.stage = ST_ITER;
-                    }
+                    after_stage2<TEST, false>(L, a, M, D, team, raw, ev);
                 }
                 __syncwarp();      // every stage of the trip is entered by the whole warp together
                 // -- yardage families: probe, then the outcome
@@ -467,39 +288,8 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                 if (have && L.stage >= ST_WAIT_PQ && L.stage <= ST_WAIT_SQ) {
                     const double q[3] = {__longlong_as_double((long long)r[0]), __longlong_as_double((long long)r[1]),
                                          __longlong_as_double((long long)r[2])};
-                    const double mz = M.mz[team];
                     have = false;
-                    if (L.stage == ST_WAIT_SQ) {                          // sack FMC:1170-1184
-                        double loss = -sample_yards(a, D, q, 0.25, -20.0, 0.0);
-                        loss = pymax(0.0, loss);
-                        loss = pymin(loss, 100.0 - (100.0 - L.ytg));
-                        L.ytg += loss; L.dist += loss; L.down += 1; L.going = 0;
-                        tick_clock(L, 24);
-                    } else {
-                        // completed pass FMC:1089-1152 / run FMC:1201-1257: the same steps with different constants
-                        const bool pass = L.stage == ST_WAIT_PQ;
-                        double yards = sample_yards(a, D, q, pass ? 0.4 : 0.35, pass ? 0.0 : -4.0, L.ytg) * M.ymul[team];
-                        if (ytg0 > 25.0 && D.u(S_U_EX) < (pass ? 0.60 : 0.5) * explosive_prob(mz, ytg0)) {
-                            const double ub = pass ? 0.35 + (0.95 - 0.35) * D.u(S_U_BOOST) : 0.2 + (0.5 - 0.2) * D.u(S_U_BOOST);
-                            yards *= 1.0 + ub * (1.0 + (pass ? 0.7 : 0.6) * mz);
-                            yards = pymin(yards, ytg0);
-                        }
-                        if (ytg0 <= (pass ? 12.0 : 9.0) && L.down <= 3) {
-                            if (D.u(S_U_FIN) < m_rz_finish_prob(ytg0, M.tanh35[team], L.down, pass)) yards = ytg0;
-                        }
-                        if (yards + 1e-9 >= ytg0) {
-                            ev.hit(EV_TD);
-                            L.score[team] += 7; L.going = 0;
-                            tick_clock(L, pass ? 20 : 28);
-                            change_possession(L, true, 75.0);
-                        } else {
-                            L.going = 0;
-                            advance_down(L, yards);
-                            tick_clock(L, pass ? 26 : 28);
-                            L.going = 0;
-                        }
-                    }
-                    L.stage = ST_ITER;
+                    after_yards<TEST, false>(L, a, M, D, team, q, ev);
                 }
                 __syncwarp();      // every stage of the trip is entered by the whole warp together
                 // -- warp tallies of this trip
@@ -524,16 +314,8 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
             }
             if (lane == 0) atomicAdd(&sh.waiting[parity], 1u);
             // ---- B: compact the requests that missed
-            const int key = parked ? stage_family(L.stage) * 2 + L.offense : -1;
-            unsigned int rank = 0;
-            {
-                const unsigned int peers = __match_any_sync(FULL, key);
-                const int leader = __ffs(peers) - 1;
-                unsigned int base = 0;
-                if (key >= 0 && lane == leader) base = atomicAdd(&sh.cnt[parity][key], (unsigned int)__popc(peers));
-                base = __shfl_sync(FULL, base, leader);
-                rank = base + (unsigned int)__popc(peers & ((1u << lane) - 1u));
-            }
+            const int key = parked ? request_key(L) : -1;
+            const unsigned int rank = request_rank(sh.cnt[parity], key, lane);
             if (__any_sync(FULL, L.stage != ST_IDLE) && lane == 0) sh.alive[parity] = 1u;
             P = pack_lane(L);
             const int total = __syncthreads_count(key >= 0);
@@ -549,21 +331,7 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                 continue;
             }
             if (tid == 0) {
-                unsigned int o = 0, it = 0;
-                for (int j = 0; j < kNumKeys; ++j) {
-                    const int k = kKeyOrder[j];
-                    unsigned int c = sh.cnt[parity][k];
-                    const unsigned int tail = c & 31u;
-                    if (tail != 0 && tail < kDeferBelow && !sh.aged[k]) { c -= tail; sh.aged[k] = 1; }
-                    else sh.aged[k] = 0;
-                    sh.evalc[k] = c;
-                    sh.off[k] = o;
-                    o += (c + 31u) & ~31u;
-                    sh.item_prefix[j] = it;
-                    it += ((c + 31u) >> 5) * (unsigned int)splits_of(k >> 1);
-                }
-                sh.item_prefix[kNumKeys] = it;
-                sh.item_next = 0;
+                plan_round(sh, parity);
                 sh.alive[parity ^ 1] = 0u;
                 sh.waiting[parity ^ 1] = 0u;
             }
@@ -575,34 +343,8 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                 requests += 1;
             }
             __syncthreads();
-            // ---- C: walk.  Work item = (key, chunk of 32 requests, output)
-            const unsigned int n_items = sh.item_prefix[kNumKeys];
-            for (;;) {
-                unsigned int it = 0;
-                if (lane == 0) it = atomicAdd(&sh.item_next, 1u);
-                it = __shfl_sync(FULL, it, 0);
-                if (it >= n_items) break;
-                int j = 0;
-                while (it >= sh.item_prefix[j + 1]) ++j;
-                const int k = kKeyOrder[j];
-                const int fam = k >> 1;
-                const unsigned int local = it - sh.item_prefix[j];
-                const int ns = splits_of(fam);
-                const unsigned int chunk = local / (unsigned int)ns;
-                const int out = (int)(local - chunk * (unsigned int)ns);
-                const unsigned int c = sh.evalc[k];
-                const unsigned int idx = chunk * 32u + (unsigned int)lane;
-                const bool live = idx < c;
-                const unsigned int p = sh.off[k] + idx;
-                uint32_t levels;
-                const double v = eval_output(fam, sh.M.tbl[fam][k & 1], out, a,
-                                             feats_saddr + (p >> 5) * (uint32_t)(kChunkFloats * 4) + (uint32_t)lane * 4u, lane, levels);
-                visits += (unsigned long long)levels * (live ? kIlp : 0);
-                if (live) {
-                    if (fam >= 2 && fam <= 4) results[(size_t)p * 3 + out] = v;
-                    else reinterpret_cast<float *>(results + (size_t)p * 3)[out] = (float)v;
-                }
-            }
+            // ---- C: walk
+            walk_requests(sh, a, feats_saddr, kChunkFloats, results, lane, visits);
             __syncthreads();
             parity ^= 1;
             rounds += 1;
@@ -618,7 +360,7 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
     if (tid < EV_N + 3) {
         unsigned long long s = 0ULL;
         for (int w = 0; w < kMemoThreads / 32; ++w) s += sh.wstat[w][tid];
-        const int ci = tid < EV_N ? kEvCounter[tid] : (tid == EV_N ? FMC_C_PLAYS : (tid == EV_N + 1 ? FMC_C_ITERS : FMC_C_MEMO_PROBES));
+        const int ci = tid < EV_N ? ev_counter(tid) : (tid == EV_N ? FMC_C_PLAYS : (tid == EV_N + 1 ? FMC_C_ITERS : FMC_C_MEMO_PROBES));
         sh.stat[ci] += s;
     }
     __syncthreads();
