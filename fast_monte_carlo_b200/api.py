@@ -26,6 +26,7 @@ from __future__ import annotations
 import os
 import threading
 import time
+from dataclasses import dataclass
 from typing import Dict, List, Optional, Sequence, Tuple
 
 import numpy as np
@@ -33,7 +34,7 @@ import pandas as pd
 
 from . import outputs
 from . import usage as _usage
-from .engine import Engine, MatchupSpec
+from .engine import Engine, GameState, MatchupSpec
 from .priors import (TeamContext, build_team_context_from_sp_flex, csv_base_from, load_sp_flex,
                      lookup_sp_flex, packaged_priors_path)
 
@@ -336,6 +337,98 @@ def simulate_slate(pairs: Sequence[Tuple[str, str]], n: int = 1000, *, sp_path: 
             entry["usage"] = uses[m]
             entry["props"] = _usage.scan_props_from_hist(ph[m], (a, b), uses[m], sheet)
         out[(a, b)] = entry
+    return out
+
+
+# ---------------------------------------------------------------------------------------------
+# live games: the rest of a game in progress, from any in-game state
+# ---------------------------------------------------------------------------------------------
+@dataclass(frozen=True)
+class LiveState:
+    """A game in progress as `simulate_live` takes it: `offense` = the NAME of the team with the ball, `score` = (points
+    of teamA, points of teamB) of the entry, `seconds` remaining in regulation, down, distance and yards to goal."""
+    offense: str
+    seconds: int
+    down: int
+    distance: float
+    yards_to_goal: float
+    score: Tuple[int, int] = (0, 0)
+
+
+def live_game_state(team_a: str, team_b: str, state) -> GameState:
+    """The engine's GameState of `state` (a LiveState, or a mapping with its fields) for the pair (team_a, team_b).
+    ValueError when the team with the ball is neither team, or a field is out of range."""
+    get = (lambda k: state[k]) if isinstance(state, dict) else (lambda k: getattr(state, k))
+    off = get("offense")
+    if off == team_a:
+        o = 0
+    elif off == team_b:
+        o = 1
+    else:
+        raise ValueError(f"Team '{off}' with the ball is neither '{team_a}' nor '{team_b}'.")
+    sc = tuple(get("score"))
+    return GameState(offense=o, seconds=int(get("seconds")), down=int(get("down")), distance=float(get("distance")),
+                     yards_to_goal=float(get("yards_to_goal")), score=(int(sc[0]), int(sc[1])))
+
+
+def simulate_live(entries: Sequence[Tuple[str, str, object]], games: int = 100_000, *, sp_path: Optional[str] = None,
+                  year: int = 2025, week: int = 1, seed: Optional[int] = None, engine: Optional[Engine] = None,
+                  markets: Optional[Dict[int, Dict[str, float]]] = None) -> List[Dict[str, object]]:
+    """Who wins from here?  Every entry (teamA, teamB, state) -- `state` a LiveState (or a mapping with its fields) --
+    plays `games` GAMES (not pairs) from its state, all entries in one launch: a win-probability curve (one pair, a state
+    per snap) and a live slate (many pairs) alike.  Entries of the same pair share one specialised table set and one memo,
+    so a curve costs little more than one entry with as many games.
+
+    Under torch.distributed every rank plays its `shard_range` slice of every entry's games and the integer histograms
+    are merged with ONE all-reduce (as in `simulate_slate`); the result does not depend on the number of ranks.
+    Returns a list in entry order of dicts: "state", "games", "hist" (the [128, 128] histogram of final (A, B) points,
+    both orientations summed), "p_win" ({teamA: p, teamB: p}), "p_tie" (regulation only, the reference has no overtime),
+    "mean_points" ({teamA: x, teamB: y}), "hist_overflow" (games in the last bin: a team with 127 or more points, which
+    the odds count as 127), and "markets": for entries whose index is in `markets` ({i: {"spread": s, "total": t}},
+    spread from teamA's side) the spread / total odds of `outputs.game_market_odds_from_hist`, else None.
+    Teams are rated from the SP+ table at `sp_path` (default: the packaged week-1 2025 table); `year` / `week` are
+    accepted as `simulate_slate` accepts them and change nothing here, since no usage data is read (every name is
+    "Unknown": player props are not returned)."""
+    import torch
+    import torch.distributed as dist
+    eng = engine if engine is not None else get_engine()
+    sp_df = load_sp_flex(sp_path if sp_path is not None else packaged_priors_path())
+    entries = list(entries)
+    if not entries:
+        raise ValueError("simulate_live needs at least one entry")
+    if int(games) < 1:
+        raise ValueError("games must be at least 1")
+    starts = []
+    sps = []
+    for a, b, st in entries:                  # same errors as the reference for unknown teams
+        sps.append((lookup_sp_flex(a, sp_df), lookup_sp_flex(b, sp_df)))
+        starts.append(live_game_state(a, b, st))
+    rank, world = 0, 1
+    if dist.is_available() and dist.is_initialized():
+        rank, world = dist.get_rank(), dist.get_world_size()
+    g0, g1 = shard_range(int(games), rank, world)
+    specs = [MatchupSpec(a, b, spa, spb, int(games), g0, g1, i * (g1 - g0), start=gs)
+             for i, ((a, b, _), (spa, spb), gs) in enumerate(zip(entries, sps, starts))]
+    dev = torch.device("cuda", eng.ctx.device)
+    hist = torch.zeros((len(specs), 2, outputs.HIST_BINS, outputs.HIST_BINS), dtype=torch.int32, device=dev)
+    with _ENGINE_LOCK:
+        eng.set_matchups(specs)
+        if g1 > g0:
+            st = torch.cuda.current_stream(dev)
+            eng.ctx.simulate_device(seed=_fresh_seed() if seed is None else int(seed), hist=hist.data_ptr(),
+                                    cuda_stream=st.cuda_stream)
+    hist64 = hist.to(torch.int64)
+    merge_histograms(hist64)
+    h = hist64.cpu().numpy()
+    out = []
+    for m, (a, b, st) in enumerate(entries):
+        h2 = h[m].sum(axis=0)
+        mk = (markets or {}).get(m) or {}
+        odds = outputs.live_odds_from_hist(h2, a, b, spread=mk.get("spread"), total=mk.get("total"))
+        last = outputs.HIST_BINS - 1
+        out.append({"state": st, "games": odds["games"], "hist": h2, "p_win": odds["p_win"], "p_tie": odds["p_tie"],
+                    "mean_points": odds["mean_points"],
+                    "hist_overflow": int(h2[last, :].sum() + h2[:last, last].sum()), "markets": odds["markets"]})
     return out
 
 

@@ -9,6 +9,7 @@
 #include <cstring>
 #include <string>
 #include <thread>
+#include <unordered_map>
 #include <vector>
 
 #include "fmc_sim.cuh"
@@ -201,6 +202,7 @@ struct fmc_ctx {
     HostForest forest[FMC_N_MODELS];
     fmc_params params;
     std::vector<fmc_matchup> matchups;
+    std::vector<fmc_game_state> starts;  // [n_matchups] start state of every entry (fmc_set_start_states), kickoff by default
     std::vector<fmc_team_usage> usage;   // [n_matchups][2] or empty (shipped configuration: every name "Unknown")
     struct NameRows { int8_t row[3][FMC_MAX_USAGE]; };
     std::vector<NameRows> name_rows;     // per team: the 0/1 feature row of every usage entry (-1: no model knows the name)
@@ -213,12 +215,14 @@ struct fmc_ctx {
     // device-side state of the last set_matchups
     TableArena sim_tables;
     MatchupDev *d_matchups = nullptr;
+    std::vector<MatchupDev> h_matchups;  // host copy of d_matchups: the range and start words are patched here, then copied
+    int n_specs = 0;                     // distinct specialisations of the current tables (memo ids 0 .. n_specs - 1)
     unsigned long long *d_next = nullptr;
     std::vector<unsigned long long> h_next;
     std::vector<int32_t> packed_slots;   // [n_matchups][FMC_N_MODELS][2]
     // exact memo (fmc_memo.hpp): rank specs of the current tables, table regions, mode
-    RankSpec *d_specs = nullptr;
-    std::vector<uint8_t> memo_ok;        // [n_matchups][kMemoFams][2] the forest's ranks fit the key
+    RankSpec *d_specs = nullptr;         // [n_specs][kMemoFams][2]
+    std::vector<uint8_t> memo_ok;        // [n_specs][kMemoFams][2] the forest's ranks fit the key
     std::vector<std::string> memo_why;   // why not, for diagnostics
     int memo_mode = 1, memo_max_trips = 8, memo_break_parked = 16, memo_break_waiting = kMemoThreads / 64;
     uint64_t memo_max_bytes = 0;
@@ -399,6 +403,20 @@ extern "C" int fmc_set_memo(fmc_ctx *c, int32_t mode, uint64_t max_bytes, int32_
     return FMC_OK;
 }
 
+static fmc_game_state kickoff_state() {
+    fmc_game_state s;
+    std::memset(&s, 0, sizeof(s));
+    s.offense = -1; s.seconds = 3600; s.down = 1; s.distance = 10.0; s.yards_to_goal = 75.0;
+    return s;
+}
+static StartDev start_dev(const fmc_game_state &s) {
+    StartDev d;
+    std::memset(&d, 0, sizeof(d));
+    d.dist = s.distance; d.ytg = s.yards_to_goal; d.sec = s.seconds; d.down = s.down; d.offense = s.offense;
+    d.score[0] = s.score[0]; d.score[1] = s.score[1];
+    return d;
+}
+
 extern "C" int fmc_set_matchups(fmc_ctx *c, int32_t n, const fmc_matchup *m) {
     if (!c || n <= 0 || !m) return fail(FMC_ERR_INVALID, "fmc_set_matchups: bad argument");
     for (int i = 0; i < n; ++i)
@@ -412,13 +430,17 @@ extern "C" int fmc_set_matchups(fmc_ctx *c, int32_t n, const fmc_matchup *m) {
                c->matchups[i].coach_col[0] == m[i].coach_col[0] && c->matchups[i].coach_col[1] == m[i].coach_col[1] &&
                // a matchup that had no games has no tables (build_tables skips it)
                (c->matchups[i].game_end > c->matchups[i].game_begin || m[i].game_end == m[i].game_begin);
+    // start states belong to a matchup list: every entry starts at the kickoff again
+    c->starts.assign(n, kickoff_state());
     if (same) {
         CK(cudaSetDevice(c->device));
         CK(cudaDeviceSynchronize());           // a launch in flight reads the ranges
         for (int i = 0; i < n; ++i) {
-            const unsigned long long r[3] = {m[i].game_begin, m[i].game_end, m[i].out_offset};
-            CK(cudaMemcpy(reinterpret_cast<char *>(c->d_matchups + i) + offsetof(MatchupDev, game_begin), r, sizeof(r), cudaMemcpyHostToDevice));
+            MatchupDev &M = c->h_matchups[i];
+            M.game_begin = m[i].game_begin; M.game_end = m[i].game_end; M.out_offset = m[i].out_offset;
+            M.start = start_dev(c->starts[i]);
         }
+        CK(cudaMemcpy(c->d_matchups, c->h_matchups.data(), c->h_matchups.size() * sizeof(MatchupDev), cudaMemcpyHostToDevice));
         c->matchups.assign(m, m + n);
         c->usage_pending = !c->usage.empty();   // the caller must repeat fmc_set_usage (or clear it): checked there
         return FMC_OK;
@@ -429,6 +451,39 @@ extern "C" int fmc_set_matchups(fmc_ctx *c, int32_t n, const fmc_matchup *m) {
     c->n_slots = 0;
     c->usage_pending = false;
     c->tables_dirty = true;
+    return FMC_OK;
+}
+
+extern "C" int fmc_set_start_states(fmc_ctx *c, int32_t n, const fmc_game_state *states) {
+    if (!c) return fail(FMC_ERR_INVALID, "fmc_set_start_states: ctx is NULL");
+    if (n != (int)c->matchups.size()) return fail(FMC_ERR_INVALID, "fmc_set_start_states: n_matchups differs from the last fmc_set_matchups");
+    std::vector<fmc_game_state> st(n, kickoff_state());
+    if (states) {
+        for (int i = 0; i < n; ++i) {
+            const fmc_game_state &s = states[i];
+            const std::string at = "fmc_set_start_states: entry " + std::to_string(i) + ": ";
+            if (s.offense < -1 || s.offense > 1) return fail(FMC_ERR_INVALID, at + "offense must be -1, 0 or 1");
+            if (s.seconds < 0 || s.seconds > 3600) return fail(FMC_ERR_INVALID, at + "seconds must be in 0..3600");
+            if (s.down < 1 || s.down > 4) return fail(FMC_ERR_INVALID, at + "down must be in 1..4");
+            if (s.score[0] < 0 || s.score[0] > 250 || s.score[1] < 0 || s.score[1] > 250)
+                return fail(FMC_ERR_INVALID, at + "scores must be in 0..250");
+            if (!std::isfinite(s.distance) || !(s.distance > 0.0) || s.distance > 100.0)
+                return fail(FMC_ERR_INVALID, at + "distance must be finite and in (0, 100]");
+            if (!(s.yards_to_goal > 0.0 && s.yards_to_goal < 100.0)) return fail(FMC_ERR_INVALID, at + "yards_to_goal must be in (0, 100)");
+            if (s.reserved != 0) return fail(FMC_ERR_INVALID, at + "reserved must be 0");
+            st[i] = s;
+        }
+    }
+    if (st.size() == c->starts.size() && std::memcmp(st.data(), c->starts.data(), st.size() * sizeof(fmc_game_state)) == 0)
+        return FMC_OK;                         // nothing changes (e.g. kickoff again after fmc_set_matchups)
+    c->starts.swap(st);
+    // the device records of the current tables get their new start words; dirty tables take them when they are built
+    if (!c->tables_dirty && c->d_matchups && c->h_matchups.size() == (size_t)n) {
+        CK(cudaSetDevice(c->device));
+        CK(cudaDeviceSynchronize());           // a launch in flight reads the start words
+        for (int i = 0; i < n; ++i) c->h_matchups[i].start = start_dev(c->starts[i]);
+        CK(cudaMemcpy(c->d_matchups, c->h_matchups.data(), c->h_matchups.size() * sizeof(MatchupDev), cudaMemcpyHostToDevice));
+    }
     return FMC_OK;
 }
 
@@ -504,7 +559,21 @@ static bool family_needed(const fmc_ctx *c, int fam) {
     return fam <= FMC_SACK_YARDS;
 }
 
-// Specialise + pack every needed forest for both orientations of every matchup; upload.
+// What the specialisation of an entry's forests depends on: the SP+ ratings folded into them, the coaches' play-model
+// columns and, in player mode, the usage tables and their name rows.  Entries with equal bytes here get the same tables.
+static std::string spec_inputs(const fmc_ctx *c, int i) {
+    const fmc_matchup &mu = c->matchups[i];
+    std::string k(reinterpret_cast<const char *>(mu.sp), sizeof(mu.sp));
+    k.append(reinterpret_cast<const char *>(mu.coach_col), sizeof(mu.coach_col));
+    if (!c->usage.empty()) {
+        k.append(reinterpret_cast<const char *>(&c->usage[(size_t)i * 2]), 2 * sizeof(fmc_team_usage));
+        k.append(reinterpret_cast<const char *>(&c->name_rows[(size_t)i * 2]), 2 * sizeof(fmc_ctx::NameRows));
+    }
+    return k;
+}
+
+// Specialise + pack every needed forest for both orientations of every distinct specialisation; upload.  Entries with
+// games whose specialisation inputs are equal share the tables, the rank specs and the memo id of the first of them.
 static int build_tables(fmc_ctx *c) {
     if (c->matchups.empty()) return fail(FMC_ERR_INVALID, "fmc_set_matchups has not been called");
     for (int fam = 0; fam < kNumFam; ++fam)
@@ -521,14 +590,28 @@ static int build_tables(fmc_ctx *c) {
     TableArena &A = c->sim_tables;
     A.clear();
     c->packed_slots.assign((size_t)n * FMC_N_MODELS * 2, 0);
-    // ---- specialise + pack every (matchup, orientation, family) forest; the jobs are independent, a slate
+    // ---- the representative of every entry with games: the first entry with games specialised alike (itself for a
+    // slate without repeated pairs); memo ids number the representatives in entry order
+    std::vector<int> rep(n, -1), memo_id(n, 0), reps;
+    {
+        std::unordered_map<std::string, int> first;
+        for (int i = 0; i < n; ++i) {
+            // a matchup without games on this context (another rank owns it: api.slate_specs(shard="matchups")) is never
+            // selected by the kernels, so it needs no tables: a rank specialises only the forests it will walk
+            if (c->matchups[i].game_end == c->matchups[i].game_begin) continue;
+            auto it = first.emplace(spec_inputs(c, i), i).first;
+            rep[i] = it->second;
+            if (rep[i] == i) { memo_id[i] = (int)reps.size(); reps.push_back(i); }
+            else memo_id[i] = memo_id[rep[i]];
+        }
+    }
+    c->n_specs = (int)reps.size();
+    const int ns = c->n_specs;
+    // ---- specialise + pack every (representative, orientation, family) forest; the jobs are independent, a slate
     // of hundreds of matchups is packed by all host threads
     struct Job { int matchup, off, fam; PackedForest pf; std::string err, memo_why; RankSpec spec; };
     std::vector<Job> jobs;
-    for (int i = 0; i < n; ++i) {
-        // a matchup without games on this context (another rank owns it: api.slate_specs(shard="matchups")) is never
-        // selected by the kernels, so it needs no tables: a rank specialises only the forests it will walk
-        if (c->matchups[i].game_end == c->matchups[i].game_begin) continue;
+    for (int i : reps) {
         for (int off = 0; off < 2; ++off)
             for (int fam = 0; fam < kNumFam; ++fam)
                 if (family_needed(c, fam)) { jobs.emplace_back(); jobs.back().matchup = i; jobs.back().off = off; jobs.back().fam = fam; }
@@ -584,6 +667,8 @@ static int build_tables(fmc_ctx *c) {
         MatchupDev &M = md[i];
         std::memset(&M, 0, sizeof(M));
         M.game_begin = mu.game_begin; M.game_end = mu.game_end; M.out_offset = mu.out_offset;
+        M.start = start_dev(c->starts[i]);
+        M.memo_id = memo_id[i];
         for (int off = 0; off < 2; ++off) {
             const int de = off ^ 1;
             const double O = mu.sp[off][1], D = mu.sp[de][2];
@@ -608,14 +693,14 @@ static int build_tables(fmc_ctx *c) {
             }
         }
     }
-    std::vector<RankSpec> specs((size_t)n * kMemoFams * 2);
+    std::vector<RankSpec> specs((size_t)(ns > 0 ? ns : 1) * kMemoFams * 2);
     std::memset(specs.data(), 0, specs.size() * sizeof(RankSpec));
-    c->memo_ok.assign((size_t)n * kMemoFams * 2, 0);
-    c->memo_why.assign((size_t)n * kMemoFams * 2, "family not in use");
+    c->memo_ok.assign((size_t)ns * kMemoFams * 2, 0);
+    c->memo_why.assign((size_t)ns * kMemoFams * 2, "family not in use");
     for (Job &j : jobs) {
         if (!j.err.empty()) return fail(FMC_ERR_CAPACITY, "packing model " + std::to_string(j.fam) + ": " + j.err);
         if (j.fam < kMemoFams) {
-            const size_t si = ((size_t)j.matchup * kMemoFams + j.fam) * 2 + j.off;
+            const size_t si = ((size_t)memo_id[j.matchup] * kMemoFams + j.fam) * 2 + j.off;
             specs[si] = j.spec;
             c->memo_ok[si] = j.spec.enabled ? 1 : 0;
             c->memo_why[si] = j.memo_why;
@@ -646,11 +731,19 @@ static int build_tables(fmc_ctx *c) {
         TableRef &T = md[q.matchup].tbl[q.fam][q.off];
         T.win_lo = (uint32_t)w; T.win_hi = (uint32_t)(w >> 32);
     }
+    // entries specialised like an earlier one share its tables
+    for (int i = 0; i < n; ++i) {
+        if (rep[i] < 0 || rep[i] == i) continue;
+        std::memcpy(md[i].tbl, md[rep[i]].tbl, sizeof(md[i].tbl));
+        std::memcpy(c->packed_slots.data() + (size_t)i * FMC_N_MODELS * 2, c->packed_slots.data() + (size_t)rep[i] * FMC_N_MODELS * 2,
+                    sizeof(int32_t) * FMC_N_MODELS * 2);
+    }
     cudaFree(c->d_matchups); cudaFree(c->d_next);
     c->d_matchups = nullptr; c->d_next = nullptr;
     CK(cudaMalloc(&c->d_matchups, md.size() * sizeof(MatchupDev)));
     CK(cudaMalloc(&c->d_next, (size_t)n * 8));
     CK(cudaMemcpy(c->d_matchups, md.data(), md.size() * sizeof(MatchupDev), cudaMemcpyHostToDevice));
+    c->h_matchups.swap(md);
     cudaFree(c->d_specs);
     c->d_specs = nullptr;
     CK(cudaMalloc(&c->d_specs, specs.size() * sizeof(RankSpec)));
@@ -812,7 +905,7 @@ extern "C" int fmc_simulate(fmc_ctx *c, const fmc_sim_args *g) {
         const size_t smem = sim_smem_bytes_players(a.name_rows);
         if (test) sim_kernel<true, true><<<grid, kSimThreads, smem, st>>>(a);
         else sim_kernel<false, true><<<grid, kSimThreads, smem, st>>>(a);
-    } else if (c->memo_mode != 0 && c->matchups.size() <= 1024) {
+    } else if (c->memo_mode != 0 && c->n_specs <= 1024) {     // the memo key has 10 bits for the specialisation
         // exact memo in front of the walk (fmc_sim_memo.cuh)
         MemoArgs mm;
         std::memset(&mm, 0, sizeof(mm));

@@ -38,7 +38,8 @@ constexpr int kMemoKeyBits = 47;        // rank bits available in the key
 constexpr int kMemoSdOffset = 256, kMemoSdLut = 512, kMemoSecLut = 3604, kMemoDownLut = 16;
 
 // What the kernel needs to turn a request of one (family, orientation) into its key.  Lives in global memory
-// (read through L1); one per (matchup, family, orientation).
+// (read through L1); one per (specialisation, family, orientation): entries of a launch whose forests are specialised
+// alike share one set.
 struct RankSpec {
     uint32_t enabled;                   // 0: this forest's ranks do not fit the key -> its requests are always walked
     uint32_t xgb;                       // compare: 1 -> right iff x >= t (xgboost), 0 -> right iff x > t (sklearn)
@@ -61,7 +62,7 @@ struct MemoRegion {
 
 struct MemoArgs {
     MemoRegion region[kMemoFams];
-    const RankSpec *specs;              // [n_matchups][kMemoFams][2]
+    const RankSpec *specs;              // [specialisations][kMemoFams][2], indexed by MatchupDev::memo_id
     int enabled;
     int max_trips;                      // stage steps a warp may run per round
     int break_parked;                   // a warp leaves the trip loop once this many of its lanes wait for the walk (or are idle)
@@ -90,12 +91,13 @@ __host__ __device__ __forceinline__ uint32_t memo_rank(const float *thr, float x
     return pos;
 }
 
-// Key of a request of (family, team on offense) in the state (down, distance, yardsToGoal, score_diff, seconds).
+// Key of a request of (family, team on offense) in the state (down, distance, yardsToGoal, score_diff, seconds) on the
+// specialisation `memo_id` (10 bits: at most 1024 specialisations per launch are memoised).
 // v1 / v2 are the distance / yardsToGoal FEATURE values as write_features forms them (float conversion, play-model
 // standardisation); the flags are derived exactly as `_fill_row` derives them (FMC:996-1021).  One implementation
 // for the kernel and for the host-side check (fmc_memo_keys_host).
 template <bool XGB>
-__host__ __device__ __forceinline__ unsigned long long memo_key(const RankSpec *rs, int fam, int team, int matchup, int down,
+__host__ __device__ __forceinline__ unsigned long long memo_key(const RankSpec *rs, int fam, int team, int memo_id, int down,
                                                                 double dist, double ytg, int sd, int sec, float v1, float v2) {
     const uint32_t fl = (ytg <= 20.0 ? 1u : 0u) | (dist >= (ytg - 0.5) ? 2u : 0u) | ((down == 4 && dist <= 2.0) ? 4u : 0u) |
                         (ytg <= 33.0 ? 8u : 0u) | (((sec % 1800) <= 120) ? 16u : 0u) | (sec > 1800 ? 0u : 32u);
@@ -113,7 +115,7 @@ __host__ __device__ __forceinline__ unsigned long long memo_key(const RankSpec *
     if (zm && v2 == 0.f) c2 = n2 + 1u;
     k |= (unsigned long long)c1 << FMC_MEMO_LD(&rs->shift[0]);
     k |= (unsigned long long)c2 << FMC_MEMO_LD(&rs->shift[1]);
-    return (1ULL << 63) | (k << 16) | ((unsigned long long)matchup << 6) | ((unsigned long long)fam << 3) | ((unsigned long long)team << 2);
+    return (1ULL << 63) | (k << 16) | ((unsigned long long)memo_id << 6) | ((unsigned long long)fam << 3) | ((unsigned long long)team << 2);
 }
 
 // ---- host: build the rank spec of one specialised forest ---------------------------------------------

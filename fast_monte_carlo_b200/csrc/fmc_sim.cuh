@@ -60,9 +60,22 @@ struct UsageDev {
     int8_t row[3][FMC_MAX_USAGE];    // 0/1 feature row of a name some model has a column for, -1 = lights nothing
 };
 
+// The state every game of a matchup entry starts from (include/fmc.h fmc_game_state); kickoff unless
+// fmc_set_start_states says otherwise.
+struct StartDev {
+    double dist, ytg;
+    int32_t sec, down;
+    int32_t offense;                 // -1: team (g & 1), the opening-kickoff rule; 0 / 1: that team
+    int32_t score[2];
+    int32_t reserved;
+};
+
 struct MatchupDev {
     double bias[2], ymul[2], mz[2], tanh35[2];
     unsigned long long game_begin, game_end, out_offset;
+    StartDev start;
+    int32_t memo_id;                 // specialisation of this entry: index of its RankSpec set and its memo key field
+    int32_t pad;
     TableRef tbl[kNumFam][2];
     UsageDev usage[2];               // player mode only
 };
@@ -470,12 +483,15 @@ static_assert(ST_WAIT_S2 == ST_WAIT_S1 + 1 && ST_WAIT_PQ == ST_WAIT_S1 + 2 && ST
 // key (family * 2 + team on offense) of the request a lane at a ST_WAIT_* stage waits for
 __device__ __forceinline__ int request_key(const Lane &L) { return stage_family(L.stage) * 2 + L.offense; }
 
-// game g of the matchup starts (simulate_game FMC:1428-1464); the parity of its id picks the team that receives first
-__device__ __forceinline__ void new_game(Lane &L, unsigned long long g) {
+// game g of the matchup starts (simulate_game FMC:1428-1464) from the entry's start record: at kickoff the parity of
+// its id picks the team that receives first.  The period follows from the clock as tick_clock derives it.
+__device__ __forceinline__ void new_game(Lane &L, const MatchupDev &M, unsigned long long g) {
     L.game = g;
-    L.offense = (int)(g & 1ULL);
-    L.sec = 3600; L.down = 1; L.dist = 10.0; L.ytg = 75.0; L.period = 1; L.going = 0;
-    L.score[0] = 0; L.score[1] = 0; L.iter = 0; L.plays = 0; L.p1 = 0; L.wr = 0;
+    L.offense = M.start.offense < 0 ? (int)(g & 1ULL) : M.start.offense;
+    L.sec = M.start.sec; L.down = M.start.down; L.dist = M.start.dist; L.ytg = M.start.ytg;
+    L.period = L.sec > 0 ? 4 - ((L.sec - 1) / 900) : 4;
+    L.going = 0;
+    L.score[0] = M.start.score[0]; L.score[1] = M.start.score[1]; L.iter = 0; L.plays = 0; L.p1 = 0; L.wr = 0;
     L.stage = ST_ITER;
 }
 
@@ -710,7 +726,7 @@ __device__ __forceinline__ int advance_lane(Lane &L, const SimKernelArgs &a, Sim
         if (L.stage == ST_NEED_GAME) {
             const unsigned long long g = atomicAdd(&a.next_game[matchup], 1ULL);
             if (g >= M.game_end) { L.stage = ST_IDLE; return -1; }
-            new_game(L, g);
+            new_game(L, M, g);
         }
         if (L.stage == ST_ITER) {
             if (L.sec <= 0) {

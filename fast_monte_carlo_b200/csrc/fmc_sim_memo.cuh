@@ -34,8 +34,9 @@ __device__ __forceinline__ void memo_st(unsigned long long addr, unsigned long l
 
 // Key of the request (family, team on offense) a lane is about to post.  The feature values are formed exactly as
 // write_features forms them (same float conversions, same play-model standardisation).
+// `memo_id` is the entry's specialisation (MatchupDev::memo_id): entries that share one share their memo entries.
 template <bool XGB>
-__device__ __forceinline__ unsigned long long lane_memo_key(const RankSpec *rs, int fam, int team, int matchup, const Lane &L,
+__device__ __forceinline__ unsigned long long lane_memo_key(const RankSpec *rs, int fam, int team, int memo_id, const Lane &L,
                                                             const SimKernelArgs &a) {
     const int sd = L.score[team] - L.score[team ^ 1];
     float v1 = (float)L.dist, v2 = (float)L.ytg;
@@ -43,7 +44,7 @@ __device__ __forceinline__ unsigned long long lane_memo_key(const RankSpec *rs, 
         if (a.pm_scaled[1]) v1 = (float)((L.dist - a.pm_mean[1]) / a.pm_scale[1]);
         if (a.pm_scaled[2]) v2 = (float)((L.ytg - a.pm_mean[2]) / a.pm_scale[2]);
     }
-    return memo_key<XGB>(rs, fam, team, matchup, L.down, L.dist, L.ytg, sd, L.sec, v1, v2);
+    return memo_key<XGB>(rs, fam, team, memo_id, L.down, L.dist, L.ytg, sd, L.sec, v1, v2);
 }
 
 __device__ __forceinline__ unsigned long long memo_slot_addr(const MemoRegion &R, unsigned long long key) {
@@ -137,7 +138,7 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
         if (tid == 0) { sh.alive[0] = 0; sh.alive[1] = 0; sh.waiting[0] = 0; sh.waiting[1] = 0; }
         __syncthreads();
         const MatchupDev &M = sh.M;
-        const RankSpec *specs = mm.specs + (size_t)m * kMemoFams * 2;
+        const RankSpec *specs = mm.specs + (size_t)M.memo_id * kMemoFams * 2;
         set_stage(P, ST_NEED_GAME);
         bool parked = false;           // the lane's request missed the memo and waits for the walk
         int pos = -1;                  // position of its request among this round's walked requests, -1 = not walked
@@ -188,7 +189,7 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                         if (need) {
                             const unsigned long long g = base + (unsigned long long)__popc(nm & ((1u << lane) - 1u));
                             if (g >= M.game_end) L.stage = ST_IDLE;
-                            else new_game(L, g);
+                            else new_game(L, M, g);
                         }
                     }
                 }
@@ -200,8 +201,8 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                 const int team = L.offense;
                 const int sd = L.score[team] - L.score[team ^ 1];
                 __syncwarp();      // every stage of the trip is entered by the whole warp together
-                // -- iteration start: fourth down and the play call
-                if (!parked && L.stage == ST_ITER) {
+                // -- iteration start: fourth down and the play call (a game that starts with the clock at 0 has none)
+                if (!parked && L.stage == ST_ITER && L.sec > 0) {
                     write_trace<TEST>(L, a, M);
                     L.iter += 1;
                     if (fourth_down(L, D, sd, ev)) L.stage = start_play<TEST, false>(L, a, M, D, sd, ev);
@@ -214,7 +215,7 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                         unsigned long long key = 0ULL;
                         bool hit = false;
                         if (mm.enabled && __ldg(&rs->enabled)) {
-                            key = lane_memo_key<true>(rs, 5, team, m, L, a);
+                            key = lane_memo_key<true>(rs, 5, team, M.memo_id, L, a);
                             hit = memo_probe<3>(memo_slot_addr(mm.region[5], key), key, r);
                             n_probes += 1; if (hit) ev.hit(EV_HIT5);
                         }
@@ -236,7 +237,7 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                     unsigned long long key = 0ULL;
                     bool hit = false;
                     if (mm.enabled && __ldg(&rs->enabled)) {
-                        key = lane_memo_key<true>(rs, 0, team, m, L, a);
+                        key = lane_memo_key<true>(rs, 0, team, M.memo_id, L, a);
                         hit = memo_probe<1>(memo_slot_addr(mm.region[0], key), key, r);
                         n_probes += 1; if (hit) ev.hit(EV_HIT0);
                     }
@@ -255,7 +256,7 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                     unsigned long long key = 0ULL;
                     bool hit = false;
                     if (mm.enabled && __ldg(&rs->enabled)) {
-                        key = lane_memo_key<true>(rs, 1, team, m, L, a);
+                        key = lane_memo_key<true>(rs, 1, team, M.memo_id, L, a);
                         hit = memo_probe<2>(memo_slot_addr(mm.region[1], key), key, r);
                         n_probes += 1; if (hit) ev.hit(EV_HIT1);
                     }
@@ -278,7 +279,7 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                     unsigned long long key = 0ULL;
                     bool hit = false;
                     if (mm.enabled && __ldg(&rs->enabled)) {
-                        key = lane_memo_key<false>(rs, fam, team, m, L, a);
+                        key = lane_memo_key<false>(rs, fam, team, M.memo_id, L, a);
                         hit = memo_probe<3>(memo_slot_addr(mm.region[fam], key), key, r);
                         n_probes += 1; if (hit) ev.w[(EV_HIT0 + fam) / 5] += 1u << (6 * ((EV_HIT0 + fam) % 5));
                     }

@@ -6,6 +6,7 @@ but as an object so that several engines (one per GPU / rank) can coexist.
 """
 from __future__ import annotations
 
+import math
 import os
 from dataclasses import dataclass
 from typing import Dict, Iterable, List, Optional, Sequence, Tuple
@@ -26,6 +27,38 @@ HEAD_COACH_MAP = {
 SIM_MODELS = ("pass_stage1", "pass_stage2", "pass_yards", "run_yards", "sack_yards", "play_model")
 
 
+@dataclass(frozen=True)
+class GameState:
+    """The state the games of a matchup entry start from: the rest of a game in progress (fmc_game_state).  The future of
+    a game depends on nothing else: the period follows from the clock and timeouts are never spent.  `offense` is a team
+    index (0 = team A, 1 = team B) or -1 = the kickoff rule (team g & 1 of game g has the ball); `score` = (points of A,
+    points of B).  The default is the opening kickoff."""
+    offense: int = -1
+    seconds: int = 3600
+    down: int = 1
+    distance: float = 10.0
+    yards_to_goal: float = 75.0
+    score: Tuple[int, int] = (0, 0)
+
+    def __post_init__(self):
+        if self.offense not in (-1, 0, 1):
+            raise ValueError("GameState.offense must be -1, 0 or 1")
+        if not (isinstance(self.seconds, (int, np.integer)) and 0 <= self.seconds <= 3600):
+            raise ValueError("GameState.seconds must be an integer in 0..3600")
+        if self.down not in (1, 2, 3, 4):
+            raise ValueError("GameState.down must be 1..4")
+        if len(self.score) != 2 or not all(isinstance(p, (int, np.integer)) and 0 <= p <= 250 for p in self.score):
+            raise ValueError("GameState.score must be two integers in 0..250")
+        d, y = float(self.distance), float(self.yards_to_goal)
+        if not (math.isfinite(d) and 0.0 < d <= 100.0):
+            raise ValueError("GameState.distance must be finite and in (0, 100]")
+        if not (0.0 < y < 100.0):
+            raise ValueError("GameState.yards_to_goal must be in (0, 100)")
+
+
+KICKOFF = GameState()
+
+
 @dataclass
 class MatchupSpec:
     """One team pair as the kernels see it."""
@@ -38,6 +71,7 @@ class MatchupSpec:
     game_end: int = 0
     out_offset: int = 0
     usage: Optional[tuple] = None        # (usage.TeamUsage of team A, of team B) or None = every name "Unknown"
+    start: Optional[GameState] = None    # state every game starts from; None = the opening kickoff
 
 
 class Engine:
@@ -119,6 +153,11 @@ class Engine:
             self.ctx.set_usage(teams, self.n_slots)
         else:
             self.n_slots = 0
+        # start states (fmc_set_start_states): an in-game state per entry, the kickoff for the others
+        if any(m.start is not None for m in self.matchups):
+            self.ctx.set_start_states([m.start if m.start is not None else KICKOFF for m in self.matchups])
+        else:
+            self.ctx.set_start_states(None)
 
     def simulate_host(self, seed: int, **kw) -> dict:
         return self.ctx.simulate_host(seed=seed, **kw)

@@ -62,6 +62,14 @@ class Matchup(C.Structure):
     ]
 
 
+class GameStateC(C.Structure):
+    """fmc_game_state"""
+    _fields_ = [
+        ("offense", C.c_int32), ("seconds", C.c_int32), ("down", C.c_int32), ("score", C.c_int32 * 2),
+        ("reserved", C.c_int32), ("distance", C.c_double), ("yards_to_goal", C.c_double),
+    ]
+
+
 class SimArgs(C.Structure):
     _fields_ = [
         ("seed", C.c_uint64), ("n_matchups", C.c_int32), ("reserved", C.c_int32),
@@ -151,6 +159,7 @@ def load_library():
     L.fmc_simulate_players_host.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                             C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.fmc_set_usage.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32]
+    L.fmc_set_start_states.argtypes = [C.c_void_p, C.c_int32, C.c_void_p]
     L.fmc_pack_forest_host_dyn.restype = C.c_int64
     L.fmc_pack_forest_host_dyn.argtypes = [C.POINTER(ForestDesc), C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32,
                                            C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64,
@@ -187,6 +196,7 @@ EXPORTED_SYMBOLS = (
     "fmc_gather_probe", "fmc_debug_errors",
     "fmc_pack_forest_host", "fmc_pack_forest_host_dyn", "fmc_set_usage", "fmc_simulate_players_host",
     "fmc_set_memo", "fmc_memo_keys_host", "fmc_gather_probe_coherent", "fmc_predict_stats", "fmc_invalidate_tables", "fmc_tree_predict_cols_host",
+    "fmc_set_start_states",
 )
 
 
@@ -396,6 +406,21 @@ class Context:
                         u.col[MODEL_INDEX[name]][e] = int(cols[e])
         _check(self._L.fmc_set_usage(self._h, len(teams), C.cast(arr, C.c_void_p), int(n_slots)))
         self.n_slots, self.has_usage = int(n_slots), True
+
+    def set_start_states(self, states) -> None:
+        """fmc_set_start_states: `states` = one state per matchup entry of the last set_matchups (objects with offense,
+        seconds, down, score, distance, yards_to_goal, such as engine.GameState; offense by team index), or None =
+        every entry starts at the kickoff."""
+        if states is None:
+            _check(self._L.fmc_set_start_states(self._h, self.n_matchups, None))
+            return
+        st = list(states)
+        arr = (GameStateC * max(len(st), 1))()
+        for i, g in enumerate(st):
+            arr[i].offense = int(g.offense); arr[i].seconds = int(g.seconds); arr[i].down = int(g.down)
+            arr[i].score[0], arr[i].score[1] = int(g.score[0]), int(g.score[1])
+            arr[i].distance = float(g.distance); arr[i].yards_to_goal = float(g.yards_to_goal)
+        _check(self._L.fmc_set_start_states(self._h, len(st), C.cast(arr, C.c_void_p)))
 
     MEMO_MODES = {"off": 0, "on": 1, "persistent": 2}
 

@@ -219,6 +219,33 @@ def game_market_odds_from_hist(hist2: np.ndarray, team: str, opp: str, *, team_i
     return out
 
 
+def live_odds_from_hist(hist2: np.ndarray, team_a: str, team_b: str, *, spread: Optional[float] = None,
+                        total: Optional[float] = None) -> Dict[str, object]:
+    """Odds of games played from a live state (api.simulate_live), over BOTH orientations: unlike a game from the
+    kickoff, the start state fixes who has the ball, so the game-id parity carries no meaning.  Returns games, p_win per
+    team, p_tie (the reference has no overtime), mean final points per team, and for `spread` (team A's line: A covers
+    when its margin beats -spread) / `total` the fields of `game_market_odds_from_hist` with team A as the team.
+    Scores past the last bin count as HIST_BINS - 1 points, as the histogram holds them."""
+    h = np.asarray(hist2).reshape(-1, HIST_BINS, HIST_BINS).sum(axis=0).astype(np.float64)
+    n = h.sum()
+    if n <= 0:
+        raise ValueError("the histogram holds no games")
+    a = np.arange(HIST_BINS, dtype=np.float64)[:, None]
+    b = np.arange(HIST_BINS, dtype=np.float64)[None, :]
+    p_a = float((h * (a > b)).sum() / n)
+    p_b = float((h * (b > a)).sum() / n)
+    out: Dict[str, object] = {
+        "games": int(n),
+        "p_win": {team_a: p_a, team_b: p_b},
+        "p_tie": float((h * (a == b)).sum() / n),
+        "mean_points": {team_a: float((h * a).sum() / n), team_b: float((h * b).sum() / n)},
+        "markets": None,
+    }
+    if spread is not None or total is not None:
+        out["markets"] = game_market_odds_from_hist(np.stack([h, np.zeros_like(h)]), team_a, team_b, spread=spread, total=total)
+    return out
+
+
 def summary_from_hist(hist2: np.ndarray, team_a: str, team_b: str) -> pd.DataFrame:
     """The `summary` frame of simulate_upcoming_matchup (FMC:1681-1687) from the histogram: each
     team's row covers the orientation in which it received the opening kickoff."""

@@ -101,6 +101,19 @@ typedef struct {
     uint64_t out_offset;  /* index of game_begin in the per-game output arrays */
 } fmc_matchup;
 
+/* The state a game starts from (fmc_set_start_states): the rest of a game in progress.  The future of a game depends on
+ * nothing else -- the period follows from the clock (4 - (seconds - 1) / 900, as the clock derives it, FMC:956-968) and
+ * timeouts are never spent (FMC:911-912).  Scores and `offense` are by team index of the matchup (0 = team A). */
+typedef struct {
+    int32_t offense;      /* team with the ball: 0 = A, 1 = B, -1 = team (g & 1) of game g (the kickoff rule) */
+    int32_t seconds;      /* seconds remaining, 0..3600 (0: the game is over, zero iterations) */
+    int32_t down;         /* 1..4 */
+    int32_t score[2];     /* points of team A, team B so far, 0..250 */
+    int32_t reserved;     /* must be 0 */
+    double distance;      /* yards to a first down, finite, in (0, 100] */
+    double yards_to_goal; /* in (0, 100) */
+} fmc_game_state;
+
 /* Usage table of one role of one team: TeamContext.qb_share / rush_share / target_share (FMC:262-264) as
  * the hot path reads them.  The engine samples an entry per play exactly as Generator.choice(len(df),
  * p=share) does (FMC:625-635: cdf = cumsum(share) / total, searchsorted(cdf, u, 'right')), feeds the models
@@ -200,6 +213,16 @@ int fmc_set_params(fmc_ctx *ctx, const fmc_params *p);
  * every loaded forest on the per-orientation constants and uploads the packed node tables. */
 int fmc_set_matchups(fmc_ctx *ctx, int32_t n, const fmc_matchup *m);
 
+/* Start states of the matchup entries of the last fmc_set_matchups: states[n_matchups], one per entry; every game of
+ * entry m starts from states[m] instead of the opening kickoff (sec 3600, 1st & 10 at the 75, 0-0, team (g & 1) with
+ * the ball).  states == NULL returns every entry to the kickoff.  fmc_set_matchups resets them to the kickoff.  Draws,
+ * outputs and the score histogram are unchanged in form: the Philox counter is (game, entry, iteration), the iteration
+ * count starts at 0 at the start state, histogram bin [m][g & 1] holds the final score.  Cheap: it neither
+ * re-specialises nor clears the memo (fmc_set_memo mode 2 keeps it); it only rewrites the start words of the device
+ * records, after the launches in flight.  FMC_ERR_INVALID for n_matchups different from the last fmc_set_matchups or a
+ * field out of range (see fmc_game_state). */
+int fmc_set_start_states(fmc_ctx *ctx, int32_t n_matchups, const fmc_game_state *states);
+
 /* Replaces the usage half of build_team_context_from_sp_flex (`_usage_from_focus_or_fallback`, FMC:228-249,
  * 1646-1659): teams[n_matchups][2] (team A, team B of each matchup of the last fmc_set_matchups), n_slots =
  * box lines per team in the per-game output.  teams == NULL returns to the shipped configuration (one
@@ -218,7 +241,9 @@ int fmc_set_usage(fmc_ctx *ctx, int32_t n_matchups, const fmc_team_usage *teams,
  * max_bytes: device memory the tables may take (0 = default: up to 1/4 of the free memory, at most 16 GiB; they
  * are sized by the games of the launch).  max_trips / break_parked: scheduling knobs of the memo kernel (stage steps a
  * warp may run per round; lanes of a warp that must wait for the walk before the warp ends its round); 0 = default.
- * Player mode (fmc_set_usage) and slates of more than 1024 matchups always run unmemoised. */
+ * Entries whose forests are specialised alike (same sp and coach_col, and in player mode the same usage tables) share
+ * one table set and one memo.  Player mode (fmc_set_usage) and launches of more than 1024 distinct specialisations
+ * always run unmemoised. */
 int fmc_set_memo(fmc_ctx *ctx, int32_t mode, uint64_t max_bytes, int32_t max_trips, int32_t break_parked);
 
 /* Replaces simulate_matchup's pool of _run_pair workers (FMC:1467-1521): plays every game of every
@@ -254,7 +279,8 @@ int fmc_tree_predict_cols_host(fmc_ctx *ctx, int32_t model_id, const double *row
                                double *out_host, int32_t tree_begin, int32_t tree_end);
 
 /* Packed-table statistics of the last fmc_set_matchups (slots per family/orientation), for
- * DESIGN.md / roofline accounting.  out[FMC_N_MODELS][2] = 8-byte slots of matchup `m`. */
+ * DESIGN.md / roofline accounting.  out[FMC_N_MODELS][2] = 8-byte slots of matchup `m` (of the table set it shares with
+ * the first entry specialised alike). */
 int fmc_packed_slots(fmc_ctx *ctx, int32_t m, int32_t *out);
 
 int fmc_sync(fmc_ctx *ctx);
