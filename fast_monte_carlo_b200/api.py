@@ -235,6 +235,37 @@ def merge_histograms(hist, counters=None):
     return hist, counters
 
 
+def _segment_buffer(n_entries: int, dev):
+    """The kernels' per-period histograms [n_entries][2][N_SEGMENTS][BINS][BINS] (768 KB an entry), zeroed."""
+    import torch
+    return torch.zeros((n_entries, 2, len(outputs.SEGMENTS), outputs.HIST_BINS, outputs.HIST_BINS), dtype=torch.int32,
+                       device=dev)
+
+
+def _merge_segments(hist, seg, counters=None):
+    """int64 copies of the score histograms and (when `seg` is not None) the period histograms, merged over ranks by ONE
+    `merge_histograms` all-reduce of the two laid end to end."""
+    import torch
+    if seg is None:
+        h64 = hist.to(torch.int64)
+        merge_histograms(h64, counters)
+        return h64, None
+    both = torch.cat([hist.reshape(-1), seg.reshape(-1)]).to(torch.int64)
+    merge_histograms(both, counters)
+    return both[:hist.numel()].reshape(hist.shape), both[hist.numel():].reshape(seg.shape)
+
+
+def _segment_lines(mk) -> None:
+    """ValueError unless every period line of a market entry ({..., "H1": {"spread": s, "total": t}}) is a mapping with
+    a spread and / or a total and nothing else."""
+    for name in outputs.SEGMENTS:
+        if name not in (mk or {}):
+            continue
+        line = mk[name]
+        if not isinstance(line, dict) or not line or not set(line) <= {"spread", "total"}:
+            raise ValueError(f"the {name} line must be a mapping with 'spread' and / or 'total', got {line!r}")
+
+
 def gather_player_box(local_rec, total_games: int):
     """The exchange step of the player path across ranks: every rank holds the per-game box of its contiguous
     game-id slice (`shard_range`), fmc_player_rec[games_local][2][n_slots]; one all-gather over the default
@@ -268,7 +299,7 @@ def gather_player_box(local_rec, total_games: int):
 def simulate_slate(pairs: Sequence[Tuple[str, str]], n: int = 1000, *, sp_path: Optional[str] = None,
                    year: int = 2025, week: int = 1, seed: Optional[int] = None,
                    engine: Optional[Engine] = None, markets: Optional[Dict[Tuple[str, str], Dict[str, float]]] = None,
-                   focus_csv: Optional[str] = None, usage_dir: str = "."):
+                   focus_csv: Optional[str] = None, usage_dir: str = ".", segments: bool = False):
     """A whole slate in one launch (BASELINE configs 3-4): every (teamA, teamB) of `pairs` is simulated for
     `n` PAIRS of games (2n games, A receives / B receives alternately, exactly like `simulate_matchup`).
 
@@ -285,6 +316,14 @@ def simulate_slate(pairs: Sequence[Tuple[str, str]], n: int = 1000, *, sp_path: 
     matchup also returns "player_hist" ([2][n_slots][PH_BINS], merged over ranks with the same all-reduce),
     "usage" and "props": `edge_finder.scan_props_for_matchup` (edge_finder.py:340-390) for the sheet's lines,
     computed from the histograms (`usage.player_prop_odds_from_hist`).
+
+    Periods: with `segments=True` every pair also returns "segments" = {name: {"hist", "odds"}} for each name of
+    `outputs.SEGMENTS` (quarters Q1..Q4, halves H1, H2; include/fmc.h defines them): "hist" = [2][BINS][BINS] of the
+    (A, B) points scored in the period per orientation (A receives first / B receives first), "odds" =
+    `outputs.segment_odds_from_hist` over BOTH orientations (the opening-kickoff coin toss is part of the pregame
+    uncertainty).  Period lines come through `markets` under the period's name:
+    {(A, B): {"spread": s, "H1": {"spread": s1, "total": t1}, "Q1": {...}}}.  The period histograms are merged over
+    ranks in the same all-reduce as the score histograms.
     """
     import torch
     import torch.distributed as dist
@@ -306,32 +345,47 @@ def simulate_slate(pairs: Sequence[Tuple[str, str]], n: int = 1000, *, sp_path: 
     eng.set_matchups(specs)
     with_players = eng.ctx.has_usage and eng.n_slots > 0
     dev = torch.device("cuda", eng.ctx.device)
+    if segments:
+        for mk in (markets or {}).values():
+            _segment_lines(mk)
     hist = torch.zeros((len(specs), 2, outputs.HIST_BINS, outputs.HIST_BINS), dtype=torch.int32, device=dev)
     counters = torch.zeros(len(native_counter_names()), dtype=torch.int64, device=dev)
     padded = torch.zeros(32, dtype=torch.int64, device=dev)
     st = torch.cuda.current_stream(dev)
     phist = (torch.zeros((len(specs), 2, eng.n_slots, _usage.PH_BINS), dtype=torch.int32, device=dev)
              if with_players else None)
+    seg = _segment_buffer(len(specs), dev) if segments else None
     eng.ctx.simulate_device(seed=_fresh_seed() if seed is None else int(seed), hist=hist.data_ptr(),
                             counters=padded.data_ptr(), cuda_stream=st.cuda_stream,
-                            player_hist=phist.data_ptr() if phist is not None else 0)
-    hist64 = hist.to(torch.int64)
+                            player_hist=phist.data_ptr() if phist is not None else 0,
+                            segment_hist=seg.data_ptr() if seg is not None else 0)
     counters.copy_(padded[:counters.numel()])
-    merge_histograms(hist64, counters)
+    hist64, seg64 = _merge_segments(hist, seg, counters)
     ph = None
     if phist is not None:
         ph64 = phist.to(torch.int64)
         merge_histograms(ph64)
         ph = ph64.cpu().numpy()
     h = hist64.cpu().numpy()
+    sgs = seg64.cpu().numpy() if seg64 is not None else None       # [pairs][2][N_SEGMENTS][BINS][BINS]
     c = counters.cpu().numpy()
     out: Dict[object, object] = {"_counters": {k: int(c[i]) for i, k in enumerate(native_counter_names())}}
     for m, (a, b) in enumerate(pairs):
         entry = {"hist": h[m], "games": int(h[m].sum()), "summary": outputs.summary_from_hist(h[m], a, b),
                  "moneyline": outputs.moneyline_from_hist(h[m], a, b), "markets": None}
         mk = (markets or {}).get((a, b))
-        if mk:
+        # with segments, a pair whose lines are all period lines has no final-score market
+        if mk and not (segments and set(mk) <= set(outputs.SEGMENTS)):
             entry["markets"] = outputs.game_market_odds_from_hist(h[m], a, b, spread=mk.get("spread"), total=mk.get("total"))
+        if sgs is not None:
+            sg = sgs[m]
+            entry["segments"] = {}
+            for k, name in enumerate(outputs.SEGMENTS):
+                both = sg[:, k].sum(axis=0)
+                line = (mk or {}).get(name) or {}
+                odds = (outputs.segment_odds_from_hist(both, a, b, spread=line.get("spread"), total=line.get("total"))
+                        if both.sum() > 0 else None)
+                entry["segments"][name] = {"hist": sg[:, k], "odds": odds}
         if ph is not None:
             entry["player_hist"] = ph[m]
             entry["usage"] = uses[m]
@@ -346,13 +400,107 @@ def simulate_slate(pairs: Sequence[Tuple[str, str]], n: int = 1000, *, sp_path: 
 @dataclass(frozen=True)
 class LiveState:
     """A game in progress as `simulate_live` takes it: `offense` = the NAME of the team with the ball, `score` = (points
-    of teamA, points of teamB) of the entry, `seconds` remaining in regulation, down, distance and yards to goal."""
+    of teamA, points of teamB) of the entry, `seconds` remaining in regulation, down, distance and yards to goal.
+    `quarter_start_score` / `half_start_score` (optional, (A, B) like `score`): the score when the current quarter and the
+    current half began; they let the odds of a period in progress cover the whole period.  A first-quarter state needs
+    neither (both are 0-0), a third-quarter state only one of them (the half and the quarter began together)."""
     offense: str
     seconds: int
     down: int
     distance: float
     yards_to_goal: float
     score: Tuple[int, int] = (0, 0)
+    quarter_start_score: Optional[Tuple[int, int]] = None
+    half_start_score: Optional[Tuple[int, int]] = None
+
+
+# (start, end) clock boundaries of every period of outputs.SEGMENTS; Q4 and H2 end with the game
+SEGMENT_BOUNDS = {"Q1": (3600, 2700), "Q2": (2700, 1800), "Q3": (1800, 900), "Q4": (900, None), "H1": (3600, 1800),
+                  "H2": (1800, None)}
+
+
+def quarter_of(seconds: int) -> int:
+    """The quarter of a clock reading, as the engine derives it: 4 - (seconds - 1) // 900, and 4 at 0."""
+    return 4 - (int(seconds) - 1) // 900 if seconds > 0 else 4
+
+
+def period_starts(state) -> Tuple[Optional[Tuple[int, int]], Optional[Tuple[int, int]]]:
+    """(score when the current quarter began, score when the current half began) of a LiveState (or a mapping with its
+    fields), each None when it is neither given nor implied (the clock implies 0-0 in the first quarter and half, and
+    the current score exactly on a quarter boundary).  ValueError for contradictory values: a start score that is not
+    componentwise half start <= quarter start <= score, a non-zero half start in the first half or a non-zero quarter
+    start in the first quarter, quarter and half start scores that differ in the third quarter, a start score of the
+    period that begins on a boundary state other than the score."""
+    get = (lambda k: state.get(k)) if isinstance(state, dict) else (lambda k: getattr(state, k, None))
+    sec = int(get("seconds"))
+    score = tuple(int(x) for x in get("score"))
+    qs, hs = get("quarter_start_score"), get("half_start_score")
+    qs = None if qs is None else tuple(int(x) for x in qs)
+    hs = None if hs is None else tuple(int(x) for x in hs)
+    for name, v in (("quarter_start_score", qs), ("half_start_score", hs)):
+        if v is not None and len(v) != 2:
+            raise ValueError(f"{name} must be (points A, points B)")
+    q = quarter_of(sec)
+    if q <= 2:
+        if hs is not None and hs != (0, 0):
+            raise ValueError(f"half_start_score {hs} in the first half: the half began at 0-0")
+        hs = (0, 0)
+    if q == 1:
+        if qs is not None and qs != (0, 0):
+            raise ValueError(f"quarter_start_score {qs} in the first quarter: the quarter began at 0-0")
+        qs = (0, 0)
+    if q == 3:
+        if qs is not None and hs is not None and qs != hs:
+            raise ValueError(f"quarter_start_score {qs} and half_start_score {hs} differ in the third quarter")
+        qs = hs = qs if qs is not None else hs
+    if sec in (2700, 1800, 900):
+        # on a boundary the quarter (and at 1800 the half) has just begun: the play that crossed it belongs to the
+        # previous quarter, so the current one began at the current score
+        for name, v in (("quarter_start_score", qs), ("half_start_score", hs if sec == 1800 else None)):
+            if v is not None and v != score:
+                raise ValueError(f"{name} {v} at {sec} s: the period began at the score {score}")
+        qs = score
+        if sec == 1800:
+            hs = score
+    le = lambda x, y: x[0] <= y[0] and x[1] <= y[1]
+    if qs is not None and not le(qs, score):
+        raise ValueError(f"quarter_start_score {qs} exceeds the score {score}")
+    if hs is not None and not le(hs, score):
+        raise ValueError(f"half_start_score {hs} exceeds the score {score}")
+    if qs is not None and hs is not None and not le(hs, qs):
+        raise ValueError(f"half_start_score {hs} exceeds quarter_start_score {qs}")
+    return qs, hs
+
+
+def live_segments(state, seg_hist: np.ndarray, team_a: str, team_b: str, lines=None) -> Dict[str, Dict[str, object]]:
+    """The periods of a live entry from its [N_SEGMENTS][BINS][BINS] histograms (both orientations summed): for every name
+    of outputs.SEGMENTS {"status", "offset", "hist", "odds"}.  status "ended": the period ended at or before the state;
+    its histogram is empty and its odds None.  "in_progress": the histogram counts from the state; `offset` = the points
+    already scored in the period (from `period_starts`), and the odds cover the whole period, or are None when the
+    period's start score is unknown (offset None).  "future": the period starts after the state.  `lines`: a market entry
+    with the period lines under the periods' names ({"H1": {"spread": s, "total": t}, ...})."""
+    get = (lambda k: state.get(k)) if isinstance(state, dict) else (lambda k: getattr(state, k, None))
+    sec = int(get("seconds"))
+    score = tuple(int(x) for x in get("score"))
+    qs, hs = period_starts(state)
+    _segment_lines(lines)
+    out: Dict[str, Dict[str, object]] = {}
+    for k, name in enumerate(outputs.SEGMENTS):
+        begin, end = SEGMENT_BOUNDS[name]
+        h = np.asarray(seg_hist[k])
+        if end is not None and sec <= end:
+            out[name] = {"status": "ended", "offset": None, "hist": np.zeros_like(h), "odds": None}
+            continue
+        if sec > begin:
+            status, offset = "future", (0, 0)
+        else:
+            base = (0, 0) if begin == 3600 else (hs if name in ("Q3", "H2") else qs)
+            status, offset = "in_progress", None if base is None else (score[0] - base[0], score[1] - base[1])
+        line = (lines or {}).get(name) or {}
+        odds = (outputs.segment_odds_from_hist(h, team_a, team_b, offset=offset, spread=line.get("spread"),
+                                               total=line.get("total")) if offset is not None and h.sum() > 0 else None)
+        out[name] = {"status": status, "offset": offset, "hist": h, "odds": odds}
+    return out
 
 
 def live_game_state(team_a: str, team_b: str, state) -> GameState:
@@ -373,7 +521,7 @@ def live_game_state(team_a: str, team_b: str, state) -> GameState:
 
 def simulate_live(entries: Sequence[Tuple[str, str, object]], games: int = 100_000, *, sp_path: Optional[str] = None,
                   year: int = 2025, week: int = 1, seed: Optional[int] = None, engine: Optional[Engine] = None,
-                  markets: Optional[Dict[int, Dict[str, float]]] = None) -> List[Dict[str, object]]:
+                  markets: Optional[Dict[int, Dict[str, float]]] = None, segments: bool = False) -> List[Dict[str, object]]:
     """Who wins from here?  Every entry (teamA, teamB, state) -- `state` a LiveState (or a mapping with its fields) --
     plays `games` GAMES (not pairs) from its state, all entries in one launch: a win-probability curve (one pair, a state
     per snap) and a live slate (many pairs) alike.  Entries of the same pair share one specialised table set and one memo,
@@ -388,7 +536,13 @@ def simulate_live(entries: Sequence[Tuple[str, str, object]], games: int = 100_0
     spread from teamA's side) the spread / total odds of `outputs.game_market_odds_from_hist`, else None.
     Teams are rated from the SP+ table at `sp_path` (default: the packaged week-1 2025 table); `year` / `week` are
     accepted as `simulate_slate` accepts them and change nothing here, since no usage data is read (every name is
-    "Unknown": player props are not returned)."""
+    "Unknown": player props are not returned).
+
+    Periods: with `segments=True` every entry also returns "segments" = `live_segments(...)`: per period of
+    `outputs.SEGMENTS` its status (ended / in_progress / future), the histogram of the points scored in it from the
+    state on (both orientations summed) and its odds, with the period lines of `markets` under the period's name
+    ({i: {"spread": s, "H2": {"spread": s2, "total": t2}}}).  A period in progress is priced as a whole when its start
+    score is known (LiveState.quarter_start_score / half_start_score, or implied by the clock)."""
     import torch
     import torch.distributed as dist
     eng = engine if engine is not None else get_engine()
@@ -400,9 +554,12 @@ def simulate_live(entries: Sequence[Tuple[str, str, object]], games: int = 100_0
         raise ValueError("games must be at least 1")
     starts = []
     sps = []
-    for a, b, st in entries:                  # same errors as the reference for unknown teams
+    for m, (a, b, st) in enumerate(entries):  # same errors as the reference for unknown teams
         sps.append((lookup_sp_flex(a, sp_df), lookup_sp_flex(b, sp_df)))
         starts.append(live_game_state(a, b, st))
+        period_starts(st)
+        if segments:
+            _segment_lines((markets or {}).get(m))
     rank, world = 0, 1
     if dist.is_available() and dist.is_initialized():
         rank, world = dist.get_rank(), dist.get_world_size()
@@ -411,15 +568,16 @@ def simulate_live(entries: Sequence[Tuple[str, str, object]], games: int = 100_0
              for i, ((a, b, _), (spa, spb), gs) in enumerate(zip(entries, sps, starts))]
     dev = torch.device("cuda", eng.ctx.device)
     hist = torch.zeros((len(specs), 2, outputs.HIST_BINS, outputs.HIST_BINS), dtype=torch.int32, device=dev)
+    seg = _segment_buffer(len(specs), dev) if segments else None
     with _ENGINE_LOCK:
         eng.set_matchups(specs)
         if g1 > g0:
             st = torch.cuda.current_stream(dev)
             eng.ctx.simulate_device(seed=_fresh_seed() if seed is None else int(seed), hist=hist.data_ptr(),
-                                    cuda_stream=st.cuda_stream)
-    hist64 = hist.to(torch.int64)
-    merge_histograms(hist64)
+                                    cuda_stream=st.cuda_stream, segment_hist=seg.data_ptr() if seg is not None else 0)
+    hist64, seg64 = _merge_segments(hist, seg)
     h = hist64.cpu().numpy()
+    sg = seg64.sum(dim=1).cpu().numpy() if seg64 is not None else None      # [entries][N_SEGMENTS][BINS][BINS]
     out = []
     for m, (a, b, st) in enumerate(entries):
         h2 = h[m].sum(axis=0)
@@ -429,6 +587,8 @@ def simulate_live(entries: Sequence[Tuple[str, str, object]], games: int = 100_0
         out.append({"state": st, "games": odds["games"], "hist": h2, "p_win": odds["p_win"], "p_tie": odds["p_tie"],
                     "mean_points": odds["mean_points"],
                     "hist_overflow": int(h2[last, :].sum() + h2[:last, last].sum()), "markets": odds["markets"]})
+        if sg is not None:
+            out[-1]["segments"] = live_segments(st, sg[m], a, b, mk)
     return out
 
 

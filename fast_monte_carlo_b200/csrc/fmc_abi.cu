@@ -235,7 +235,7 @@ struct fmc_ctx {
     bool launched = false;
     // fmc_simulate_host: device scratch + pinned staging, kept between calls
     struct Scratch { void *dev = nullptr; size_t dev_bytes = 0; };
-    Scratch scr[8];
+    Scratch scr[11];     // 0..7 fmc_simulate_host's buffers, 8 the period rows of fmc_simulate_segments, 9..10 its host path
     // pinned staging of the large device -> host copies of fmc_simulate_host (two buffers: the DMA of one chunk overlaps
     // the host copy of the previous one into the caller's pageable buffer)
     void *pin[2] = {nullptr, nullptr};
@@ -295,12 +295,19 @@ extern "C" int fmc_create(int device, fmc_ctx **out) {
     c->params.stage2_standin[0] = (double)0.78f;
     c->params.stage2_standin[1] = (double)0.05f;
     c->params.stage2_standin[2] = (double)0.17f;
-    CKC(cudaFuncSetAttribute(sim_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_smem_bytes(false)));
-    CKC(cudaFuncSetAttribute(sim_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_smem_bytes(false)));
-    CKC(cudaFuncSetAttribute(sim_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_smem_bytes(true)));
-    CKC(cudaFuncSetAttribute(sim_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_smem_bytes(true)));
-    CKC(cudaFuncSetAttribute(sim_memo_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_memo_smem_bytes()));
-    CKC(cudaFuncSetAttribute(sim_memo_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_memo_smem_bytes()));
+    CKC(cudaFuncSetAttribute(sim_kernel<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_smem_bytes(false)));
+    CKC(cudaFuncSetAttribute(sim_kernel<true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_smem_bytes(false)));
+    CKC(cudaFuncSetAttribute(sim_kernel<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_smem_bytes(true)));
+    CKC(cudaFuncSetAttribute(sim_kernel<true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_smem_bytes(true)));
+    CKC(cudaFuncSetAttribute(sim_memo_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_memo_smem_bytes()));
+    CKC(cudaFuncSetAttribute(sim_memo_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_memo_smem_bytes()));
+    // the instantiations with the period hooks (fmc_simulate_segments)
+    CKC(cudaFuncSetAttribute(sim_kernel<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_smem_bytes(false)));
+    CKC(cudaFuncSetAttribute(sim_kernel<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_smem_bytes(false)));
+    CKC(cudaFuncSetAttribute(sim_kernel<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_smem_bytes(true)));
+    CKC(cudaFuncSetAttribute(sim_kernel<true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_smem_bytes(true)));
+    CKC(cudaFuncSetAttribute(sim_memo_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_memo_smem_bytes()));
+    CKC(cudaFuncSetAttribute(sim_memo_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_memo_smem_bytes()));
     CKC(cudaEventCreateWithFlags(&c->ev_done, cudaEventDisableTiming));
     CKC(cudaMalloc(&c->d_pred_stats, 16));
     CKC(cudaMemset(c->d_pred_stats, 0, 16));
@@ -840,7 +847,26 @@ static size_t memo_layout(fmc_ctx *c, uint64_t games, MemoRegion (&R)[kMemoFams]
     return need;
 }
 
-extern "C" int fmc_simulate(fmc_ctx *c, const fmc_sim_args *g) {
+static cudaError_t scratch(fmc_ctx *c, int slot, size_t bytes, void **out);
+
+// The kernel of a launch: player mode, the memo kernel or the plain one; injected draws / traces (TEST); period
+// outputs (SEG).
+template <bool SEG>
+static void launch_sim(const SimKernelArgs &a, const MemoArgs *mm, bool players, bool test, int grid, int mgrid, size_t smem,
+                       cudaStream_t st) {
+    if (players) {
+        if (test) sim_kernel<true, true, SEG><<<grid, kSimThreads, smem, st>>>(a);
+        else sim_kernel<false, true, SEG><<<grid, kSimThreads, smem, st>>>(a);
+    } else if (mm) {
+        if (test) sim_memo_kernel<true, SEG><<<mgrid, kMemoThreads, sim_memo_smem_bytes(), st>>>(a, *mm);
+        else sim_memo_kernel<false, SEG><<<mgrid, kMemoThreads, sim_memo_smem_bytes(), st>>>(a, *mm);
+    } else {
+        if (test) sim_kernel<true, false, SEG><<<grid, kSimThreads, sim_smem_bytes(false), st>>>(a);
+        else sim_kernel<false, false, SEG><<<grid, kSimThreads, sim_smem_bytes(false), st>>>(a);
+    }
+}
+
+static int simulate_impl(fmc_ctx *c, const fmc_sim_args *g, const fmc_segment_args *seg) {
     if (!c || !g) return fail(FMC_ERR_INVALID, "fmc_simulate: bad argument");
     CK(cudaSetDevice(c->device));
     settle_usage(c);
@@ -853,10 +879,20 @@ extern "C" int fmc_simulate(fmc_ctx *c, const fmc_sim_args *g) {
     cudaStream_t st = (cudaStream_t)g->stream;
     // one launch in flight per context: the work counters, the running player boxes and the memo are per context
     if (c->launched) CK(cudaStreamWaitEvent(st, c->ev_done, 0));
-    uint64_t games = 0;
+    uint64_t games = 0, out_games = 0;
     for (size_t i = 0; i < c->matchups.size(); ++i) {
         c->h_next[i] = c->matchups[i].game_begin;
         games += c->matchups[i].game_end - c->matchups[i].game_begin;
+        const uint64_t hi = c->matchups[i].out_offset + (c->matchups[i].game_end - c->matchups[i].game_begin);
+        if (hi > out_games) out_games = hi;
+    }
+    const bool segs = seg && (seg->period_scores_dev || seg->segment_hist_dev);
+    uint32_t *rows = segs ? seg->period_scores_dev : nullptr;
+    if (segs && !rows && out_games) {
+        // the per-game rows are the state of the period hooks: device scratch when the caller only wants the histograms
+        void *p = nullptr;
+        CK(scratch(c, 8, (size_t)out_games * 3 * sizeof(uint32_t), &p));
+        rows = (uint32_t *)p;
     }
     CK(cudaMemcpyAsync(c->d_next, c->h_next.data(), c->h_next.size() * 8, cudaMemcpyHostToDevice, st));
     SimKernelArgs a;
@@ -878,6 +914,7 @@ extern "C" int fmc_simulate(fmc_ctx *c, const fmc_sim_args *g) {
     }
     a.scores = g->scores_dev; a.hist = g->hist_dev; a.counters = (unsigned long long *)g->counters_dev;
     a.stream = g->stream_dev; a.trace = g->trace_dev; a.iters = g->iters_dev;
+    a.period_scores = rows; a.segment_hist = segs ? seg->segment_hist_dev : nullptr;
     const bool players = !c->usage.empty();
     if ((g->players_dev || g->player_hist_dev) && !players)
         return fail(FMC_ERR_INVALID, "fmc_simulate: players_dev / player_hist_dev need fmc_set_usage");
@@ -899,15 +936,16 @@ extern "C" int fmc_simulate(fmc_ctx *c, const fmc_sim_args *g) {
     debug_set_range(c->sim_tables);
 #endif
     const bool test = a.stream || a.trace;      // parity-test instantiation
+    size_t smem = 0;
+    MemoArgs mm;
+    bool memo = false;
     if (players) {
         a.n_prow = c->n_prow; a.n_trow = c->n_trow; a.n_rrow = c->n_rrow;
         a.name_rows = c->n_prow + c->n_trow > c->n_rrow ? c->n_prow + c->n_trow : c->n_rrow;
-        const size_t smem = sim_smem_bytes_players(a.name_rows);
-        if (test) sim_kernel<true, true><<<grid, kSimThreads, smem, st>>>(a);
-        else sim_kernel<false, true><<<grid, kSimThreads, smem, st>>>(a);
+        smem = sim_smem_bytes_players(a.name_rows);
     } else if (c->memo_mode != 0 && c->n_specs <= 1024) {     // the memo key has 10 bits for the specialisation
         // exact memo in front of the walk (fmc_sim_memo.cuh)
-        MemoArgs mm;
+        memo = true;
         std::memset(&mm, 0, sizeof(mm));
         const bool was_valid = c->memo_valid;
         size_t bytes = memo_layout(c, games, c->memo_region);
@@ -919,17 +957,20 @@ extern "C" int fmc_simulate(fmc_ctx *c, const fmc_sim_args *g) {
         mm.break_parked = c->memo_break_parked;
         mm.break_waiting = c->memo_break_waiting;
         c->memo_valid = bytes != 0;
-        const int mgrid = c->prop.multiProcessorCount * kMemoCtasPerSm;
-        if (test) sim_memo_kernel<true><<<mgrid, kMemoThreads, sim_memo_smem_bytes(), st>>>(a, mm);
-        else sim_memo_kernel<false><<<mgrid, kMemoThreads, sim_memo_smem_bytes(), st>>>(a, mm);
-    } else {
-        if (test) sim_kernel<true, false><<<grid, kSimThreads, sim_smem_bytes(false), st>>>(a);
-        else sim_kernel<false, false><<<grid, kSimThreads, sim_smem_bytes(false), st>>>(a);
     }
+    const int mgrid = c->prop.multiProcessorCount * kMemoCtasPerSm;
+    if (segs) launch_sim<true>(a, memo ? &mm : nullptr, players, test, grid, mgrid, smem, st);
+    else launch_sim<false>(a, memo ? &mm : nullptr, players, test, grid, mgrid, smem, st);
     CK(cudaGetLastError());
     CK(cudaEventRecord(c->ev_done, st));
     c->launched = true;
     return FMC_OK;
+}
+
+extern "C" int fmc_simulate(fmc_ctx *c, const fmc_sim_args *g) { return simulate_impl(c, g, nullptr); }
+
+extern "C" int fmc_simulate_segments(fmc_ctx *c, const fmc_sim_args *g, const fmc_segment_args *seg) {
+    return simulate_impl(c, g, seg);
 }
 
 // Device scratch of fmc_simulate_host, kept in the context between calls (grow-only): no cudaMalloc / cudaFree per call.
@@ -978,7 +1019,8 @@ static cudaError_t d2h_staged(fmc_ctx *c, void *dst, const void *src, size_t byt
 
 static int simulate_host_impl(fmc_ctx *c, uint64_t seed, uint32_t *scores_host, uint32_t *hist_host,
                               uint64_t *counters_host, const double *stream_host, double *trace_host,
-                              uint16_t *iters_host, fmc_player_rec *players_host, uint32_t *player_hist_host) {
+                              uint16_t *iters_host, fmc_player_rec *players_host, uint32_t *player_hist_host,
+                              uint32_t *period_host, uint32_t *seg_hist_host) {
     if (!c) return fail(FMC_ERR_INVALID, "ctx is NULL");
     if (c->matchups.empty()) return fail(FMC_ERR_INVALID, "fmc_set_matchups has not been called");
     CK(cudaSetDevice(c->device));
@@ -997,7 +1039,8 @@ static int simulate_host_impl(fmc_ctx *c, uint64_t seed, uint32_t *scores_host, 
     fmc_player_rec *d_players = nullptr;
     const size_t players_n = games * 2 * (size_t)c->n_slots;
     if ((players_host || player_hist_host) && c->usage.empty()) return fail(FMC_ERR_INVALID, "players output needs fmc_set_usage");
-    uint32_t *d_phist = nullptr;
+    uint32_t *d_phist = nullptr, *d_period = nullptr, *d_seg = nullptr;
+    const size_t seg_n = nm * 2 * FMC_N_SEGMENTS * FMC_HIST_BINS * FMC_HIST_BINS;
     const size_t phist_n = c->matchups.size() * 2 * (size_t)c->n_slots * FMC_PH_BINS;
     int rc = FMC_OK;
     cudaError_t e = cudaSuccess;
@@ -1030,13 +1073,22 @@ static int simulate_host_impl(fmc_ctx *c, uint64_t seed, uint32_t *scores_host, 
             if ((e = scratch(c, 7, phist_n * 4, (void **)&d_phist)) != cudaSuccess) { bail(e, "cudaMalloc player hist"); break; }
             if ((e = cudaMemsetAsync(d_phist, 0, phist_n * 4)) != cudaSuccess) { bail(e, "memset player hist"); break; }
         }
+        if (period_host && games) {
+            if ((e = scratch(c, 9, games * 3 * 4, (void **)&d_period)) != cudaSuccess) { bail(e, "cudaMalloc period scores"); break; }
+        }
+        if (seg_hist_host) {
+            if ((e = scratch(c, 10, seg_n * 4, (void **)&d_seg)) != cudaSuccess) { bail(e, "cudaMalloc segment hist"); break; }
+            if ((e = cudaMemsetAsync(d_seg, 0, seg_n * 4)) != cudaSuccess) { bail(e, "memset segment hist"); break; }
+        }
         fmc_sim_args g;
         std::memset(&g, 0, sizeof(g));
         g.player_hist_dev = d_phist;
         g.seed = seed; g.n_matchups = (int)nm; g.scores_dev = d_scores; g.hist_dev = d_hist; g.counters_dev = d_cnt;
         g.stream_dev = d_stream; g.trace_dev = d_trace; g.iters_dev = d_iters; g.stream = nullptr;
         g.players_dev = d_players;
-        rc = fmc_simulate(c, &g);
+        fmc_segment_args sg;
+        sg.period_scores_dev = d_period; sg.segment_hist_dev = d_seg;
+        rc = simulate_impl(c, &g, &sg);
         if (rc) break;
         if ((e = cudaDeviceSynchronize()) != cudaSuccess) { bail(e, "sim_kernel"); break; }
         if (scores_host && games && (e = d2h_staged(c, scores_host, d_scores, games * 4)) != cudaSuccess) { bail(e, "D2H scores"); break; }
@@ -1046,6 +1098,8 @@ static int simulate_host_impl(fmc_ctx *c, uint64_t seed, uint32_t *scores_host, 
         if (iters_host && games && (e = cudaMemcpy(iters_host, d_iters, games * 2, cudaMemcpyDeviceToHost)) != cudaSuccess) { bail(e, "D2H iters"); break; }
         if (d_players && (e = d2h_staged(c, players_host, d_players, players_n * sizeof(fmc_player_rec))) != cudaSuccess) { bail(e, "D2H players"); break; }
         if (d_phist && (e = cudaMemcpy(player_hist_host, d_phist, phist_n * 4, cudaMemcpyDeviceToHost)) != cudaSuccess) { bail(e, "D2H player hist"); break; }
+        if (d_period && (e = d2h_staged(c, period_host, d_period, games * 3 * 4)) != cudaSuccess) { bail(e, "D2H period scores"); break; }
+        if (d_seg && (e = cudaMemcpy(seg_hist_host, d_seg, seg_n * 4, cudaMemcpyDeviceToHost)) != cudaSuccess) { bail(e, "D2H segment hist"); break; }
     } while (0);
     // big test-mode buffers (injected draws, traces: 46 KB per game) are not worth keeping
     for (int slot : {3, 4})
@@ -1056,14 +1110,23 @@ static int simulate_host_impl(fmc_ctx *c, uint64_t seed, uint32_t *scores_host, 
 extern "C" int fmc_simulate_host(fmc_ctx *c, uint64_t seed, uint32_t *scores_host, uint32_t *hist_host,
                                  uint64_t *counters_host, const double *stream_host, double *trace_host,
                                  uint16_t *iters_host) {
-    return simulate_host_impl(c, seed, scores_host, hist_host, counters_host, stream_host, trace_host, iters_host, nullptr, nullptr);
+    return simulate_host_impl(c, seed, scores_host, hist_host, counters_host, stream_host, trace_host, iters_host, nullptr, nullptr,
+                              nullptr, nullptr);
 }
 
 extern "C" int fmc_simulate_players_host(fmc_ctx *c, uint64_t seed, uint32_t *scores_host, uint32_t *hist_host,
                                          uint64_t *counters_host, const double *stream_host, double *trace_host,
                                          uint16_t *iters_host, fmc_player_rec *players_host, uint32_t *player_hist_host) {
     return simulate_host_impl(c, seed, scores_host, hist_host, counters_host, stream_host, trace_host, iters_host, players_host,
-                              player_hist_host);
+                              player_hist_host, nullptr, nullptr);
+}
+
+extern "C" int fmc_simulate_segments_host(fmc_ctx *c, uint64_t seed, uint32_t *scores_host, uint32_t *hist_host,
+                                          uint64_t *counters_host, const double *stream_host, double *trace_host,
+                                          uint16_t *iters_host, fmc_player_rec *players_host, uint32_t *player_hist_host,
+                                          uint32_t *period_scores_host, uint32_t *segment_hist_host) {
+    return simulate_host_impl(c, seed, scores_host, hist_host, counters_host, stream_host, trace_host, iters_host, players_host,
+                              player_hist_host, period_scores_host, segment_hist_host);
 }
 
 extern "C" int fmc_tree_predict(fmc_ctx *c, int32_t id, const double *rows_dev, int64_t n, double *out_dev,

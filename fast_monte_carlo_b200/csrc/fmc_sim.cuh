@@ -115,6 +115,11 @@ struct SimKernelArgs {
     // player mode: name rows actually needed by the matchups of this launch (a chunk has kSimRows + name_rows rows):
     // passer rows [kDynRow0, +n_prow), target rows behind them, rusher rows [kDynRow0, +n_rrow)
     int n_prow, n_trow, n_rrow, name_rows;
+    // period outputs (fmc_simulate_segments; read only by the SEG instantiations): the Q1..Q3 end scores of every game
+    // (never NULL there: the library supplies device scratch when the caller did not ask for them) and the optional
+    // per-segment histograms
+    uint32_t *period_scores;           // [games][3]
+    uint32_t *segment_hist;            // [n_matchups][2][FMC_N_SEGMENTS][BINS][BINS]
 };
 
 enum Stage : int {
@@ -235,11 +240,73 @@ __device__ __forceinline__ void advance_down(Lane &L, double gained) {          
         if (L.down > 4) change_possession(L, false, 0.0);
     }
 }
-__device__ __forceinline__ void tick_clock(Lane &L, int base) {                             // FMC:956-968
+// ---- period outputs (fmc_simulate_segments, include/fmc.h FMC_N_SEGMENTS) --------------------------------------------
+// The hooks of the clock and of the end of a game.  Periods<false> is empty: the instantiations without period outputs
+// compile to the code they had before the hooks existed.  Periods<true> keeps no lane state: the game's own
+// period_scores row is its state.  The score at the end of quarter q goes to row[q - 1] when the clock crosses the
+// boundary; later boundaries read the earlier words as their segment bases.  The writes and the later reads of one
+// game's row are made by threads of ONE CTA in different rounds, with a __syncthreads() between them (sim_kernel moves
+// games between the threads of its CTA only, at the regrouping barriers; sim_memo_kernel never moves a game, so there
+// it is the same thread).
+__device__ __forceinline__ uint32_t score_word(const Lane &L) { return (uint32_t)L.score[0] | ((uint32_t)L.score[1] << 16); }
+
+template <bool SEG> struct Periods;
+template <> struct Periods<false> {
+    static constexpr bool kOn = false;
+    __device__ __forceinline__ Periods(const SimKernelArgs &, const MatchupDev &, int) {}
+    __device__ __forceinline__ void quarter_end(const Lane &, int) const {}
+    __device__ __forceinline__ void game_end(const Lane &) const {}
+};
+template <> struct Periods<true> {
+    static constexpr bool kOn = true;
+    const SimKernelArgs &a;
+    const MatchupDev &M;
+    int matchup;
+    __device__ __forceinline__ Periods(const SimKernelArgs &a_, const MatchupDev &M_, int m) : a(a_), M(M_), matchup(m) {}
+    __device__ __forceinline__ uint32_t *row(const Lane &L) const {
+        return a.period_scores + (size_t)(M.out_offset + (L.game - M.game_begin)) * 3;
+    }
+    __device__ __forceinline__ uint32_t start_word() const { return (uint32_t)M.start.score[0] | ((uint32_t)M.start.score[1] << 16); }
+    // base of a segment that starts at boundary b: the score there if the game was simulated across it, else the start
+    __device__ __forceinline__ uint32_t base(const uint32_t *r, int q_before) const {
+        return M.start.sec > 3600 - 900 * q_before ? r[q_before - 1] : start_word();
+    }
+    __device__ __forceinline__ void add(const Lane &L, int seg, uint32_t end, uint32_t base) const {
+        const int pa = (int)(end & 0xFFFFu) - (int)(base & 0xFFFFu), pb = (int)(end >> 16) - (int)(base >> 16);
+        const int ha = pa < FMC_HIST_BINS ? pa : FMC_HIST_BINS - 1, hb = pb < FMC_HIST_BINS ? pb : FMC_HIST_BINS - 1;
+        atomicAdd(a.segment_hist + ((((size_t)matchup * 2 + (L.game & 1ULL)) * FMC_N_SEGMENTS + seg) * FMC_HIST_BINS + ha) * FMC_HIST_BINS + hb, 1u);
+    }
+    // quarter q (1..3) ended with the play just ticked
+    __device__ __forceinline__ void quarter_end(const Lane &L, int q) const {
+        uint32_t *r = row(L);
+        const uint32_t w = score_word(L);
+        r[q - 1] = w;
+        if (a.segment_hist) {
+            add(L, FMC_SEG_Q1 + q - 1, w, q > 1 ? base(r, q - 1) : start_word());
+            if (q == 2) add(L, FMC_SEG_H1, w, start_word());
+        }
+    }
+    // the game is over: sentinels for the quarter ends at or before the start state; Q4 and H2 end here
+    __device__ __forceinline__ void game_end(const Lane &L) const {
+        uint32_t *r = row(L);
+#pragma unroll
+        for (int q = 1; q <= 3; ++q)
+            if (M.start.sec <= 3600 - 900 * q) r[q - 1] = FMC_PERIOD_NONE;
+        if (a.segment_hist) {
+            const uint32_t w = score_word(L);
+            add(L, FMC_SEG_Q4, w, base(r, 3));
+            add(L, FMC_SEG_H2, w, base(r, 2));
+        }
+    }
+};
+
+template <class Pk>
+__device__ __forceinline__ void tick_clock(Lane &L, int base, const Pk &pk) {                // FMC:956-968
     const int v = L.sec - base;
     L.sec = v > 0 ? v : 0;
     const int old = L.period;
     L.period = L.sec > 0 ? 4 - ((L.sec - 1) / 900) : 4;
+    if (L.period != old) pk.quarter_end(L, old);
     if (L.period != old && L.period == 3) change_possession(L, true, 75.0);
 }
 __device__ __forceinline__ double pass_prob_v1(int down, double distance, double ytg, int sec, int sd) {  // FMC:719-735
@@ -498,9 +565,9 @@ __device__ __forceinline__ void new_game(Lane &L, const MatchupDev &M, unsigned 
 // Game over (FMC:1456-1464, 1501-1503): score word, iteration count and player box to the outputs.  Returns the game's
 // bin in the score histogram of its matchup ([orientation][score 0][score 1]; a score past the last bin is clamped into
 // it and counted as an overflow); the kernel adds it.
-template <bool PLAYERS, class Ev>
+template <bool PLAYERS, class Ev, class Pk>
 __device__ __forceinline__ unsigned int end_game_record(const Lane &L, const SimKernelArgs &a, const MatchupDev &M, int matchup,
-                                                        unsigned long long *stat, Ev &ev) {
+                                                        unsigned long long *stat, Ev &ev, const Pk &pk) {
     const size_t oi = (size_t)(M.out_offset + (L.game - M.game_begin));
     if (a.scores) a.scores[oi] = (uint32_t)L.score[0] | ((uint32_t)L.score[1] << 16);
     if (a.iters) a.iters[oi] = (uint16_t)L.iter;
@@ -513,6 +580,7 @@ __device__ __forceinline__ unsigned int end_game_record(const Lane &L, const Sim
                   a.player_hist ? a.player_hist + (size_t)matchup * (size_t)lines * FMC_PH_BINS : nullptr, lines,
                   &stat[FMC_C_PH_OVERFLOW]);
     }
+    pk.game_end(L);
     ev.hit(EV_GAMES);
     return (unsigned int)(((L.game & 1ULL) * FMC_HIST_BINS + ha) * FMC_HIST_BINS + hb);
 }
@@ -531,8 +599,8 @@ __device__ __forceinline__ void write_trace(const Lane &L, const SimKernelArgs &
 
 // Fourth down (handle_fourth FMC:1382-1421): go for it, kick a field goal or punt (attempt_punt FMC:876-896).  Returns
 // whether a play follows; sd = score difference for the team on offense.
-template <bool TEST, class Ev>
-__device__ __forceinline__ bool fourth_down(Lane &L, Draws<TEST> &D, int sd, Ev &ev) {
+template <bool TEST, class Ev, class Pk>
+__device__ __forceinline__ bool fourth_down(Lane &L, Draws<TEST> &D, int sd, Ev &ev, const Pk &pk) {
     if (L.down != 4) return true;
     const int team = L.offense;
     const double ytg = L.ytg, dist = L.dist;
@@ -545,8 +613,12 @@ __device__ __forceinline__ bool fourth_down(Lane &L, Draws<TEST> &D, int sd, Ev 
     if (ytg <= 38.0) {
         ev.hit(EV_FGA);
         const bool good = D.u(S_U_FG) < field_goal_prob(ytg + 17.0);
-        tick_clock(L, 12);
-        if (good) { ev.hit(EV_FG); L.score[team] += 3; change_possession(L, true, 75.0); }
+        // With period hooks the kick's points go on before its tick, as a touchdown's do, so that a quarter that ends on
+        // the kick holds them.  tick_clock and change_possession read no score, so the order changes nothing else; the
+        // instantiations without hooks keep the original order, which compiles to fewer spills there.
+        if (Pk::kOn && good) L.score[team] += 3;
+        tick_clock(L, 12, pk);
+        if (good) { ev.hit(EV_FG); if (!Pk::kOn) L.score[team] += 3; change_possession(L, true, 75.0); }
         else change_possession(L, true, 100.0 - ytg);
         return false;
     }
@@ -560,7 +632,7 @@ __device__ __forceinline__ bool fourth_down(Lane &L, Draws<TEST> &D, int sd, Ev 
     }
     net = softclip(net, 15.0, ytg - 1.0);
     const int inet = (int)net;
-    tick_clock(L, 16);
+    tick_clock(L, 16, pk);
     change_possession(L, true, softclip(100.0 - (ytg - (double)inet), 1.0, 99.0));
     return false;
 }
@@ -640,15 +712,15 @@ __device__ __forceinline__ void stage2_raw(bool model, const float *m, const Sim
 }
 
 // The not-complete outcome (FMC:1157-1199): incomplete, interception, or a sack that waits for its yards
-template <bool TEST, bool PLAYERS, class Ev>
+template <bool TEST, bool PLAYERS, class Ev, class Pk>
 __device__ __forceinline__ void after_stage2(Lane &L, const SimKernelArgs &a, const MatchupDev &M, Draws<TEST> &D, int team,
-                                             const double raw[3], Ev &ev) {
+                                             const double raw[3], Ev &ev, const Pk &pk) {
     const int outcome = stage2_outcome(raw, D.u(S_U_S2));
     if (outcome == 0) {                                   // incomplete FMC:1160-1168
         ev.hit(EV_INC);
         if (PLAYERS) credit(a, M, L, team, 0, L.p1, PC_ATT, false, 0.0);
         L.down += 1; L.going = 0;
-        tick_clock(L, 10);
+        tick_clock(L, 10, pk);
         L.stage = ST_ITER;
     } else if (outcome == 2) {                            // sack FMC:1170-1174
         ev.hit(EV_SACK);
@@ -661,22 +733,22 @@ __device__ __forceinline__ void after_stage2(Lane &L, const SimKernelArgs &a, co
         const double spot = 100.0 - (L.ytg - ret);
         L.going = 0;
         change_possession(L, true, spot);
-        tick_clock(L, 12);
+        tick_clock(L, 12, pk);
         L.stage = ST_ITER;
     }
 }
 
 // The yards of a play from the quantiles q of its yardage model: sack FMC:1170-1184, completed pass FMC:1089-1152 and
 // run FMC:1201-1257 (the same steps with different constants).  The play ends.
-template <bool TEST, bool PLAYERS, class Ev>
+template <bool TEST, bool PLAYERS, class Ev, class Pk>
 __device__ __forceinline__ void after_yards(Lane &L, const SimKernelArgs &a, const MatchupDev &M, Draws<TEST> &D, int team,
-                                            const double q[3], Ev &ev) {
+                                            const double q[3], Ev &ev, const Pk &pk) {
     if (L.stage == ST_WAIT_SQ) {
         double loss = -sample_yards(a, D, q, 0.25, -20.0, 0.0);
         loss = pymax(0.0, loss);
         loss = pymin(loss, 100.0 - (100.0 - L.ytg));
         L.ytg += loss; L.dist += loss; L.down += 1; L.going = 0;
-        tick_clock(L, 24);
+        tick_clock(L, 24, pk);
     } else {
         const bool pass = L.stage == ST_WAIT_PQ;
         const double ytg0 = L.ytg, mz = M.mz[team];
@@ -703,12 +775,12 @@ __device__ __forceinline__ void after_yards(Lane &L, const SimKernelArgs &a, con
         if (td) {
             ev.hit(EV_TD);
             L.score[team] += 7; L.going = 0;
-            tick_clock(L, pass ? 20 : 28);
+            tick_clock(L, pass ? 20 : 28, pk);
             change_possession(L, true, 75.0);
         } else {
             L.going = 0;
             advance_down(L, yards);
-            tick_clock(L, pass ? 26 : 28);
+            tick_clock(L, pass ? 26 : 28, pk);
         }
     }
     L.stage = ST_ITER;
@@ -716,11 +788,12 @@ __device__ __forceinline__ void after_yards(Lane &L, const SimKernelArgs &a, con
 
 // Advance one lane until it posts a request (returns its key, family * 2 + offense) or has nothing
 // left to do (returns -1).  `res` points at this lane's result record of the previous round.
-template <bool TEST, bool PLAYERS>
+template <bool TEST, bool PLAYERS, bool SEG>
 __device__ __forceinline__ int advance_lane(Lane &L, const SimKernelArgs &a, SimShared &sh, const double *res) {
     const MatchupDev &M = sh.M;
     const int matchup = sh.cur_matchup;
     StatEvents ev{sh.stat};
+    const Periods<SEG> pk(a, M, matchup);
     for (;;) {
         if (L.stage == ST_IDLE) return -1;
         if (L.stage == ST_NEED_GAME) {
@@ -730,7 +803,7 @@ __device__ __forceinline__ int advance_lane(Lane &L, const SimKernelArgs &a, Sim
         }
         if (L.stage == ST_ITER) {
             if (L.sec <= 0) {
-                const unsigned int bin = end_game_record<PLAYERS>(L, a, M, matchup, sh.stat, ev);
+                const unsigned int bin = end_game_record<PLAYERS>(L, a, M, matchup, sh.stat, ev, pk);
                 if (a.hist) atomicAdd(&a.hist[(size_t)matchup * 2 * FMC_HIST_BINS * FMC_HIST_BINS + bin], 1u);
                 atomicAdd(&sh.stat[FMC_C_PLAYS], (unsigned long long)L.plays);
                 atomicAdd(&sh.stat[FMC_C_ITERS], (unsigned long long)L.iter);
@@ -741,7 +814,7 @@ __device__ __forceinline__ int advance_lane(Lane &L, const SimKernelArgs &a, Sim
             Draws<TEST> D(a, M, matchup, L);
             L.iter += 1;
             const int sd = L.score[L.offense] - L.score[L.offense ^ 1];
-            if (!fourth_down(L, D, sd, ev)) continue;
+            if (!fourth_down(L, D, sd, ev, pk)) continue;
             L.stage = start_play<TEST, PLAYERS>(L, a, M, D, sd, ev);
             return request_key(L);
         }
@@ -759,12 +832,12 @@ __device__ __forceinline__ int advance_lane(Lane &L, const SimKernelArgs &a, Sim
         if (L.stage == ST_WAIT_S1 || L.stage == ST_WAIT_S2) {
             double raw[3];
             stage2_raw(L.stage == ST_WAIT_S2, mg, a, raw);
-            after_stage2<TEST, PLAYERS>(L, a, M, D, team, raw, ev);
+            after_stage2<TEST, PLAYERS>(L, a, M, D, team, raw, ev, pk);
             if (L.stage == ST_WAIT_SQ) return request_key(L);
             continue;
         }
         const double q[3] = {res[0], res[1], res[2]};
-        after_yards<TEST, PLAYERS>(L, a, M, D, team, q, ev);
+        after_yards<TEST, PLAYERS>(L, a, M, D, team, q, ev, pk);
     }
 }
 
@@ -963,8 +1036,9 @@ __device__ __forceinline__ void walk_requests(RoundShared &sh, const SimKernelAr
 
 // PLAYERS = true: usage tables are set (fmc_set_usage): names are sampled per play, requests carry kDynRows
 // more feature rows, tracked names get per-game box lines.  The shipped configuration (every name "Unknown")
-// runs the PLAYERS = false instantiation, which carries none of it.
-template <bool TEST, bool PLAYERS>
+// runs the PLAYERS = false instantiation, which carries none of it.  SEG = true: the launch has period outputs
+// (fmc_simulate_segments, Periods<true>); the SEG = false instantiations are the code without the hooks.
+template <bool TEST, bool PLAYERS, bool SEG>
 __global__ void __launch_bounds__(kSimThreads, kSimCtasPerSm) sim_kernel(const SimKernelArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     // player mode sizes a chunk by the name rows the launch needs (runtime); the shipped configuration is compile-time
@@ -1000,7 +1074,7 @@ __global__ void __launch_bounds__(kSimThreads, kSimCtasPerSm) sim_kernel(const S
             // ---- A: advance to the next request (a held-back lane re-posts the one it has)
             Lane L = unpack_lane(P);
             L.home = home;
-            const int key = held >= 0 ? held : advance_lane<TEST, PLAYERS>(L, a, sh, results + (size_t)pos * 3);
+            const int key = held >= 0 ? held : advance_lane<TEST, PLAYERS, SEG>(L, a, sh, results + (size_t)pos * 3);
             __syncwarp();
             // ---- B: compaction
             const unsigned int rank = request_rank(sh.cnt[parity], key, lane);

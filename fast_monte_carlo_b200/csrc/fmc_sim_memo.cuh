@@ -110,7 +110,8 @@ inline size_t sim_memo_smem_bytes() { return kMemoSharedBytes + kMemoFeatBytes +
 // (bounds of a full CTA whatever kMemoThreads: builds of this kernel with __launch_bounds__(512 | 768, ...) die on the B200
 // with "an illegal instruction was encountered" at the first launch; the same source with bounds 1024 and a 512-thread
 // launch is fine -- ptxas 12.9)
-template <bool TEST>
+// SEG: the launch has period outputs (sim_kernel's SEG)
+template <bool TEST, bool SEG>
 __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a, const MemoArgs mm) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     constexpr int kChunkFloats = chunk_floats(false);
@@ -138,6 +139,7 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
         if (tid == 0) { sh.alive[0] = 0; sh.alive[1] = 0; sh.waiting[0] = 0; sh.waiting[1] = 0; }
         __syncthreads();
         const MatchupDev &M = sh.M;
+        const Periods<SEG> pk(a, M, m);
         const RankSpec *specs = mm.specs + (size_t)M.memo_id * kMemoFams * 2;
         set_stage(P, ST_NEED_GAME);
         bool parked = false;           // the lane's request missed the memo and waits for the walk
@@ -167,7 +169,7 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                 const bool over = !parked && L.stage == ST_ITER && L.sec <= 0;
                 const unsigned int over_mask = __ballot_sync(FULL, over);
                 if (over) {
-                    const unsigned int bin = end_game_record<false>(L, a, M, m, sh.stat, ev);
+                    const unsigned int bin = end_game_record<false>(L, a, M, m, sh.stat, ev, pk);
                     if (a.hist) {
                         // warp-level reduce: lanes finishing in the same bin add once
                         const unsigned int peers = __match_any_sync(over_mask, bin);
@@ -205,7 +207,7 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                 if (!parked && L.stage == ST_ITER && L.sec > 0) {
                     write_trace<TEST>(L, a, M);
                     L.iter += 1;
-                    if (fourth_down(L, D, sd, ev)) L.stage = start_play<TEST, false>(L, a, M, D, sd, ev);
+                    if (fourth_down(L, D, sd, ev, pk)) L.stage = start_play<TEST, false>(L, a, M, D, sd, ev);
                 }
                 __syncwarp();      // every stage of the trip is entered by the whole warp together
                 // -- play model (policy 1): probe, then the play call
@@ -269,7 +271,7 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                     double raw[3];
                     stage2_raw(!s2_standin, mg, a, raw);
                     have = false;
-                    after_stage2<TEST, false>(L, a, M, D, team, raw, ev);
+                    after_stage2<TEST, false>(L, a, M, D, team, raw, ev, pk);
                 }
                 __syncwarp();      // every stage of the trip is entered by the whole warp together
                 // -- yardage families: probe, then the outcome
@@ -290,7 +292,7 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                     const double q[3] = {__longlong_as_double((long long)r[0]), __longlong_as_double((long long)r[1]),
                                          __longlong_as_double((long long)r[2])};
                     have = false;
-                    after_yards<TEST, false>(L, a, M, D, team, q, ev);
+                    after_yards<TEST, false>(L, a, M, D, team, q, ev, pk);
                 }
                 __syncwarp();      // every stage of the trip is entered by the whole warp together
                 // -- warp tallies of this trip

@@ -30,6 +30,8 @@ COUNTER_NAMES = ("games", "plays", "iters", "pass", "comp", "inc", "int", "sack"
                  "memo_hits_sq", "memo_hits_pm")
 PH_YDS_BINS, PH_YDS_OFFSET, PH_CNT_BINS = 8192, 1000, 128
 PH_BINS = PH_YDS_BINS + 5 * PH_CNT_BINS
+N_SEGMENTS = 6                     # FMC_N_SEGMENTS: Q1, Q2, Q3, Q4, H1, H2
+PERIOD_NONE = 0xFFFFFFFF           # FMC_PERIOD_NONE: a quarter end at or before the start state
 
 
 class FmcError(RuntimeError):
@@ -77,6 +79,11 @@ class SimArgs(C.Structure):
         ("stream_dev", C.c_void_p), ("trace_dev", C.c_void_p), ("iters_dev", C.c_void_p),
         ("stream", C.c_void_p), ("players_dev", C.c_void_p), ("player_hist_dev", C.c_void_p),
     ]
+
+
+class SegmentArgs(C.Structure):
+    """fmc_segment_args"""
+    _fields_ = [("period_scores_dev", C.c_void_p), ("segment_hist_dev", C.c_void_p)]
 
 
 MAX_USAGE = 32
@@ -158,6 +165,8 @@ def load_library():
                                     C.c_void_p, C.c_void_p]
     L.fmc_simulate_players_host.argtypes = [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                             C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
+    L.fmc_simulate_segments.argtypes = [C.c_void_p, C.POINTER(SimArgs), C.POINTER(SegmentArgs)]
+    L.fmc_simulate_segments_host.argtypes = [C.c_void_p, C.c_uint64] + [C.c_void_p] * 10
     L.fmc_set_usage.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32]
     L.fmc_set_start_states.argtypes = [C.c_void_p, C.c_int32, C.c_void_p]
     L.fmc_pack_forest_host_dyn.restype = C.c_int64
@@ -196,7 +205,7 @@ EXPORTED_SYMBOLS = (
     "fmc_gather_probe", "fmc_debug_errors",
     "fmc_pack_forest_host", "fmc_pack_forest_host_dyn", "fmc_set_usage", "fmc_simulate_players_host",
     "fmc_set_memo", "fmc_memo_keys_host", "fmc_gather_probe_coherent", "fmc_predict_stats", "fmc_invalidate_tables", "fmc_tree_predict_cols_host",
-    "fmc_set_start_states",
+    "fmc_set_start_states", "fmc_simulate_segments", "fmc_simulate_segments_host",
 )
 
 
@@ -437,8 +446,10 @@ class Context:
 
     # -- simulation ------------------------------------------------------------------------------
     def simulate_device(self, *, seed: int, scores=0, hist=0, counters=0, stream_in=0, trace=0, iters=0,
-                        cuda_stream=0, players=0, player_hist=0) -> None:
-        """Asynchronous launch on raw device pointers (ints; 0 = not requested)."""
+                        cuda_stream=0, players=0, player_hist=0, period_scores=0, segment_hist=0) -> None:
+        """Asynchronous launch on raw device pointers (ints; 0 = not requested).  `period_scores` (uint32[games][3]) and
+        `segment_hist` (uint32[n_matchups][2][N_SEGMENTS][BINS][BINS], zeroed by the caller) are the per-period outputs
+        of fmc_simulate_segments; without them the call is fmc_simulate."""
         a = SimArgs()
         a.seed = int(seed) & 0xFFFFFFFFFFFFFFFF
         a.n_matchups = self.n_matchups
@@ -447,11 +458,20 @@ class Context:
         a.stream = cuda_stream or None
         a.players_dev = players or None      # fmc_player_rec[games][2][n_slots]
         a.player_hist_dev = player_hist or None   # uint32[n_matchups][2][n_slots][PH_BINS], zeroed by the caller
-        _check(self._L.fmc_simulate(self._h, C.byref(a)))
+        if period_scores or segment_hist:
+            sg = SegmentArgs()
+            sg.period_scores_dev = period_scores or None; sg.segment_hist_dev = segment_hist or None
+            _check(self._L.fmc_simulate_segments(self._h, C.byref(a), C.byref(sg)))
+        else:
+            _check(self._L.fmc_simulate(self._h, C.byref(a)))
 
     def simulate_host(self, *, seed: int, want_scores=True, want_hist=True, stream: Optional[np.ndarray] = None,
-                      want_trace=False, want_iters=False, want_players=False, want_player_hist=False) -> dict:
-        """End-to-end call with host buffers (fmc_simulate_host / fmc_simulate_players_host)."""
+                      want_trace=False, want_iters=False, want_players=False, want_player_hist=False,
+                      want_period_scores=False, want_segments=False) -> dict:
+        """End-to-end call with host buffers (fmc_simulate_host / fmc_simulate_players_host, and
+        fmc_simulate_segments_host when `want_period_scores` / `want_segments` ask for the per-period outputs: "period_scores"
+        uint32[games][3] score words at the end of Q1..Q3 (PERIOD_NONE before the start state), "segment_hist"
+        uint32[n_matchups][2][N_SEGMENTS][BINS][BINS])."""
         n = self.total_games
         scores = np.zeros(n, dtype=np.uint32) if want_scores else None
         hist = np.zeros((self.n_matchups, 2, HIST_BINS, HIST_BINS), dtype=np.uint32) if want_hist else None
@@ -464,6 +484,8 @@ class Context:
                 raise ValueError(f"stream must be [{n},{MAX_ITERS},{N_SLOTS}]")
         vp = lambda a: None if a is None else a.ctypes.data
         players = phist = None
+        period = np.zeros((n, 3), dtype=np.uint32) if want_period_scores else None
+        seg = (np.zeros((self.n_matchups, 2, N_SEGMENTS, HIST_BINS, HIST_BINS), dtype=np.uint32) if want_segments else None)
         if want_players or want_player_hist:
             if not self.has_usage:
                 raise FmcError("want_players / want_player_hist need set_usage")
@@ -471,6 +493,12 @@ class Context:
                 players = np.zeros((n, 2, max(self.n_slots, 1)), dtype=PLAYER_REC)
             if want_player_hist:
                 phist = np.zeros((self.n_matchups, 2, max(self.n_slots, 1), PH_BINS), dtype=np.uint32)
+        if period is not None or seg is not None:
+            _check(self._L.fmc_simulate_segments_host(
+                self._h, int(seed) & 0xFFFFFFFFFFFFFFFF, vp(scores), vp(hist), vp(counters), vp(stream), vp(trace), vp(iters),
+                players.ctypes.data if (players is not None and self.n_slots) else None,
+                phist.ctypes.data if (phist is not None and self.n_slots) else None, vp(period), vp(seg)))
+        elif players is not None or phist is not None:
             _check(self._L.fmc_simulate_players_host(self._h, int(seed) & 0xFFFFFFFFFFFFFFFF, vp(scores), vp(hist),
                                                      vp(counters), vp(stream), vp(trace), vp(iters),
                                                      players.ctypes.data if (players is not None and self.n_slots) else None,
@@ -493,6 +521,10 @@ class Context:
             out["trace"] = trace
         if iters is not None:
             out["iters"] = iters.astype(np.int32)
+        if period is not None:
+            out["period_scores"] = period
+        if seg is not None:
+            out["segment_hist"] = seg
         return out
 
     # -- tree prediction -------------------------------------------------------------------------------

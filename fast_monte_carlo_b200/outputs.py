@@ -246,6 +246,49 @@ def live_odds_from_hist(hist2: np.ndarray, team_a: str, team_b: str, *, spread: 
     return out
 
 
+# periods of a game (include/fmc.h FMC_N_SEGMENTS), in the order of the kernels' segment histograms
+SEGMENTS = ("Q1", "Q2", "Q3", "Q4", "H1", "H2")
+
+
+def segment_odds_from_hist(h2: np.ndarray, team_a: str, team_b: str, *, offset=(0, 0), spread: Optional[float] = None,
+                           total: Optional[float] = None) -> Dict[str, object]:
+    """Odds of one period (quarter or half) from a [BINS, BINS] histogram of the (A, B) points scored in it: games,
+    p_win per team, p_tie (a period can end level), mean points per team, and for `spread` (team A's line) / `total`
+    the fields of `game_market_odds_from_hist` with team A as the team.  `offset` = (A, B) points already scored in the
+    period (a live period in progress whose histogram counts from the live state) and is added to every bin, without
+    clamping.  Points past the last bin count as HIST_BINS - 1, as the histogram holds them.  With offset (0, 0) on a
+    final-score histogram this is `live_odds_from_hist`."""
+    h = np.asarray(h2).reshape(HIST_BINS, HIST_BINS).astype(np.float64)
+    n = h.sum()
+    if n <= 0:
+        raise ValueError("the histogram holds no games")
+    oa, ob = int(offset[0]), int(offset[1])
+    a = np.arange(HIST_BINS, dtype=np.float64)[:, None] + oa
+    b = np.arange(HIST_BINS, dtype=np.float64)[None, :] + ob
+    out: Dict[str, object] = {
+        "games": int(n),
+        "p_win": {team_a: float((h * (a > b)).sum() / n), team_b: float((h * (b > a)).sum() / n)},
+        "p_tie": float((h * (a == b)).sum() / n),
+        "mean_points": {team_a: float((h * a).sum() / n), team_b: float((h * b).sum() / n)},
+        "markets": None,
+    }
+    if spread is not None or total is not None:
+        # the offset moves every margin by oa - ob and every total by oa + ob: price the lines moved the other way on the
+        # histogram as it is, then put the line and the margin / total statistics back where the period has them
+        d, s = oa - ob, oa + ob
+        mk = game_market_odds_from_hist(np.stack([h, np.zeros_like(h)]), team_a, team_b,
+                                        spread=None if spread is None else float(spread) + d,
+                                        total=None if total is None else float(total) - s)
+        if "spread" in mk:
+            mk["spread"].update(spread=float(spread), mean_margin=mk["spread"]["mean_margin"] + d,
+                                median_margin=mk["spread"]["median_margin"] + d)
+        if "total" in mk:
+            mk["total"].update(total=float(total), mean_total=mk["total"]["mean_total"] + s,
+                               median_total=mk["total"]["median_total"] + s)
+        out["markets"] = mk
+    return out
+
+
 def summary_from_hist(hist2: np.ndarray, team_a: str, team_b: str) -> pd.DataFrame:
     """The `summary` frame of simulate_upcoming_matchup (FMC:1681-1687) from the histogram: each
     team's row covers the orientation in which it received the opening kickoff."""

@@ -170,6 +170,20 @@ enum {
                                  sack yards = sack, play model = plays under policy 1 */
 };
 
+/* Periods (quarter and half markets, fmc_simulate_segments).  Quarter q (1..3) ends when the clock crosses
+ * 3600 - 900 q (2700, 1800, 900): the period is 4 - (seconds - 1) / 900, as the clock derives it.  A play's points
+ * count in the quarter in which it was snapped, so the score at the end of quarter q is the score after the play whose
+ * clock tick crossed the boundary (the score at the next iteration start or, if the game is over, the final score).
+ * Segments, in this order: Q1, Q2, Q3, Q4, H1 (= Q1 + Q2), H2 (= Q3 + Q4).  A segment's value for a game is the
+ * (points A, points B) scored in it: the score at its end minus the score at its base, which is the score at its start
+ * boundary or the game's start state (fmc_set_start_states) if that is later.  A segment that ends at or before the
+ * start state is not counted (boundary B lies in the simulated future iff start seconds > B); one in progress counts
+ * from the start state.  Q4 and H2 end at the game's end: a game that starts with the clock at 0 counts (0, 0) in Q4
+ * and H2 and nothing else. */
+#define FMC_N_SEGMENTS 6
+enum { FMC_SEG_Q1 = 0, FMC_SEG_Q2, FMC_SEG_Q3, FMC_SEG_Q4, FMC_SEG_H1, FMC_SEG_H2 };
+#define FMC_PERIOD_NONE 0xFFFFFFFFu  /* period_scores word of a quarter end at or before the start state */
+
 #define FMC_N_SLOTS 16           /* injected-draw record per (game, loop iteration); see DESIGN.md */
 #define FMC_MAX_ITERS 360
 #define FMC_TRACE_COLS 8
@@ -250,6 +264,25 @@ int fmc_set_memo(fmc_ctx *ctx, int32_t mode, uint64_t max_bytes, int32_t max_tri
  * matchup range to completion on the GPU.  Asynchronous on args->stream. */
 int fmc_simulate(fmc_ctx *ctx, const fmc_sim_args *args);
 
+/* Per-period outputs of a launch (see FMC_N_SEGMENTS for the definitions); both optional.
+ *   period_scores_dev  [games][3]: score word (points A) | (points B) << 16 at the end of Q1, Q2, Q3, at
+ *                      out_offset + (g - game_begin) like scores_dev; FMC_PERIOD_NONE for a quarter end at or before
+ *                      the start state.
+ *   segment_hist_dev   [n_matchups][2][FMC_N_SEGMENTS][BINS][BINS], += 1 at [m][g & 1][segment][min(A, BINS-1)]
+ *                      [min(B, BINS-1)] with A, B the points scored in the segment (zero it first, like hist_dev).
+ *                      Without period_scores_dev the library keeps the per-game rows in device scratch (12 B a game);
+ *                      the first such call, and one that needs more rows than any before it, grows that scratch and
+ *                      synchronises the device (grow-only, like the running player boxes). */
+typedef struct {
+    uint32_t *period_scores_dev;
+    uint32_t *segment_hist_dev;
+} fmc_segment_args;
+
+/* fmc_simulate plus the per-period outputs.  seg == NULL, or both pointers NULL, is exactly fmc_simulate; otherwise the
+ * launch runs the kernel instantiation with the period hooks (the one without them is unchanged).  Every other output,
+ * draw and game is the same as without them. */
+int fmc_simulate_segments(fmc_ctx *ctx, const fmc_sim_args *args, const fmc_segment_args *seg);
+
 /* Same, with HOST result buffers (any may be NULL): allocates device scratch, runs, copies back and
  * synchronises.  This is the call the reference-facing Python API makes (end-to-end path). */
 int fmc_simulate_host(fmc_ctx *ctx, uint64_t seed, uint32_t *scores_host, uint32_t *hist_host,
@@ -261,6 +294,14 @@ int fmc_simulate_host(fmc_ctx *ctx, uint64_t seed, uint32_t *scores_host, uint32
 int fmc_simulate_players_host(fmc_ctx *ctx, uint64_t seed, uint32_t *scores_host, uint32_t *hist_host,
                               uint64_t *counters_host, const double *stream_host, double *trace_host,
                               uint16_t *iters_host, fmc_player_rec *players_host, uint32_t *player_hist_host);
+
+/* fmc_simulate_players_host plus the per-period outputs: period_scores_host [games][3] and segment_hist_host
+ * [n_matchups][2][FMC_N_SEGMENTS][BINS][BINS] (either may be NULL; see fmc_segment_args).  Player outputs need
+ * fmc_set_usage, as there. */
+int fmc_simulate_segments_host(fmc_ctx *ctx, uint64_t seed, uint32_t *scores_host, uint32_t *hist_host,
+                               uint64_t *counters_host, const double *stream_host, double *trace_host,
+                               uint16_t *iters_host, fmc_player_rec *players_host, uint32_t *player_hist_host,
+                               uint32_t *period_scores_host, uint32_t *segment_hist_host);
 
 /* Raw margins of one model on n rows of the 17 numerics (play_model: first 12), NUM order of
  * FMC:676-682, float64 row-major [n][17]; out float64 [n][n_outputs].  Trees [tree_begin, tree_end)
