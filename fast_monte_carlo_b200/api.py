@@ -242,17 +242,28 @@ def _segment_buffer(n_entries: int, dev):
                        device=dev)
 
 
-def _merge_segments(hist, seg, counters=None):
-    """int64 copies of the score histograms and (when `seg` is not None) the period histograms, merged over ranks by ONE
-    `merge_histograms` all-reduce of the two laid end to end."""
+def _merge_segments(hist, seg, counters=None, seq=None):
+    """int64 copies of the score histograms, the period histograms `seg` and the scoring-sequence histograms `seq` (each
+    may be None), merged over ranks by ONE `merge_histograms` all-reduce of them laid end to end.  Returns (hist, seg,
+    seq), None where None was given."""
     import torch
-    if seg is None:
-        h64 = hist.to(torch.int64)
-        merge_histograms(h64, counters)
-        return h64, None
-    both = torch.cat([hist.reshape(-1), seg.reshape(-1)]).to(torch.int64)
-    merge_histograms(both, counters)
-    return both[:hist.numel()].reshape(hist.shape), both[hist.numel():].reshape(seg.shape)
+    parts = [t for t in (hist, seg, seq) if t is not None]
+    flat = torch.cat([t.reshape(-1) for t in parts]).to(torch.int64)
+    merge_histograms(flat, counters)
+    out, at = [], 0
+    for t in (hist, seg, seq):
+        if t is None:
+            out.append(None)
+            continue
+        out.append(flat[at:at + t.numel()].reshape(t.shape))
+        at += t.numel()
+    return tuple(out)
+
+
+def _sequence_buffer(n_entries: int, dev):
+    """The kernels' scoring-sequence histograms [n_entries][2][SEQ_BINS] (2 KB an entry), zeroed."""
+    import torch
+    return torch.zeros((n_entries, 2, outputs.SEQ_BINS), dtype=torch.int32, device=dev)
 
 
 def _segment_lines(mk) -> None:
@@ -299,7 +310,8 @@ def gather_player_box(local_rec, total_games: int):
 def simulate_slate(pairs: Sequence[Tuple[str, str]], n: int = 1000, *, sp_path: Optional[str] = None,
                    year: int = 2025, week: int = 1, seed: Optional[int] = None,
                    engine: Optional[Engine] = None, markets: Optional[Dict[Tuple[str, str], Dict[str, float]]] = None,
-                   focus_csv: Optional[str] = None, usage_dir: str = ".", segments: bool = False):
+                   focus_csv: Optional[str] = None, usage_dir: str = ".", segments: bool = False,
+                   sequence: bool = False):
     """A whole slate in one launch (BASELINE configs 3-4): every (teamA, teamB) of `pairs` is simulated for
     `n` PAIRS of games (2n games, A receives / B receives alternately, exactly like `simulate_matchup`).
 
@@ -324,6 +336,12 @@ def simulate_slate(pairs: Sequence[Tuple[str, str]], n: int = 1000, *, sp_path: 
     uncertainty).  Period lines come through `markets` under the period's name:
     {(A, B): {"spread": s, "H1": {"spread": s1, "total": t1}, "Q1": {...}}}.  The period histograms are merged over
     ranks in the same all-reduce as the score histograms.
+
+    Scoring sequence: with `sequence=True` every pair also returns "sequence_hist" ([2][SEQ_BINS] per orientation, A
+    receives first / B receives first; include/fmc.h defines the bins), "first_score" and "race" (the next-score and
+    race-to-N parts of `outputs.sequence_odds_from_hist` over BOTH orientations) and "opening_drive" = {receiving team:
+    the drive part of `outputs.sequence_odds_from_hist` of the orientation in which that team receives the kickoff}.
+    These histograms ride in the same all-reduce too.
     """
     import torch
     import torch.distributed as dist
@@ -355,12 +373,14 @@ def simulate_slate(pairs: Sequence[Tuple[str, str]], n: int = 1000, *, sp_path: 
     phist = (torch.zeros((len(specs), 2, eng.n_slots, _usage.PH_BINS), dtype=torch.int32, device=dev)
              if with_players else None)
     seg = _segment_buffer(len(specs), dev) if segments else None
+    sq = _sequence_buffer(len(specs), dev) if sequence else None
     eng.ctx.simulate_device(seed=_fresh_seed() if seed is None else int(seed), hist=hist.data_ptr(),
                             counters=padded.data_ptr(), cuda_stream=st.cuda_stream,
                             player_hist=phist.data_ptr() if phist is not None else 0,
-                            segment_hist=seg.data_ptr() if seg is not None else 0)
+                            segment_hist=seg.data_ptr() if seg is not None else 0,
+                            sequence_hist=sq.data_ptr() if sq is not None else 0)
     counters.copy_(padded[:counters.numel()])
-    hist64, seg64 = _merge_segments(hist, seg, counters)
+    hist64, seg64, sq64 = _merge_segments(hist, seg, counters, sq)
     ph = None
     if phist is not None:
         ph64 = phist.to(torch.int64)
@@ -368,6 +388,7 @@ def simulate_slate(pairs: Sequence[Tuple[str, str]], n: int = 1000, *, sp_path: 
         ph = ph64.cpu().numpy()
     h = hist64.cpu().numpy()
     sgs = seg64.cpu().numpy() if seg64 is not None else None       # [pairs][2][N_SEGMENTS][BINS][BINS]
+    sqs = sq64.cpu().numpy() if sq64 is not None else None          # [pairs][2][SEQ_BINS]
     c = counters.cpu().numpy()
     out: Dict[object, object] = {"_counters": {k: int(c[i]) for i, k in enumerate(native_counter_names())}}
     for m, (a, b) in enumerate(pairs):
@@ -386,6 +407,15 @@ def simulate_slate(pairs: Sequence[Tuple[str, str]], n: int = 1000, *, sp_path: 
                 odds = (outputs.segment_odds_from_hist(both, a, b, spread=line.get("spread"), total=line.get("total"))
                         if both.sum() > 0 else None)
                 entry["segments"][name] = {"hist": sg[:, k], "odds": odds}
+        if sqs is not None:
+            entry["sequence_hist"] = sqs[m]
+            if entry["games"] > 0:
+                both = outputs.sequence_odds_from_hist(sqs[m], a, b)
+                entry["first_score"], entry["race"] = both["next_score"], both["race"]
+                entry["opening_drive"] = {t: outputs.sequence_odds_from_hist(sqs[m][o], a, b)["drive"]
+                                          for o, t in enumerate((a, b))}
+            else:
+                entry["first_score"] = entry["race"] = entry["opening_drive"] = None
         if ph is not None:
             entry["player_hist"] = ph[m]
             entry["usage"] = uses[m]
@@ -521,7 +551,8 @@ def live_game_state(team_a: str, team_b: str, state) -> GameState:
 
 def simulate_live(entries: Sequence[Tuple[str, str, object]], games: int = 100_000, *, sp_path: Optional[str] = None,
                   year: int = 2025, week: int = 1, seed: Optional[int] = None, engine: Optional[Engine] = None,
-                  markets: Optional[Dict[int, Dict[str, float]]] = None, segments: bool = False) -> List[Dict[str, object]]:
+                  markets: Optional[Dict[int, Dict[str, float]]] = None, segments: bool = False,
+                  sequence: bool = False) -> List[Dict[str, object]]:
     """Who wins from here?  Every entry (teamA, teamB, state) -- `state` a LiveState (or a mapping with its fields) --
     plays `games` GAMES (not pairs) from its state, all entries in one launch: a win-probability curve (one pair, a state
     per snap) and a live slate (many pairs) alike.  Entries of the same pair share one specialised table set and one memo,
@@ -542,7 +573,12 @@ def simulate_live(entries: Sequence[Tuple[str, str, object]], games: int = 100_0
     `outputs.SEGMENTS` its status (ended / in_progress / future), the histogram of the points scored in it from the
     state on (both orientations summed) and its odds, with the period lines of `markets` under the period's name
     ({i: {"spread": s, "H2": {"spread": s2, "total": t2}}}).  A period in progress is priced as a whole when its start
-    score is known (LiveState.quarter_start_score / half_start_score, or implied by the clock)."""
+    score is known (LiveState.quarter_start_score / half_start_score, or implied by the clock).
+
+    Scoring sequence: with `sequence=True` every entry also returns "sequence_hist" ([SEQ_BINS], both orientations
+    summed) and, from `outputs.sequence_odds_from_hist` with the state's score as the start score, "next_score" (which
+    team scores next and how, or no further score), "drive" (how the drive in progress ends) and "race" (first to
+    10 / 15 / 20 / 25 / 30, targets already reached reported as settled)."""
     import torch
     import torch.distributed as dist
     eng = engine if engine is not None else get_engine()
@@ -569,15 +605,18 @@ def simulate_live(entries: Sequence[Tuple[str, str, object]], games: int = 100_0
     dev = torch.device("cuda", eng.ctx.device)
     hist = torch.zeros((len(specs), 2, outputs.HIST_BINS, outputs.HIST_BINS), dtype=torch.int32, device=dev)
     seg = _segment_buffer(len(specs), dev) if segments else None
+    sq = _sequence_buffer(len(specs), dev) if sequence else None
     with _ENGINE_LOCK:
         eng.set_matchups(specs)
         if g1 > g0:
             st = torch.cuda.current_stream(dev)
             eng.ctx.simulate_device(seed=_fresh_seed() if seed is None else int(seed), hist=hist.data_ptr(),
-                                    cuda_stream=st.cuda_stream, segment_hist=seg.data_ptr() if seg is not None else 0)
-    hist64, seg64 = _merge_segments(hist, seg)
+                                    cuda_stream=st.cuda_stream, segment_hist=seg.data_ptr() if seg is not None else 0,
+                                    sequence_hist=sq.data_ptr() if sq is not None else 0)
+    hist64, seg64, sq64 = _merge_segments(hist, seg, None, sq)
     h = hist64.cpu().numpy()
     sg = seg64.sum(dim=1).cpu().numpy() if seg64 is not None else None      # [entries][N_SEGMENTS][BINS][BINS]
+    sqh = sq64.sum(dim=1).cpu().numpy() if sq64 is not None else None       # [entries][SEQ_BINS]
     out = []
     for m, (a, b, st) in enumerate(entries):
         h2 = h[m].sum(axis=0)
@@ -589,6 +628,9 @@ def simulate_live(entries: Sequence[Tuple[str, str, object]], games: int = 100_0
                     "hist_overflow": int(h2[last, :].sum() + h2[:last, last].sum()), "markets": odds["markets"]})
         if sg is not None:
             out[-1]["segments"] = live_segments(st, sg[m], a, b, mk)
+        if sqh is not None:
+            seq = outputs.sequence_odds_from_hist(sqh[m], a, b, start_score=tuple(starts[m].score))
+            out[-1].update(sequence_hist=sqh[m], next_score=seq["next_score"], drive=seq["drive"], race=seq["race"])
     return out
 
 

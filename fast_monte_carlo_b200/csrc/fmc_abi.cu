@@ -235,7 +235,9 @@ struct fmc_ctx {
     bool launched = false;
     // fmc_simulate_host: device scratch + pinned staging, kept between calls
     struct Scratch { void *dev = nullptr; size_t dev_bytes = 0; };
-    Scratch scr[11];     // 0..7 fmc_simulate_host's buffers, 8 the period rows of fmc_simulate_segments, 9..10 its host path
+    // 0..7 fmc_simulate_host's buffers, 8 the period rows of fmc_simulate_segments, 9..10 its host path, 11 the sequence
+    // rows of fmc_simulate_markets, 12..13 its host path
+    Scratch scr[14];
     // pinned staging of the large device -> host copies of fmc_simulate_host (two buffers: the DMA of one chunk overlaps
     // the host copy of the previous one into the caller's pageable buffer)
     void *pin[2] = {nullptr, nullptr};
@@ -271,6 +273,22 @@ extern "C" void fmc_destroy(fmc_ctx *c);
 extern "C" const char *fmc_last_error(void) { return g_err.c_str(); }
 extern "C" int fmc_abi_version(void) { return FMC_ABI_VERSION; }
 
+// the dynamic shared memory every instantiation of one hook mask may use
+template <int HOOKS>
+static cudaError_t set_smem_limits() {
+    cudaError_t e = cudaSuccess;
+    auto set = [&](const void *f, size_t bytes) {
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    };
+    set((const void *)sim_kernel<false, false, HOOKS>, sim_smem_bytes(false));
+    set((const void *)sim_kernel<true, false, HOOKS>, sim_smem_bytes(false));
+    set((const void *)sim_kernel<false, true, HOOKS>, sim_smem_bytes(true));
+    set((const void *)sim_kernel<true, true, HOOKS>, sim_smem_bytes(true));
+    set((const void *)sim_memo_kernel<false, HOOKS>, sim_memo_smem_bytes());
+    set((const void *)sim_memo_kernel<true, HOOKS>, sim_memo_smem_bytes());
+    return e;
+}
+
 extern "C" int fmc_create(int device, fmc_ctx **out) {
     if (!out) return fail(FMC_ERR_INVALID, "fmc_create: out is NULL");
     int n = 0;
@@ -295,19 +313,11 @@ extern "C" int fmc_create(int device, fmc_ctx **out) {
     c->params.stage2_standin[0] = (double)0.78f;
     c->params.stage2_standin[1] = (double)0.05f;
     c->params.stage2_standin[2] = (double)0.17f;
-    CKC(cudaFuncSetAttribute(sim_kernel<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_smem_bytes(false)));
-    CKC(cudaFuncSetAttribute(sim_kernel<true, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_smem_bytes(false)));
-    CKC(cudaFuncSetAttribute(sim_kernel<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_smem_bytes(true)));
-    CKC(cudaFuncSetAttribute(sim_kernel<true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_smem_bytes(true)));
-    CKC(cudaFuncSetAttribute(sim_memo_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_memo_smem_bytes()));
-    CKC(cudaFuncSetAttribute(sim_memo_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_memo_smem_bytes()));
-    // the instantiations with the period hooks (fmc_simulate_segments)
-    CKC(cudaFuncSetAttribute(sim_kernel<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_smem_bytes(false)));
-    CKC(cudaFuncSetAttribute(sim_kernel<true, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_smem_bytes(false)));
-    CKC(cudaFuncSetAttribute(sim_kernel<false, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_smem_bytes(true)));
-    CKC(cudaFuncSetAttribute(sim_kernel<true, true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_smem_bytes(true)));
-    CKC(cudaFuncSetAttribute(sim_memo_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_memo_smem_bytes()));
-    CKC(cudaFuncSetAttribute(sim_memo_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sim_memo_smem_bytes()));
+    CKC(set_smem_limits<0>());
+    // the instantiations with hooks: period outputs (fmc_simulate_segments), sequence outputs, both (fmc_simulate_markets)
+    CKC(set_smem_limits<kHookPeriods>());
+    CKC(set_smem_limits<kHookSequence>());
+    CKC(set_smem_limits<kHookPeriods | kHookSequence>());
     CKC(cudaEventCreateWithFlags(&c->ev_done, cudaEventDisableTiming));
     CKC(cudaMalloc(&c->d_pred_stats, 16));
     CKC(cudaMemset(c->d_pred_stats, 0, 16));
@@ -849,24 +859,34 @@ static size_t memo_layout(fmc_ctx *c, uint64_t games, MemoRegion (&R)[kMemoFams]
 
 static cudaError_t scratch(fmc_ctx *c, int slot, size_t bytes, void **out);
 
-// The kernel of a launch: player mode, the memo kernel or the plain one; injected draws / traces (TEST); period
-// outputs (SEG).
-template <bool SEG>
+// The kernel of a launch: player mode, the memo kernel or the plain one; injected draws / traces (TEST); the hooks of
+// the optional outputs (HOOKS).
+template <int HOOKS>
 static void launch_sim(const SimKernelArgs &a, const MemoArgs *mm, bool players, bool test, int grid, int mgrid, size_t smem,
                        cudaStream_t st) {
     if (players) {
-        if (test) sim_kernel<true, true, SEG><<<grid, kSimThreads, smem, st>>>(a);
-        else sim_kernel<false, true, SEG><<<grid, kSimThreads, smem, st>>>(a);
+        if (test) sim_kernel<true, true, HOOKS><<<grid, kSimThreads, smem, st>>>(a);
+        else sim_kernel<false, true, HOOKS><<<grid, kSimThreads, smem, st>>>(a);
     } else if (mm) {
-        if (test) sim_memo_kernel<true, SEG><<<mgrid, kMemoThreads, sim_memo_smem_bytes(), st>>>(a, *mm);
-        else sim_memo_kernel<false, SEG><<<mgrid, kMemoThreads, sim_memo_smem_bytes(), st>>>(a, *mm);
+        if (test) sim_memo_kernel<true, HOOKS><<<mgrid, kMemoThreads, sim_memo_smem_bytes(), st>>>(a, *mm);
+        else sim_memo_kernel<false, HOOKS><<<mgrid, kMemoThreads, sim_memo_smem_bytes(), st>>>(a, *mm);
     } else {
-        if (test) sim_kernel<true, false, SEG><<<grid, kSimThreads, sim_smem_bytes(false), st>>>(a);
-        else sim_kernel<false, false, SEG><<<grid, kSimThreads, sim_smem_bytes(false), st>>>(a);
+        if (test) sim_kernel<true, false, HOOKS><<<grid, kSimThreads, sim_smem_bytes(false), st>>>(a);
+        else sim_kernel<false, false, HOOKS><<<grid, kSimThreads, sim_smem_bytes(false), st>>>(a);
     }
 }
 
-static int simulate_impl(fmc_ctx *c, const fmc_sim_args *g, const fmc_segment_args *seg) {
+// grow-only device scratch for the per-game rows of a hook when the caller did not ask for them
+static int hook_rows(fmc_ctx *c, int slot, uint64_t out_games, int words, uint32_t **rows) {
+    if (*rows || !out_games) return FMC_OK;
+    void *p = nullptr;
+    CK(scratch(c, slot, (size_t)out_games * words * sizeof(uint32_t), &p));
+    *rows = (uint32_t *)p;
+    return FMC_OK;
+}
+
+// Every simulation entry point: seg / seq may be NULL or hold only NULL pointers.
+static int simulate_impl(fmc_ctx *c, const fmc_sim_args *g, const fmc_segment_args *seg, const fmc_sequence_args *seq) {
     if (!c || !g) return fail(FMC_ERR_INVALID, "fmc_simulate: bad argument");
     CK(cudaSetDevice(c->device));
     settle_usage(c);
@@ -886,14 +906,13 @@ static int simulate_impl(fmc_ctx *c, const fmc_sim_args *g, const fmc_segment_ar
         const uint64_t hi = c->matchups[i].out_offset + (c->matchups[i].game_end - c->matchups[i].game_begin);
         if (hi > out_games) out_games = hi;
     }
+    // the per-game rows are the state of the hooks: device scratch when the caller only wants the histograms
     const bool segs = seg && (seg->period_scores_dev || seg->segment_hist_dev);
     uint32_t *rows = segs ? seg->period_scores_dev : nullptr;
-    if (segs && !rows && out_games) {
-        // the per-game rows are the state of the period hooks: device scratch when the caller only wants the histograms
-        void *p = nullptr;
-        CK(scratch(c, 8, (size_t)out_games * 3 * sizeof(uint32_t), &p));
-        rows = (uint32_t *)p;
-    }
+    if (segs) { int rc = hook_rows(c, 8, out_games, 3, &rows); if (rc) return rc; }
+    const bool seqs = seq && (seq->sequence_dev || seq->sequence_hist_dev);
+    uint32_t *seq_rows = seqs ? seq->sequence_dev : nullptr;
+    if (seqs) { int rc = hook_rows(c, 11, out_games, 2, &seq_rows); if (rc) return rc; }
     CK(cudaMemcpyAsync(c->d_next, c->h_next.data(), c->h_next.size() * 8, cudaMemcpyHostToDevice, st));
     SimKernelArgs a;
     std::memset(&a, 0, sizeof(a));
@@ -915,6 +934,7 @@ static int simulate_impl(fmc_ctx *c, const fmc_sim_args *g, const fmc_segment_ar
     a.scores = g->scores_dev; a.hist = g->hist_dev; a.counters = (unsigned long long *)g->counters_dev;
     a.stream = g->stream_dev; a.trace = g->trace_dev; a.iters = g->iters_dev;
     a.period_scores = rows; a.segment_hist = segs ? seg->segment_hist_dev : nullptr;
+    a.sequence = seq_rows; a.sequence_hist = seqs ? seq->sequence_hist_dev : nullptr;
     const bool players = !c->usage.empty();
     if ((g->players_dev || g->player_hist_dev) && !players)
         return fail(FMC_ERR_INVALID, "fmc_simulate: players_dev / player_hist_dev need fmc_set_usage");
@@ -959,18 +979,27 @@ static int simulate_impl(fmc_ctx *c, const fmc_sim_args *g, const fmc_segment_ar
         c->memo_valid = bytes != 0;
     }
     const int mgrid = c->prop.multiProcessorCount * kMemoCtasPerSm;
-    if (segs) launch_sim<true>(a, memo ? &mm : nullptr, players, test, grid, mgrid, smem, st);
-    else launch_sim<false>(a, memo ? &mm : nullptr, players, test, grid, mgrid, smem, st);
+    const MemoArgs *mp = memo ? &mm : nullptr;
+    switch ((segs ? kHookPeriods : 0) | (seqs ? kHookSequence : 0)) {
+    case 0: launch_sim<0>(a, mp, players, test, grid, mgrid, smem, st); break;
+    case kHookPeriods: launch_sim<kHookPeriods>(a, mp, players, test, grid, mgrid, smem, st); break;
+    case kHookSequence: launch_sim<kHookSequence>(a, mp, players, test, grid, mgrid, smem, st); break;
+    default: launch_sim<kHookPeriods | kHookSequence>(a, mp, players, test, grid, mgrid, smem, st); break;
+    }
     CK(cudaGetLastError());
     CK(cudaEventRecord(c->ev_done, st));
     c->launched = true;
     return FMC_OK;
 }
 
-extern "C" int fmc_simulate(fmc_ctx *c, const fmc_sim_args *g) { return simulate_impl(c, g, nullptr); }
+extern "C" int fmc_simulate(fmc_ctx *c, const fmc_sim_args *g) { return simulate_impl(c, g, nullptr, nullptr); }
 
 extern "C" int fmc_simulate_segments(fmc_ctx *c, const fmc_sim_args *g, const fmc_segment_args *seg) {
-    return simulate_impl(c, g, seg);
+    return simulate_impl(c, g, seg, nullptr);
+}
+
+extern "C" int fmc_simulate_markets(fmc_ctx *c, const fmc_sim_args *g, const fmc_segment_args *seg, const fmc_sequence_args *seq) {
+    return simulate_impl(c, g, seg, seq);
 }
 
 // Device scratch of fmc_simulate_host, kept in the context between calls (grow-only): no cudaMalloc / cudaFree per call.
@@ -1020,7 +1049,7 @@ static cudaError_t d2h_staged(fmc_ctx *c, void *dst, const void *src, size_t byt
 static int simulate_host_impl(fmc_ctx *c, uint64_t seed, uint32_t *scores_host, uint32_t *hist_host,
                               uint64_t *counters_host, const double *stream_host, double *trace_host,
                               uint16_t *iters_host, fmc_player_rec *players_host, uint32_t *player_hist_host,
-                              uint32_t *period_host, uint32_t *seg_hist_host) {
+                              uint32_t *period_host, uint32_t *seg_hist_host, uint32_t *seq_host, uint32_t *seq_hist_host) {
     if (!c) return fail(FMC_ERR_INVALID, "ctx is NULL");
     if (c->matchups.empty()) return fail(FMC_ERR_INVALID, "fmc_set_matchups has not been called");
     CK(cudaSetDevice(c->device));
@@ -1039,8 +1068,9 @@ static int simulate_host_impl(fmc_ctx *c, uint64_t seed, uint32_t *scores_host, 
     fmc_player_rec *d_players = nullptr;
     const size_t players_n = games * 2 * (size_t)c->n_slots;
     if ((players_host || player_hist_host) && c->usage.empty()) return fail(FMC_ERR_INVALID, "players output needs fmc_set_usage");
-    uint32_t *d_phist = nullptr, *d_period = nullptr, *d_seg = nullptr;
+    uint32_t *d_phist = nullptr, *d_period = nullptr, *d_seg = nullptr, *d_seq = nullptr, *d_seqh = nullptr;
     const size_t seg_n = nm * 2 * FMC_N_SEGMENTS * FMC_HIST_BINS * FMC_HIST_BINS;
+    const size_t seqh_n = nm * 2 * FMC_SEQ_BINS;
     const size_t phist_n = c->matchups.size() * 2 * (size_t)c->n_slots * FMC_PH_BINS;
     int rc = FMC_OK;
     cudaError_t e = cudaSuccess;
@@ -1080,6 +1110,13 @@ static int simulate_host_impl(fmc_ctx *c, uint64_t seed, uint32_t *scores_host, 
             if ((e = scratch(c, 10, seg_n * 4, (void **)&d_seg)) != cudaSuccess) { bail(e, "cudaMalloc segment hist"); break; }
             if ((e = cudaMemsetAsync(d_seg, 0, seg_n * 4)) != cudaSuccess) { bail(e, "memset segment hist"); break; }
         }
+        if (seq_host && games) {
+            if ((e = scratch(c, 12, games * 2 * 4, (void **)&d_seq)) != cudaSuccess) { bail(e, "cudaMalloc sequence"); break; }
+        }
+        if (seq_hist_host) {
+            if ((e = scratch(c, 13, seqh_n * 4, (void **)&d_seqh)) != cudaSuccess) { bail(e, "cudaMalloc sequence hist"); break; }
+            if ((e = cudaMemsetAsync(d_seqh, 0, seqh_n * 4)) != cudaSuccess) { bail(e, "memset sequence hist"); break; }
+        }
         fmc_sim_args g;
         std::memset(&g, 0, sizeof(g));
         g.player_hist_dev = d_phist;
@@ -1088,7 +1125,9 @@ static int simulate_host_impl(fmc_ctx *c, uint64_t seed, uint32_t *scores_host, 
         g.players_dev = d_players;
         fmc_segment_args sg;
         sg.period_scores_dev = d_period; sg.segment_hist_dev = d_seg;
-        rc = simulate_impl(c, &g, &sg);
+        fmc_sequence_args sq;
+        sq.sequence_dev = d_seq; sq.sequence_hist_dev = d_seqh;
+        rc = simulate_impl(c, &g, &sg, &sq);
         if (rc) break;
         if ((e = cudaDeviceSynchronize()) != cudaSuccess) { bail(e, "sim_kernel"); break; }
         if (scores_host && games && (e = d2h_staged(c, scores_host, d_scores, games * 4)) != cudaSuccess) { bail(e, "D2H scores"); break; }
@@ -1100,6 +1139,8 @@ static int simulate_host_impl(fmc_ctx *c, uint64_t seed, uint32_t *scores_host, 
         if (d_phist && (e = cudaMemcpy(player_hist_host, d_phist, phist_n * 4, cudaMemcpyDeviceToHost)) != cudaSuccess) { bail(e, "D2H player hist"); break; }
         if (d_period && (e = d2h_staged(c, period_host, d_period, games * 3 * 4)) != cudaSuccess) { bail(e, "D2H period scores"); break; }
         if (d_seg && (e = cudaMemcpy(seg_hist_host, d_seg, seg_n * 4, cudaMemcpyDeviceToHost)) != cudaSuccess) { bail(e, "D2H segment hist"); break; }
+        if (d_seq && (e = d2h_staged(c, seq_host, d_seq, games * 2 * 4)) != cudaSuccess) { bail(e, "D2H sequence"); break; }
+        if (d_seqh && (e = cudaMemcpy(seq_hist_host, d_seqh, seqh_n * 4, cudaMemcpyDeviceToHost)) != cudaSuccess) { bail(e, "D2H sequence hist"); break; }
     } while (0);
     // big test-mode buffers (injected draws, traces: 46 KB per game) are not worth keeping
     for (int slot : {3, 4})
@@ -1111,14 +1152,14 @@ extern "C" int fmc_simulate_host(fmc_ctx *c, uint64_t seed, uint32_t *scores_hos
                                  uint64_t *counters_host, const double *stream_host, double *trace_host,
                                  uint16_t *iters_host) {
     return simulate_host_impl(c, seed, scores_host, hist_host, counters_host, stream_host, trace_host, iters_host, nullptr, nullptr,
-                              nullptr, nullptr);
+                              nullptr, nullptr, nullptr, nullptr);
 }
 
 extern "C" int fmc_simulate_players_host(fmc_ctx *c, uint64_t seed, uint32_t *scores_host, uint32_t *hist_host,
                                          uint64_t *counters_host, const double *stream_host, double *trace_host,
                                          uint16_t *iters_host, fmc_player_rec *players_host, uint32_t *player_hist_host) {
     return simulate_host_impl(c, seed, scores_host, hist_host, counters_host, stream_host, trace_host, iters_host, players_host,
-                              player_hist_host, nullptr, nullptr);
+                              player_hist_host, nullptr, nullptr, nullptr, nullptr);
 }
 
 extern "C" int fmc_simulate_segments_host(fmc_ctx *c, uint64_t seed, uint32_t *scores_host, uint32_t *hist_host,
@@ -1126,7 +1167,16 @@ extern "C" int fmc_simulate_segments_host(fmc_ctx *c, uint64_t seed, uint32_t *s
                                           uint16_t *iters_host, fmc_player_rec *players_host, uint32_t *player_hist_host,
                                           uint32_t *period_scores_host, uint32_t *segment_hist_host) {
     return simulate_host_impl(c, seed, scores_host, hist_host, counters_host, stream_host, trace_host, iters_host, players_host,
-                              player_hist_host, period_scores_host, segment_hist_host);
+                              player_hist_host, period_scores_host, segment_hist_host, nullptr, nullptr);
+}
+
+extern "C" int fmc_simulate_markets_host(fmc_ctx *c, uint64_t seed, uint32_t *scores_host, uint32_t *hist_host,
+                                         uint64_t *counters_host, const double *stream_host, double *trace_host,
+                                         uint16_t *iters_host, fmc_player_rec *players_host, uint32_t *player_hist_host,
+                                         uint32_t *period_scores_host, uint32_t *segment_hist_host, uint32_t *sequence_host,
+                                         uint32_t *sequence_hist_host) {
+    return simulate_host_impl(c, seed, scores_host, hist_host, counters_host, stream_host, trace_host, iters_host, players_host,
+                              player_hist_host, period_scores_host, segment_hist_host, sequence_host, sequence_hist_host);
 }
 
 extern "C" int fmc_tree_predict(fmc_ctx *c, int32_t id, const double *rows_dev, int64_t n, double *out_dev,

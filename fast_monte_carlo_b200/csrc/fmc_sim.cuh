@@ -115,11 +115,16 @@ struct SimKernelArgs {
     // player mode: name rows actually needed by the matchups of this launch (a chunk has kSimRows + name_rows rows):
     // passer rows [kDynRow0, +n_prow), target rows behind them, rusher rows [kDynRow0, +n_rrow)
     int n_prow, n_trow, n_rrow, name_rows;
-    // period outputs (fmc_simulate_segments; read only by the SEG instantiations): the Q1..Q3 end scores of every game
+    // period outputs (fmc_simulate_segments; read only by the instantiations with the period hooks): the Q1..Q3 end scores of every game
     // (never NULL there: the library supplies device scratch when the caller did not ask for them) and the optional
     // per-segment histograms
     uint32_t *period_scores;           // [games][3]
     uint32_t *segment_hist;            // [n_matchups][2][FMC_N_SEGMENTS][BINS][BINS]
+    // scoring-sequence outputs (fmc_simulate_markets; read only by the instantiations with the sequence hooks): the
+    // next-score and drive-result words of every game (never NULL there, device scratch like period_scores) and the
+    // optional per-entry histogram
+    uint32_t *sequence;                // [games][2]
+    uint32_t *sequence_hist;           // [n_matchups][2][FMC_SEQ_BINS]
 };
 
 enum Stage : int {
@@ -300,13 +305,106 @@ template <> struct Periods<true> {
     }
 };
 
+// ---- scoring-sequence outputs (fmc_simulate_markets, include/fmc.h FMC_SEQ_NONE) -------------------------------------
+// The hooks of the scoring plays and of the plays that end a drive, called before the play's tick so that they see the
+// clock at the snap (a play's own result therefore comes before the end of the half its tick crosses).  Sequence<false>
+// is empty.  Sequence<true> keeps no lane state: the game's own sequence row is its state, set at the start of the game
+// (next score FMC_SEQ_NONE, drive open) and read back by the later hooks, under the same rule as the period rows.  The
+// race needs no state: scores only grow, so the one play that takes a team from below N to N or more while the other is
+// below N decides target N; a target either team had reached at the start state can never be decided that way, nor end
+// with both teams below it, so it is counted nowhere.
+constexpr uint32_t kDriveOpen = 0xFFFFFFFFu;
+
+template <bool SEQ> struct Sequence;
+template <> struct Sequence<false> {
+    __device__ __forceinline__ Sequence(const SimKernelArgs &, const MatchupDev &, int) {}
+    __device__ __forceinline__ void game_start(const Lane &) const {}
+    __device__ __forceinline__ void scored(const Lane &, int, int, int) const {}
+    __device__ __forceinline__ void drive_end(const Lane &, int, int) const {}
+    __device__ __forceinline__ void game_end(const Lane &) const {}
+};
+template <> struct Sequence<true> {
+    const SimKernelArgs &a;
+    const MatchupDev &M;
+    int matchup;
+    __device__ __forceinline__ Sequence(const SimKernelArgs &a_, const MatchupDev &M_, int m) : a(a_), M(M_), matchup(m) {}
+    __device__ __forceinline__ uint32_t *row(const Lane &L) const {
+        return a.sequence + (size_t)(M.out_offset + (L.game - M.game_begin)) * 2;
+    }
+    __device__ __forceinline__ void count(const Lane &L, int bin) const {
+        if (a.sequence_hist) atomicAdd(a.sequence_hist + ((size_t)matchup * 2 + (L.game & 1ULL)) * FMC_SEQ_BINS + bin, 1u);
+    }
+    __device__ __forceinline__ void game_start(const Lane &L) const {
+        uint32_t *r = row(L);
+        r[0] = FMC_SEQ_NONE;
+        r[1] = kDriveOpen;
+    }
+    // `team` scored (kind FMC_SEQ_TD / FMC_SEQ_FG) on the play snapped at `clock`; L.score already holds the points
+    __device__ __forceinline__ void scored(const Lane &L, int team, int kind, int clock) const {
+        uint32_t *r = row(L);
+        if (r[0] == FMC_SEQ_NONE) {
+            r[0] = FMC_SEQ_WORD(team, kind, clock);
+            count(L, FMC_SEQ_BIN_NEXT(team, kind, clock));
+        }
+        if (a.sequence_hist) {
+            constexpr int targets[FMC_N_RACE] = FMC_RACE_TARGETS;
+            const int now = L.score[team], before = now - (kind == FMC_SEQ_TD ? 7 : 3), other = L.score[team ^ 1];
+#pragma unroll
+            for (int t = 0; t < FMC_N_RACE; ++t)
+                if (before < targets[t] && now >= targets[t] && other < targets[t]) count(L, FMC_SEQ_BIN_RACE(t, team));
+        }
+    }
+    // the play snapped at `clock` ends the drive with result `code`, unless an earlier play ended it
+    __device__ __forceinline__ void drive_end(const Lane &L, int code, int clock) const {
+        uint32_t *r = row(L);
+        if (r[1] == kDriveOpen) {
+            r[1] = FMC_DRIVE_WORD(code, clock);
+            count(L, FMC_SEQ_BIN_DRIVE(code));
+        }
+    }
+    __device__ __forceinline__ void game_end(const Lane &L) const {
+        if (row(L)[0] == FMC_SEQ_NONE) count(L, FMC_SEQ_BIN_NONE);
+        drive_end(L, FMC_DRIVE_GAME, 0);
+        if (a.sequence_hist) {
+            constexpr int targets[FMC_N_RACE] = FMC_RACE_TARGETS;
+#pragma unroll
+            for (int t = 0; t < FMC_N_RACE; ++t)
+                if (L.score[0] < targets[t] && L.score[1] < targets[t]) count(L, FMC_SEQ_BIN_RACE(t, FMC_RACE_NEITHER));
+        }
+    }
+};
+
+// The hook policy of the step functions: HOOKS is a mask of the launch's optional outputs.  Hooks<0> compiles to the code
+// without hooks; kOn says whether any hook is in (a hooked field goal adds its points before its tick).
+enum { kHookPeriods = 1, kHookSequence = 2 };
+template <int HOOKS>
+struct Hooks {
+    static constexpr bool kOn = HOOKS != 0;
+    Periods<(HOOKS & kHookPeriods) != 0> per;
+    Sequence<(HOOKS & kHookSequence) != 0> seq;
+    __device__ __forceinline__ Hooks(const SimKernelArgs &a, const MatchupDev &M, int m) : per(a, M, m), seq(a, M, m) {}
+    __device__ __forceinline__ void game_start(const Lane &L) const { seq.game_start(L); }
+    // quarter q ended with the play snapped at `snap`; the end of the half ends the drive if nothing else did
+    __device__ __forceinline__ void quarter_end(const Lane &L, int q, int snap) const {
+        per.quarter_end(L, q);
+        if (q == 2) seq.drive_end(L, FMC_DRIVE_HALF, snap);
+    }
+    __device__ __forceinline__ void scored(const Lane &L, int team, int kind, int clock) const { seq.scored(L, team, kind, clock); }
+    __device__ __forceinline__ void drive_end(const Lane &L, int code, int clock) const { seq.drive_end(L, code, clock); }
+    __device__ __forceinline__ void game_end(const Lane &L) const {
+        per.game_end(L);
+        seq.game_end(L);
+    }
+};
+
 template <class Pk>
 __device__ __forceinline__ void tick_clock(Lane &L, int base, const Pk &pk) {                // FMC:956-968
+    const int snap = L.sec;
     const int v = L.sec - base;
     L.sec = v > 0 ? v : 0;
     const int old = L.period;
     L.period = L.sec > 0 ? 4 - ((L.sec - 1) / 900) : 4;
-    if (L.period != old) pk.quarter_end(L, old);
+    if (L.period != old) pk.quarter_end(L, old, snap);
     if (L.period != old && L.period == 3) change_possession(L, true, 75.0);
 }
 __device__ __forceinline__ double pass_prob_v1(int down, double distance, double ytg, int sec, int sd) {  // FMC:719-735
@@ -613,10 +711,12 @@ __device__ __forceinline__ bool fourth_down(Lane &L, Draws<TEST> &D, int sd, Ev 
     if (ytg <= 38.0) {
         ev.hit(EV_FGA);
         const bool good = D.u(S_U_FG) < field_goal_prob(ytg + 17.0);
-        // With period hooks the kick's points go on before its tick, as a touchdown's do, so that a quarter that ends on
-        // the kick holds them.  tick_clock and change_possession read no score, so the order changes nothing else; the
+        // With hooks the kick's points go on before its tick, as a touchdown's do, so that a quarter that ends on the
+        // kick holds them and the scoring hook sees them.  tick_clock and change_possession read no score, so the order changes nothing else; the
         // instantiations without hooks keep the original order, which compiles to fewer spills there.
         if (Pk::kOn && good) L.score[team] += 3;
+        if (good) pk.scored(L, team, FMC_SEQ_FG, L.sec);
+        pk.drive_end(L, good ? FMC_DRIVE_FG : FMC_DRIVE_MISSED_FG, L.sec);
         tick_clock(L, 12, pk);
         if (good) { ev.hit(EV_FG); if (!Pk::kOn) L.score[team] += 3; change_possession(L, true, 75.0); }
         else change_possession(L, true, 100.0 - ytg);
@@ -632,6 +732,7 @@ __device__ __forceinline__ bool fourth_down(Lane &L, Draws<TEST> &D, int sd, Ev 
     }
     net = softclip(net, 15.0, ytg - 1.0);
     const int inet = (int)net;
+    pk.drive_end(L, FMC_DRIVE_PUNT, L.sec);
     tick_clock(L, 16, pk);
     change_possession(L, true, softclip(100.0 - (ytg - (double)inet), 1.0, 99.0));
     return false;
@@ -732,6 +833,7 @@ __device__ __forceinline__ void after_stage2(Lane &L, const SimKernelArgs &a, co
         const double ret = softclip(6.0 + 5.0 * D.z(S_Z_INT), 0.0, L.ytg);
         const double spot = 100.0 - (L.ytg - ret);
         L.going = 0;
+        pk.drive_end(L, FMC_DRIVE_INT, L.sec);
         change_possession(L, true, spot);
         tick_clock(L, 12, pk);
         L.stage = ST_ITER;
@@ -775,11 +877,14 @@ __device__ __forceinline__ void after_yards(Lane &L, const SimKernelArgs &a, con
         if (td) {
             ev.hit(EV_TD);
             L.score[team] += 7; L.going = 0;
+            pk.scored(L, team, FMC_SEQ_TD, L.sec);
+            pk.drive_end(L, FMC_DRIVE_TD, L.sec);
             tick_clock(L, pass ? 20 : 28, pk);
             change_possession(L, true, 75.0);
         } else {
             L.going = 0;
             advance_down(L, yards);
+            if (L.offense != team) pk.drive_end(L, FMC_DRIVE_DOWNS, L.sec);      // turnover on downs
             tick_clock(L, pass ? 26 : 28, pk);
         }
     }
@@ -788,18 +893,19 @@ __device__ __forceinline__ void after_yards(Lane &L, const SimKernelArgs &a, con
 
 // Advance one lane until it posts a request (returns its key, family * 2 + offense) or has nothing
 // left to do (returns -1).  `res` points at this lane's result record of the previous round.
-template <bool TEST, bool PLAYERS, bool SEG>
+template <bool TEST, bool PLAYERS, int HOOKS>
 __device__ __forceinline__ int advance_lane(Lane &L, const SimKernelArgs &a, SimShared &sh, const double *res) {
     const MatchupDev &M = sh.M;
     const int matchup = sh.cur_matchup;
     StatEvents ev{sh.stat};
-    const Periods<SEG> pk(a, M, matchup);
+    const Hooks<HOOKS> pk(a, M, matchup);
     for (;;) {
         if (L.stage == ST_IDLE) return -1;
         if (L.stage == ST_NEED_GAME) {
             const unsigned long long g = atomicAdd(&a.next_game[matchup], 1ULL);
             if (g >= M.game_end) { L.stage = ST_IDLE; return -1; }
             new_game(L, M, g);
+            pk.game_start(L);
         }
         if (L.stage == ST_ITER) {
             if (L.sec <= 0) {
@@ -1036,9 +1142,10 @@ __device__ __forceinline__ void walk_requests(RoundShared &sh, const SimKernelAr
 
 // PLAYERS = true: usage tables are set (fmc_set_usage): names are sampled per play, requests carry kDynRows
 // more feature rows, tracked names get per-game box lines.  The shipped configuration (every name "Unknown")
-// runs the PLAYERS = false instantiation, which carries none of it.  SEG = true: the launch has period outputs
-// (fmc_simulate_segments, Periods<true>); the SEG = false instantiations are the code without the hooks.
-template <bool TEST, bool PLAYERS, bool SEG>
+// runs the PLAYERS = false instantiation, which carries none of it.  HOOKS: the optional outputs of the launch
+// (kHookPeriods: fmc_simulate_segments, Periods<true>; kHookSequence: fmc_simulate_markets, Sequence<true>); the
+// HOOKS = 0 instantiations are the code without the hooks.
+template <bool TEST, bool PLAYERS, int HOOKS>
 __global__ void __launch_bounds__(kSimThreads, kSimCtasPerSm) sim_kernel(const SimKernelArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     // player mode sizes a chunk by the name rows the launch needs (runtime); the shipped configuration is compile-time
@@ -1074,7 +1181,7 @@ __global__ void __launch_bounds__(kSimThreads, kSimCtasPerSm) sim_kernel(const S
             // ---- A: advance to the next request (a held-back lane re-posts the one it has)
             Lane L = unpack_lane(P);
             L.home = home;
-            const int key = held >= 0 ? held : advance_lane<TEST, PLAYERS, SEG>(L, a, sh, results + (size_t)pos * 3);
+            const int key = held >= 0 ? held : advance_lane<TEST, PLAYERS, HOOKS>(L, a, sh, results + (size_t)pos * 3);
             __syncwarp();
             // ---- B: compaction
             const unsigned int rank = request_rank(sh.cnt[parity], key, lane);

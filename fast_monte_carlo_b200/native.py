@@ -13,6 +13,9 @@ from typing import Optional
 
 import numpy as np
 
+from . import outputs as _out
+from .outputs import DRIVE_RESULTS, RACE_TARGETS, SEQ_BINS  # noqa: F401  (scoring-sequence layout, include/fmc.h)
+
 HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("FMC_LIB_PATH") or os.path.join(HERE, "libfmc_b200.so")
 
@@ -32,6 +35,14 @@ PH_YDS_BINS, PH_YDS_OFFSET, PH_CNT_BINS = 8192, 1000, 128
 PH_BINS = PH_YDS_BINS + 5 * PH_CNT_BINS
 N_SEGMENTS = 6                     # FMC_N_SEGMENTS: Q1, Q2, Q3, Q4, H1, H2
 PERIOD_NONE = 0xFFFFFFFF           # FMC_PERIOD_NONE: a quarter end at or before the start state
+# scoring sequence (include/fmc.h FMC_SEQ_NONE): the per-game words; the histogram layout is outputs'
+SEQ_NONE = 0xFFFFFFFF              # FMC_SEQ_NONE: no score after the start state
+SEQ_TD, SEQ_FG = 0, 1              # kind of a scoring play
+
+
+def seq_bin_next(team, kind, clock):
+    """FMC_SEQ_BIN_NEXT: bin of a next score by `team` of `kind` snapped with `clock` (1..3600) seconds left"""
+    return (team * 2 + kind) * _out.SEQ_MINUTES + (np.asarray(clock) - 1) // 60
 
 
 class FmcError(RuntimeError):
@@ -84,6 +95,11 @@ class SimArgs(C.Structure):
 class SegmentArgs(C.Structure):
     """fmc_segment_args"""
     _fields_ = [("period_scores_dev", C.c_void_p), ("segment_hist_dev", C.c_void_p)]
+
+
+class SequenceArgs(C.Structure):
+    """fmc_sequence_args"""
+    _fields_ = [("sequence_dev", C.c_void_p), ("sequence_hist_dev", C.c_void_p)]
 
 
 MAX_USAGE = 32
@@ -167,6 +183,8 @@ def load_library():
                                             C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]
     L.fmc_simulate_segments.argtypes = [C.c_void_p, C.POINTER(SimArgs), C.POINTER(SegmentArgs)]
     L.fmc_simulate_segments_host.argtypes = [C.c_void_p, C.c_uint64] + [C.c_void_p] * 10
+    L.fmc_simulate_markets.argtypes = [C.c_void_p, C.POINTER(SimArgs), C.POINTER(SegmentArgs), C.POINTER(SequenceArgs)]
+    L.fmc_simulate_markets_host.argtypes = [C.c_void_p, C.c_uint64] + [C.c_void_p] * 12
     L.fmc_set_usage.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32]
     L.fmc_set_start_states.argtypes = [C.c_void_p, C.c_int32, C.c_void_p]
     L.fmc_pack_forest_host_dyn.restype = C.c_int64
@@ -206,6 +224,7 @@ EXPORTED_SYMBOLS = (
     "fmc_pack_forest_host", "fmc_pack_forest_host_dyn", "fmc_set_usage", "fmc_simulate_players_host",
     "fmc_set_memo", "fmc_memo_keys_host", "fmc_gather_probe_coherent", "fmc_predict_stats", "fmc_invalidate_tables", "fmc_tree_predict_cols_host",
     "fmc_set_start_states", "fmc_simulate_segments", "fmc_simulate_segments_host",
+    "fmc_simulate_markets", "fmc_simulate_markets_host",
 )
 
 
@@ -446,10 +465,12 @@ class Context:
 
     # -- simulation ------------------------------------------------------------------------------
     def simulate_device(self, *, seed: int, scores=0, hist=0, counters=0, stream_in=0, trace=0, iters=0,
-                        cuda_stream=0, players=0, player_hist=0, period_scores=0, segment_hist=0) -> None:
+                        cuda_stream=0, players=0, player_hist=0, period_scores=0, segment_hist=0, sequence=0,
+                        sequence_hist=0) -> None:
         """Asynchronous launch on raw device pointers (ints; 0 = not requested).  `period_scores` (uint32[games][3]) and
-        `segment_hist` (uint32[n_matchups][2][N_SEGMENTS][BINS][BINS], zeroed by the caller) are the per-period outputs
-        of fmc_simulate_segments; without them the call is fmc_simulate."""
+        `segment_hist` (uint32[n_matchups][2][N_SEGMENTS][BINS][BINS], zeroed by the caller) are the per-period outputs,
+        `sequence` (uint32[games][2]) and `sequence_hist` (uint32[n_matchups][2][SEQ_BINS], zeroed by the caller) the
+        scoring-sequence outputs of fmc_simulate_markets; without any of them the call is fmc_simulate."""
         a = SimArgs()
         a.seed = int(seed) & 0xFFFFFFFFFFFFFFFF
         a.n_matchups = self.n_matchups
@@ -458,20 +479,24 @@ class Context:
         a.stream = cuda_stream or None
         a.players_dev = players or None      # fmc_player_rec[games][2][n_slots]
         a.player_hist_dev = player_hist or None   # uint32[n_matchups][2][n_slots][PH_BINS], zeroed by the caller
-        if period_scores or segment_hist:
+        if period_scores or segment_hist or sequence or sequence_hist:
             sg = SegmentArgs()
             sg.period_scores_dev = period_scores or None; sg.segment_hist_dev = segment_hist or None
-            _check(self._L.fmc_simulate_segments(self._h, C.byref(a), C.byref(sg)))
+            sq = SequenceArgs()
+            sq.sequence_dev = sequence or None; sq.sequence_hist_dev = sequence_hist or None
+            _check(self._L.fmc_simulate_markets(self._h, C.byref(a), C.byref(sg), C.byref(sq)))
         else:
             _check(self._L.fmc_simulate(self._h, C.byref(a)))
 
     def simulate_host(self, *, seed: int, want_scores=True, want_hist=True, stream: Optional[np.ndarray] = None,
                       want_trace=False, want_iters=False, want_players=False, want_player_hist=False,
-                      want_period_scores=False, want_segments=False) -> dict:
+                      want_period_scores=False, want_segments=False, want_sequence=False, want_sequence_hist=False) -> dict:
         """End-to-end call with host buffers (fmc_simulate_host / fmc_simulate_players_host, and
         fmc_simulate_segments_host when `want_period_scores` / `want_segments` ask for the per-period outputs: "period_scores"
         uint32[games][3] score words at the end of Q1..Q3 (PERIOD_NONE before the start state), "segment_hist"
-        uint32[n_matchups][2][N_SEGMENTS][BINS][BINS])."""
+        uint32[n_matchups][2][N_SEGMENTS][BINS][BINS]), and fmc_simulate_markets_host when `want_sequence` /
+        `want_sequence_hist` ask for the scoring-sequence outputs: "sequence" uint32[games][2] (next-score word, drive-result
+        word) and "sequence_hist" uint32[n_matchups][2][SEQ_BINS]."""
         n = self.total_games
         scores = np.zeros(n, dtype=np.uint32) if want_scores else None
         hist = np.zeros((self.n_matchups, 2, HIST_BINS, HIST_BINS), dtype=np.uint32) if want_hist else None
@@ -493,11 +518,13 @@ class Context:
                 players = np.zeros((n, 2, max(self.n_slots, 1)), dtype=PLAYER_REC)
             if want_player_hist:
                 phist = np.zeros((self.n_matchups, 2, max(self.n_slots, 1), PH_BINS), dtype=np.uint32)
-        if period is not None or seg is not None:
-            _check(self._L.fmc_simulate_segments_host(
+        seq = np.zeros((n, 2), dtype=np.uint32) if want_sequence else None
+        seqh = np.zeros((self.n_matchups, 2, SEQ_BINS), dtype=np.uint32) if want_sequence_hist else None
+        if period is not None or seg is not None or seq is not None or seqh is not None:
+            _check(self._L.fmc_simulate_markets_host(
                 self._h, int(seed) & 0xFFFFFFFFFFFFFFFF, vp(scores), vp(hist), vp(counters), vp(stream), vp(trace), vp(iters),
                 players.ctypes.data if (players is not None and self.n_slots) else None,
-                phist.ctypes.data if (phist is not None and self.n_slots) else None, vp(period), vp(seg)))
+                phist.ctypes.data if (phist is not None and self.n_slots) else None, vp(period), vp(seg), vp(seq), vp(seqh)))
         elif players is not None or phist is not None:
             _check(self._L.fmc_simulate_players_host(self._h, int(seed) & 0xFFFFFFFFFFFFFFFF, vp(scores), vp(hist),
                                                      vp(counters), vp(stream), vp(trace), vp(iters),
@@ -525,6 +552,10 @@ class Context:
             out["period_scores"] = period
         if seg is not None:
             out["segment_hist"] = seg
+        if seq is not None:
+            out["sequence"] = seq
+        if seqh is not None:
+            out["sequence_hist"] = seqh
         return out
 
     # -- tree prediction -------------------------------------------------------------------------------

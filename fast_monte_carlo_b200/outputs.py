@@ -289,6 +289,81 @@ def segment_odds_from_hist(h2: np.ndarray, team_a: str, team_b: str, *, offset=(
     return out
 
 
+# scoring sequence (include/fmc.h FMC_SEQ_NONE): layout of one orientation's sequence histogram
+DRIVE_RESULTS = ("td", "fg", "missed_fg", "punt", "interception", "downs", "end_of_half", "end_of_game")
+RACE_TARGETS = (10, 15, 20, 25, 30)
+SEQ_MINUTES = 60
+SEQ_BIN_NONE = 4 * SEQ_MINUTES
+SEQ_BIN_DRIVE0 = SEQ_BIN_NONE + 1
+SEQ_BIN_RACE0 = SEQ_BIN_DRIVE0 + len(DRIVE_RESULTS)
+SEQ_BINS = SEQ_BIN_RACE0 + 3 * len(RACE_TARGETS)
+SCORE_KINDS = ("td", "fg")
+
+
+def sequence_odds_from_hist(h, team_a: str, team_b: str, *, start_score=(0, 0), before=()) -> Dict[str, object]:
+    """Next-score, drive-result and race-to-N odds from a scoring-sequence histogram: [SEQ_BINS] of one orientation or
+    [..., SEQ_BINS] (summed over the leading axes, e.g. both orientations).  `start_score` = (A, B) points at the start
+    state the histogram was played from: a race target either team had reached there is settled.  `before` = clocks C
+    (multiples of 60 in 0..3600) for P(the next score is by a team and snapped with more than C seconds left).
+    Returns {"games",
+             "next_score": {"p": {team: {"td", "fg", "any"}}, "none", "american": {team: {...}}, "before": {C: {team: p}}},
+             "drive": {"p": {result: p}, "p_scores", "american": {result: odds}},
+             "race": {N: {"settled": False, "p": {team_a, team_b, "neither"}, "american": {...}} or
+                         {"settled": True, "winner": team or None (both teams had reached N)}}}.
+    ValueError for a histogram of another shape, negative or empty counts, drive or race bins that do not hold every
+    game, or a malformed start score or clock."""
+    a = np.asarray(h)
+    if a.ndim < 1 or a.shape[-1] != SEQ_BINS:
+        raise ValueError(f"a sequence histogram has {SEQ_BINS} bins in its last axis, got shape {a.shape}")
+    if not np.issubdtype(a.dtype, np.integer) or (a < 0).any():
+        raise ValueError("a sequence histogram holds non-negative integer counts")
+    a = a.reshape(-1, SEQ_BINS).astype(np.int64).sum(axis=0)
+    sc = tuple(start_score)
+    if len(sc) != 2 or any(int(x) != x or x < 0 for x in sc):
+        raise ValueError(f"start_score must be (points A, points B) >= 0, got {start_score!r}")
+    nxt = a[:SEQ_BIN_NONE].reshape(2, 2, SEQ_MINUTES)              # [team][kind][minute]
+    n = int(nxt.sum() + a[SEQ_BIN_NONE])
+    if n <= 0:
+        raise ValueError("the histogram holds no games")
+    drive = a[SEQ_BIN_DRIVE0:SEQ_BIN_RACE0]
+    if int(drive.sum()) != n:
+        raise ValueError(f"the drive bins hold {int(drive.sum())} games, the next-score bins {n}")
+    teams = (team_a, team_b)
+    p_next = {teams[t]: {SCORE_KINDS[k]: float(nxt[t, k].sum() / n) for k in range(2)} for t in range(2)}
+    for t in teams:
+        p_next[t]["any"] = p_next[t]["td"] + p_next[t]["fg"]
+    p_none = float(a[SEQ_BIN_NONE] / n)
+    out_before = {}
+    for c in before:
+        if int(c) != c or c < 0 or c > 3600 or int(c) % 60:
+            raise ValueError(f"a clock of `before` must be a multiple of 60 in 0..3600, got {c!r}")
+        # snap clock > C  <=>  minute bin (clock - 1) // 60 >= C // 60
+        out_before[int(c)] = {teams[t]: float(nxt[t, :, int(c) // 60:].sum() / n) for t in range(2)}
+    p_drive = {r: float(drive[i] / n) for i, r in enumerate(DRIVE_RESULTS)}
+    race = {}
+    for i, target in enumerate(RACE_TARGETS):
+        bins = a[SEQ_BIN_RACE0 + 3 * i:SEQ_BIN_RACE0 + 3 * i + 3]
+        if sc[0] >= target or sc[1] >= target:
+            if bins.sum():
+                raise ValueError(f"race to {target} was settled at the start score {sc} but its bins hold games")
+            race[target] = {"settled": True,
+                            "winner": None if (sc[0] >= target and sc[1] >= target) else teams[0 if sc[0] >= target else 1]}
+            continue
+        if int(bins.sum()) != n:
+            raise ValueError(f"the race-to-{target} bins hold {int(bins.sum())} games, the next-score bins {n}")
+        p = {team_a: float(bins[0] / n), team_b: float(bins[1] / n), "neither": float(bins[2] / n)}
+        race[target] = {"settled": False, "p": p, "american": {k: prob_to_american(v) for k, v in p.items()}}
+    return {
+        "games": n,
+        "next_score": {"p": p_next, "none": p_none,
+                       "american": {t: {k: prob_to_american(v) for k, v in p_next[t].items()} for t in teams},
+                       "before": out_before},
+        "drive": {"p": p_drive, "p_scores": p_drive["td"] + p_drive["fg"],
+                  "american": {k: prob_to_american(v) for k, v in p_drive.items()}},
+        "race": race,
+    }
+
+
 def summary_from_hist(hist2: np.ndarray, team_a: str, team_b: str) -> pd.DataFrame:
     """The `summary` frame of simulate_upcoming_matchup (FMC:1681-1687) from the histogram: each
     team's row covers the orientation in which it received the opening kickoff."""

@@ -184,6 +184,40 @@ enum {
 enum { FMC_SEG_Q1 = 0, FMC_SEG_Q2, FMC_SEG_Q3, FMC_SEG_Q4, FMC_SEG_H1, FMC_SEG_H2 };
 #define FMC_PERIOD_NONE 0xFFFFFFFFu  /* period_scores word of a quarter end at or before the start state */
 
+/* Scoring sequence (next-score, drive-result and race-to-N markets, fmc_simulate_markets).  Everything counts from the
+ * game's start state (the kickoff, or fmc_set_start_states); teams are the matchup's (0 = A).  The engine scores only
+ * touchdowns (7) and made field goals (3), always by the team on offense.
+ *  - Next score: the first play after the start state that adds points: (team, kind, clock at its snap = the seconds at
+ *    the start of the iteration that played it).  FMC_SEQ_NONE if the game ends with the start score.
+ *  - Drive result: the drive is the possession of the team on offense at the start state (g & 1 at the kickoff).  It
+ *    ends at the first of: TD, FG made, FG missed, punt, interception, turnover on downs (advance_down's change of
+ *    possession), end of half (the halftime change of possession when the clock crosses 1800), end of game (the clock
+ *    reaches 0 with the drive on).  A play's own result comes before the end of the half its tick crosses.  A down
+ *    that passes 4 without a change of possession (incomplete pass, sack) does not end it.
+ *  - Race to N (N in FMC_RACE_TARGETS): won by the team whose score (start points included) first reaches N, decided
+ *    at the scoring play that takes it from below N to N or more while the other team is below N; "neither" if no team
+ *    reaches N.  A target either team had reached at the start state is settled and not counted. */
+#define FMC_SEQ_NONE 0xFFFFFFFFu     /* sequence word 0 of a game without a score after the start state */
+enum { FMC_SEQ_TD = 0, FMC_SEQ_FG = 1 };          /* kind of a scoring play */
+enum { FMC_DRIVE_TD = 0, FMC_DRIVE_FG, FMC_DRIVE_MISSED_FG, FMC_DRIVE_PUNT, FMC_DRIVE_INT, FMC_DRIVE_DOWNS,
+       FMC_DRIVE_HALF, FMC_DRIVE_GAME, FMC_N_DRIVE };
+#define FMC_N_RACE 5
+#define FMC_RACE_TARGETS {10, 15, 20, 25, 30}
+enum { FMC_RACE_A = 0, FMC_RACE_B, FMC_RACE_NEITHER };
+/* sequence word 0: next score team:1 | kind:1 | clock:12 (or FMC_SEQ_NONE); word 1: drive result | clock at the snap of
+ * the play that ended it << 8 (0 for the end of the game) */
+#define FMC_SEQ_WORD(team, kind, clock) ((uint32_t)(team) | ((uint32_t)(kind) << 1) | ((uint32_t)(clock) << 2))
+#define FMC_DRIVE_WORD(code, clock) ((uint32_t)(code) | ((uint32_t)(clock) << 8))
+/* bins of one orientation's sequence histogram: next score by (team, kind) and minute of regulation at its snap
+ * (clock 1..3600 -> minute bin (clock - 1) / 60, aligned with the quarter ends), no further score, the drive results,
+ * then the race targets x (A, B, neither) */
+#define FMC_SEQ_MINUTES 60
+#define FMC_SEQ_BIN_NEXT(team, kind, clock) (((team) * 2 + (kind)) * FMC_SEQ_MINUTES + ((clock) - 1) / 60)
+#define FMC_SEQ_BIN_NONE (4 * FMC_SEQ_MINUTES)
+#define FMC_SEQ_BIN_DRIVE(code) (FMC_SEQ_BIN_NONE + 1 + (code))
+#define FMC_SEQ_BIN_RACE(target, r) (FMC_SEQ_BIN_DRIVE(FMC_N_DRIVE) + (target) * 3 + (r))
+#define FMC_SEQ_BINS FMC_SEQ_BIN_RACE(FMC_N_RACE, 0)      /* 264 */
+
 #define FMC_N_SLOTS 16           /* injected-draw record per (game, loop iteration); see DESIGN.md */
 #define FMC_MAX_ITERS 360
 #define FMC_TRACE_COLS 8
@@ -302,6 +336,31 @@ int fmc_simulate_segments_host(fmc_ctx *ctx, uint64_t seed, uint32_t *scores_hos
                                uint64_t *counters_host, const double *stream_host, double *trace_host,
                                uint16_t *iters_host, fmc_player_rec *players_host, uint32_t *player_hist_host,
                                uint32_t *period_scores_host, uint32_t *segment_hist_host);
+
+/* Scoring-sequence outputs of a launch (see FMC_SEQ_NONE for the definitions); both optional.
+ *   sequence_dev       [games][2] at out_offset + (g - game_begin) like scores_dev: word 0 the next score
+ *                      (FMC_SEQ_WORD or FMC_SEQ_NONE), word 1 the drive result (FMC_DRIVE_WORD).
+ *   sequence_hist_dev  [n_matchups][2][FMC_SEQ_BINS], += 1 at [m][g & 1][bin] for the next score (or none), the drive
+ *                      result and every race target that is not settled (zero it first, like hist_dev).
+ *                      Without sequence_dev the library keeps the per-game rows in device scratch (8 B a game), grown
+ *                      like the period rows of fmc_segment_args. */
+typedef struct {
+    uint32_t *sequence_dev;
+    uint32_t *sequence_hist_dev;
+} fmc_sequence_args;
+
+/* fmc_simulate plus the per-period and the scoring-sequence outputs; seg and seq may each be NULL (or hold only NULL
+ * pointers).  Neither is fmc_simulate, seg alone fmc_simulate_segments.  The launch runs the kernel instantiation with
+ * the hooks it asks for; every other output, draw and game is the same as without them. */
+int fmc_simulate_markets(fmc_ctx *ctx, const fmc_sim_args *args, const fmc_segment_args *seg, const fmc_sequence_args *seq);
+
+/* fmc_simulate_segments_host plus the scoring-sequence outputs: sequence_host [games][2] and sequence_hist_host
+ * [n_matchups][2][FMC_SEQ_BINS] (any output may be NULL). */
+int fmc_simulate_markets_host(fmc_ctx *ctx, uint64_t seed, uint32_t *scores_host, uint32_t *hist_host,
+                              uint64_t *counters_host, const double *stream_host, double *trace_host,
+                              uint16_t *iters_host, fmc_player_rec *players_host, uint32_t *player_hist_host,
+                              uint32_t *period_scores_host, uint32_t *segment_hist_host, uint32_t *sequence_host,
+                              uint32_t *sequence_hist_host);
 
 /* Raw margins of one model on n rows of the 17 numerics (play_model: first 12), NUM order of
  * FMC:676-682, float64 row-major [n][17]; out float64 [n][n_outputs].  Trees [tree_begin, tree_end)
