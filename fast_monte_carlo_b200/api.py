@@ -34,7 +34,7 @@ import pandas as pd
 
 from . import outputs
 from . import usage as _usage
-from .engine import Engine, GameState, MatchupSpec
+from .engine import Engine, GameState, MatchupSpec, OvertimeRules, overtime_rules  # noqa: F401
 from .priors import (TeamContext, build_team_context_from_sp_flex, csv_base_from, load_sp_flex,
                      lookup_sp_flex, packaged_priors_path)
 
@@ -88,10 +88,15 @@ def simulate_matchup(teamA: TeamContext, teamB: TeamContext, n: int = 100, seed:
                      show_progress: bool = True, collect_players: bool = False,
                      players_csv: Optional[str] = None, processes: Optional[int] = None,
                      *, engine: Optional[Engine] = None,
-                     game_range: Optional[Tuple[int, int]] = None) -> Tuple[pd.DataFrame, Optional[pd.DataFrame]]:
+                     game_range: Optional[Tuple[int, int]] = None,
+                     overtime=False) -> Tuple[pd.DataFrame, Optional[pd.DataFrame]]:
     """`game_range=(g0, g1)` (ours, for one process per GPU): simulate only games [g0, g1) of the 2n -- `shard_range`
     gives a rank its slice; the rows returned are those games, and the histograms of the ranks add up to the run's
-    (`merge_histograms`).  A given seed gives the same games whatever the split."""
+    (`merge_histograms`).  A given seed gives the same games whatever the split.
+    `overtime` (False, True or an engine.OvertimeRules): play games level after regulation to a result under college
+    overtime rules.  The scores are then final scores, overtime included, and sims_df.attrs["overtime"] holds
+    `outputs.overtime_odds_from_hist` of the games.  The default is the reference's end of the game at 0:00."""
+    rules = overtime_rules(overtime)
     eng = engine if engine is not None else get_engine()
     games = 2 * int(n)
     g0, g1 = (0, games) if game_range is None else (int(game_range[0]), int(game_range[1]))
@@ -110,13 +115,16 @@ def simulate_matchup(teamA: TeamContext, teamB: TeamContext, n: int = 100, seed:
                 # the sampled names feed the models whether or not the box is collected (FMC:1058-1081, 1203-1216)
                 eng.set_matchups([MatchupSpec(teamA.name, teamB.name, teamA.sp, teamB.sp, games, g0, g1, 0, usage=use)])
                 want_box = bool(collect_players) and eng.n_slots > 0
+                ot_kw = dict(overtime=rules, want_ot_hist=True) if rules is not None else {}
                 res = eng.simulate_host(_fresh_seed() if seed is None else int(seed), want_scores=True, want_hist=True,
-                                        want_players=want_box)
+                                        want_players=want_box, **ot_kw)
             names = names_f.result()
         box = res.get("players")
         sims_df = outputs.sims_frame(teamA.name, teamB.name, res["scores"], first_game=g0, names=names)
         sims_df.attrs["counters"] = dict(res["counters"])
         sims_df.attrs["hist"] = _Attached(res["hist"][0])
+        if rules is not None:
+            sims_df.attrs["overtime"] = outputs.overtime_odds_from_hist(res["ot_hist"][0], teamA.name, teamB.name)
         LAST_RUN.clear()
         LAST_RUN.update(hist=res["hist"][0], counters=dict(res["counters"]), teams=(teamA.name, teamB.name),
                         scores=res["scores"], player_box=box, usage=use, game_range=(g0, g1))
@@ -137,7 +145,9 @@ def simulate_upcoming_matchup(teamA: str, teamB: str, *, year: int = 2025, week:
                               show_progress: bool = True, collect_players: bool = True,
                               save_csv: Optional[str] = None, processes: Optional[int] = None,
                               seed: Optional[int] = None, engine: Optional[Engine] = None,
-                              focus_csv: Optional[str] = None, usage_dir: str = "."):
+                              focus_csv: Optional[str] = None, usage_dir: str = ".", overtime=False):
+    """`overtime` as in `simulate_matchup`; with it, meta["overtime"] holds `outputs.overtime_odds_from_hist`."""
+    overtime_rules(overtime)
     sp_df = load_sp_flex(sp_path)
     # FMC:605 builds the focus tables at import from `2025_week1_players.csv` in the working directory
     focus = _usage.build_focus_usage_tables(focus_csv if focus_csv is not None else _usage.FOCUS_PLAYERS_CSV)
@@ -146,7 +156,8 @@ def simulate_upcoming_matchup(teamA: str, teamB: str, *, year: int = 2025, week:
 
     t0 = time.perf_counter()
     sims_df, players_df = simulate_matchup(A, B, n=n, seed=seed, show_progress=show_progress,
-                                           collect_players=collect_players, processes=processes, engine=engine)
+                                           collect_players=collect_players, processes=processes, engine=engine,
+                                           overtime=overtime)
     t1 = time.perf_counter()
     # FMC:1681-1687.  The group-by over the 2n rows and the joint score histogram the kernel accumulated hold the same
     # information; the histogram gives the five statistics in microseconds (tests check the two agree)
@@ -188,6 +199,8 @@ def simulate_upcoming_matchup(teamA: str, teamB: str, *, year: int = 2025, week:
     if c:
         meta["plays"] = c["plays"]
         meta["games"] = c["games"]
+    if "overtime" in sims_df.attrs:
+        meta["overtime"] = sims_df.attrs["overtime"]
     return sims_df, players_df, summary, A, B, meta
 
 
@@ -242,22 +255,43 @@ def _segment_buffer(n_entries: int, dev):
                        device=dev)
 
 
-def _merge_segments(hist, seg, counters=None, seq=None):
-    """int64 copies of the score histograms, the period histograms `seg` and the scoring-sequence histograms `seq` (each
-    may be None), merged over ranks by ONE `merge_histograms` all-reduce of them laid end to end.  Returns (hist, seg,
-    seq), None where None was given."""
+def _merge_all(counters, *hists):
+    """int64 copies of the integer histograms `hists` (each may be None), merged over ranks by ONE `merge_histograms`
+    all-reduce of them laid end to end.  Returns them in order, None where None was given."""
     import torch
-    parts = [t for t in (hist, seg, seq) if t is not None]
+    parts = [t for t in hists if t is not None]
     flat = torch.cat([t.reshape(-1) for t in parts]).to(torch.int64)
     merge_histograms(flat, counters)
     out, at = [], 0
-    for t in (hist, seg, seq):
+    for t in hists:
         if t is None:
             out.append(None)
             continue
         out.append(flat[at:at + t.numel()].reshape(t.shape))
         at += t.numel()
     return tuple(out)
+
+
+def _merge_segments(hist, seg, counters=None, seq=None):
+    """int64 copies of the score histograms, the period histograms `seg` and the scoring-sequence histograms `seq` (each
+    may be None), merged over ranks by ONE `merge_histograms` all-reduce of them laid end to end.  Returns (hist, seg,
+    seq), None where None was given."""
+    return _merge_all(counters, hist, seg, seq)
+
+
+def _overtime_buffer(n_entries: int, dev):
+    """The kernels' overtime histograms [n_entries][2][OT_MAX_PERIODS + 1][3] (408 B an entry), zeroed."""
+    import torch
+    return torch.zeros((n_entries, 2, outputs.OT_MAX_PERIODS + 1, 3), dtype=torch.int32, device=dev)
+
+
+def _overtime_args(overtime, segments: bool, sequence: bool):
+    """The OvertimeRules of an API call; ValueError when combined with period or sequence outputs (their definitions
+    are for regulation)."""
+    rules = overtime_rules(overtime)
+    if rules is not None and (segments or sequence):
+        raise ValueError("overtime cannot be combined with segments=True or sequence=True")
+    return rules
 
 
 def _sequence_buffer(n_entries: int, dev):
@@ -311,7 +345,7 @@ def simulate_slate(pairs: Sequence[Tuple[str, str]], n: int = 1000, *, sp_path: 
                    year: int = 2025, week: int = 1, seed: Optional[int] = None,
                    engine: Optional[Engine] = None, markets: Optional[Dict[Tuple[str, str], Dict[str, float]]] = None,
                    focus_csv: Optional[str] = None, usage_dir: str = ".", segments: bool = False,
-                   sequence: bool = False):
+                   sequence: bool = False, overtime=False):
     """A whole slate in one launch (BASELINE configs 3-4): every (teamA, teamB) of `pairs` is simulated for
     `n` PAIRS of games (2n games, A receives / B receives alternately, exactly like `simulate_matchup`).
 
@@ -342,9 +376,15 @@ def simulate_slate(pairs: Sequence[Tuple[str, str]], n: int = 1000, *, sp_path: 
     race-to-N parts of `outputs.sequence_odds_from_hist` over BOTH orientations) and "opening_drive" = {receiving team:
     the drive part of `outputs.sequence_odds_from_hist` of the orientation in which that team receives the kickoff}.
     These histograms ride in the same all-reduce too.
+
+    Overtime: `overtime` (False, True or an engine.OvertimeRules) plays games level after regulation to a result under
+    college overtime rules; "hist", "summary", "moneyline" and "markets" then come from the final scores, overtime
+    included, and every pair also returns "overtime" = `outputs.overtime_odds_from_hist` over both orientations (its
+    histogram rides in the same all-reduce).  ValueError with `segments=True` or `sequence=True`.
     """
     import torch
     import torch.distributed as dist
+    rules = _overtime_args(overtime, segments, sequence)
     eng = engine if engine is not None else get_engine()
     sp_df = load_sp_flex(sp_path if sp_path is not None else packaged_priors_path())
     sheet = focus_csv if focus_csv is not None else _usage.FOCUS_PLAYERS_CSV
@@ -374,13 +414,16 @@ def simulate_slate(pairs: Sequence[Tuple[str, str]], n: int = 1000, *, sp_path: 
              if with_players else None)
     seg = _segment_buffer(len(specs), dev) if segments else None
     sq = _sequence_buffer(len(specs), dev) if sequence else None
+    ot = _overtime_buffer(len(specs), dev) if rules is not None else None
     eng.ctx.simulate_device(seed=_fresh_seed() if seed is None else int(seed), hist=hist.data_ptr(),
                             counters=padded.data_ptr(), cuda_stream=st.cuda_stream,
                             player_hist=phist.data_ptr() if phist is not None else 0,
                             segment_hist=seg.data_ptr() if seg is not None else 0,
-                            sequence_hist=sq.data_ptr() if sq is not None else 0)
+                            sequence_hist=sq.data_ptr() if sq is not None else 0,
+                            overtime=rules, ot_hist=ot.data_ptr() if ot is not None else 0)
     counters.copy_(padded[:counters.numel()])
-    hist64, seg64, sq64 = _merge_segments(hist, seg, counters, sq)
+    hist64, seg64, sq64, ot64 = _merge_all(counters, hist, seg, sq, ot)
+    oth = ot64.cpu().numpy() if ot64 is not None else None           # [pairs][2][OT_MAX_PERIODS + 1][3]
     ph = None
     if phist is not None:
         ph64 = phist.to(torch.int64)
@@ -416,6 +459,8 @@ def simulate_slate(pairs: Sequence[Tuple[str, str]], n: int = 1000, *, sp_path: 
                                           for o, t in enumerate((a, b))}
             else:
                 entry["first_score"] = entry["race"] = entry["opening_drive"] = None
+        if oth is not None:
+            entry["overtime"] = outputs.overtime_odds_from_hist(oth[m], a, b) if entry["games"] > 0 else None
         if ph is not None:
             entry["player_hist"] = ph[m]
             entry["usage"] = uses[m]
@@ -552,7 +597,7 @@ def live_game_state(team_a: str, team_b: str, state) -> GameState:
 def simulate_live(entries: Sequence[Tuple[str, str, object]], games: int = 100_000, *, sp_path: Optional[str] = None,
                   year: int = 2025, week: int = 1, seed: Optional[int] = None, engine: Optional[Engine] = None,
                   markets: Optional[Dict[int, Dict[str, float]]] = None, segments: bool = False,
-                  sequence: bool = False) -> List[Dict[str, object]]:
+                  sequence: bool = False, overtime=False) -> List[Dict[str, object]]:
     """Who wins from here?  Every entry (teamA, teamB, state) -- `state` a LiveState (or a mapping with its fields) --
     plays `games` GAMES (not pairs) from its state, all entries in one launch: a win-probability curve (one pair, a state
     per snap) and a live slate (many pairs) alike.  Entries of the same pair share one specialised table set and one memo,
@@ -561,7 +606,8 @@ def simulate_live(entries: Sequence[Tuple[str, str, object]], games: int = 100_0
     Under torch.distributed every rank plays its `shard_range` slice of every entry's games and the integer histograms
     are merged with ONE all-reduce (as in `simulate_slate`); the result does not depend on the number of ranks.
     Returns a list in entry order of dicts: "state", "games", "hist" (the [128, 128] histogram of final (A, B) points,
-    both orientations summed), "p_win" ({teamA: p, teamB: p}), "p_tie" (regulation only, the reference has no overtime),
+    both orientations summed), "p_win" ({teamA: p, teamB: p}), "p_tie" (without overtime the games level at 0:00, as in
+    the reference; with it only those level at the cap of periods),
     "mean_points" ({teamA: x, teamB: y}), "hist_overflow" (games in the last bin: a team with 127 or more points, which
     the odds count as 127), and "markets": for entries whose index is in `markets` ({i: {"spread": s, "total": t}},
     spread from teamA's side) the spread / total odds of `outputs.game_market_odds_from_hist`, else None.
@@ -578,9 +624,16 @@ def simulate_live(entries: Sequence[Tuple[str, str, object]], games: int = 100_0
     Scoring sequence: with `sequence=True` every entry also returns "sequence_hist" ([SEQ_BINS], both orientations
     summed) and, from `outputs.sequence_odds_from_hist` with the state's score as the start score, "next_score" (which
     team scores next and how, or no further score), "drive" (how the drive in progress ends) and "race" (first to
-    10 / 15 / 20 / 25 / 30, targets already reached reported as settled)."""
+    10 / 15 / 20 / 25 / 30, targets already reached reported as settled).
+
+    Overtime: `overtime` (False, True or an engine.OvertimeRules) plays games level after regulation to a result under
+    college overtime rules, also from a state at 0:00 with the score level; "hist", "p_win", "p_tie", "mean_points" and
+    "markets" then come from the final scores, and every entry also returns "overtime" =
+    `outputs.overtime_odds_from_hist` (P(overtime), the 3-way result at the end of regulation, P(win in overtime) per
+    team, the distribution of overtime periods).  ValueError with `segments=True` or `sequence=True`."""
     import torch
     import torch.distributed as dist
+    rules = _overtime_args(overtime, segments, sequence)
     eng = engine if engine is not None else get_engine()
     sp_df = load_sp_flex(sp_path if sp_path is not None else packaged_priors_path())
     entries = list(entries)
@@ -606,14 +659,17 @@ def simulate_live(entries: Sequence[Tuple[str, str, object]], games: int = 100_0
     hist = torch.zeros((len(specs), 2, outputs.HIST_BINS, outputs.HIST_BINS), dtype=torch.int32, device=dev)
     seg = _segment_buffer(len(specs), dev) if segments else None
     sq = _sequence_buffer(len(specs), dev) if sequence else None
+    ot = _overtime_buffer(len(specs), dev) if rules is not None else None
     with _ENGINE_LOCK:
         eng.set_matchups(specs)
         if g1 > g0:
             st = torch.cuda.current_stream(dev)
             eng.ctx.simulate_device(seed=_fresh_seed() if seed is None else int(seed), hist=hist.data_ptr(),
                                     cuda_stream=st.cuda_stream, segment_hist=seg.data_ptr() if seg is not None else 0,
-                                    sequence_hist=sq.data_ptr() if sq is not None else 0)
-    hist64, seg64, sq64 = _merge_segments(hist, seg, None, sq)
+                                    sequence_hist=sq.data_ptr() if sq is not None else 0,
+                                    overtime=rules, ot_hist=ot.data_ptr() if ot is not None else 0)
+    hist64, seg64, sq64, ot64 = _merge_all(None, hist, seg, sq, ot)
+    oth = ot64.cpu().numpy() if ot64 is not None else None
     h = hist64.cpu().numpy()
     sg = seg64.sum(dim=1).cpu().numpy() if seg64 is not None else None      # [entries][N_SEGMENTS][BINS][BINS]
     sqh = sq64.sum(dim=1).cpu().numpy() if sq64 is not None else None       # [entries][SEQ_BINS]
@@ -631,6 +687,8 @@ def simulate_live(entries: Sequence[Tuple[str, str, object]], games: int = 100_0
         if sqh is not None:
             seq = outputs.sequence_odds_from_hist(sqh[m], a, b, start_score=tuple(starts[m].score))
             out[-1].update(sequence_hist=sqh[m], next_score=seq["next_score"], drive=seq["drive"], race=seq["race"])
+        if oth is not None:
+            out[-1]["overtime"] = outputs.overtime_odds_from_hist(oth[m], a, b)
     return out
 
 

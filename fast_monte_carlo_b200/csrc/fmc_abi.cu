@@ -236,8 +236,8 @@ struct fmc_ctx {
     // fmc_simulate_host: device scratch + pinned staging, kept between calls
     struct Scratch { void *dev = nullptr; size_t dev_bytes = 0; };
     // 0..7 fmc_simulate_host's buffers, 8 the period rows of fmc_simulate_segments, 9..10 its host path, 11 the sequence
-    // rows of fmc_simulate_markets, 12..13 its host path
-    Scratch scr[14];
+    // rows of fmc_simulate_markets, 12..13 its host path, 14..15 the host path of fmc_simulate_overtime
+    Scratch scr[16];
     // pinned staging of the large device -> host copies of fmc_simulate_host (two buffers: the DMA of one chunk overlaps
     // the host copy of the previous one into the caller's pageable buffer)
     void *pin[2] = {nullptr, nullptr};
@@ -273,19 +273,19 @@ extern "C" void fmc_destroy(fmc_ctx *c);
 extern "C" const char *fmc_last_error(void) { return g_err.c_str(); }
 extern "C" int fmc_abi_version(void) { return FMC_ABI_VERSION; }
 
-// the dynamic shared memory every instantiation of one hook mask may use
-template <int HOOKS>
+// the dynamic shared memory every instantiation of one hook mask (and overtime rule) may use
+template <int HOOKS, bool OT = false>
 static cudaError_t set_smem_limits() {
     cudaError_t e = cudaSuccess;
     auto set = [&](const void *f, size_t bytes) {
         if (e == cudaSuccess) e = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
     };
-    set((const void *)sim_kernel<false, false, HOOKS>, sim_smem_bytes(false));
-    set((const void *)sim_kernel<true, false, HOOKS>, sim_smem_bytes(false));
-    set((const void *)sim_kernel<false, true, HOOKS>, sim_smem_bytes(true));
-    set((const void *)sim_kernel<true, true, HOOKS>, sim_smem_bytes(true));
-    set((const void *)sim_memo_kernel<false, HOOKS>, sim_memo_smem_bytes());
-    set((const void *)sim_memo_kernel<true, HOOKS>, sim_memo_smem_bytes());
+    set((const void *)sim_kernel<false, false, HOOKS, OT>, sim_smem_bytes(false));
+    set((const void *)sim_kernel<true, false, HOOKS, OT>, sim_smem_bytes(false));
+    set((const void *)sim_kernel<false, true, HOOKS, OT>, sim_smem_bytes(true));
+    set((const void *)sim_kernel<true, true, HOOKS, OT>, sim_smem_bytes(true));
+    set((const void *)sim_memo_kernel<false, HOOKS, OT>, sim_memo_smem_bytes());
+    set((const void *)sim_memo_kernel<true, HOOKS, OT>, sim_memo_smem_bytes());
     return e;
 }
 
@@ -318,6 +318,7 @@ extern "C" int fmc_create(int device, fmc_ctx **out) {
     CKC(set_smem_limits<kHookPeriods>());
     CKC(set_smem_limits<kHookSequence>());
     CKC(set_smem_limits<kHookPeriods | kHookSequence>());
+    CKC((set_smem_limits<0, true>()));      // overtime (fmc_simulate_overtime)
     CKC(cudaEventCreateWithFlags(&c->ev_done, cudaEventDisableTiming));
     CKC(cudaMalloc(&c->d_pred_stats, 16));
     CKC(cudaMemset(c->d_pred_stats, 0, 16));
@@ -860,19 +861,19 @@ static size_t memo_layout(fmc_ctx *c, uint64_t games, MemoRegion (&R)[kMemoFams]
 static cudaError_t scratch(fmc_ctx *c, int slot, size_t bytes, void **out);
 
 // The kernel of a launch: player mode, the memo kernel or the plain one; injected draws / traces (TEST); the hooks of
-// the optional outputs (HOOKS).
-template <int HOOKS>
+// the optional outputs (HOOKS); overtime (OT).
+template <int HOOKS, bool OT = false>
 static void launch_sim(const SimKernelArgs &a, const MemoArgs *mm, bool players, bool test, int grid, int mgrid, size_t smem,
                        cudaStream_t st) {
     if (players) {
-        if (test) sim_kernel<true, true, HOOKS><<<grid, kSimThreads, smem, st>>>(a);
-        else sim_kernel<false, true, HOOKS><<<grid, kSimThreads, smem, st>>>(a);
+        if (test) sim_kernel<true, true, HOOKS, OT><<<grid, kSimThreads, smem, st>>>(a);
+        else sim_kernel<false, true, HOOKS, OT><<<grid, kSimThreads, smem, st>>>(a);
     } else if (mm) {
-        if (test) sim_memo_kernel<true, HOOKS><<<mgrid, kMemoThreads, sim_memo_smem_bytes(), st>>>(a, *mm);
-        else sim_memo_kernel<false, HOOKS><<<mgrid, kMemoThreads, sim_memo_smem_bytes(), st>>>(a, *mm);
+        if (test) sim_memo_kernel<true, HOOKS, OT><<<mgrid, kMemoThreads, sim_memo_smem_bytes(), st>>>(a, *mm);
+        else sim_memo_kernel<false, HOOKS, OT><<<mgrid, kMemoThreads, sim_memo_smem_bytes(), st>>>(a, *mm);
     } else {
-        if (test) sim_kernel<true, false, HOOKS><<<grid, kSimThreads, sim_smem_bytes(false), st>>>(a);
-        else sim_kernel<false, false, HOOKS><<<grid, kSimThreads, sim_smem_bytes(false), st>>>(a);
+        if (test) sim_kernel<true, false, HOOKS, OT><<<grid, kSimThreads, sim_smem_bytes(false), st>>>(a);
+        else sim_kernel<false, false, HOOKS, OT><<<grid, kSimThreads, sim_smem_bytes(false), st>>>(a);
     }
 }
 
@@ -885,9 +886,18 @@ static int hook_rows(fmc_ctx *c, int slot, uint64_t out_games, int words, uint32
     return FMC_OK;
 }
 
-// Every simulation entry point: seg / seq may be NULL or hold only NULL pointers.
-static int simulate_impl(fmc_ctx *c, const fmc_sim_args *g, const fmc_segment_args *seg, const fmc_sequence_args *seq) {
+// Every simulation entry point: seg / seq may be NULL or hold only NULL pointers; ot NULL is the reference's end at 0:00.
+static int simulate_impl(fmc_ctx *c, const fmc_sim_args *g, const fmc_segment_args *seg, const fmc_sequence_args *seq,
+                         const fmc_overtime_args *ot) {
     if (!c || !g) return fail(FMC_ERR_INVALID, "fmc_simulate: bad argument");
+    if (ot) {
+        if (ot->max_periods < 1 || ot->max_periods > FMC_OT_MAX_PERIODS)
+            return fail(FMC_ERR_INVALID, "fmc_simulate_overtime: max_periods must be 1.." + std::to_string(FMC_OT_MAX_PERIODS));
+        if (ot->snap_clock < 1 || ot->snap_clock > 900)
+            return fail(FMC_ERR_INVALID, "fmc_simulate_overtime: snap_clock must be 1..900");
+        if ((seg && (seg->period_scores_dev || seg->segment_hist_dev)) || (seq && (seq->sequence_dev || seq->sequence_hist_dev)))
+            return fail(FMC_ERR_INVALID, "fmc_simulate_overtime: overtime has no period or sequence outputs");
+    }
     CK(cudaSetDevice(c->device));
     settle_usage(c);
     if (c->tables_dirty) {
@@ -935,6 +945,10 @@ static int simulate_impl(fmc_ctx *c, const fmc_sim_args *g, const fmc_segment_ar
     a.stream = g->stream_dev; a.trace = g->trace_dev; a.iters = g->iters_dev;
     a.period_scores = rows; a.segment_hist = segs ? seg->segment_hist_dev : nullptr;
     a.sequence = seq_rows; a.sequence_hist = seqs ? seq->sequence_hist_dev : nullptr;
+    if (ot) {
+        a.ot_max_periods = ot->max_periods; a.ot_snap_clock = ot->snap_clock;
+        a.ot_periods = ot->ot_periods_dev; a.ot_hist = ot->ot_hist_dev;
+    }
     const bool players = !c->usage.empty();
     if ((g->players_dev || g->player_hist_dev) && !players)
         return fail(FMC_ERR_INVALID, "fmc_simulate: players_dev / player_hist_dev need fmc_set_usage");
@@ -980,7 +994,8 @@ static int simulate_impl(fmc_ctx *c, const fmc_sim_args *g, const fmc_segment_ar
     }
     const int mgrid = c->prop.multiProcessorCount * kMemoCtasPerSm;
     const MemoArgs *mp = memo ? &mm : nullptr;
-    switch ((segs ? kHookPeriods : 0) | (seqs ? kHookSequence : 0)) {
+    if (ot) launch_sim<0, true>(a, mp, players, test, grid, mgrid, smem, st);
+    else switch ((segs ? kHookPeriods : 0) | (seqs ? kHookSequence : 0)) {
     case 0: launch_sim<0>(a, mp, players, test, grid, mgrid, smem, st); break;
     case kHookPeriods: launch_sim<kHookPeriods>(a, mp, players, test, grid, mgrid, smem, st); break;
     case kHookSequence: launch_sim<kHookSequence>(a, mp, players, test, grid, mgrid, smem, st); break;
@@ -992,14 +1007,18 @@ static int simulate_impl(fmc_ctx *c, const fmc_sim_args *g, const fmc_segment_ar
     return FMC_OK;
 }
 
-extern "C" int fmc_simulate(fmc_ctx *c, const fmc_sim_args *g) { return simulate_impl(c, g, nullptr, nullptr); }
+extern "C" int fmc_simulate(fmc_ctx *c, const fmc_sim_args *g) { return simulate_impl(c, g, nullptr, nullptr, nullptr); }
 
 extern "C" int fmc_simulate_segments(fmc_ctx *c, const fmc_sim_args *g, const fmc_segment_args *seg) {
-    return simulate_impl(c, g, seg, nullptr);
+    return simulate_impl(c, g, seg, nullptr, nullptr);
 }
 
 extern "C" int fmc_simulate_markets(fmc_ctx *c, const fmc_sim_args *g, const fmc_segment_args *seg, const fmc_sequence_args *seq) {
-    return simulate_impl(c, g, seg, seq);
+    return simulate_impl(c, g, seg, seq, nullptr);
+}
+
+extern "C" int fmc_simulate_overtime(fmc_ctx *c, const fmc_sim_args *g, const fmc_overtime_args *ot) {
+    return simulate_impl(c, g, nullptr, nullptr, ot);
 }
 
 // Device scratch of fmc_simulate_host, kept in the context between calls (grow-only): no cudaMalloc / cudaFree per call.
@@ -1049,7 +1068,8 @@ static cudaError_t d2h_staged(fmc_ctx *c, void *dst, const void *src, size_t byt
 static int simulate_host_impl(fmc_ctx *c, uint64_t seed, uint32_t *scores_host, uint32_t *hist_host,
                               uint64_t *counters_host, const double *stream_host, double *trace_host,
                               uint16_t *iters_host, fmc_player_rec *players_host, uint32_t *player_hist_host,
-                              uint32_t *period_host, uint32_t *seg_hist_host, uint32_t *seq_host, uint32_t *seq_hist_host) {
+                              uint32_t *period_host, uint32_t *seg_hist_host, uint32_t *seq_host, uint32_t *seq_hist_host,
+                              const fmc_overtime_args *ot_host = nullptr) {
     if (!c) return fail(FMC_ERR_INVALID, "ctx is NULL");
     if (c->matchups.empty()) return fail(FMC_ERR_INVALID, "fmc_set_matchups has not been called");
     CK(cudaSetDevice(c->device));
@@ -1071,6 +1091,9 @@ static int simulate_host_impl(fmc_ctx *c, uint64_t seed, uint32_t *scores_host, 
     uint32_t *d_phist = nullptr, *d_period = nullptr, *d_seg = nullptr, *d_seq = nullptr, *d_seqh = nullptr;
     const size_t seg_n = nm * 2 * FMC_N_SEGMENTS * FMC_HIST_BINS * FMC_HIST_BINS;
     const size_t seqh_n = nm * 2 * FMC_SEQ_BINS;
+    const size_t oth_n = nm * 2 * (FMC_OT_MAX_PERIODS + 1) * 3;
+    uint8_t *d_otp = nullptr;
+    uint32_t *d_oth = nullptr;
     const size_t phist_n = c->matchups.size() * 2 * (size_t)c->n_slots * FMC_PH_BINS;
     int rc = FMC_OK;
     cudaError_t e = cudaSuccess;
@@ -1117,6 +1140,13 @@ static int simulate_host_impl(fmc_ctx *c, uint64_t seed, uint32_t *scores_host, 
             if ((e = scratch(c, 13, seqh_n * 4, (void **)&d_seqh)) != cudaSuccess) { bail(e, "cudaMalloc sequence hist"); break; }
             if ((e = cudaMemsetAsync(d_seqh, 0, seqh_n * 4)) != cudaSuccess) { bail(e, "memset sequence hist"); break; }
         }
+        if (ot_host && ot_host->ot_periods_dev && games) {
+            if ((e = scratch(c, 14, games, (void **)&d_otp)) != cudaSuccess) { bail(e, "cudaMalloc overtime periods"); break; }
+        }
+        if (ot_host && ot_host->ot_hist_dev) {
+            if ((e = scratch(c, 15, oth_n * 4, (void **)&d_oth)) != cudaSuccess) { bail(e, "cudaMalloc overtime hist"); break; }
+            if ((e = cudaMemsetAsync(d_oth, 0, oth_n * 4)) != cudaSuccess) { bail(e, "memset overtime hist"); break; }
+        }
         fmc_sim_args g;
         std::memset(&g, 0, sizeof(g));
         g.player_hist_dev = d_phist;
@@ -1127,7 +1157,9 @@ static int simulate_host_impl(fmc_ctx *c, uint64_t seed, uint32_t *scores_host, 
         sg.period_scores_dev = d_period; sg.segment_hist_dev = d_seg;
         fmc_sequence_args sq;
         sq.sequence_dev = d_seq; sq.sequence_hist_dev = d_seqh;
-        rc = simulate_impl(c, &g, &sg, &sq);
+        fmc_overtime_args ov;
+        if (ot_host) { ov = *ot_host; ov.ot_periods_dev = d_otp; ov.ot_hist_dev = d_oth; }
+        rc = simulate_impl(c, &g, &sg, &sq, ot_host ? &ov : nullptr);
         if (rc) break;
         if ((e = cudaDeviceSynchronize()) != cudaSuccess) { bail(e, "sim_kernel"); break; }
         if (scores_host && games && (e = d2h_staged(c, scores_host, d_scores, games * 4)) != cudaSuccess) { bail(e, "D2H scores"); break; }
@@ -1141,6 +1173,8 @@ static int simulate_host_impl(fmc_ctx *c, uint64_t seed, uint32_t *scores_host, 
         if (d_seg && (e = cudaMemcpy(seg_hist_host, d_seg, seg_n * 4, cudaMemcpyDeviceToHost)) != cudaSuccess) { bail(e, "D2H segment hist"); break; }
         if (d_seq && (e = d2h_staged(c, seq_host, d_seq, games * 2 * 4)) != cudaSuccess) { bail(e, "D2H sequence"); break; }
         if (d_seqh && (e = cudaMemcpy(seq_hist_host, d_seqh, seqh_n * 4, cudaMemcpyDeviceToHost)) != cudaSuccess) { bail(e, "D2H sequence hist"); break; }
+        if (d_otp && (e = cudaMemcpy(ot_host->ot_periods_dev, d_otp, games, cudaMemcpyDeviceToHost)) != cudaSuccess) { bail(e, "D2H overtime periods"); break; }
+        if (d_oth && (e = cudaMemcpy(ot_host->ot_hist_dev, d_oth, oth_n * 4, cudaMemcpyDeviceToHost)) != cudaSuccess) { bail(e, "D2H overtime hist"); break; }
     } while (0);
     // big test-mode buffers (injected draws, traces: 46 KB per game) are not worth keeping
     for (int slot : {3, 4})
@@ -1177,6 +1211,16 @@ extern "C" int fmc_simulate_markets_host(fmc_ctx *c, uint64_t seed, uint32_t *sc
                                          uint32_t *sequence_hist_host) {
     return simulate_host_impl(c, seed, scores_host, hist_host, counters_host, stream_host, trace_host, iters_host, players_host,
                               player_hist_host, period_scores_host, segment_hist_host, sequence_host, sequence_hist_host);
+}
+
+extern "C" int fmc_simulate_overtime_host(fmc_ctx *c, uint64_t seed, uint32_t *scores_host, uint32_t *hist_host,
+                                          uint64_t *counters_host, const double *stream_host, double *trace_host,
+                                          uint16_t *iters_host, fmc_player_rec *players_host, uint32_t *player_hist_host,
+                                          int32_t max_periods, int32_t snap_clock, uint8_t *ot_periods_host, uint32_t *ot_hist_host) {
+    // host pointers in the device fields: simulate_host_impl stages them through device scratch
+    const fmc_overtime_args ot{max_periods, snap_clock, ot_periods_host, ot_hist_host};
+    return simulate_host_impl(c, seed, scores_host, hist_host, counters_host, stream_host, trace_host, iters_host, players_host,
+                              player_hist_host, nullptr, nullptr, nullptr, nullptr, &ot);
 }
 
 extern "C" int fmc_tree_predict(fmc_ctx *c, int32_t id, const double *rows_dev, int64_t n, double *out_dev,

@@ -24,6 +24,8 @@
 // trip loop of sim_memo_kernel (fmc_sim_memo.cuh) both call them: a rule is changed in one place for both kernels.
 #pragma once
 
+#include <type_traits>
+
 #include "fmc_device.cuh"
 #include "fmc_pack.hpp"
 
@@ -125,6 +127,11 @@ struct SimKernelArgs {
     // optional per-entry histogram
     uint32_t *sequence;                // [games][2]
     uint32_t *sequence_hist;           // [n_matchups][2][FMC_SEQ_BINS]
+    // overtime (fmc_simulate_overtime; read only by the instantiations with overtime): the rules' two parameters and the
+    // optional outputs
+    int ot_max_periods, ot_snap_clock;
+    uint8_t *ot_periods;               // [games]
+    uint32_t *ot_hist;                 // [n_matchups][2][FMC_OT_MAX_PERIODS + 1][3]
 };
 
 enum Stage : int {
@@ -145,35 +152,54 @@ struct Lane {
     int p1, wr;                // player mode: usage entries sampled for the current play (passer | rusher, target)
     int home;                  // index of the running player box this game (and its successors) accumulates in
 };
+// The lane of the instantiations with overtime: the overtime state (Overtime<true>), 0 in regulation.  A type of its own so
+// that the lane of every other instantiation keeps its layout.
+struct OtLane : Lane {
+    int ot;
+};
+template <bool OT> using LaneT = typename std::conditional<OT, OtLane, Lane>::type;
 
 // A game's state between rounds: nine registers instead of sixteen, so that the tree walk (which runs with
 // every lane's game parked) has room for its eight gather chains.
 struct PackedLane {
     unsigned long long game;
     double dist, ytg;
-    uint32_t a;     // sec:12 | down:10 | period:3 | offense:1 | going:1 | stage:4
+    uint32_t a;     // sec:12 | down:10 | period:3 | offense:1 | going:1 | stage:4 | overtime:1
     uint32_t b;     // iter:10 | plays:10 | p1:5 | wr:5 (player mode)
     uint32_t c;     // score[0]:16 | score[1]:16
 };
-__device__ __forceinline__ PackedLane pack_lane(const Lane &L) {
+// OT: the instantiations with overtime.  In overtime the clock does not run: every snap is played at the snap clock of
+// the launch, so the sec field holds the overtime state instead (bit 31 set) and unpacking restores the clock from a.
+template <bool OT = false>
+__device__ __forceinline__ PackedLane pack_lane(const LaneT<OT> &L) {
     PackedLane P;
     P.game = L.game; P.dist = L.dist; P.ytg = L.ytg;
     P.a = (uint32_t)L.sec | ((uint32_t)L.down << 12) | ((uint32_t)L.period << 22) | ((uint32_t)L.offense << 25) |
           ((uint32_t)L.going << 26) | ((uint32_t)L.stage << 27);
+    if constexpr (OT) {
+        if (L.ot) P.a = (P.a & ~0xFFFu) | (uint32_t)L.ot | 0x80000000u;
+    }
     P.b = (uint32_t)L.iter | ((uint32_t)L.plays << 10) | ((uint32_t)L.p1 << 20) | ((uint32_t)L.wr << 25);
     P.c = (uint32_t)L.score[0] | ((uint32_t)L.score[1] << 16);
     return P;
 }
-__device__ __forceinline__ Lane unpack_lane(const PackedLane &P) {
-    Lane L;
+template <bool OT = false>
+__device__ __forceinline__ LaneT<OT> unpack_lane(const PackedLane &P, const SimKernelArgs &a) {
+    LaneT<OT> L;
     L.game = P.game; L.dist = P.dist; L.ytg = P.ytg;
     L.sec = (int)(P.a & 0xFFFu); L.down = (int)((P.a >> 12) & 0x3FFu); L.period = (int)((P.a >> 22) & 7u);
     L.offense = (int)((P.a >> 25) & 1u); L.going = (int)((P.a >> 26) & 1u); L.stage = (int)(P.a >> 27);
     L.iter = (int)(P.b & 0x3FFu); L.plays = (int)((P.b >> 10) & 0x3FFu);
     L.p1 = (int)((P.b >> 20) & 0x1Fu); L.wr = (int)((P.b >> 25) & 0x1Fu);
     L.score[0] = (int)(P.c & 0xFFFFu); L.score[1] = (int)(P.c >> 16);
+    if constexpr (OT) {
+        L.stage &= 15;
+        L.ot = 0;
+        if (P.a >> 31) { L.ot = L.sec; L.sec = a.ot_snap_clock; }
+    }
     return L;
 }
+// (a lane gets a new stage this way only between matchups, without a game: the overtime bit is cleared with the stage)
 __device__ __forceinline__ void set_stage(PackedLane &P, int stage) { P.a = (P.a & 0x07FFFFFFu) | ((uint32_t)stage << 27); }
 // the state of a lane without a game
 __device__ __forceinline__ PackedLane idle_lane() {
@@ -374,15 +400,111 @@ template <> struct Sequence<true> {
     }
 };
 
+// ---- overtime (fmc_simulate_overtime, include/fmc.h FMC_OT_MAX_PERIODS) ------------------------------------------------
+// The rule that plays a game level at the end of regulation to a result.  Overtime<false> is the reference's end of the
+// game at 0:00.  Overtime<true> keeps its state in OtLane::ot: the period k (1..FMC_OT_MAX_PERIODS), whether the second
+// possession of the period is on, whether the snap is a two-point try, and a period-2 touchdown whose try is still due.
+// The team with the first possession of period k is (g & 1) in period 1 and alternates; a possession ends when the
+// offense changes (every place that calls change_possession) or, for a try, after its one snap.  All bookkeeping runs at
+// the start of an iteration (over), before the trace row, except the points of a touchdown, which after_yards adds.
+enum : int { kOtPeriod = 31, kOtSecond = 32, kOtTry = 64, kOtTd = 128 };
+
+template <bool OT> struct Overtime;
+template <> struct Overtime<false> {
+    __device__ __forceinline__ Overtime(const SimKernelArgs &, int) {}
+    __device__ __forceinline__ void game_start(const Lane &) const {}
+    // the game is over at the start of an iteration
+    __device__ __forceinline__ bool over(const Lane &L) const { return L.sec <= 0; }
+    // points of a touchdown just scored
+    __device__ __forceinline__ int touchdown(const Lane &) const { return 7; }
+    // the snap credits player box lines
+    __device__ __forceinline__ bool credits(const Lane &) const { return true; }
+    __device__ __forceinline__ void game_end(const Lane &, unsigned long long *, size_t) const {}
+};
+template <> struct Overtime<true> {
+    const SimKernelArgs &a;
+    int matchup;
+    __device__ __forceinline__ Overtime(const SimKernelArgs &a_, int m) : a(a_), matchup(m) {}
+    // the step functions see a Lane; the lanes of these instantiations are OtLanes
+    __device__ __forceinline__ static int &st(Lane &L) { return static_cast<OtLane &>(L).ot; }
+    __device__ __forceinline__ static int st(const Lane &L) { return static_cast<const OtLane &>(L).ot; }
+    __device__ __forceinline__ void game_start(Lane &L) const { st(L) = 0; }
+    // the team whose possession is on
+    __device__ __forceinline__ static int team(const Lane &L) {
+        const int o = st(L);
+        return (int)(L.game & 1ULL) ^ (((o & kOtPeriod) - 1) & 1) ^ ((o & kOtSecond) ? 1 : 0);
+    }
+    __device__ __forceinline__ static void two_point_try(Lane &L) {
+        st(L) |= kOtTry;
+        L.down = 1; L.dist = 3.0; L.ytg = 3.0; L.going = 0;
+    }
+    // the possession the state names starts: 1st & 10 at the opponent's 25 in periods 1 and 2, a two-point try from period 3
+    __device__ __forceinline__ static void possession(Lane &L) {
+        L.offense = team(L);
+        if ((st(L) & kOtPeriod) >= 3) two_point_try(L);
+        else { L.down = 1; L.dist = 10.0; L.ytg = 25.0; L.going = 0; }
+    }
+    __device__ __forceinline__ bool over(Lane &L) const {
+        int &o = st(L);
+        if (o == 0) {
+            if (L.sec > 0) return false;
+            if (L.score[0] != L.score[1]) return true;
+            o = 1;                                             // level at 0:00: period 1, first possession
+            possession(L);
+        } else {
+            const int t = team(L), k = o & kOtPeriod;
+            if (o & kOtTd) {                                   // a period-2 touchdown: its try, unless it already won
+                if ((o & kOtSecond) && L.score[t] > L.score[t ^ 1]) return true;
+                o &= ~kOtTd;
+                L.offense = t;
+                two_point_try(L);
+            } else if ((o & kOtTry) || L.offense != t) {      // the possession is over
+                if (!(o & kOtSecond)) o = k | kOtSecond;
+                else if (L.score[0] != L.score[1] || k >= a.ot_max_periods) return true;
+                else o = k + 1;
+                possession(L);
+            }
+        }
+        if (L.iter >= FMC_MAX_ITERS) return true;
+        L.sec = a.ot_snap_clock;
+        return false;
+    }
+    __device__ __forceinline__ int touchdown(Lane &L) const {
+        int &o = st(L);
+        if (o & kOtTry) return 2;
+        if ((o & kOtPeriod) == 2) { o |= kOtTd; return 6; }
+        return 7;
+    }
+    __device__ __forceinline__ bool credits(const Lane &L) const { return !(st(L) & kOtTry); }
+    // periods played to the per-game output, the game to the overtime histogram and counters
+    __device__ __forceinline__ void game_end(const Lane &L, unsigned long long *stat, size_t oi) const {
+        const int k = st(L) & kOtPeriod;
+        if (a.ot_periods) a.ot_periods[oi] = (uint8_t)k;
+        if (a.ot_hist) {
+            const int r = L.score[0] > L.score[1] ? FMC_OT_A : (L.score[1] > L.score[0] ? FMC_OT_B : FMC_OT_LEVEL);
+            atomicAdd(a.ot_hist + (((size_t)matchup * 2 + (L.game & 1ULL)) * (FMC_OT_MAX_PERIODS + 1) + k) * 3 + r, 1u);
+        }
+        if (k) {
+            atomicAdd(&stat[FMC_C_OT_GAMES], 1ULL);
+            atomicAdd(&stat[FMC_C_OT_PERIODS], (unsigned long long)k);
+        }
+    }
+};
+
 // The hook policy of the step functions: HOOKS is a mask of the launch's optional outputs.  Hooks<0> compiles to the code
-// without hooks; kOn says whether any hook is in (a hooked field goal adds its points before its tick).
+// without hooks; kOn says whether any hook is in (a hooked field goal adds its points before its tick).  OT: the overtime
+// rule, instantiated with HOOKS = 0 only.  Overtime<OT> is a base, so that Hooks<HOOKS, false> keeps the layout it had
+// before overtime existed (an empty member would not).
 enum { kHookPeriods = 1, kHookSequence = 2 };
-template <int HOOKS>
-struct Hooks {
+template <int HOOKS, bool OT = false>
+struct Hooks : Overtime<OT> {
+    static_assert(!(OT && HOOKS), "overtime has no period or sequence outputs");
     static constexpr bool kOn = HOOKS != 0;
     Periods<(HOOKS & kHookPeriods) != 0> per;
     Sequence<(HOOKS & kHookSequence) != 0> seq;
-    __device__ __forceinline__ Hooks(const SimKernelArgs &a, const MatchupDev &M, int m) : per(a, M, m), seq(a, M, m) {}
+    __device__ __forceinline__ Hooks(const SimKernelArgs &a, const MatchupDev &M, int m)
+        : Overtime<OT>(a, m), per(a, M, m), seq(a, M, m) {}
+    __device__ __forceinline__ const Overtime<OT> &ot() const { return *this; }
     __device__ __forceinline__ void game_start(const Lane &L) const { seq.game_start(L); }
     // quarter q ended with the play snapped at `snap`; the end of the half ends the drive if nothing else did
     __device__ __forceinline__ void quarter_end(const Lane &L, int q, int snap) const {
@@ -679,6 +801,7 @@ __device__ __forceinline__ unsigned int end_game_record(const Lane &L, const Sim
                   &stat[FMC_C_PH_OVERFLOW]);
     }
     pk.game_end(L);
+    pk.ot().game_end(L, stat, oi);
     ev.hit(EV_GAMES);
     return (unsigned int)(((L.game & 1ULL) * FMC_HIST_BINS + ha) * FMC_HIST_BINS + hb);
 }
@@ -741,9 +864,9 @@ __device__ __forceinline__ bool fourth_down(Lane &L, Draws<TEST> &D, int sd, Ev 
 // The play call from P(pass) (FMC:1058-1075, 1203-1208; P(run) after the two normalisations of FMC:1064-1066).  Returns
 // the stage the play waits at.  Player mode samples the passer and target (credits the target) or the rusher (credits
 // the carry).
-template <bool TEST, bool PLAYERS, class Ev>
+template <bool TEST, bool PLAYERS, class Ev, class Pk>
 __device__ __forceinline__ int call_play(Lane &L, const SimKernelArgs &a, const MatchupDev &M, Draws<TEST> &D, int team,
-                                         double p_pass, Ev &ev) {
+                                         double p_pass, Ev &ev, const Pk &pk) {
     double a0 = 1.0 - p_pass, a1 = p_pass;
     const double s = a0 + a1;
     a0 = a0 / s; a1 = a1 / s;
@@ -753,7 +876,7 @@ __device__ __forceinline__ int call_play(Lane &L, const SimKernelArgs &a, const 
         if (PLAYERS) {
             L.p1 = sample_usage(M.usage[team], 1, D.u(S_U_P1));
             L.wr = 0;
-            credit(a, M, L, team, 1, L.p1, PC_ATT, false, 0.0);
+            if (pk.ot().credits(L)) credit(a, M, L, team, 1, L.p1, PC_ATT, false, 0.0);
         }
         return ST_WAIT_RQ;
     }
@@ -761,18 +884,19 @@ __device__ __forceinline__ int call_play(Lane &L, const SimKernelArgs &a, const 
     if (PLAYERS) {
         L.p1 = sample_usage(M.usage[team], 0, D.u(S_U_P1));
         L.wr = sample_usage(M.usage[team], 2, D.u(S_U_WR));
-        credit(a, M, L, team, 2, L.wr, PC_ATT, false, 0.0);
+        if (pk.ot().credits(L)) credit(a, M, L, team, 2, L.wr, PC_ATT, false, 0.0);
     }
     return ST_WAIT_S1;
 }
 
 // A play starts (simulate_play FMC:1026-...).  Returns the stage it waits at: the play model's margins (policy 1), or
 // the model of the play called with the heuristic P(pass).
-template <bool TEST, bool PLAYERS, class Ev>
-__device__ __forceinline__ int start_play(Lane &L, const SimKernelArgs &a, const MatchupDev &M, Draws<TEST> &D, int sd, Ev &ev) {
+template <bool TEST, bool PLAYERS, class Ev, class Pk>
+__device__ __forceinline__ int start_play(Lane &L, const SimKernelArgs &a, const MatchupDev &M, Draws<TEST> &D, int sd, Ev &ev,
+                                          const Pk &pk) {
     L.plays += 1;
     if (a.policy == 1) return ST_WAIT_PM;
-    return call_play<TEST, PLAYERS>(L, a, M, D, L.offense, pass_prob_v1(L.down, L.dist, L.ytg, L.sec, sd), ev);
+    return call_play<TEST, PLAYERS>(L, a, M, D, L.offense, pass_prob_v1(L.down, L.dist, L.ytg, L.sec, sd), ev, pk);
 }
 
 // P(pass) from the play model's nc margins m (FMC:420-425): float32 softmax of m / T, clipped to [.02, .98]
@@ -819,17 +943,17 @@ __device__ __forceinline__ void after_stage2(Lane &L, const SimKernelArgs &a, co
     const int outcome = stage2_outcome(raw, D.u(S_U_S2));
     if (outcome == 0) {                                   // incomplete FMC:1160-1168
         ev.hit(EV_INC);
-        if (PLAYERS) credit(a, M, L, team, 0, L.p1, PC_ATT, false, 0.0);
+        if (PLAYERS && pk.ot().credits(L)) credit(a, M, L, team, 0, L.p1, PC_ATT, false, 0.0);
         L.down += 1; L.going = 0;
         tick_clock(L, 10, pk);
         L.stage = ST_ITER;
     } else if (outcome == 2) {                            // sack FMC:1170-1174
         ev.hit(EV_SACK);
-        if (PLAYERS) credit(a, M, L, team, 0, L.p1, PC_SACK, false, 0.0);
+        if (PLAYERS && pk.ot().credits(L)) credit(a, M, L, team, 0, L.p1, PC_SACK, false, 0.0);
         L.stage = ST_WAIT_SQ;
     } else {                                              // intercepted FMC:1186-1199
         ev.hit(EV_INT);
-        if (PLAYERS) credit(a, M, L, team, 0, L.p1, PC_ATT | PC_INT, false, 0.0);
+        if (PLAYERS && pk.ot().credits(L)) credit(a, M, L, team, 0, L.p1, PC_ATT | PC_INT, false, 0.0);
         const double ret = softclip(6.0 + 5.0 * D.z(S_Z_INT), 0.0, L.ytg);
         const double spot = 100.0 - (L.ytg - ret);
         L.going = 0;
@@ -864,7 +988,7 @@ __device__ __forceinline__ void after_yards(Lane &L, const SimKernelArgs &a, con
             if (D.u(S_U_FIN) < rz_finish_prob(ytg0, M.tanh35[team], L.down, pass)) yards = ytg0;
         }
         const bool td = yards + 1e-9 >= ytg0;
-        if (PLAYERS) {                  // FMC:1108-1127, 1140-1145 (pass), 1232-1234, 1246-1247 (run)
+        if (PLAYERS && pk.ot().credits(L)) {      // FMC:1108-1127, 1140-1145 (pass), 1232-1234, 1246-1247 (run)
             const double y = td ? ytg0 : yards;
             const unsigned long long c_td = td ? PC_TD : 0ULL;
             if (pass) {
@@ -876,7 +1000,7 @@ __device__ __forceinline__ void after_yards(Lane &L, const SimKernelArgs &a, con
         }
         if (td) {
             ev.hit(EV_TD);
-            L.score[team] += 7; L.going = 0;
+            L.score[team] += pk.ot().touchdown(L); L.going = 0;
             pk.scored(L, team, FMC_SEQ_TD, L.sec);
             pk.drive_end(L, FMC_DRIVE_TD, L.sec);
             tick_clock(L, pass ? 20 : 28, pk);
@@ -893,12 +1017,12 @@ __device__ __forceinline__ void after_yards(Lane &L, const SimKernelArgs &a, con
 
 // Advance one lane until it posts a request (returns its key, family * 2 + offense) or has nothing
 // left to do (returns -1).  `res` points at this lane's result record of the previous round.
-template <bool TEST, bool PLAYERS, int HOOKS>
-__device__ __forceinline__ int advance_lane(Lane &L, const SimKernelArgs &a, SimShared &sh, const double *res) {
+template <bool TEST, bool PLAYERS, int HOOKS, bool OT>
+__device__ __forceinline__ int advance_lane(LaneT<OT> &L, const SimKernelArgs &a, SimShared &sh, const double *res) {
     const MatchupDev &M = sh.M;
     const int matchup = sh.cur_matchup;
     StatEvents ev{sh.stat};
-    const Hooks<HOOKS> pk(a, M, matchup);
+    const Hooks<HOOKS, OT> pk(a, M, matchup);
     for (;;) {
         if (L.stage == ST_IDLE) return -1;
         if (L.stage == ST_NEED_GAME) {
@@ -906,9 +1030,12 @@ __device__ __forceinline__ int advance_lane(Lane &L, const SimKernelArgs &a, Sim
             if (g >= M.game_end) { L.stage = ST_IDLE; return -1; }
             new_game(L, M, g);
             pk.game_start(L);
+            pk.ot().game_start(L);
         }
         if (L.stage == ST_ITER) {
-            if (L.sec <= 0) {
+            // (the instantiations without overtime keep the clock test of their own: calling Overtime<false>::over here, inline
+            // as it is, reorders the code of those with the sequence hooks)
+            if (OT ? pk.ot().over(L) : L.sec <= 0) {
                 const unsigned int bin = end_game_record<PLAYERS>(L, a, M, matchup, sh.stat, ev, pk);
                 if (a.hist) atomicAdd(&a.hist[(size_t)matchup * 2 * FMC_HIST_BINS * FMC_HIST_BINS + bin], 1u);
                 atomicAdd(&sh.stat[FMC_C_PLAYS], (unsigned long long)L.plays);
@@ -921,7 +1048,7 @@ __device__ __forceinline__ int advance_lane(Lane &L, const SimKernelArgs &a, Sim
             L.iter += 1;
             const int sd = L.score[L.offense] - L.score[L.offense ^ 1];
             if (!fourth_down(L, D, sd, ev, pk)) continue;
-            L.stage = start_play<TEST, PLAYERS>(L, a, M, D, sd, ev);
+            L.stage = start_play<TEST, PLAYERS>(L, a, M, D, sd, ev, pk);
             return request_key(L);
         }
         // ---- resuming a parked play: the iteration counter already points past this iteration
@@ -931,7 +1058,7 @@ __device__ __forceinline__ int advance_lane(Lane &L, const SimKernelArgs &a, Sim
         const int team = L.offense;
         const float *mg = reinterpret_cast<const float *>(res);
         if (L.stage == ST_WAIT_PM) {
-            L.stage = call_play<TEST, PLAYERS>(L, a, M, D, team, p_pass_from_play_model(mg, M.tbl[5][team].n_outputs, a), ev);
+            L.stage = call_play<TEST, PLAYERS>(L, a, M, D, team, p_pass_from_play_model(mg, M.tbl[5][team].n_outputs, a), ev, pk);
             return request_key(L);
         }
         if (L.stage == ST_WAIT_S1 && !after_stage1(L, a, M, D, team, mg[0], ev)) return request_key(L);
@@ -1144,8 +1271,9 @@ __device__ __forceinline__ void walk_requests(RoundShared &sh, const SimKernelAr
 // more feature rows, tracked names get per-game box lines.  The shipped configuration (every name "Unknown")
 // runs the PLAYERS = false instantiation, which carries none of it.  HOOKS: the optional outputs of the launch
 // (kHookPeriods: fmc_simulate_segments, Periods<true>; kHookSequence: fmc_simulate_markets, Sequence<true>); the
-// HOOKS = 0 instantiations are the code without the hooks.
-template <bool TEST, bool PLAYERS, int HOOKS>
+// HOOKS = 0 instantiations are the code without the hooks.  OT: overtime (fmc_simulate_overtime, Overtime<true>), with
+// HOOKS = 0 only.
+template <bool TEST, bool PLAYERS, int HOOKS, bool OT = false>
 __global__ void __launch_bounds__(kSimThreads, kSimCtasPerSm) sim_kernel(const SimKernelArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     // player mode sizes a chunk by the name rows the launch needs (runtime); the shipped configuration is compile-time
@@ -1179,9 +1307,9 @@ __global__ void __launch_bounds__(kSimThreads, kSimCtasPerSm) sim_kernel(const S
         int held = -1;                 // key of a request that was held back last round
         for (;;) {
             // ---- A: advance to the next request (a held-back lane re-posts the one it has)
-            Lane L = unpack_lane(P);
+            LaneT<OT> L = unpack_lane<OT>(P, a);
             L.home = home;
-            const int key = held >= 0 ? held : advance_lane<TEST, PLAYERS, HOOKS>(L, a, sh, results + (size_t)pos * 3);
+            const int key = held >= 0 ? held : advance_lane<TEST, PLAYERS, HOOKS, OT>(L, a, sh, results + (size_t)pos * 3);
             __syncwarp();
             // ---- B: compaction
             const unsigned int rank = request_rank(sh.cnt[parity], key, lane);
@@ -1206,7 +1334,7 @@ __global__ void __launch_bounds__(kSimThreads, kSimCtasPerSm) sim_kernel(const S
             {
                 const unsigned int slot = evald ? sh.dense_off[key] + rank : sh.n_eval + atomicAdd(&sh.rest, 1u);
                 const unsigned int npos = evald ? sh.off[key] + rank : 0u;
-                P = pack_lane(L);
+                P = pack_lane<OT>(L);
                 xchg[0 * kSimThreads + slot] = (uint32_t)P.game;
                 xchg[1 * kSimThreads + slot] = (uint32_t)(P.game >> 32);
                 xchg[2 * kSimThreads + slot] = (uint32_t)__double2loint(P.dist);
@@ -1235,7 +1363,7 @@ __global__ void __launch_bounds__(kSimThreads, kSimCtasPerSm) sim_kernel(const S
             }
             held = (!evald && mykey >= 0) ? mykey : -1;
             if (evald) {
-                const Lane Ln = unpack_lane(P);
+                const LaneT<OT> Ln = unpack_lane<OT>(P, a);
                 write_features<PLAYERS>(feats + (size_t)(pos >> 5) * kChunkFloats + (pos & 31), Ln, mykey >> 1, a, sh.M);
             }
             __syncthreads();

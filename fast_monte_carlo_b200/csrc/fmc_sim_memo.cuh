@@ -110,8 +110,8 @@ inline size_t sim_memo_smem_bytes() { return kMemoSharedBytes + kMemoFeatBytes +
 // (bounds of a full CTA whatever kMemoThreads: builds of this kernel with __launch_bounds__(512 | 768, ...) die on the B200
 // with "an illegal instruction was encountered" at the first launch; the same source with bounds 1024 and a 512-thread
 // launch is fine -- ptxas 12.9)
-// HOOKS: the optional outputs of the launch (sim_kernel's HOOKS)
-template <bool TEST, int HOOKS>
+// HOOKS, OT: the optional outputs of the launch and overtime (sim_kernel's)
+template <bool TEST, int HOOKS, bool OT = false>
 __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a, const MemoArgs mm) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     constexpr int kChunkFloats = chunk_floats(false);
@@ -139,14 +139,14 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
         if (tid == 0) { sh.alive[0] = 0; sh.alive[1] = 0; sh.waiting[0] = 0; sh.waiting[1] = 0; }
         __syncthreads();
         const MatchupDev &M = sh.M;
-        const Hooks<HOOKS> pk(a, M, m);
+        const Hooks<HOOKS, OT> pk(a, M, m);
         const RankSpec *specs = mm.specs + (size_t)M.memo_id * kMemoFams * 2;
         set_stage(P, ST_NEED_GAME);
         bool parked = false;           // the lane's request missed the memo and waits for the walk
         int pos = -1;                  // position of its request among this round's walked requests, -1 = not walked
         int parity = 0;
         for (;;) {
-            Lane L = unpack_lane(P);
+            LaneT<OT> L = unpack_lane<OT>(P, a);
             unsigned long long r[3] = {0ULL, 0ULL, 0ULL};
             bool have = false;         // r[] holds the outputs the lane's stage waits for
             // ---- D: walked requests come back; they also enter the memo
@@ -166,7 +166,7 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                 EvTally ev;
                 uint32_t fin_plays = 0, fin_iters = 0, n_probes = 0;
                 // -- game over
-                const bool over = !parked && L.stage == ST_ITER && L.sec <= 0;
+                const bool over = !parked && L.stage == ST_ITER && pk.ot().over(L);
                 const unsigned int over_mask = __ballot_sync(FULL, over);
                 if (over) {
                     const unsigned int bin = end_game_record<false>(L, a, M, m, sh.stat, ev, pk);
@@ -191,7 +191,7 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                         if (need) {
                             const unsigned long long g = base + (unsigned long long)__popc(nm & ((1u << lane) - 1u));
                             if (g >= M.game_end) L.stage = ST_IDLE;
-                            else { new_game(L, M, g); pk.game_start(L); }
+                            else { new_game(L, M, g); pk.game_start(L); pk.ot().game_start(L); }
                         }
                     }
                 }
@@ -207,7 +207,7 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                 if (!parked && L.stage == ST_ITER && L.sec > 0) {
                     write_trace<TEST>(L, a, M);
                     L.iter += 1;
-                    if (fourth_down(L, D, sd, ev, pk)) L.stage = start_play<TEST, false>(L, a, M, D, sd, ev);
+                    if (fourth_down(L, D, sd, ev, pk)) L.stage = start_play<TEST, false>(L, a, M, D, sd, ev, pk);
                 }
                 __syncwarp();      // every stage of the trip is entered by the whole warp together
                 // -- play model (policy 1): probe, then the play call
@@ -228,7 +228,7 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                         mg[0] = __uint_as_float((uint32_t)r[0]); mg[1] = __uint_as_float((uint32_t)(r[0] >> 32));
                         mg[2] = __uint_as_float((uint32_t)r[1]); mg[3] = __uint_as_float((uint32_t)(r[1] >> 32));
                         mg[4] = __uint_as_float((uint32_t)r[2]); mg[5] = 0.f;
-                        L.stage = call_play<TEST, false>(L, a, M, D, team, p_pass_from_play_model(mg, M.tbl[5][team].n_outputs, a), ev);
+                        L.stage = call_play<TEST, false>(L, a, M, D, team, p_pass_from_play_model(mg, M.tbl[5][team].n_outputs, a), ev, pk);
                         have = false;
                     }
                 }
@@ -320,7 +320,7 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
             const int key = parked ? request_key(L) : -1;
             const unsigned int rank = request_rank(sh.cnt[parity], key, lane);
             if (__any_sync(FULL, L.stage != ST_IDLE) && lane == 0) sh.alive[parity] = 1u;
-            P = pack_lane(L);
+            P = pack_lane<OT>(L);
             const int total = __syncthreads_count(key >= 0);
             const bool alive = sh.alive[parity] != 0u;
             if (total == 0 && !alive) break;   // every game of the matchup is played

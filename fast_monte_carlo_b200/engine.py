@@ -59,6 +59,35 @@ class GameState:
 KICKOFF = GameState()
 
 
+@dataclass(frozen=True)
+class OvertimeRules:
+    """College overtime (include/fmc.h FMC_OT_MAX_PERIODS): a game level after regulation is played on in periods of one
+    possession per team from the opponent's 25 (a period-2 touchdown is followed by a two-point try; from period 3 every
+    possession is a two-point try) until it has a result.  `max_periods` (1..16): a game still level after that many
+    periods ends level.  `snap_clock` (1..900): the clock does not run in overtime, and every overtime snap is played
+    with this many seconds left, so that the models and the fourth-down logic see end-of-game urgency."""
+    max_periods: int = native.OT_MAX_PERIODS
+    snap_clock: int = 120
+
+    def __post_init__(self):
+        if not (isinstance(self.max_periods, (int, np.integer)) and 1 <= self.max_periods <= native.OT_MAX_PERIODS):
+            raise ValueError(f"OvertimeRules.max_periods must be an integer in 1..{native.OT_MAX_PERIODS}")
+        if not (isinstance(self.snap_clock, (int, np.integer)) and 1 <= self.snap_clock <= 900):
+            raise ValueError("OvertimeRules.snap_clock must be an integer in 1..900")
+
+
+def overtime_rules(overtime) -> Optional[OvertimeRules]:
+    """The rules an API `overtime=` argument asks for: False / None = none (the game ends at 0:00, as in the reference),
+    True = the defaults, or an OvertimeRules."""
+    if overtime is None or overtime is False:
+        return None
+    if overtime is True:
+        return OvertimeRules()
+    if isinstance(overtime, OvertimeRules):
+        return overtime
+    raise ValueError("overtime must be False, True or an OvertimeRules")
+
+
 @dataclass
 class MatchupSpec:
     """One team pair as the kernels see it."""

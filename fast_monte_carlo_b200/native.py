@@ -30,7 +30,7 @@ TRACE_COLS = 8
 COUNTER_NAMES = ("games", "plays", "iters", "pass", "comp", "inc", "int", "sack", "run", "td", "fga", "fg",
                  "punt", "go", "hist_overflow", "rounds", "requests", "visits", "ph_overflow", "warp_steps",
                  "memo_probes", "memo_hits", "trips", "_23", "memo_hits_s1", "memo_hits_s2", "memo_hits_pq", "memo_hits_rq",
-                 "memo_hits_sq", "memo_hits_pm")
+                 "memo_hits_sq", "memo_hits_pm", "ot_games", "ot_periods")
 PH_YDS_BINS, PH_YDS_OFFSET, PH_CNT_BINS = 8192, 1000, 128
 PH_BINS = PH_YDS_BINS + 5 * PH_CNT_BINS
 N_SEGMENTS = 6                     # FMC_N_SEGMENTS: Q1, Q2, Q3, Q4, H1, H2
@@ -38,6 +38,8 @@ PERIOD_NONE = 0xFFFFFFFF           # FMC_PERIOD_NONE: a quarter end at or before
 # scoring sequence (include/fmc.h FMC_SEQ_NONE): the per-game words; the histogram layout is outputs'
 SEQ_NONE = 0xFFFFFFFF              # FMC_SEQ_NONE: no score after the start state
 SEQ_TD, SEQ_FG = 0, 1              # kind of a scoring play
+OT_MAX_PERIODS = 16                # FMC_OT_MAX_PERIODS; the overtime histogram is [n_matchups][2][OT_MAX_PERIODS + 1][3]
+OT_A, OT_B, OT_LEVEL = 0, 1, 2      # its last index: the final result
 
 
 def seq_bin_next(team, kind, clock):
@@ -100,6 +102,12 @@ class SegmentArgs(C.Structure):
 class SequenceArgs(C.Structure):
     """fmc_sequence_args"""
     _fields_ = [("sequence_dev", C.c_void_p), ("sequence_hist_dev", C.c_void_p)]
+
+
+class OvertimeArgs(C.Structure):
+    """fmc_overtime_args"""
+    _fields_ = [("max_periods", C.c_int32), ("snap_clock", C.c_int32), ("ot_periods_dev", C.c_void_p),
+                ("ot_hist_dev", C.c_void_p)]
 
 
 MAX_USAGE = 32
@@ -185,6 +193,9 @@ def load_library():
     L.fmc_simulate_segments_host.argtypes = [C.c_void_p, C.c_uint64] + [C.c_void_p] * 10
     L.fmc_simulate_markets.argtypes = [C.c_void_p, C.POINTER(SimArgs), C.POINTER(SegmentArgs), C.POINTER(SequenceArgs)]
     L.fmc_simulate_markets_host.argtypes = [C.c_void_p, C.c_uint64] + [C.c_void_p] * 12
+    L.fmc_simulate_overtime.argtypes = [C.c_void_p, C.POINTER(SimArgs), C.POINTER(OvertimeArgs)]
+    L.fmc_simulate_overtime_host.argtypes = ([C.c_void_p, C.c_uint64] + [C.c_void_p] * 8 + [C.c_int32, C.c_int32] +
+                                             [C.c_void_p] * 2)
     L.fmc_set_usage.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32]
     L.fmc_set_start_states.argtypes = [C.c_void_p, C.c_int32, C.c_void_p]
     L.fmc_pack_forest_host_dyn.restype = C.c_int64
@@ -224,7 +235,7 @@ EXPORTED_SYMBOLS = (
     "fmc_pack_forest_host", "fmc_pack_forest_host_dyn", "fmc_set_usage", "fmc_simulate_players_host",
     "fmc_set_memo", "fmc_memo_keys_host", "fmc_gather_probe_coherent", "fmc_predict_stats", "fmc_invalidate_tables", "fmc_tree_predict_cols_host",
     "fmc_set_start_states", "fmc_simulate_segments", "fmc_simulate_segments_host",
-    "fmc_simulate_markets", "fmc_simulate_markets_host",
+    "fmc_simulate_markets", "fmc_simulate_markets_host", "fmc_simulate_overtime", "fmc_simulate_overtime_host",
 )
 
 
@@ -466,11 +477,14 @@ class Context:
     # -- simulation ------------------------------------------------------------------------------
     def simulate_device(self, *, seed: int, scores=0, hist=0, counters=0, stream_in=0, trace=0, iters=0,
                         cuda_stream=0, players=0, player_hist=0, period_scores=0, segment_hist=0, sequence=0,
-                        sequence_hist=0) -> None:
+                        sequence_hist=0, overtime=None, ot_periods=0, ot_hist=0) -> None:
         """Asynchronous launch on raw device pointers (ints; 0 = not requested).  `period_scores` (uint32[games][3]) and
         `segment_hist` (uint32[n_matchups][2][N_SEGMENTS][BINS][BINS], zeroed by the caller) are the per-period outputs,
         `sequence` (uint32[games][2]) and `sequence_hist` (uint32[n_matchups][2][SEQ_BINS], zeroed by the caller) the
-        scoring-sequence outputs of fmc_simulate_markets; without any of them the call is fmc_simulate."""
+        scoring-sequence outputs of fmc_simulate_markets; without any of them the call is fmc_simulate.  `overtime` (an
+        engine.OvertimeRules) plays level games to a result (fmc_simulate_overtime), with the optional outputs
+        `ot_periods` (uint8[games]) and `ot_hist` (uint32[n_matchups][2][OT_MAX_PERIODS + 1][3], zeroed by the caller);
+        it has no period or sequence outputs."""
         a = SimArgs()
         a.seed = int(seed) & 0xFFFFFFFFFFFFFFFF
         a.n_matchups = self.n_matchups
@@ -479,7 +493,14 @@ class Context:
         a.stream = cuda_stream or None
         a.players_dev = players or None      # fmc_player_rec[games][2][n_slots]
         a.player_hist_dev = player_hist or None   # uint32[n_matchups][2][n_slots][PH_BINS], zeroed by the caller
-        if period_scores or segment_hist or sequence or sequence_hist:
+        if overtime is not None:
+            if period_scores or segment_hist or sequence or sequence_hist:
+                raise ValueError("overtime has no period or sequence outputs")
+            ot = OvertimeArgs(int(overtime.max_periods), int(overtime.snap_clock), ot_periods or None, ot_hist or None)
+            _check(self._L.fmc_simulate_overtime(self._h, C.byref(a), C.byref(ot)))
+        elif ot_periods or ot_hist:
+            raise ValueError("ot_periods / ot_hist need overtime")
+        elif period_scores or segment_hist or sequence or sequence_hist:
             sg = SegmentArgs()
             sg.period_scores_dev = period_scores or None; sg.segment_hist_dev = segment_hist or None
             sq = SequenceArgs()
@@ -490,13 +511,17 @@ class Context:
 
     def simulate_host(self, *, seed: int, want_scores=True, want_hist=True, stream: Optional[np.ndarray] = None,
                       want_trace=False, want_iters=False, want_players=False, want_player_hist=False,
-                      want_period_scores=False, want_segments=False, want_sequence=False, want_sequence_hist=False) -> dict:
+                      want_period_scores=False, want_segments=False, want_sequence=False, want_sequence_hist=False,
+                      overtime=None, want_ot_periods=False, want_ot_hist=False) -> dict:
         """End-to-end call with host buffers (fmc_simulate_host / fmc_simulate_players_host, and
         fmc_simulate_segments_host when `want_period_scores` / `want_segments` ask for the per-period outputs: "period_scores"
         uint32[games][3] score words at the end of Q1..Q3 (PERIOD_NONE before the start state), "segment_hist"
         uint32[n_matchups][2][N_SEGMENTS][BINS][BINS]), and fmc_simulate_markets_host when `want_sequence` /
         `want_sequence_hist` ask for the scoring-sequence outputs: "sequence" uint32[games][2] (next-score word, drive-result
-        word) and "sequence_hist" uint32[n_matchups][2][SEQ_BINS]."""
+        word) and "sequence_hist" uint32[n_matchups][2][SEQ_BINS].  With `overtime` (an engine.OvertimeRules) level games
+        are played to a result (fmc_simulate_overtime_host); `want_ot_periods` / `want_ot_hist` add "ot_periods"
+        uint8[games] and "ot_hist" uint32[n_matchups][2][OT_MAX_PERIODS + 1][3].  Overtime has no period or sequence
+        outputs."""
         n = self.total_games
         scores = np.zeros(n, dtype=np.uint32) if want_scores else None
         hist = np.zeros((self.n_matchups, 2, HIST_BINS, HIST_BINS), dtype=np.uint32) if want_hist else None
@@ -520,7 +545,20 @@ class Context:
                 phist = np.zeros((self.n_matchups, 2, max(self.n_slots, 1), PH_BINS), dtype=np.uint32)
         seq = np.zeros((n, 2), dtype=np.uint32) if want_sequence else None
         seqh = np.zeros((self.n_matchups, 2, SEQ_BINS), dtype=np.uint32) if want_sequence_hist else None
-        if period is not None or seg is not None or seq is not None or seqh is not None:
+        hooks = period is not None or seg is not None or seq is not None or seqh is not None
+        if overtime is None and (want_ot_periods or want_ot_hist):
+            raise ValueError("want_ot_periods / want_ot_hist need overtime")
+        otp = np.zeros(n, dtype=np.uint8) if want_ot_periods else None
+        oth = np.zeros((self.n_matchups, 2, OT_MAX_PERIODS + 1, 3), dtype=np.uint32) if want_ot_hist else None
+        if overtime is not None:
+            if hooks:
+                raise ValueError("overtime has no period or sequence outputs")
+            _check(self._L.fmc_simulate_overtime_host(
+                self._h, int(seed) & 0xFFFFFFFFFFFFFFFF, vp(scores), vp(hist), vp(counters), vp(stream), vp(trace), vp(iters),
+                players.ctypes.data if (players is not None and self.n_slots) else None,
+                phist.ctypes.data if (phist is not None and self.n_slots) else None,
+                int(overtime.max_periods), int(overtime.snap_clock), vp(otp), vp(oth)))
+        elif hooks:
             _check(self._L.fmc_simulate_markets_host(
                 self._h, int(seed) & 0xFFFFFFFFFFFFFFFF, vp(scores), vp(hist), vp(counters), vp(stream), vp(trace), vp(iters),
                 players.ctypes.data if (players is not None and self.n_slots) else None,
@@ -556,6 +594,10 @@ class Context:
             out["sequence"] = seq
         if seqh is not None:
             out["sequence_hist"] = seqh
+        if otp is not None:
+            out["ot_periods"] = otp
+        if oth is not None:
+            out["ot_hist"] = oth
         return out
 
     # -- tree prediction -------------------------------------------------------------------------------

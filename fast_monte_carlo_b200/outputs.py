@@ -119,7 +119,9 @@ def sims_frame(team_a: str, team_b: str, scores: np.ndarray, first_game: int = 0
 
 
 def summary_frame(sims_df: pd.DataFrame) -> pd.DataFrame:
-    """groupby(team) mean/sd/win_rate exactly as FMC:1681-1687 (sample std, ties are not wins)."""
+    """groupby(team) mean/sd/win_rate exactly as FMC:1681-1687 (sample std, ties are not wins).  The scores are final
+    scores: without overtime a game level at 0:00 is a tie; with it (engine.OvertimeRules) only a game still level at the
+    cap of periods is."""
     win = (sims_df["pts"].to_numpy() > sims_df["opp_pts"].to_numpy())
     tmp = sims_df.assign(_win=win)
     out = tmp.groupby("team").agg(
@@ -171,7 +173,8 @@ def prob_to_american(p: float) -> int:
 
 def moneyline_from_hist(hist2: np.ndarray, team: str, opp: str) -> Dict[str, Dict]:
     """edge_finder.moneyline_from_sims (edge_finder.py:249-281) with `team` = A: p_team from the
-    A-first orientation, p_opp from the B-first one (they need not sum to 1)."""
+    A-first orientation, p_opp from the B-first one (they need not sum to 1).  Ties are not wins: without overtime the
+    games level at 0:00, with it only those level at the cap of periods."""
     a, b, w = _oriented(hist2, True)
     p_team = float((w * (a > b)).sum() / w.sum())
     b2, a2, w2 = _oriented(hist2, False)
@@ -223,7 +226,8 @@ def live_odds_from_hist(hist2: np.ndarray, team_a: str, team_b: str, *, spread: 
                         total: Optional[float] = None) -> Dict[str, object]:
     """Odds of games played from a live state (api.simulate_live), over BOTH orientations: unlike a game from the
     kickoff, the start state fixes who has the ball, so the game-id parity carries no meaning.  Returns games, p_win per
-    team, p_tie (the reference has no overtime), mean final points per team, and for `spread` (team A's line: A covers
+    team, p_tie (without overtime the games level at 0:00, as in the reference; with it, engine.OvertimeRules, only the
+    games still level at the cap of periods), mean final points per team, and for `spread` (team A's line: A covers
     when its margin beats -spread) / `total` the fields of `game_market_odds_from_hist` with team A as the team.
     Scores past the last bin count as HIST_BINS - 1 points, as the histogram holds them."""
     h = np.asarray(hist2).reshape(-1, HIST_BINS, HIST_BINS).sum(axis=0).astype(np.float64)
@@ -244,6 +248,33 @@ def live_odds_from_hist(hist2: np.ndarray, team_a: str, team_b: str, *, spread: 
     if spread is not None or total is not None:
         out["markets"] = game_market_odds_from_hist(np.stack([h, np.zeros_like(h)]), team_a, team_b, spread=spread, total=total)
     return out
+
+
+OT_MAX_PERIODS = 16        # include/fmc.h FMC_OT_MAX_PERIODS
+
+
+def overtime_odds_from_hist(ot_hist2: np.ndarray, team_a: str, team_b: str) -> Dict[str, object]:
+    """Overtime markets of one entry from its overtime histogram ([2][OT_MAX_PERIODS + 1][3] or [OT_MAX_PERIODS + 1][3]:
+    games by overtime periods played and final result A won / B won / level; both orientations are summed).  Returns
+    games; p_ot, the probability of overtime; "regulation", the 3-way result at the end of regulation (A, B, level =
+    p_ot) with fair American odds; "ot_win", the probability per team of winning in overtime (unconditional: the two sum
+    to p_ot - p_level); "periods", P(the game ends after exactly k overtime periods) for k = 0..OT_MAX_PERIODS; and
+    p_level, the probability that a game is still level when the cap of periods ends it."""
+    h = np.asarray(ot_hist2, dtype=np.float64).reshape(-1, OT_MAX_PERIODS + 1, 3).sum(axis=0)
+    n = h.sum()
+    if n <= 0:
+        raise ValueError("the overtime histogram holds no games")
+    p = h / n
+    p_ot = float(p[1:].sum())
+    reg = {team_a: float(p[0, 0]), team_b: float(p[0, 1]), "level": float(p[0, 2]) + p_ot}
+    return {
+        "games": int(n),
+        "p_ot": p_ot,
+        "regulation": {k: {"p": v, "american": prob_to_american(v)} for k, v in reg.items()},
+        "ot_win": {team_a: float(p[1:, 0].sum()), team_b: float(p[1:, 1].sum())},
+        "periods": [float(x) for x in p.sum(axis=1)],
+        "p_level": float(p[1:, 2].sum()),
+    }
 
 
 # periods of a game (include/fmc.h FMC_N_SEGMENTS), in the order of the kernels' segment histograms

@@ -167,7 +167,9 @@ enum {
     FMC_C_TRIPS,       /* warp-level passes of the state machine (memo kernel) */
     FMC_C_MEMO_HITS_FAM0 = 24 /* ... 29: memo hits per family (model ids 0..5); probes per family follow from the event
                                  counters: stage 1 = pass, stage 2 = pass - comp, pass yards = comp, run yards = run,
-                                 sack yards = sack, play model = plays under policy 1 */
+                                 sack yards = sack, play model = plays under policy 1 */,
+    FMC_C_OT_GAMES = 30,      /* games that went to overtime (fmc_simulate_overtime) */
+    FMC_C_OT_PERIODS = 31     /* overtime periods they played */
 };
 
 /* Periods (quarter and half markets, fmc_simulate_segments).  Quarter q (1..3) ends when the clock crosses
@@ -217,6 +219,29 @@ enum { FMC_RACE_A = 0, FMC_RACE_B, FMC_RACE_NEITHER };
 #define FMC_SEQ_BIN_DRIVE(code) (FMC_SEQ_BIN_NONE + 1 + (code))
 #define FMC_SEQ_BIN_RACE(target, r) (FMC_SEQ_BIN_DRIVE(FMC_N_DRIVE) + (target) * 3 + (r))
 #define FMC_SEQ_BINS FMC_SEQ_BIN_RACE(FMC_N_RACE, 0)      /* 264 */
+
+/* Overtime (fmc_simulate_overtime; opt-in: without it a game ends at 0:00, level or not, as in the reference).  The NCAA
+ * rules in force since 2021, played with the reference's plays, models and fourth-down logic:
+ *  - A game level when regulation ends (the clock reaches 0, or a start state at 0 s) goes to overtime.
+ *  - Periods k = 1, 2, ...; each team has one possession per period.  Team (g & 1), the opening-kickoff receiver, has the
+ *    first possession of period 1; the order alternates every period.
+ *  - Periods 1 and 2: a possession starts at 1st & 10 at the opponent's 25 (down 1, distance 10, yards to goal 25) and
+ *    is played by the reference's rules until the offense changes (TD, FG made or missed, punt, interception, turnover
+ *    on downs).  A TD is 7 in period 1; in period 2 it is 6 and is followed by a two-point try.  A FG is 3.
+ *  - From period 3 every possession is one two-point try.  A try is one snap at down 1, distance 3, yards to goal 3: 2
+ *    points iff the snap is a TD by the reference's rules, else 0; the rest of its result is discarded and it credits
+ *    no player box line (its event counters count as for any snap).
+ *  - The clock does not run: every overtime snap is played with seconds = snap_clock (1..900; 120 puts it in the last
+ *    two minutes of the fourth quarter, so the models and the fourth-down logic see end-of-game urgency).
+ *  - The game ends as soon as the team with the second possession of a period leads (a period-2 TD that wins plays no
+ *    try), after the second possession of a period if the score is not level, level after max_periods periods
+ *    (1..FMC_OT_MAX_PERIODS), and as it stands when its iteration count reaches FMC_MAX_ITERS.
+ *  - Every overtime snap is one iteration: the Philox counter (game, entry, iteration) keeps counting from regulation,
+ *    so a game not level after regulation is the same game with overtime on or off, and the trace row of an overtime
+ *    iteration holds the state after the bookkeeping of its start (possession, try, period).
+ * Scores, score words, the score histogram, iteration counts, traces, counters and player boxes include overtime. */
+#define FMC_OT_MAX_PERIODS 16
+enum { FMC_OT_A = 0, FMC_OT_B, FMC_OT_LEVEL };    /* last index of the overtime histogram: the game's result */
 
 #define FMC_N_SLOTS 16           /* injected-draw record per (game, loop iteration); see DESIGN.md */
 #define FMC_MAX_ITERS 360
@@ -361,6 +386,34 @@ int fmc_simulate_markets_host(fmc_ctx *ctx, uint64_t seed, uint32_t *scores_host
                               uint16_t *iters_host, fmc_player_rec *players_host, uint32_t *player_hist_host,
                               uint32_t *period_scores_host, uint32_t *segment_hist_host, uint32_t *sequence_host,
                               uint32_t *sequence_hist_host);
+
+/* Overtime of a launch (see FMC_OT_MAX_PERIODS for the rules).
+ *   max_periods   1..FMC_OT_MAX_PERIODS: a game still level after this many periods ends level.
+ *   snap_clock    1..900: the seconds every overtime snap is played with.
+ *   ot_periods_dev optional [games] at out_offset + (g - game_begin) like scores_dev: overtime periods played (0: the
+ *                 game was decided in regulation).
+ *   ot_hist_dev   optional [n_matchups][2][FMC_OT_MAX_PERIODS + 1][3], += 1 at [m][g & 1][periods][FMC_OT_A | FMC_OT_B |
+ *                 FMC_OT_LEVEL] by the final score (zero it first, like hist_dev).  Bin [.][.][0] holds the games decided
+ *                 in regulation. */
+typedef struct {
+    int32_t max_periods;
+    int32_t snap_clock;
+    uint8_t *ot_periods_dev;
+    uint32_t *ot_hist_dev;
+} fmc_overtime_args;
+
+/* fmc_simulate with overtime; ot == NULL is exactly fmc_simulate.  The launch runs the kernel instantiation with the
+ * overtime rule.  FMC_ERR_INVALID for a field out of range.  Overtime has no period or sequence outputs (the markets of
+ * fmc_simulate_markets are defined for regulation). */
+int fmc_simulate_overtime(fmc_ctx *ctx, const fmc_sim_args *args, const fmc_overtime_args *ot);
+
+/* fmc_simulate_players_host with overtime: max_periods and snap_clock as in fmc_overtime_args, ot_periods_host [games]
+ * and ot_hist_host [n_matchups][2][FMC_OT_MAX_PERIODS + 1][3] (any output may be NULL; player outputs need
+ * fmc_set_usage). */
+int fmc_simulate_overtime_host(fmc_ctx *ctx, uint64_t seed, uint32_t *scores_host, uint32_t *hist_host,
+                               uint64_t *counters_host, const double *stream_host, double *trace_host,
+                               uint16_t *iters_host, fmc_player_rec *players_host, uint32_t *player_hist_host,
+                               int32_t max_periods, int32_t snap_clock, uint8_t *ot_periods_host, uint32_t *ot_hist_host);
 
 /* Raw margins of one model on n rows of the 17 numerics (play_model: first 12), NUM order of
  * FMC:676-682, float64 row-major [n][17]; out float64 [n][n_outputs].  Trees [tree_begin, tree_end)
