@@ -23,6 +23,7 @@ usage data every name is "Unknown" and `players_df` is empty, as in the shipped 
 """
 from __future__ import annotations
 
+import dataclasses
 import os
 import threading
 import time
@@ -478,7 +479,10 @@ class LiveState:
     of teamA, points of teamB) of the entry, `seconds` remaining in regulation, down, distance and yards to goal.
     `quarter_start_score` / `half_start_score` (optional, (A, B) like `score`): the score when the current quarter and the
     current half began; they let the odds of a period in progress cover the whole period.  A first-quarter state needs
-    neither (both are 0-0), a third-quarter state only one of them (the half and the quarter began together)."""
+    neither (both are 0-0), a third-quarter state only one of them (the half and the quarter began together).
+    `fourth_down` (optional, a fourth down with time left only): "go", "fg" or "punt" forces that choice at the state's
+    snap of every game (engine.GameState.fourth_down); None lets the reference's rule decide, as at every later fourth
+    down."""
     offense: str
     seconds: int
     down: int
@@ -487,6 +491,7 @@ class LiveState:
     score: Tuple[int, int] = (0, 0)
     quarter_start_score: Optional[Tuple[int, int]] = None
     half_start_score: Optional[Tuple[int, int]] = None
+    fourth_down: Optional[str] = None
 
 
 # (start, end) clock boundaries of every period of outputs.SEGMENTS; Q4 and H2 end with the game
@@ -582,6 +587,9 @@ def live_game_state(team_a: str, team_b: str, state) -> GameState:
     """The engine's GameState of `state` (a LiveState, or a mapping with its fields) for the pair (team_a, team_b).
     ValueError when the team with the ball is neither team, or a field is out of range."""
     get = (lambda k: state[k]) if isinstance(state, dict) else (lambda k: getattr(state, k))
+    fd = state.get("fourth_down") if isinstance(state, dict) else getattr(state, "fourth_down", None)
+    if fd is not None and fd not in outputs.FOURTH_DOWN_CHOICES:
+        raise ValueError(f"fourth_down must be None or one of {outputs.FOURTH_DOWN_CHOICES}, got {fd!r}")
     off = get("offense")
     if off == team_a:
         o = 0
@@ -591,7 +599,8 @@ def live_game_state(team_a: str, team_b: str, state) -> GameState:
         raise ValueError(f"Team '{off}' with the ball is neither '{team_a}' nor '{team_b}'.")
     sc = tuple(get("score"))
     return GameState(offense=o, seconds=int(get("seconds")), down=int(get("down")), distance=float(get("distance")),
-                     yards_to_goal=float(get("yards_to_goal")), score=(int(sc[0]), int(sc[1])))
+                     yards_to_goal=float(get("yards_to_goal")), score=(int(sc[0]), int(sc[1])),
+                     fourth_down=0 if fd is None else 1 + outputs.FOURTH_DOWN_CHOICES.index(fd))
 
 
 def simulate_live(entries: Sequence[Tuple[str, str, object]], games: int = 100_000, *, sp_path: Optional[str] = None,
@@ -630,15 +639,24 @@ def simulate_live(entries: Sequence[Tuple[str, str, object]], games: int = 100_0
     college overtime rules, also from a state at 0:00 with the score level; "hist", "p_win", "p_tie", "mean_points" and
     "markets" then come from the final scores, and every entry also returns "overtime" =
     `outputs.overtime_odds_from_hist` (P(overtime), the 3-way result at the end of regulation, P(win in overtime) per
-    team, the distribution of overtime periods).  ValueError with `segments=True` or `sequence=True`."""
+    team, the distribution of overtime periods).  ValueError with `segments=True` or `sequence=True`.
+
+    Fourth downs: a state's `fourth_down` ("go" | "fg" | "punt") forces that choice at its snap; ValueError with
+    `segments=True` or `sequence=True`.  `fourth_down_decisions` prices every choice of a state at once."""
+    return _live(entries, games, sp_path=sp_path, seed=seed, engine=engine, markets=markets, segments=segments,
+                 sequence=sequence, overtime=overtime, caller="simulate_live")
+
+
+def _live(entries, games, *, sp_path, seed, engine, markets, segments, sequence, overtime, caller):
+    """The body of `simulate_live`: every entry in one launch, the histograms merged by one all-reduce, a result dict
+    per entry."""
     import torch
     import torch.distributed as dist
     rules = _overtime_args(overtime, segments, sequence)
-    eng = engine if engine is not None else get_engine()
     sp_df = load_sp_flex(sp_path if sp_path is not None else packaged_priors_path())
     entries = list(entries)
     if not entries:
-        raise ValueError("simulate_live needs at least one entry")
+        raise ValueError(f"{caller} needs at least one entry")
     if int(games) < 1:
         raise ValueError("games must be at least 1")
     starts = []
@@ -649,6 +667,9 @@ def simulate_live(entries: Sequence[Tuple[str, str, object]], games: int = 100_0
         period_starts(st)
         if segments:
             _segment_lines((markets or {}).get(m))
+    if (segments or sequence) and any(gs.fourth_down for gs in starts):
+        raise ValueError("a forced fourth-down choice cannot be combined with segments=True or sequence=True")
+    eng = engine if engine is not None else get_engine()
     rank, world = 0, 1
     if dist.is_available() and dist.is_initialized():
         rank, world = dist.get_rank(), dist.get_world_size()
@@ -668,6 +689,12 @@ def simulate_live(entries: Sequence[Tuple[str, str, object]], games: int = 100_0
                                     cuda_stream=st.cuda_stream, segment_hist=seg.data_ptr() if seg is not None else 0,
                                     sequence_hist=sq.data_ptr() if sq is not None else 0,
                                     overtime=rules, ot_hist=ot.data_ptr() if ot is not None else 0)
+    return _live_results(entries, starts, markets, hist, seg, sq, ot)
+
+
+def _live_results(entries, starts, markets, hist, seg, sq, ot) -> List[Dict[str, object]]:
+    """The result dicts of `simulate_live` from the kernels' histograms of this rank (each but `hist` may be None),
+    merged over ranks by ONE all-reduce."""
     hist64, seg64, sq64, ot64 = _merge_all(None, hist, seg, sq, ot)
     oth = ot64.cpu().numpy() if ot64 is not None else None
     h = hist64.cpu().numpy()
@@ -690,6 +717,86 @@ def simulate_live(entries: Sequence[Tuple[str, str, object]], games: int = 100_0
         if oth is not None:
             out[-1]["overtime"] = outputs.overtime_odds_from_hist(oth[m], a, b)
     return out
+
+
+def _fourth_down_plan(entries, markets):
+    """The entries of one `fourth_down_decisions` launch: per state its policy entry, then one entry per available choice.
+    Returns (launch entries, their markets, per state [(key, launch index)], per state {choice: reason} of the choices
+    left out)."""
+    launch, mk, plan, unavailable = [], {}, [], []
+    for i, (a, b, st) in enumerate(entries):
+        get = (lambda k: st.get(k)) if isinstance(st, dict) else (lambda k: getattr(st, k, None))
+        if int(get("down")) != 4 or int(get("seconds")) <= 0:
+            raise ValueError(f"state {i}: fourth_down_decisions needs a fourth down (down 4) with time left")
+        if get("fourth_down") is not None:
+            raise ValueError(f"state {i}: leave fourth_down None; every choice is priced")
+        ytg = float(get("yards_to_goal"))
+        why = {}
+        if not ytg <= 38.0:
+            why["fg"] = f"a field goal is modelled from yards_to_goal <= 38 only (a try of at most 55 yards), not {ytg:g}"
+        if not ytg >= 16.0:
+            why["punt"] = f"a punt needs yards_to_goal >= 16 (the net distance is clipped to [15, yards_to_goal - 1]), not {ytg:g}"
+        rows = []
+        for key in (None,) + outputs.FOURTH_DOWN_CHOICES:
+            if key in why:
+                continue
+            if isinstance(st, dict):
+                s2 = dict(st, fourth_down=key)
+            else:
+                s2 = dataclasses.replace(st, fourth_down=key)
+            rows.append(("policy" if key is None else key, len(launch)))
+            if (markets or {}).get(i) is not None:
+                mk[len(launch)] = markets[i]
+            launch.append((a, b, s2))
+        plan.append(rows)
+        unavailable.append(why)
+    return launch, mk, plan, unavailable
+
+
+def _fourth_down_group(entries, plan, unavailable, results) -> List[Dict[str, object]]:
+    """Per state of `fourth_down_decisions`: its entries' results and the decision arithmetic of their histograms."""
+    out = []
+    for (a, b, st), rows, why in zip(entries, plan, unavailable):
+        got = {k: results[j] for k, j in rows}
+        off = st.get("offense") if isinstance(st, dict) else st.offense
+        dec = outputs.fourth_down_from_hists({k: r["hist"] for k, r in got.items()}, offense_is_a=off == a)
+        out.append({"state": st, "policy": got["policy"],
+                    "choices": {c: got.get(c) for c in outputs.FOURTH_DOWN_CHOICES}, "unavailable": dict(why),
+                    "equity": dec["equity"], "best": dec["best"], "delta": dec["delta"]})
+    return out
+
+
+def fourth_down_decisions(entries: Sequence[Tuple[str, str, object]], games: int = 100_000, *, overtime=True,
+                          markets: Optional[Dict[int, Dict[str, float]]] = None, seed: Optional[int] = None,
+                          engine: Optional[Engine] = None, sp_path: Optional[str] = None, year: int = 2025,
+                          week: int = 1) -> List[Dict[str, object]]:
+    """Go for it, kick or punt?  Every entry (teamA, teamB, state) -- `state` a LiveState (or a mapping with its fields)
+    at a fourth down with time left and `fourth_down` None -- is priced under the reference's own rule ("policy") and
+    under each choice forced at its snap: "go" always, "fg" with yards_to_goal <= 38 (the range in which the reference
+    kicks), "punt" with yards_to_goal >= 16.  Each of these plays `games` games, and every entry of every state runs in
+    ONE launch (entries of one pair share tables and the memo, so a whole fourth-down chart costs one call).  Every later
+    fourth down of a game follows the reference's rule.
+
+    `overtime` defaults to True here (False, True or an engine.OvertimeRules, as in `simulate_live`): a decision priced on
+    games left level at 0:00 undervalues the kick that ties.  `markets` ({i: {"spread": s, "total": t}}) prices lines
+    on every entry of state i.  Under torch.distributed the games are sharded and the histograms merged with one
+    all-reduce, as in `simulate_live`.
+
+    Returns, per state in entry order: "state"; "policy" and "choices" ({"go" | "fg" | "punt": result or None}), each
+    result with the keys of a `simulate_live` entry ("hist", "p_win", "p_tie", "mean_points", "markets", and "overtime"
+    with overtime); "unavailable" ({choice: reason} of the choices left out); and from `outputs.fourth_down_from_hists`
+    "equity" ({"policy" | choice: {"equity", "se", "games"}}, the offense's P(win) + P(level) / 2 and its standard
+    error), "best" (the choice of highest equity) and "delta" ({other choice: {"equity": best - other, "se"}}).
+    Forced choices run the kernels' decision instantiations; `year` / `week` are accepted as in `simulate_live`."""
+    entries = list(entries)
+    if not entries:
+        raise ValueError("fourth_down_decisions needs at least one entry")
+    for a, b, st in entries:
+        live_game_state(a, b, st)          # the team with the ball and the state's ranges first
+    launch, mk, plan, why = _fourth_down_plan(entries, markets)
+    results = _live(launch, games, sp_path=sp_path, seed=seed, engine=engine, markets=mk, segments=False,
+                    sequence=False, overtime=overtime, caller="fourth_down_decisions")
+    return _fourth_down_group(entries, plan, why, results)
 
 
 def native_counter_names():

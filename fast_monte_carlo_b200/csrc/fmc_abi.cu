@@ -273,19 +273,19 @@ extern "C" void fmc_destroy(fmc_ctx *c);
 extern "C" const char *fmc_last_error(void) { return g_err.c_str(); }
 extern "C" int fmc_abi_version(void) { return FMC_ABI_VERSION; }
 
-// the dynamic shared memory every instantiation of one hook mask (and overtime rule) may use
-template <int HOOKS, bool OT = false>
+// the dynamic shared memory every instantiation of one hook mask (overtime rule, decision rule) may use
+template <int HOOKS, bool OT = false, bool DEC = false>
 static cudaError_t set_smem_limits() {
     cudaError_t e = cudaSuccess;
     auto set = [&](const void *f, size_t bytes) {
         if (e == cudaSuccess) e = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
     };
-    set((const void *)sim_kernel<false, false, HOOKS, OT>, sim_smem_bytes(false));
-    set((const void *)sim_kernel<true, false, HOOKS, OT>, sim_smem_bytes(false));
-    set((const void *)sim_kernel<false, true, HOOKS, OT>, sim_smem_bytes(true));
-    set((const void *)sim_kernel<true, true, HOOKS, OT>, sim_smem_bytes(true));
-    set((const void *)sim_memo_kernel<false, HOOKS, OT>, sim_memo_smem_bytes());
-    set((const void *)sim_memo_kernel<true, HOOKS, OT>, sim_memo_smem_bytes());
+    set((const void *)sim_kernel<false, false, HOOKS, OT, DEC>, sim_smem_bytes(false));
+    set((const void *)sim_kernel<true, false, HOOKS, OT, DEC>, sim_smem_bytes(false));
+    set((const void *)sim_kernel<false, true, HOOKS, OT, DEC>, sim_smem_bytes(true));
+    set((const void *)sim_kernel<true, true, HOOKS, OT, DEC>, sim_smem_bytes(true));
+    set((const void *)sim_memo_kernel<false, HOOKS, OT, DEC>, sim_memo_smem_bytes());
+    set((const void *)sim_memo_kernel<true, HOOKS, OT, DEC>, sim_memo_smem_bytes());
     return e;
 }
 
@@ -319,6 +319,8 @@ extern "C" int fmc_create(int device, fmc_ctx **out) {
     CKC(set_smem_limits<kHookSequence>());
     CKC(set_smem_limits<kHookPeriods | kHookSequence>());
     CKC((set_smem_limits<0, true>()));      // overtime (fmc_simulate_overtime)
+    CKC((set_smem_limits<0, false, true>()));   // forced fourth-down choices (fmc_game_state.fourth_down) ...
+    CKC((set_smem_limits<0, true, true>()));    // ... with overtime
     CKC(cudaEventCreateWithFlags(&c->ev_done, cudaEventDisableTiming));
     CKC(cudaMalloc(&c->d_pred_stats, 16));
     CKC(cudaMemset(c->d_pred_stats, 0, 16));
@@ -431,7 +433,7 @@ static StartDev start_dev(const fmc_game_state &s) {
     StartDev d;
     std::memset(&d, 0, sizeof(d));
     d.dist = s.distance; d.ytg = s.yards_to_goal; d.sec = s.seconds; d.down = s.down; d.offense = s.offense;
-    d.score[0] = s.score[0]; d.score[1] = s.score[1];
+    d.score[0] = s.score[0]; d.score[1] = s.score[1]; d.fourth_down = s.fourth_down;
     return d;
 }
 
@@ -488,7 +490,14 @@ extern "C" int fmc_set_start_states(fmc_ctx *c, int32_t n, const fmc_game_state 
             if (!std::isfinite(s.distance) || !(s.distance > 0.0) || s.distance > 100.0)
                 return fail(FMC_ERR_INVALID, at + "distance must be finite and in (0, 100]");
             if (!(s.yards_to_goal > 0.0 && s.yards_to_goal < 100.0)) return fail(FMC_ERR_INVALID, at + "yards_to_goal must be in (0, 100)");
-            if (s.reserved != 0) return fail(FMC_ERR_INVALID, at + "reserved must be 0");
+            if (s.fourth_down < FMC_4TH_POLICY || s.fourth_down > FMC_4TH_PUNT)
+                return fail(FMC_ERR_INVALID, at + "fourth_down must be FMC_4TH_POLICY, _GO, _FG or _PUNT");
+            if (s.fourth_down != FMC_4TH_POLICY && (s.down != 4 || s.seconds == 0))
+                return fail(FMC_ERR_INVALID, at + "a forced fourth-down choice needs a fourth down with time left");
+            if (s.fourth_down == FMC_4TH_FG && !(s.yards_to_goal <= 38.0))
+                return fail(FMC_ERR_INVALID, at + "a forced field goal needs yards_to_goal <= 38");
+            if (s.fourth_down == FMC_4TH_PUNT && !(s.yards_to_goal >= 16.0))
+                return fail(FMC_ERR_INVALID, at + "a forced punt needs yards_to_goal >= 16");
             st[i] = s;
         }
     }
@@ -861,19 +870,19 @@ static size_t memo_layout(fmc_ctx *c, uint64_t games, MemoRegion (&R)[kMemoFams]
 static cudaError_t scratch(fmc_ctx *c, int slot, size_t bytes, void **out);
 
 // The kernel of a launch: player mode, the memo kernel or the plain one; injected draws / traces (TEST); the hooks of
-// the optional outputs (HOOKS); overtime (OT).
-template <int HOOKS, bool OT = false>
+// the optional outputs (HOOKS); overtime (OT); forced fourth-down choices (DEC).
+template <int HOOKS, bool OT = false, bool DEC = false>
 static void launch_sim(const SimKernelArgs &a, const MemoArgs *mm, bool players, bool test, int grid, int mgrid, size_t smem,
                        cudaStream_t st) {
     if (players) {
-        if (test) sim_kernel<true, true, HOOKS, OT><<<grid, kSimThreads, smem, st>>>(a);
-        else sim_kernel<false, true, HOOKS, OT><<<grid, kSimThreads, smem, st>>>(a);
+        if (test) sim_kernel<true, true, HOOKS, OT, DEC><<<grid, kSimThreads, smem, st>>>(a);
+        else sim_kernel<false, true, HOOKS, OT, DEC><<<grid, kSimThreads, smem, st>>>(a);
     } else if (mm) {
-        if (test) sim_memo_kernel<true, HOOKS, OT><<<mgrid, kMemoThreads, sim_memo_smem_bytes(), st>>>(a, *mm);
-        else sim_memo_kernel<false, HOOKS, OT><<<mgrid, kMemoThreads, sim_memo_smem_bytes(), st>>>(a, *mm);
+        if (test) sim_memo_kernel<true, HOOKS, OT, DEC><<<mgrid, kMemoThreads, sim_memo_smem_bytes(), st>>>(a, *mm);
+        else sim_memo_kernel<false, HOOKS, OT, DEC><<<mgrid, kMemoThreads, sim_memo_smem_bytes(), st>>>(a, *mm);
     } else {
-        if (test) sim_kernel<true, false, HOOKS, OT><<<grid, kSimThreads, sim_smem_bytes(false), st>>>(a);
-        else sim_kernel<false, false, HOOKS, OT><<<grid, kSimThreads, sim_smem_bytes(false), st>>>(a);
+        if (test) sim_kernel<true, false, HOOKS, OT, DEC><<<grid, kSimThreads, sim_smem_bytes(false), st>>>(a);
+        else sim_kernel<false, false, HOOKS, OT, DEC><<<grid, kSimThreads, sim_smem_bytes(false), st>>>(a);
     }
 }
 
@@ -890,6 +899,12 @@ static int hook_rows(fmc_ctx *c, int slot, uint64_t out_games, int words, uint32
 static int simulate_impl(fmc_ctx *c, const fmc_sim_args *g, const fmc_segment_args *seg, const fmc_sequence_args *seq,
                          const fmc_overtime_args *ot) {
     if (!c || !g) return fail(FMC_ERR_INVALID, "fmc_simulate: bad argument");
+    // forced fourth-down choices (fmc_game_state.fourth_down) run the decision instantiations; every other launch runs
+    // the kernels it ran before they existed
+    bool dec = false;
+    for (const fmc_game_state &s : c->starts) dec = dec || s.fourth_down != FMC_4TH_POLICY;
+    if (dec && ((seg && (seg->period_scores_dev || seg->segment_hist_dev)) || (seq && (seq->sequence_dev || seq->sequence_hist_dev))))
+        return fail(FMC_ERR_INVALID, "fmc_simulate: forced fourth-down choices have no period or sequence outputs");
     if (ot) {
         if (ot->max_periods < 1 || ot->max_periods > FMC_OT_MAX_PERIODS)
             return fail(FMC_ERR_INVALID, "fmc_simulate_overtime: max_periods must be 1.." + std::to_string(FMC_OT_MAX_PERIODS));
@@ -994,7 +1009,9 @@ static int simulate_impl(fmc_ctx *c, const fmc_sim_args *g, const fmc_segment_ar
     }
     const int mgrid = c->prop.multiProcessorCount * kMemoCtasPerSm;
     const MemoArgs *mp = memo ? &mm : nullptr;
-    if (ot) launch_sim<0, true>(a, mp, players, test, grid, mgrid, smem, st);
+    if (dec && ot) launch_sim<0, true, true>(a, mp, players, test, grid, mgrid, smem, st);
+    else if (dec) launch_sim<0, false, true>(a, mp, players, test, grid, mgrid, smem, st);
+    else if (ot) launch_sim<0, true>(a, mp, players, test, grid, mgrid, smem, st);
     else switch ((segs ? kHookPeriods : 0) | (seqs ? kHookSequence : 0)) {
     case 0: launch_sim<0>(a, mp, players, test, grid, mgrid, smem, st); break;
     case kHookPeriods: launch_sim<kHookPeriods>(a, mp, players, test, grid, mgrid, smem, st); break;

@@ -69,7 +69,7 @@ struct StartDev {
     int32_t sec, down;
     int32_t offense;                 // -1: team (g & 1), the opening-kickoff rule; 0 / 1: that team
     int32_t score[2];
-    int32_t reserved;
+    int32_t fourth_down;             // FMC_4TH_*: the forced choice of the first iteration of every game (0: the policy)
 };
 
 struct MatchupDev {
@@ -491,20 +491,38 @@ template <> struct Overtime<true> {
     }
 };
 
+// ---- fourth-down decisions (fmc_game_state.fourth_down, include/fmc.h FMC_4TH_POLICY) -------------------------------
+// The choice fourth_down makes at a game's first iteration.  Decision<false> has none to make: fourth_down draws it, as
+// the reference does.  Decision<true> reads the forced choice of the entry from the CTA's copy of its MatchupDev (the
+// record new_game started the game from): no lane state.  Both kernels count the iteration before they call fourth_down,
+// so the first iteration is the call that sees L.iter == 1.
+template <bool DEC> struct Decision;
+template <> struct Decision<false> {
+    __device__ __forceinline__ Decision(const MatchupDev &) {}
+    __device__ __forceinline__ int forced(const Lane &) const { return FMC_4TH_POLICY; }
+};
+template <> struct Decision<true> {
+    const MatchupDev &M;
+    __device__ __forceinline__ Decision(const MatchupDev &M_) : M(M_) {}
+    __device__ __forceinline__ int forced(const Lane &L) const { return L.iter == 1 ? M.start.fourth_down : FMC_4TH_POLICY; }
+};
+
 // The hook policy of the step functions: HOOKS is a mask of the launch's optional outputs.  Hooks<0> compiles to the code
 // without hooks; kOn says whether any hook is in (a hooked field goal adds its points before its tick).  OT: the overtime
-// rule, instantiated with HOOKS = 0 only.  Overtime<OT> is a base, so that Hooks<HOOKS, false> keeps the layout it had
-// before overtime existed (an empty member would not).
+// rule, DEC: the forced fourth-down choices, both instantiated with HOOKS = 0 only.  Overtime<OT> and Decision<DEC> are
+// bases, so that Hooks<HOOKS, false, false> keeps the layout it had before either existed (an empty member would not).
 enum { kHookPeriods = 1, kHookSequence = 2 };
-template <int HOOKS, bool OT = false>
-struct Hooks : Overtime<OT> {
+template <int HOOKS, bool OT = false, bool DEC = false>
+struct Hooks : Overtime<OT>, Decision<DEC> {
     static_assert(!(OT && HOOKS), "overtime has no period or sequence outputs");
+    static_assert(!(DEC && HOOKS), "forced fourth-down choices have no period or sequence outputs");
     static constexpr bool kOn = HOOKS != 0;
     Periods<(HOOKS & kHookPeriods) != 0> per;
     Sequence<(HOOKS & kHookSequence) != 0> seq;
     __device__ __forceinline__ Hooks(const SimKernelArgs &a, const MatchupDev &M, int m)
-        : Overtime<OT>(a, m), per(a, M, m), seq(a, M, m) {}
+        : Overtime<OT>(a, m), Decision<DEC>(M), per(a, M, m), seq(a, M, m) {}
     __device__ __forceinline__ const Overtime<OT> &ot() const { return *this; }
+    __device__ __forceinline__ const Decision<DEC> &dec() const { return *this; }
     __device__ __forceinline__ void game_start(const Lane &L) const { seq.game_start(L); }
     // quarter q ended with the play snapped at `snap`; the end of the half ends the drive if nothing else did
     __device__ __forceinline__ void quarter_end(const Lane &L, int q, int snap) const {
@@ -819,19 +837,21 @@ __device__ __forceinline__ void write_trace(const Lane &L, const SimKernelArgs &
 }
 
 // Fourth down (handle_fourth FMC:1382-1421): go for it, kick a field goal or punt (attempt_punt FMC:876-896).  Returns
-// whether a play follows; sd = score difference for the team on offense.
+// whether a play follows; sd = score difference for the team on offense.  A forced choice (Decision<true>, the first
+// iteration of a game) takes its branch without the go / kick draws; the branch reads the slots it always reads.
 template <bool TEST, class Ev, class Pk>
 __device__ __forceinline__ bool fourth_down(Lane &L, Draws<TEST> &D, int sd, Ev &ev, const Pk &pk) {
     if (L.down != 4) return true;
     const int team = L.offense;
     const double ytg = L.ytg, dist = L.dist;
+    const int forced = pk.dec().forced(L);
     const double p_go = pymin(1.0, go_for_it_prob(ytg, dist, sd, L.sec) * 1.15);
-    if (D.u(S_U_GO) < p_go) {
+    if (forced == FMC_4TH_GO || (forced == FMC_4TH_POLICY && D.u(S_U_GO) < p_go)) {
         L.going = 1;
         ev.hit(EV_GO);
         return true;
     }
-    if (ytg <= 38.0) {
+    if (forced == FMC_4TH_FG || (forced == FMC_4TH_POLICY && ytg <= 38.0)) {
         ev.hit(EV_FGA);
         const bool good = D.u(S_U_FG) < field_goal_prob(ytg + 17.0);
         // With hooks the kick's points go on before its tick, as a touchdown's do, so that a quarter that ends on the
@@ -1017,12 +1037,12 @@ __device__ __forceinline__ void after_yards(Lane &L, const SimKernelArgs &a, con
 
 // Advance one lane until it posts a request (returns its key, family * 2 + offense) or has nothing
 // left to do (returns -1).  `res` points at this lane's result record of the previous round.
-template <bool TEST, bool PLAYERS, int HOOKS, bool OT>
+template <bool TEST, bool PLAYERS, int HOOKS, bool OT, bool DEC>
 __device__ __forceinline__ int advance_lane(LaneT<OT> &L, const SimKernelArgs &a, SimShared &sh, const double *res) {
     const MatchupDev &M = sh.M;
     const int matchup = sh.cur_matchup;
     StatEvents ev{sh.stat};
-    const Hooks<HOOKS, OT> pk(a, M, matchup);
+    const Hooks<HOOKS, OT, DEC> pk(a, M, matchup);
     for (;;) {
         if (L.stage == ST_IDLE) return -1;
         if (L.stage == ST_NEED_GAME) {
@@ -1271,9 +1291,9 @@ __device__ __forceinline__ void walk_requests(RoundShared &sh, const SimKernelAr
 // more feature rows, tracked names get per-game box lines.  The shipped configuration (every name "Unknown")
 // runs the PLAYERS = false instantiation, which carries none of it.  HOOKS: the optional outputs of the launch
 // (kHookPeriods: fmc_simulate_segments, Periods<true>; kHookSequence: fmc_simulate_markets, Sequence<true>); the
-// HOOKS = 0 instantiations are the code without the hooks.  OT: overtime (fmc_simulate_overtime, Overtime<true>), with
-// HOOKS = 0 only.
-template <bool TEST, bool PLAYERS, int HOOKS, bool OT = false>
+// HOOKS = 0 instantiations are the code without the hooks.  OT: overtime (fmc_simulate_overtime, Overtime<true>), DEC:
+// forced fourth-down choices (fmc_game_state.fourth_down, Decision<true>), both with HOOKS = 0 only.
+template <bool TEST, bool PLAYERS, int HOOKS, bool OT = false, bool DEC = false>
 __global__ void __launch_bounds__(kSimThreads, kSimCtasPerSm) sim_kernel(const SimKernelArgs a) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     // player mode sizes a chunk by the name rows the launch needs (runtime); the shipped configuration is compile-time
@@ -1309,7 +1329,7 @@ __global__ void __launch_bounds__(kSimThreads, kSimCtasPerSm) sim_kernel(const S
             // ---- A: advance to the next request (a held-back lane re-posts the one it has)
             LaneT<OT> L = unpack_lane<OT>(P, a);
             L.home = home;
-            const int key = held >= 0 ? held : advance_lane<TEST, PLAYERS, HOOKS, OT>(L, a, sh, results + (size_t)pos * 3);
+            const int key = held >= 0 ? held : advance_lane<TEST, PLAYERS, HOOKS, OT, DEC>(L, a, sh, results + (size_t)pos * 3);
             __syncwarp();
             // ---- B: compaction
             const unsigned int rank = request_rank(sh.cnt[parity], key, lane);

@@ -110,8 +110,8 @@ inline size_t sim_memo_smem_bytes() { return kMemoSharedBytes + kMemoFeatBytes +
 // (bounds of a full CTA whatever kMemoThreads: builds of this kernel with __launch_bounds__(512 | 768, ...) die on the B200
 // with "an illegal instruction was encountered" at the first launch; the same source with bounds 1024 and a 512-thread
 // launch is fine -- ptxas 12.9)
-// HOOKS, OT: the optional outputs of the launch and overtime (sim_kernel's)
-template <bool TEST, int HOOKS, bool OT = false>
+// HOOKS, OT, DEC: the optional outputs of the launch, overtime and forced fourth-down choices (sim_kernel's)
+template <bool TEST, int HOOKS, bool OT = false, bool DEC = false>
 __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a, const MemoArgs mm) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     constexpr int kChunkFloats = chunk_floats(false);
@@ -139,7 +139,7 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
         if (tid == 0) { sh.alive[0] = 0; sh.alive[1] = 0; sh.waiting[0] = 0; sh.waiting[1] = 0; }
         __syncthreads();
         const MatchupDev &M = sh.M;
-        const Hooks<HOOKS, OT> pk(a, M, m);
+        const Hooks<HOOKS, OT, DEC> pk(a, M, m);
         const RankSpec *specs = mm.specs + (size_t)M.memo_id * kMemoFams * 2;
         set_stage(P, ST_NEED_GAME);
         bool parked = false;           // the lane's request missed the memo and waits for the walk

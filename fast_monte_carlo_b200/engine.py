@@ -27,18 +27,28 @@ HEAD_COACH_MAP = {
 SIM_MODELS = ("pass_stage1", "pass_stage2", "pass_yards", "run_yards", "sack_yards", "play_model")
 
 
+# fmc_game_state.fourth_down (include/fmc.h FMC_4TH_POLICY)
+FOURTH_DOWN_POLICY, FOURTH_DOWN_GO, FOURTH_DOWN_FG, FOURTH_DOWN_PUNT = 0, 1, 2, 3
+
+
 @dataclass(frozen=True)
 class GameState:
     """The state the games of a matchup entry start from: the rest of a game in progress (fmc_game_state).  The future of
     a game depends on nothing else: the period follows from the clock and timeouts are never spent.  `offense` is a team
     index (0 = team A, 1 = team B) or -1 = the kickoff rule (team g & 1 of game g has the ball); `score` = (points of A,
-    points of B).  The default is the opening kickoff."""
+    points of B).  The default is the opening kickoff.
+
+    `fourth_down` (FOURTH_DOWN_POLICY = 0, FOURTH_DOWN_GO, _FG, _PUNT; include/fmc.h FMC_4TH_POLICY) forces the choice
+    of a fourth-down state (down 4, seconds > 0) at the first snap of every game: go for it, kick (yards_to_goal <= 38
+    only, the range in which the reference kicks) or punt (yards_to_goal >= 16 only).  Every later fourth down follows
+    the reference's rule.  A game whose own draw picks that branch plays the same game forced to it."""
     offense: int = -1
     seconds: int = 3600
     down: int = 1
     distance: float = 10.0
     yards_to_goal: float = 75.0
     score: Tuple[int, int] = (0, 0)
+    fourth_down: int = 0
 
     def __post_init__(self):
         if self.offense not in (-1, 0, 1):
@@ -54,6 +64,15 @@ class GameState:
             raise ValueError("GameState.distance must be finite and in (0, 100]")
         if not (0.0 < y < 100.0):
             raise ValueError("GameState.yards_to_goal must be in (0, 100)")
+        c = self.fourth_down
+        if not (isinstance(c, (int, np.integer)) and FOURTH_DOWN_POLICY <= c <= FOURTH_DOWN_PUNT):
+            raise ValueError("GameState.fourth_down must be FOURTH_DOWN_POLICY, _GO, _FG or _PUNT (0..3)")
+        if c != FOURTH_DOWN_POLICY and (self.down != 4 or self.seconds == 0):
+            raise ValueError("a forced fourth-down choice needs a fourth down (down 4) with time left")
+        if c == FOURTH_DOWN_FG and not y <= 38.0:
+            raise ValueError("a forced field goal needs yards_to_goal <= 38")
+        if c == FOURTH_DOWN_PUNT and not y >= 16.0:
+            raise ValueError("a forced punt needs yards_to_goal >= 16")
 
 
 KICKOFF = GameState()

@@ -81,7 +81,7 @@ class GameStateC(C.Structure):
     """fmc_game_state"""
     _fields_ = [
         ("offense", C.c_int32), ("seconds", C.c_int32), ("down", C.c_int32), ("score", C.c_int32 * 2),
-        ("reserved", C.c_int32), ("distance", C.c_double), ("yards_to_goal", C.c_double),
+        ("fourth_down", C.c_int32), ("distance", C.c_double), ("yards_to_goal", C.c_double),
     ]
 
 
@@ -448,8 +448,8 @@ class Context:
 
     def set_start_states(self, states) -> None:
         """fmc_set_start_states: `states` = one state per matchup entry of the last set_matchups (objects with offense,
-        seconds, down, score, distance, yards_to_goal, such as engine.GameState; offense by team index), or None =
-        every entry starts at the kickoff."""
+        seconds, down, score, distance, yards_to_goal and optionally fourth_down, such as engine.GameState; offense by
+        team index), or None = every entry starts at the kickoff."""
         if states is None:
             _check(self._L.fmc_set_start_states(self._h, self.n_matchups, None))
             return
@@ -459,6 +459,7 @@ class Context:
             arr[i].offense = int(g.offense); arr[i].seconds = int(g.seconds); arr[i].down = int(g.down)
             arr[i].score[0], arr[i].score[1] = int(g.score[0]), int(g.score[1])
             arr[i].distance = float(g.distance); arr[i].yards_to_goal = float(g.yards_to_goal)
+            arr[i].fourth_down = int(getattr(g, "fourth_down", 0))
         _check(self._L.fmc_set_start_states(self._h, len(st), C.cast(arr, C.c_void_p)))
 
     MEMO_MODES = {"off": 0, "on": 1, "persistent": 2}

@@ -277,6 +277,43 @@ def overtime_odds_from_hist(ot_hist2: np.ndarray, team_a: str, team_b: str) -> D
     }
 
 
+# the forced choices of a fourth down (include/fmc.h FMC_4TH_GO, _FG, _PUNT), in code order
+FOURTH_DOWN_CHOICES = ("go", "fg", "punt")
+
+
+def _equity(hist2: np.ndarray, offense_is_a: bool) -> Dict[str, float]:
+    """The offense's equity P(win) + P(level) / 2 over the games of a histogram of final (A, B) points (orientations
+    summed), and its standard error: the sample standard deviation of the per-game value (1, 1/2 or 0) over sqrt(n)."""
+    h = np.asarray(hist2, dtype=np.float64).reshape(-1, HIST_BINS, HIST_BINS).sum(axis=0)
+    n = h.sum()
+    if n <= 1:
+        raise ValueError("a choice's histogram needs at least two games")
+    a = np.arange(HIST_BINS)[:, None]
+    b = np.arange(HIST_BINS)[None, :]
+    win, level = (a > b, a == b) if offense_is_a else (b > a, a == b)
+    w, t = float((h * win).sum()), float((h * level).sum())
+    e = (w + 0.5 * t) / n
+    var = max((w + 0.25 * t) / n - e * e, 0.0) * n / (n - 1)
+    return {"equity": e, "se": float(np.sqrt(var / n)), "games": int(n)}
+
+
+def fourth_down_from_hists(hists: Dict[str, Optional[np.ndarray]], offense_is_a: bool) -> Dict[str, object]:
+    """Fourth-down decision arithmetic from the final-score histograms of one state ([..., BINS, BINS] final (A, B)
+    points, orientations summed): `hists` maps "policy" and each of FOURTH_DOWN_CHOICES to its histogram, None for a
+    choice left out.  Returns "equity": {"policy" | choice: {"equity", "se", "games"}} for every histogram given, where
+    equity is the offense's P(win) + P(level) / 2; "best": the choice of highest equity; "delta": for each other choice
+    {"equity": best - choice, "se": sqrt(se_best^2 + se_choice^2)} (the entries' games are independent, so the variances
+    add)."""
+    eq = {k: _equity(h, offense_is_a) for k, h in hists.items() if h is not None}
+    choices = [c for c in FOURTH_DOWN_CHOICES if c in eq]
+    if not choices:
+        raise ValueError("no choice has a histogram")
+    best = max(choices, key=lambda c: eq[c]["equity"])
+    delta = {c: {"equity": eq[best]["equity"] - eq[c]["equity"],
+                 "se": float(np.hypot(eq[best]["se"], eq[c]["se"]))} for c in choices if c != best}
+    return {"equity": eq, "best": best, "delta": delta}
+
+
 # periods of a game (include/fmc.h FMC_N_SEGMENTS), in the order of the kernels' segment histograms
 SEGMENTS = ("Q1", "Q2", "Q3", "Q4", "H1", "H2")
 

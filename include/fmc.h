@@ -109,10 +109,26 @@ typedef struct {
     int32_t seconds;      /* seconds remaining, 0..3600 (0: the game is over, zero iterations) */
     int32_t down;         /* 1..4 */
     int32_t score[2];     /* points of team A, team B so far, 0..250 */
-    int32_t reserved;     /* must be 0 */
+    int32_t fourth_down;  /* FMC_4TH_POLICY (0), or the forced choice of a fourth-down start state: FMC_4TH_GO / _FG / _PUNT */
     double distance;      /* yards to a first down, finite, in (0, 100] */
     double yards_to_goal; /* in (0, 100) */
 } fmc_game_state;
+
+/* Fourth-down decisions (fmc_game_state.fourth_down).  A forced choice belongs to an entry whose start state is a fourth
+ * down (down 4, seconds > 0) and applies to the first iteration of each of its games only, the start state's snap;
+ * every later fourth down follows the reference's handle_fourth (FMC:1382-1421).
+ *  - FMC_4TH_POLICY: the reference's draw, go iff u(S_U_GO) < min(1, 1.15 go_for_it_prob), else kick iff
+ *    yards_to_goal <= 38, else punt.
+ *  - FMC_4TH_GO: the down-4 snap is played, as when the draw says go.
+ *  - FMC_4TH_FG: the field-goal branch: made iff u(S_U_FG) < field_goal_prob(yards_to_goal + 17), 12 s, change of
+ *    possession.  Only with yards_to_goal <= 38, the range in which the reference kicks.
+ *  - FMC_4TH_PUNT: the punt branch (S_Z_GROSS, S_Z_RET, S_U_TB), 16 s, change of possession.  Only with
+ *    yards_to_goal >= 16: below that the clip of the net distance to [15, yards_to_goal - 1] is empty.
+ * A forced iteration reads only the draw slots its branch reads, from the same record (game, entry, iteration 0): a game
+ * whose own draws pick branch X plays, forced to X, the same game bit for bit (score, iterations, trace, box lines,
+ * overtime periods, event counters).  FMC_ERR_INVALID for any other code, a non-zero code on a state that is not a
+ * fourth down with time left or outside the choice's range, and forced choices with period or sequence outputs. */
+enum { FMC_4TH_POLICY = 0, FMC_4TH_GO, FMC_4TH_FG, FMC_4TH_PUNT };
 
 /* Usage table of one role of one team: TeamContext.qb_share / rush_share / target_share (FMC:262-264) as
  * the hot path reads them.  The engine samples an entry per play exactly as Generator.choice(len(df),
@@ -293,7 +309,8 @@ int fmc_set_matchups(fmc_ctx *ctx, int32_t n, const fmc_matchup *m);
  * count starts at 0 at the start state, histogram bin [m][g & 1] holds the final score.  Cheap: it neither
  * re-specialises nor clears the memo (fmc_set_memo mode 2 keeps it); it only rewrites the start words of the device
  * records, after the launches in flight.  FMC_ERR_INVALID for n_matchups different from the last fmc_set_matchups or a
- * field out of range (see fmc_game_state). */
+ * field out of range (see fmc_game_state and FMC_4TH_POLICY).  While some entry has a forced fourth-down choice, a launch
+ * runs the kernel instantiations with the decision rule; entries with FMC_4TH_POLICY play the same games in them. */
 int fmc_set_start_states(fmc_ctx *ctx, int32_t n_matchups, const fmc_game_state *states);
 
 /* Replaces the usage half of build_team_context_from_sp_flex (`_usage_from_focus_or_fallback`, FMC:228-249,
