@@ -35,7 +35,7 @@ import pandas as pd
 
 from . import outputs
 from . import usage as _usage
-from .engine import Engine, GameState, MatchupSpec, OvertimeRules, overtime_rules  # noqa: F401
+from .engine import Engine, GameState, MatchupSpec, OvertimeRules, OvertimeState, overtime_rules  # noqa: F401
 from .priors import (TeamContext, build_team_context_from_sp_flex, csv_base_from, load_sp_flex,
                      lookup_sp_flex, packaged_priors_path)
 
@@ -482,7 +482,9 @@ class LiveState:
     neither (both are 0-0), a third-quarter state only one of them (the half and the quarter began together).
     `fourth_down` (optional, a fourth down with time left only): "go", "fg" or "punt" forces that choice at the state's
     snap of every game (engine.GameState.fourth_down); None lets the reference's rule decide, as at every later fourth
-    down."""
+    down.  `overtime` (optional, an OvertimeState(period, possession=1, two_point_try=False)): the snap is in overtime,
+    in that period and possession; `seconds` must then be 0, and the score one the overtime rules can reach there
+    (engine.GameState.overtime).  A fourth-down choice is allowed at an overtime fourth down that is not a try."""
     offense: str
     seconds: int
     down: int
@@ -492,6 +494,7 @@ class LiveState:
     quarter_start_score: Optional[Tuple[int, int]] = None
     half_start_score: Optional[Tuple[int, int]] = None
     fourth_down: Optional[str] = None
+    overtime: Optional[OvertimeState] = None
 
 
 # (start, end) clock boundaries of every period of outputs.SEGMENTS; Q4 and H2 end with the game
@@ -584,10 +587,14 @@ def live_segments(state, seg_hist: np.ndarray, team_a: str, team_b: str, lines=N
 
 
 def live_game_state(team_a: str, team_b: str, state) -> GameState:
-    """The engine's GameState of `state` (a LiveState, or a mapping with its fields) for the pair (team_a, team_b).
-    ValueError when the team with the ball is neither team, or a field is out of range."""
+    """The engine's GameState of `state` (a LiveState, or a mapping with its fields) for the pair (team_a, team_b).  In a
+    mapping, "overtime" may be an OvertimeState or a mapping with its fields.  ValueError when the team with the ball is
+    neither team, or a field is out of range."""
     get = (lambda k: state[k]) if isinstance(state, dict) else (lambda k: getattr(state, k))
     fd = state.get("fourth_down") if isinstance(state, dict) else getattr(state, "fourth_down", None)
+    ot = state.get("overtime") if isinstance(state, dict) else getattr(state, "overtime", None)
+    if isinstance(ot, dict):
+        ot = OvertimeState(**ot)
     if fd is not None and fd not in outputs.FOURTH_DOWN_CHOICES:
         raise ValueError(f"fourth_down must be None or one of {outputs.FOURTH_DOWN_CHOICES}, got {fd!r}")
     off = get("offense")
@@ -600,7 +607,7 @@ def live_game_state(team_a: str, team_b: str, state) -> GameState:
     sc = tuple(get("score"))
     return GameState(offense=o, seconds=int(get("seconds")), down=int(get("down")), distance=float(get("distance")),
                      yards_to_goal=float(get("yards_to_goal")), score=(int(sc[0]), int(sc[1])),
-                     fourth_down=0 if fd is None else 1 + outputs.FOURTH_DOWN_CHOICES.index(fd))
+                     fourth_down=0 if fd is None else 1 + outputs.FOURTH_DOWN_CHOICES.index(fd), overtime=ot)
 
 
 def simulate_live(entries: Sequence[Tuple[str, str, object]], games: int = 100_000, *, sp_path: Optional[str] = None,
@@ -641,6 +648,12 @@ def simulate_live(entries: Sequence[Tuple[str, str, object]], games: int = 100_0
     `outputs.overtime_odds_from_hist` (P(overtime), the 3-way result at the end of regulation, P(win in overtime) per
     team, the distribution of overtime periods).  ValueError with `segments=True` or `sequence=True`.
 
+    States inside overtime (LiveState.overtime) play the rest of overtime from that snap: a curve can follow a game
+    through overtime snap by snap.  They need `overtime` on, with max_periods at least the state's period (ValueError
+    otherwise).  Their "overtime" result is the same `outputs.overtime_odds_from_hist`, of games that are all in
+    overtime: P(overtime) is 1, the regulation result is level, and the periods distribution counts the last period
+    played, so it starts at the state's period.
+
     Fourth downs: a state's `fourth_down` ("go" | "fg" | "punt") forces that choice at its snap; ValueError with
     `segments=True` or `sequence=True`.  `fourth_down_decisions` prices every choice of a state at once."""
     return _live(entries, games, sp_path=sp_path, seed=seed, engine=engine, markets=markets, segments=segments,
@@ -669,6 +682,10 @@ def _live(entries, games, *, sp_path, seed, engine, markets, segments, sequence,
             _segment_lines((markets or {}).get(m))
     if (segments or sequence) and any(gs.fourth_down for gs in starts):
         raise ValueError("a forced fourth-down choice cannot be combined with segments=True or sequence=True")
+    for i, gs in enumerate(starts):
+        if gs.overtime is not None and (rules is None or rules.max_periods < gs.overtime.period):
+            raise ValueError(f"state {i} is in overtime period {gs.overtime.period}: it needs overtime on, with "
+                             f"max_periods >= {gs.overtime.period}")
     eng = engine if engine is not None else get_engine()
     rank, world = 0, 1
     if dist.is_available() and dist.is_initialized():
@@ -726,8 +743,11 @@ def _fourth_down_plan(entries, markets):
     launch, mk, plan, unavailable = [], {}, [], []
     for i, (a, b, st) in enumerate(entries):
         get = (lambda k: st.get(k)) if isinstance(st, dict) else (lambda k: getattr(st, k, None))
-        if int(get("down")) != 4 or int(get("seconds")) <= 0:
-            raise ValueError(f"state {i}: fourth_down_decisions needs a fourth down (down 4) with time left")
+        gs = live_game_state(a, b, st)
+        if gs.down != 4 or (gs.seconds <= 0 and gs.overtime is None):
+            raise ValueError(f"state {i}: fourth_down_decisions needs a fourth down (down 4) with time left, or in overtime")
+        if gs.overtime is not None and gs.overtime.two_point_try:
+            raise ValueError(f"state {i}: a two-point try has no fourth-down choice")
         if get("fourth_down") is not None:
             raise ValueError(f"state {i}: leave fourth_down None; every choice is priced")
         ytg = float(get("yards_to_goal"))
@@ -771,7 +791,7 @@ def fourth_down_decisions(entries: Sequence[Tuple[str, str, object]], games: int
                           engine: Optional[Engine] = None, sp_path: Optional[str] = None, year: int = 2025,
                           week: int = 1) -> List[Dict[str, object]]:
     """Go for it, kick or punt?  Every entry (teamA, teamB, state) -- `state` a LiveState (or a mapping with its fields)
-    at a fourth down with time left and `fourth_down` None -- is priced under the reference's own rule ("policy") and
+    at a fourth down with time left, or at an overtime fourth down that is not a try, and `fourth_down` None -- is priced under the reference's own rule ("policy") and
     under each choice forced at its snap: "go" always, "fg" with yards_to_goal <= 38 (the range in which the reference
     kicks), "punt" with yards_to_goal >= 16.  Each of these plays `games` games, and every entry of every state runs in
     ONE launch (entries of one pair share tables and the memo, so a whole fourth-down chart costs one call).  Every later
@@ -779,7 +799,8 @@ def fourth_down_decisions(entries: Sequence[Tuple[str, str, object]], games: int
 
     `overtime` defaults to True here (False, True or an engine.OvertimeRules, as in `simulate_live`): a decision priced on
     games left level at 0:00 undervalues the kick that ties.  `markets` ({i: {"spread": s, "total": t}}) prices lines
-    on every entry of state i.  Under torch.distributed the games are sharded and the histograms merged with one
+    on every entry of state i.  An overtime state (LiveState.overtime) is priced the same way, with the same kick and
+    punt ranges; it needs overtime on.  Under torch.distributed the games are sharded and the histograms merged with one
     all-reduce, as in `simulate_live`.
 
     Returns, per state in entry order: "state"; "policy" and "choices" ({"go" | "fg" | "punt": result or None}), each

@@ -203,6 +203,7 @@ struct fmc_ctx {
     fmc_params params;
     std::vector<fmc_matchup> matchups;
     std::vector<fmc_game_state> starts;  // [n_matchups] start state of every entry (fmc_set_start_states), kickoff by default
+    std::vector<fmc_overtime_state> ot_starts;   // [n_matchups] its overtime state (fmc_set_start_states_overtime), period 0 by default
     std::vector<fmc_team_usage> usage;   // [n_matchups][2] or empty (shipped configuration: every name "Unknown")
     struct NameRows { int8_t row[3][FMC_MAX_USAGE]; };
     std::vector<NameRows> name_rows;     // per team: the 0/1 feature row of every usage entry (-1: no model knows the name)
@@ -436,6 +437,59 @@ static StartDev start_dev(const fmc_game_state &s) {
     d.score[0] = s.score[0]; d.score[1] = s.score[1]; d.fourth_down = s.fourth_down;
     return d;
 }
+// Overtime<true>'s start word of an overtime state (fmc_sim.cuh kOtPeriod ...): the state before the bookkeeping of
+// iteration 0 that produces the start snap, and kOtFlip when team 1 had the first possession of period 1
+static int32_t ot_start_word(const fmc_game_state &s, const fmc_overtime_state &o) {
+    const int k = o.period, second = o.possession == 2;
+    if (k == 0) return 0;
+    const int first_of_1 = (s.offense ^ second ^ ((k - 1) & 1)) & 1;
+    int w;
+    if (!o.two_point_try) w = k | (second ? kOtSecond : 0);
+    else if (k == 2) w = 2 | (second ? kOtSecond : 0) | kOtTd;
+    else w = second ? (k | kOtTry) : ((k - 1) | kOtSecond | kOtTry);
+    return w | (first_of_1 ? kOtFlip : 0);
+}
+static void set_start(MatchupDev &M, const fmc_game_state &s, const fmc_overtime_state &o) {
+    M.start = start_dev(s);
+    M.ot_start = ot_start_word(s, o);
+}
+// Why the start state (s, o) is refused ("" = valid); o == nullptr: regulation
+static std::string start_error(const fmc_game_state &s, const fmc_overtime_state *o) {
+    if (s.offense < -1 || s.offense > 1) return "offense must be -1, 0 or 1";
+    if (s.seconds < 0 || s.seconds > 3600) return "seconds must be in 0..3600";
+    if (s.down < 1 || s.down > 4) return "down must be in 1..4";
+    if (s.score[0] < 0 || s.score[0] > 250 || s.score[1] < 0 || s.score[1] > 250) return "scores must be in 0..250";
+    if (!std::isfinite(s.distance) || !(s.distance > 0.0) || s.distance > 100.0) return "distance must be finite and in (0, 100]";
+    if (!(s.yards_to_goal > 0.0 && s.yards_to_goal < 100.0)) return "yards_to_goal must be in (0, 100)";
+    if (s.fourth_down < FMC_4TH_POLICY || s.fourth_down > FMC_4TH_PUNT)
+        return "fourth_down must be FMC_4TH_POLICY, _GO, _FG or _PUNT";
+    const bool ot = o && o->period != 0;
+    if (o && !ot && (o->possession || o->two_point_try || o->reserved)) return "a regulation state (period 0) has no overtime fields";
+    if (s.fourth_down != FMC_4TH_POLICY && (s.down != 4 || (!ot && s.seconds == 0) || (ot && o->two_point_try)))
+        return "a forced fourth-down choice needs a fourth down with time left or an overtime fourth down that is not a try";
+    if (s.fourth_down == FMC_4TH_FG && !(s.yards_to_goal <= 38.0)) return "a forced field goal needs yards_to_goal <= 38";
+    if (s.fourth_down == FMC_4TH_PUNT && !(s.yards_to_goal >= 16.0)) return "a forced punt needs yards_to_goal >= 16";
+    if (!ot) return "";
+    const int k = o->period, p = o->possession, t = o->two_point_try;
+    if (k < 1 || k > FMC_OT_MAX_PERIODS) return "overtime period must be in 0.." + std::to_string(FMC_OT_MAX_PERIODS);
+    if (p != 1 && p != 2) return "overtime possession must be 1 or 2";
+    if (t != 0 && t != 1) return "two_point_try must be 0 or 1";
+    if (o->reserved != 0) return "overtime reserved field must be 0";
+    if (s.seconds != 0) return "an overtime state has seconds 0";
+    if (s.offense < 0) return "an overtime state names the team with the ball (offense 0 or 1)";
+    if (t && k == 1) return "period 1 has no two-point try";
+    if (!t && k >= 3) return "from period 3 every snap is a two-point try";
+    if (t && !(s.down == 1 && s.distance == 3.0 && s.yards_to_goal == 3.0))
+        return "a two-point try is down 1, distance 3, yards_to_goal 3";
+    // the margins the rules can reach: d = the offense's points minus the opponent's
+    const int d = s.score[s.offense] - s.score[s.offense ^ 1];
+    bool ok;
+    if (!t) ok = p == 1 ? d == 0 : (k == 1 ? (d == 0 || d == -3 || d == -7) : (d == 0 || d == -3 || d == -6 || d == -8));
+    else if (k == 2 && p == 1) ok = d == 6;
+    else ok = p == 1 ? d == 0 : (d == 0 || d == -2);
+    if (!ok) return "the rules cannot reach this overtime score margin (" + std::to_string(d) + " for the offense)";
+    return "";
+}
 
 extern "C" int fmc_set_matchups(fmc_ctx *c, int32_t n, const fmc_matchup *m) {
     if (!c || n <= 0 || !m) return fail(FMC_ERR_INVALID, "fmc_set_matchups: bad argument");
@@ -452,13 +506,14 @@ extern "C" int fmc_set_matchups(fmc_ctx *c, int32_t n, const fmc_matchup *m) {
                (c->matchups[i].game_end > c->matchups[i].game_begin || m[i].game_end == m[i].game_begin);
     // start states belong to a matchup list: every entry starts at the kickoff again
     c->starts.assign(n, kickoff_state());
+    c->ot_starts.assign(n, fmc_overtime_state{});
     if (same) {
         CK(cudaSetDevice(c->device));
         CK(cudaDeviceSynchronize());           // a launch in flight reads the ranges
         for (int i = 0; i < n; ++i) {
             MatchupDev &M = c->h_matchups[i];
             M.game_begin = m[i].game_begin; M.game_end = m[i].game_end; M.out_offset = m[i].out_offset;
-            M.start = start_dev(c->starts[i]);
+            set_start(M, c->starts[i], c->ot_starts[i]);
         }
         CK(cudaMemcpy(c->d_matchups, c->h_matchups.data(), c->h_matchups.size() * sizeof(MatchupDev), cudaMemcpyHostToDevice));
         c->matchups.assign(m, m + n);
@@ -475,40 +530,33 @@ extern "C" int fmc_set_matchups(fmc_ctx *c, int32_t n, const fmc_matchup *m) {
 }
 
 extern "C" int fmc_set_start_states(fmc_ctx *c, int32_t n, const fmc_game_state *states) {
+    return fmc_set_start_states_overtime(c, n, states, nullptr);
+}
+
+extern "C" int fmc_set_start_states_overtime(fmc_ctx *c, int32_t n, const fmc_game_state *states, const fmc_overtime_state *ot) {
     if (!c) return fail(FMC_ERR_INVALID, "fmc_set_start_states: ctx is NULL");
     if (n != (int)c->matchups.size()) return fail(FMC_ERR_INVALID, "fmc_set_start_states: n_matchups differs from the last fmc_set_matchups");
+    if (ot && !states) return fail(FMC_ERR_INVALID, "fmc_set_start_states_overtime: overtime states need game states");
     std::vector<fmc_game_state> st(n, kickoff_state());
+    std::vector<fmc_overtime_state> ots(n, fmc_overtime_state{});
     if (states) {
         for (int i = 0; i < n; ++i) {
-            const fmc_game_state &s = states[i];
-            const std::string at = "fmc_set_start_states: entry " + std::to_string(i) + ": ";
-            if (s.offense < -1 || s.offense > 1) return fail(FMC_ERR_INVALID, at + "offense must be -1, 0 or 1");
-            if (s.seconds < 0 || s.seconds > 3600) return fail(FMC_ERR_INVALID, at + "seconds must be in 0..3600");
-            if (s.down < 1 || s.down > 4) return fail(FMC_ERR_INVALID, at + "down must be in 1..4");
-            if (s.score[0] < 0 || s.score[0] > 250 || s.score[1] < 0 || s.score[1] > 250)
-                return fail(FMC_ERR_INVALID, at + "scores must be in 0..250");
-            if (!std::isfinite(s.distance) || !(s.distance > 0.0) || s.distance > 100.0)
-                return fail(FMC_ERR_INVALID, at + "distance must be finite and in (0, 100]");
-            if (!(s.yards_to_goal > 0.0 && s.yards_to_goal < 100.0)) return fail(FMC_ERR_INVALID, at + "yards_to_goal must be in (0, 100)");
-            if (s.fourth_down < FMC_4TH_POLICY || s.fourth_down > FMC_4TH_PUNT)
-                return fail(FMC_ERR_INVALID, at + "fourth_down must be FMC_4TH_POLICY, _GO, _FG or _PUNT");
-            if (s.fourth_down != FMC_4TH_POLICY && (s.down != 4 || s.seconds == 0))
-                return fail(FMC_ERR_INVALID, at + "a forced fourth-down choice needs a fourth down with time left");
-            if (s.fourth_down == FMC_4TH_FG && !(s.yards_to_goal <= 38.0))
-                return fail(FMC_ERR_INVALID, at + "a forced field goal needs yards_to_goal <= 38");
-            if (s.fourth_down == FMC_4TH_PUNT && !(s.yards_to_goal >= 16.0))
-                return fail(FMC_ERR_INVALID, at + "a forced punt needs yards_to_goal >= 16");
-            st[i] = s;
+            const std::string why = start_error(states[i], ot ? ot + i : nullptr);
+            if (!why.empty()) return fail(FMC_ERR_INVALID, "fmc_set_start_states: entry " + std::to_string(i) + ": " + why);
+            st[i] = states[i];
+            if (ot) ots[i] = ot[i];
         }
     }
-    if (st.size() == c->starts.size() && std::memcmp(st.data(), c->starts.data(), st.size() * sizeof(fmc_game_state)) == 0)
+    if (st.size() == c->starts.size() && std::memcmp(st.data(), c->starts.data(), st.size() * sizeof(fmc_game_state)) == 0 &&
+        std::memcmp(ots.data(), c->ot_starts.data(), ots.size() * sizeof(fmc_overtime_state)) == 0)
         return FMC_OK;                         // nothing changes (e.g. kickoff again after fmc_set_matchups)
     c->starts.swap(st);
+    c->ot_starts.swap(ots);
     // the device records of the current tables get their new start words; dirty tables take them when they are built
     if (!c->tables_dirty && c->d_matchups && c->h_matchups.size() == (size_t)n) {
         CK(cudaSetDevice(c->device));
         CK(cudaDeviceSynchronize());           // a launch in flight reads the start words
-        for (int i = 0; i < n; ++i) c->h_matchups[i].start = start_dev(c->starts[i]);
+        for (int i = 0; i < n; ++i) set_start(c->h_matchups[i], c->starts[i], c->ot_starts[i]);
         CK(cudaMemcpy(c->d_matchups, c->h_matchups.data(), c->h_matchups.size() * sizeof(MatchupDev), cudaMemcpyHostToDevice));
     }
     return FMC_OK;
@@ -694,7 +742,7 @@ static int build_tables(fmc_ctx *c) {
         MatchupDev &M = md[i];
         std::memset(&M, 0, sizeof(M));
         M.game_begin = mu.game_begin; M.game_end = mu.game_end; M.out_offset = mu.out_offset;
-        M.start = start_dev(c->starts[i]);
+        set_start(M, c->starts[i], c->ot_starts[i]);
         M.memo_id = memo_id[i];
         for (int off = 0; off < 2; ++off) {
             const int de = off ^ 1;
@@ -905,6 +953,14 @@ static int simulate_impl(fmc_ctx *c, const fmc_sim_args *g, const fmc_segment_ar
     for (const fmc_game_state &s : c->starts) dec = dec || s.fourth_down != FMC_4TH_POLICY;
     if (dec && ((seg && (seg->period_scores_dev || seg->segment_hist_dev)) || (seq && (seq->sequence_dev || seq->sequence_hist_dev))))
         return fail(FMC_ERR_INVALID, "fmc_simulate: forced fourth-down choices have no period or sequence outputs");
+    // entries that start in overtime (fmc_set_start_states_overtime) need the overtime rule and its periods
+    int ot_period = 0;
+    for (const fmc_overtime_state &o : c->ot_starts) ot_period = std::max(ot_period, (int)o.period);
+    if (ot_period && !ot)
+        return fail(FMC_ERR_INVALID, "fmc_simulate: an entry starts in overtime; the launch needs overtime (fmc_simulate_overtime)");
+    if (ot_period && ot && ot->max_periods < ot_period)
+        return fail(FMC_ERR_INVALID, "fmc_simulate_overtime: an entry starts in overtime period " + std::to_string(ot_period) +
+                                         ", after max_periods");
     if (ot) {
         if (ot->max_periods < 1 || ot->max_periods > FMC_OT_MAX_PERIODS)
             return fail(FMC_ERR_INVALID, "fmc_simulate_overtime: max_periods must be 1.." + std::to_string(FMC_OT_MAX_PERIODS));

@@ -77,7 +77,7 @@ struct MatchupDev {
     unsigned long long game_begin, game_end, out_offset;
     StartDev start;
     int32_t memo_id;                 // specialisation of this entry: index of its RankSpec set and its memo key field
-    int32_t pad;
+    int32_t ot_start;                // overtime state every game starts from (Overtime<true>::game_start), 0: regulation
     TableRef tbl[kNumFam][2];
     UsageDev usage[2];               // player mode only
 };
@@ -404,15 +404,21 @@ template <> struct Sequence<true> {
 // The rule that plays a game level at the end of regulation to a result.  Overtime<false> is the reference's end of the
 // game at 0:00.  Overtime<true> keeps its state in OtLane::ot: the period k (1..FMC_OT_MAX_PERIODS), whether the second
 // possession of the period is on, whether the snap is a two-point try, and a period-2 touchdown whose try is still due.
-// The team with the first possession of period k is (g & 1) in period 1 and alternates; a possession ends when the
-// offense changes (every place that calls change_possession) or, for a try, after its one snap.  All bookkeeping runs at
-// the start of an iteration (over), before the trace row, except the points of a touchdown, which after_yards adds.
-enum : int { kOtPeriod = 31, kOtSecond = 32, kOtTry = 64, kOtTd = 128 };
+// The team with the first possession of period k is (g & 1) in period 1 and alternates, or the other team when kOtFlip is
+// set (a game started in overtime, fmc_set_start_states_overtime); a possession ends when the offense changes (every place
+// that calls change_possession) or, for a try, after its one snap.  All bookkeeping runs at the start of an iteration
+// (over), before the trace row, except the points of a touchdown, which after_yards adds.
+//
+// A start in overtime (MatchupDev::ot_start, written by the library) is the state before the bookkeeping of iteration 0
+// that produces the start snap: k | second for a snap of a possession (offense = team()); for a try, 2 | second | kOtTd
+// in period 2, (k - 1) | kOtSecond | kOtTry for the first try of period k >= 3 and k | kOtTry for its second.  Its kOtFlip
+// says that team 1 had the first possession of period 1; game_start turns that into the game's own bit.
+enum : int { kOtPeriod = 31, kOtSecond = 32, kOtTry = 64, kOtTd = 128, kOtFlip = 256 };
 
 template <bool OT> struct Overtime;
 template <> struct Overtime<false> {
     __device__ __forceinline__ Overtime(const SimKernelArgs &, int) {}
-    __device__ __forceinline__ void game_start(const Lane &) const {}
+    __device__ __forceinline__ void game_start(const Lane &, const MatchupDev &) const {}
     // the game is over at the start of an iteration
     __device__ __forceinline__ bool over(const Lane &L) const { return L.sec <= 0; }
     // points of a touchdown just scored
@@ -428,11 +434,14 @@ template <> struct Overtime<true> {
     // the step functions see a Lane; the lanes of these instantiations are OtLanes
     __device__ __forceinline__ static int &st(Lane &L) { return static_cast<OtLane &>(L).ot; }
     __device__ __forceinline__ static int st(const Lane &L) { return static_cast<const OtLane &>(L).ot; }
-    __device__ __forceinline__ void game_start(Lane &L) const { st(L) = 0; }
+    __device__ __forceinline__ void game_start(Lane &L, const MatchupDev &M) const {
+        const int s = M.ot_start;
+        st(L) = s ? s ^ ((int)(L.game & 1ULL) << 8) : 0;
+    }
     // the team whose possession is on
     __device__ __forceinline__ static int team(const Lane &L) {
         const int o = st(L);
-        return (int)(L.game & 1ULL) ^ (((o & kOtPeriod) - 1) & 1) ^ ((o & kOtSecond) ? 1 : 0);
+        return (int)(L.game & 1ULL) ^ ((o >> 8) & 1) ^ (((o & kOtPeriod) - 1) & 1) ^ ((o & kOtSecond) ? 1 : 0);
     }
     __device__ __forceinline__ static void two_point_try(Lane &L) {
         st(L) |= kOtTry;
@@ -459,9 +468,9 @@ template <> struct Overtime<true> {
                 L.offense = t;
                 two_point_try(L);
             } else if ((o & kOtTry) || L.offense != t) {      // the possession is over
-                if (!(o & kOtSecond)) o = k | kOtSecond;
+                if (!(o & kOtSecond)) o = (o & kOtFlip) | k | kOtSecond;
                 else if (L.score[0] != L.score[1] || k >= a.ot_max_periods) return true;
-                else o = k + 1;
+                else o = (o & kOtFlip) | (k + 1);
                 possession(L);
             }
         }
@@ -1050,7 +1059,7 @@ __device__ __forceinline__ int advance_lane(LaneT<OT> &L, const SimKernelArgs &a
             if (g >= M.game_end) { L.stage = ST_IDLE; return -1; }
             new_game(L, M, g);
             pk.game_start(L);
-            pk.ot().game_start(L);
+            pk.ot().game_start(L, M);
         }
         if (L.stage == ST_ITER) {
             // (the instantiations without overtime keep the clock test of their own: calling Overtime<false>::over here, inline

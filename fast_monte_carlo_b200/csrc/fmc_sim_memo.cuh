@@ -191,7 +191,7 @@ __global__ void __launch_bounds__(1024, 1) sim_memo_kernel(const SimKernelArgs a
                         if (need) {
                             const unsigned long long g = base + (unsigned long long)__popc(nm & ((1u << lane) - 1u));
                             if (g >= M.game_end) L.stage = ST_IDLE;
-                            else { new_game(L, M, g); pk.game_start(L); pk.ot().game_start(L); }
+                            else { new_game(L, M, g); pk.game_start(L); pk.ot().game_start(L, M); }
                         }
                     }
                 }

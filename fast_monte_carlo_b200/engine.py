@@ -32,6 +32,39 @@ FOURTH_DOWN_POLICY, FOURTH_DOWN_GO, FOURTH_DOWN_FG, FOURTH_DOWN_PUNT = 0, 1, 2, 
 
 
 @dataclass(frozen=True)
+class OvertimeState:
+    """Where in overtime a start state is (include/fmc.h fmc_overtime_state): `period` 1..16, `possession` 1 or 2 (the
+    first or second possession of the period), `two_point_try` (the snap is a two-point try: always from period 3, after
+    a touchdown in period 2, never in period 1)."""
+    period: int
+    possession: int = 1
+    two_point_try: bool = False
+
+    def __post_init__(self):
+        if not (isinstance(self.period, (int, np.integer)) and 1 <= self.period <= native.OT_MAX_PERIODS):
+            raise ValueError(f"OvertimeState.period must be an integer in 1..{native.OT_MAX_PERIODS}")
+        if self.possession not in (1, 2):
+            raise ValueError("OvertimeState.possession must be 1 or 2")
+        if self.two_point_try not in (False, True):
+            raise ValueError("OvertimeState.two_point_try must be a bool")
+        if self.two_point_try and self.period == 1:
+            raise ValueError("period 1 of overtime has no two-point try")
+        if not self.two_point_try and self.period >= 3:
+            raise ValueError("from period 3 of overtime every snap is a two-point try")
+
+
+def overtime_margins(ot: OvertimeState) -> Tuple[int, ...]:
+    """The margins (points of the team with the ball minus the opponent's) the overtime rules can reach at `ot`."""
+    if not ot.two_point_try:
+        if ot.possession == 1:
+            return (0,)
+        return (0, -3, -7) if ot.period == 1 else (0, -3, -6, -8)
+    if ot.period == 2 and ot.possession == 1:
+        return (6,)
+    return (0,) if ot.possession == 1 else (0, -2)
+
+
+@dataclass(frozen=True)
 class GameState:
     """The state the games of a matchup entry start from: the rest of a game in progress (fmc_game_state).  The future of
     a game depends on nothing else: the period follows from the clock and timeouts are never spent.  `offense` is a team
@@ -41,7 +74,12 @@ class GameState:
     `fourth_down` (FOURTH_DOWN_POLICY = 0, FOURTH_DOWN_GO, _FG, _PUNT; include/fmc.h FMC_4TH_POLICY) forces the choice
     of a fourth-down state (down 4, seconds > 0) at the first snap of every game: go for it, kick (yards_to_goal <= 38
     only, the range in which the reference kicks) or punt (yards_to_goal >= 16 only).  Every later fourth down follows
-    the reference's rule.  A game whose own draw picks that branch plays the same game forced to it."""
+    the reference's rule.  A game whose own draw picks that branch plays the same game forced to it.
+
+    `overtime` (an OvertimeState, None = regulation) puts the state inside overtime: the snap about to be played in that
+    period and possession, played at the launch's snap clock.  It needs seconds 0 and offense 0 or 1, a try is 1st & 3 at
+    the 3, and the score must be one the rules can reach there (`overtime_margins`); a forced choice is allowed at any
+    overtime fourth down that is not a try.  A launch of such a state needs overtime rules with max_periods >= period."""
     offense: int = -1
     seconds: int = 3600
     down: int = 1
@@ -49,6 +87,7 @@ class GameState:
     yards_to_goal: float = 75.0
     score: Tuple[int, int] = (0, 0)
     fourth_down: int = 0
+    overtime: Optional[OvertimeState] = None
 
     def __post_init__(self):
         if self.offense not in (-1, 0, 1):
@@ -67,12 +106,29 @@ class GameState:
         c = self.fourth_down
         if not (isinstance(c, (int, np.integer)) and FOURTH_DOWN_POLICY <= c <= FOURTH_DOWN_PUNT):
             raise ValueError("GameState.fourth_down must be FOURTH_DOWN_POLICY, _GO, _FG or _PUNT (0..3)")
-        if c != FOURTH_DOWN_POLICY and (self.down != 4 or self.seconds == 0):
-            raise ValueError("a forced fourth-down choice needs a fourth down (down 4) with time left")
+        ot = self.overtime
+        if ot is not None and not isinstance(ot, OvertimeState):
+            raise ValueError("GameState.overtime must be None or an OvertimeState")
+        if c != FOURTH_DOWN_POLICY and (self.down != 4 or (ot is None and self.seconds == 0)):
+            raise ValueError("a forced fourth-down choice needs a fourth down (down 4) with time left, or in overtime")
+        if c != FOURTH_DOWN_POLICY and ot is not None and ot.two_point_try:
+            raise ValueError("a two-point try has no fourth-down choice")
         if c == FOURTH_DOWN_FG and not y <= 38.0:
             raise ValueError("a forced field goal needs yards_to_goal <= 38")
         if c == FOURTH_DOWN_PUNT and not y >= 16.0:
             raise ValueError("a forced punt needs yards_to_goal >= 16")
+        if ot is None:
+            return
+        if self.seconds != 0:
+            raise ValueError("an overtime state has seconds 0 (regulation is over)")
+        if self.offense not in (0, 1):
+            raise ValueError("an overtime state names the team with the ball (offense 0 or 1)")
+        if ot.two_point_try and (self.down, d, y) != (1, 3.0, 3.0):
+            raise ValueError("a two-point try is down 1, distance 3, yards_to_goal 3")
+        m = int(self.score[self.offense]) - int(self.score[self.offense ^ 1])
+        if m not in overtime_margins(ot):
+            raise ValueError(f"the overtime rules cannot reach a margin of {m} for the team with the ball at {ot} "
+                             f"(possible: {overtime_margins(ot)})")
 
 
 KICKOFF = GameState()

@@ -85,6 +85,11 @@ class GameStateC(C.Structure):
     ]
 
 
+class OvertimeStateC(C.Structure):
+    """fmc_overtime_state"""
+    _fields_ = [("period", C.c_int32), ("possession", C.c_int32), ("two_point_try", C.c_int32), ("reserved", C.c_int32)]
+
+
 class SimArgs(C.Structure):
     _fields_ = [
         ("seed", C.c_uint64), ("n_matchups", C.c_int32), ("reserved", C.c_int32),
@@ -198,6 +203,7 @@ def load_library():
                                              [C.c_void_p] * 2)
     L.fmc_set_usage.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_int32]
     L.fmc_set_start_states.argtypes = [C.c_void_p, C.c_int32, C.c_void_p]
+    L.fmc_set_start_states_overtime.argtypes = [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p]
     L.fmc_pack_forest_host_dyn.restype = C.c_int64
     L.fmc_pack_forest_host_dyn.argtypes = [C.POINTER(ForestDesc), C.c_int32, C.c_int32, C.c_int32, C.c_void_p, C.c_int32,
                                            C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64,
@@ -236,6 +242,7 @@ EXPORTED_SYMBOLS = (
     "fmc_set_memo", "fmc_memo_keys_host", "fmc_gather_probe_coherent", "fmc_predict_stats", "fmc_invalidate_tables", "fmc_tree_predict_cols_host",
     "fmc_set_start_states", "fmc_simulate_segments", "fmc_simulate_segments_host",
     "fmc_simulate_markets", "fmc_simulate_markets_host", "fmc_simulate_overtime", "fmc_simulate_overtime_host",
+    "fmc_set_start_states_overtime",
 )
 
 
@@ -447,20 +454,26 @@ class Context:
         self.n_slots, self.has_usage = int(n_slots), True
 
     def set_start_states(self, states) -> None:
-        """fmc_set_start_states: `states` = one state per matchup entry of the last set_matchups (objects with offense,
-        seconds, down, score, distance, yards_to_goal and optionally fourth_down, such as engine.GameState; offense by
-        team index), or None = every entry starts at the kickoff."""
+        """fmc_set_start_states_overtime: `states` = one state per matchup entry of the last set_matchups (objects with
+        offense, seconds, down, score, distance, yards_to_goal and optionally fourth_down and overtime, such as
+        engine.GameState; offense by team index; overtime None or an object with period, possession and two_point_try),
+        or None = every entry starts at the kickoff."""
         if states is None:
-            _check(self._L.fmc_set_start_states(self._h, self.n_matchups, None))
+            _check(self._L.fmc_set_start_states_overtime(self._h, self.n_matchups, None, None))
             return
         st = list(states)
         arr = (GameStateC * max(len(st), 1))()
+        ot = (OvertimeStateC * max(len(st), 1))()
         for i, g in enumerate(st):
             arr[i].offense = int(g.offense); arr[i].seconds = int(g.seconds); arr[i].down = int(g.down)
             arr[i].score[0], arr[i].score[1] = int(g.score[0]), int(g.score[1])
             arr[i].distance = float(g.distance); arr[i].yards_to_goal = float(g.yards_to_goal)
             arr[i].fourth_down = int(getattr(g, "fourth_down", 0))
-        _check(self._L.fmc_set_start_states(self._h, len(st), C.cast(arr, C.c_void_p)))
+            o = getattr(g, "overtime", None)
+            if o is not None:
+                ot[i].period, ot[i].possession = int(o.period), int(o.possession)
+                ot[i].two_point_try = int(bool(o.two_point_try))
+        _check(self._L.fmc_set_start_states_overtime(self._h, len(st), C.cast(arr, C.c_void_p), C.cast(ot, C.c_void_p)))
 
     MEMO_MODES = {"off": 0, "on": 1, "persistent": 2}
 

@@ -115,7 +115,8 @@ typedef struct {
 } fmc_game_state;
 
 /* Fourth-down decisions (fmc_game_state.fourth_down).  A forced choice belongs to an entry whose start state is a fourth
- * down (down 4, seconds > 0) and applies to the first iteration of each of its games only, the start state's snap;
+ * down (down 4, seconds > 0, or an overtime fourth down that is not a try: fmc_overtime_state) and applies to the first
+ * iteration of each of its games only, the start state's snap;
  * every later fourth down follows the reference's handle_fourth (FMC:1382-1421).
  *  - FMC_4TH_POLICY: the reference's draw, go iff u(S_U_GO) < min(1, 1.15 go_for_it_prob), else kick iff
  *    yards_to_goal <= 38, else punt.
@@ -259,6 +260,30 @@ enum { FMC_RACE_A = 0, FMC_RACE_B, FMC_RACE_NEITHER };
 #define FMC_OT_MAX_PERIODS 16
 enum { FMC_OT_A = 0, FMC_OT_B, FMC_OT_LEVEL };    /* last index of the overtime histogram: the game's result */
 
+/* A start state inside overtime (fmc_set_start_states_overtime): with the fmc_game_state of the entry (offense, down,
+ * distance, yards_to_goal, score) it names the overtime snap about to be played, the state the trace row of an overtime
+ * iteration holds.  period 0 is regulation (the other fields 0); otherwise
+ *  - period k in 1..FMC_OT_MAX_PERIODS, possession 1 or 2 (the first or second possession of period k), two_point_try
+ *    0 or 1.  seconds must be 0 (every snap is played at the launch's snap_clock) and offense 0 or 1; a try is down 1,
+ *    distance 3, yards to goal 3.  The team with the first possession of period 1 follows from offense, possession and
+ *    k (it need not be team g & 1).
+ *  - d = the offense's points minus the opponent's must be one the rules can reach: 0 on the first possession of
+ *    periods 1 and 2; 0, -3 or -7 on the second possession of period 1; 0, -3, -6 or -8 on the second possession of
+ *    period 2; +6 on a first-possession try of period 2; 0 or -2 on a second-possession try of period 2 (a
+ *    second-possession touchdown that wins plays no try); 0 on a first-possession try from period 3, 0 or -2 on a
+ *    second-possession try.  No try in period 1, only tries from period 3.
+ *  - A forced fourth-down choice (fmc_game_state.fourth_down) is allowed at any fourth down that is not a try, with its
+ *    ranges; it applies to the first snap.
+ * A launch with such an entry needs overtime with max_periods >= period (FMC_ERR_INVALID otherwise).  Draws count
+ * iterations from the start state, as for every start state; the overtime histogram bin is the last period played, and
+ * the overtime periods output and counters count periods, not periods from the start. */
+typedef struct {
+    int32_t period;
+    int32_t possession;
+    int32_t two_point_try;
+    int32_t reserved;     /* 0 */
+} fmc_overtime_state;
+
 #define FMC_N_SLOTS 16           /* injected-draw record per (game, loop iteration); see DESIGN.md */
 #define FMC_MAX_ITERS 360
 #define FMC_TRACE_COLS 8
@@ -312,6 +337,14 @@ int fmc_set_matchups(fmc_ctx *ctx, int32_t n, const fmc_matchup *m);
  * field out of range (see fmc_game_state and FMC_4TH_POLICY).  While some entry has a forced fourth-down choice, a launch
  * runs the kernel instantiations with the decision rule; entries with FMC_4TH_POLICY play the same games in them. */
 int fmc_set_start_states(fmc_ctx *ctx, int32_t n_matchups, const fmc_game_state *states);
+
+/* fmc_set_start_states with an overtime state per entry: ot[n_matchups] (see fmc_overtime_state; period 0 =
+ * regulation).  ot == NULL is fmc_set_start_states; states == NULL needs ot == NULL.  fmc_set_matchups and
+ * fmc_set_start_states return every entry to regulation.  FMC_ERR_INVALID for a state the rules cannot reach; a launch
+ * with an entry in overtime fails with FMC_ERR_INVALID without overtime, with max_periods below the entry's period, or
+ * with period or sequence outputs. */
+int fmc_set_start_states_overtime(fmc_ctx *ctx, int32_t n_matchups, const fmc_game_state *states,
+                                  const fmc_overtime_state *ot);
 
 /* Replaces the usage half of build_team_context_from_sp_flex (`_usage_from_focus_or_fallback`, FMC:228-249,
  * 1646-1659): teams[n_matchups][2] (team A, team B of each matchup of the last fmc_set_matchups), n_slots =
